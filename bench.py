@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the rolling-window Bayesian tangency-weight hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], "C2"): one full daily-rebalance backtest, 4,150 rebalance dates,
 N = 500 synthetic assets, conjugate (VIX-scaled HF prior) + Jeffreys priors = 8,300 windows per step:
@@ -42,6 +42,7 @@ if ROOT not in sys.path:
 
 METRIC = "posterior tangency-weight windows/sec at N=500"
 UNIT = "windows/s"
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 # ----------------------------------------------------------------------------- workload
@@ -89,6 +90,26 @@ def intraday_config(mkt, conj, d_idx, hf_days):
     return dict(intraday_rows_uploaded=int(hi - lo), intraday_rows_in_market=int(mkt.hf_prices.shape[0]),
                 intraday_note="bars before the first window's look-back (history only the daily windows need) are "
                               "read by no window and are not uploaded")
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as ``out_dir/<name>.npy`` in float64, so that two builds can be compared output for output.
+    Past DUMP_LIMIT_BYTES in all, every 2-D array (one row per window, all with the same rows) keeps the same seeded
+    sample of rows, so runs with the same arguments write the same rows."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        rows2d = [a for a in arrays.values() if a.ndim == 2]
+        row_bytes = sum(a.shape[1] * a.itemsize for a in rows2d)
+        other = total - sum(a.nbytes for a in rows2d)
+        keep = max(1, (DUMP_LIMIT_BYTES - other) // row_bytes)
+        rows = np.sort(np.random.default_rng(0).choice(rows2d[0].shape[0], keep, replace=False))
+        arrays = {k: a[rows] if a.ndim == 2 else a for k, a in arrays.items()}
+        print(f"bench.py: outputs exceed {DUMP_LIMIT_BYTES >> 20} MB, writing a seeded sample of {keep} rows",
+              file=sys.stderr)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -507,16 +528,21 @@ def run_ours(args):
     launches = (eng.launch_count - launches0) // args.steps + (2 if world > 1 else 0)      # + the two all-gathers
     status_bad = int((out_c["status"] != 0).sum().item() + (out_j["status"] != 0).sum().item())
     value = n_gpus * 2 * W / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives from its last step: the (all-gathered) weights and the status flags
+        wc, wj = (out_c["weights"], out_j["weights"]) if world == 1 else (gathered_c.view(-1, N), gathered_j.view(-1, N))
+        dump_outputs(args.dump_outputs, {"conjugate_weights": wc.cpu().numpy(), "jeffreys_weights": wj.cpu().numpy(),
+                                         "conjugate_status": out_c["status"].cpu().numpy(),
+                                         "jeffreys_status": out_j["status"].cpu().numpy()})
 
     # ---- end-to-end timing through the host-buffer API
-    e2e_steps = max(1, min(args.steps, 3))
     step_e2e()
     barrier()
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         step_e2e()
     torch.cuda.synchronize()
-    e2e_s = max_over_ranks((time.perf_counter() - t0) / e2e_steps)
+    e2e_s = max_over_ranks((time.perf_counter() - t0) / args.steps)
     e2e_value = n_gpus * 2 * W / e2e_s
     if sub_batches:      # sub-batches anchor their block grids differently: same sums, different association
         ref_w = out_c["weights"].cpu().numpy()
@@ -625,7 +651,7 @@ def run_ours(args):
                            **intraday_config(mkt, conj, d_idx, args.hf_days)),
             "clocks": clocks,
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": d2h_bytes,
-                    "ms_per_step": e2e_s * 1e3, "matches_device_path": e2e_match, "steps": e2e_steps,
+                    "ms_per_step": e2e_s * 1e3, "matches_device_path": e2e_match, "steps": args.steps,
                     "inputs": "host buffers pinned once outside the timed region; windows planned once outside it",
                     "conjugate_sub_batches": len(sub_batches) if sub_batches else 1,
                     "h2d_ceiling": h2d_ceiling,
@@ -844,7 +870,13 @@ def main():
                     help="N > 1: weak = one independent path per GPU; strong = ONE backtest split by date range (north star)")
     ap.add_argument("--paths", type=int, default=64, help="C5: independent synthetic paths in total")
     ap.add_argument("--path-pool", type=int, default=2, help="C5: distinct generated markets per GPU the paths cycle through")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="C2: write the weights and status flags of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "C2" or args.scaling != "weak"):
+        ap.error("--dump-outputs applies to the C2 workload of --impl ours with --scaling weak")
     if args.impl == "reference":
         run_reference(args)
     elif args.config != "C2" or args.scaling == "strong":

@@ -2,7 +2,8 @@
 prices inside the look-back), stocks without intraday data, NaN and TIED market caps, a constituent list that names
 unknown tickers, portfolios larger than the eligible universe, partially overlapping turnover frames.
 
-Runs on the CPU (no CUDA call) wherever /root/reference exists; index order and membership are compared exactly.
+Runs on the CPU (no CUDA call); the tests that import the reference's own functions run where its sources are found
+(``$REF_SRC``, see oracle/ref_import.py). Index order and membership are compared exactly.
 """
 import numpy as np
 import pandas as pd
@@ -12,7 +13,7 @@ from incorporating_different_sources_b200 import backtest as bt
 from incorporating_different_sources_b200.synthetic import generate_market
 from oracle.ref_import import load_reference, reference_available, set_universe
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference sources not present on this machine")
+needs_reference = pytest.mark.skipif(not reference_available(), reason="reference sources not present on this machine")
 
 
 def _damaged_market():
@@ -30,6 +31,7 @@ def _damaged_market():
     return mkt, prices, caps, intr
 
 
+@needs_reference
 @pytest.mark.parametrize("freq", ["daily", "weekly", "monthly"])
 @pytest.mark.parametrize("size", [3, 7, 50])
 def test_universe_selection_matches_reference(freq, size):
@@ -51,6 +53,7 @@ def test_universe_selection_matches_reference(freq, size):
         bt.UNIVERSE_PROVIDER = None
 
 
+@needs_reference
 @pytest.mark.parametrize("freq", ["daily", "weekly", "monthly"])
 @pytest.mark.parametrize("size", [3, 7, 50])
 def test_vectorised_universe_selection_matches_reference_on_every_date(freq, size):
@@ -76,6 +79,7 @@ def test_vectorised_universe_selection_matches_reference_on_every_date(freq, siz
         bt.UNIVERSE_PROVIDER = None
 
 
+@needs_reference
 def test_vectorised_universe_selection_without_provider_and_missing_cap_date():
     pc = load_reference(check=True)
     mkt, prices, caps, intr = _damaged_market()
@@ -92,17 +96,21 @@ def test_vectorised_universe_selection_without_provider_and_missing_cap_date():
 
 
 def test_universe_selection_errors_match_reference():
-    pc = load_reference(check=True)
+    """The exception types are the reference's; its own function is checked beside ours where its sources are found."""
     mkt, prices, caps, intr = _damaged_market()
     set_universe(mkt.tickers)
     d = prices.index[60]
-    for fn in (pc.get_k_largest_stocks_market_caps, bt.get_k_largest_stocks_market_caps):
+    fns = [bt.get_k_largest_stocks_market_caps]
+    if reference_available():
+        fns.insert(0, load_reference(check=True).get_k_largest_stocks_market_caps)
+    for fn in fns:
         with pytest.raises(RuntimeError):
             fn(caps, prices, intr, d, 5, 30, "hourly")                              # :637
         with pytest.raises(ValueError):
             fn(caps.drop(index=d), prices, intr, d, 5, 30, "daily")                  # :657
 
 
+@needs_reference
 def test_turnover_and_window_helpers_match_reference():
     pc = load_reference(check=True)
     from incorporating_different_sources_b200 import portfolio_calculations as ours
@@ -145,6 +153,7 @@ def test_rebalance_calendar_matches_reference_loop():
         bt.rebalance_flags(days, "yearly")
 
 
+@needs_reference
 @pytest.mark.parametrize("freq", ["daily", "weekly"])
 def test_mcm_prior_n_on_the_series_own_calendar_matches_reference(freq):
     """FRED's daily EPU index has an observation on every CALENDAR day: the reference averages the last n
