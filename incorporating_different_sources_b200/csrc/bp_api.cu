@@ -5,17 +5,14 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
-#include <array>
-#include <cstdarg>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
-#include <map>
 #include <string>
-#include <utility>
 #include <vector>
 
 #include "../../include/bayes_portfolio.h"
+#include "batch_plan.h"
 #include "kernels.h"
 
 using namespace bp;
@@ -24,17 +21,9 @@ static_assert(BP_NSCAL == bp::BP_S_COUNT, "scalar record size mismatch between h
 
 namespace {
 
-thread_local std::string g_err;
+thread_local std::string g_err;      // bp_last_error
 
-int fail(int code, const char* fmt, ...) {
-    char buf[1024];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof(buf), fmt, ap);
-    va_end(ap);
-    g_err = buf;
-    return code;
-}
+#define fail(...) fail_to(&g_err, __VA_ARGS__)
 
 #define CU_TRY(expr)                                                                                     \
     do {                                                                                                 \
@@ -52,6 +41,22 @@ bool is_device_ptr(const void* p) {
         return false;
     }
     return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+}
+
+// A grow-only buffer of `cap` elements: device memory, or page-locked host memory when `pinned` (see grow)
+template <class T>
+struct DevBuf {
+    T* p = nullptr;
+    size_t cap = 0;
+    bool pinned = false;
+};
+
+template <class T>
+void free_buf(DevBuf<T>& b) {
+    if (b.pinned) cudaFreeHost(b.p);
+    else cudaFree(b.p);
+    b.p = nullptr;
+    b.cap = 0;
 }
 
 }  // namespace
@@ -75,8 +80,7 @@ struct bp_handle {
     double *pool_prices = nullptr, *pool_caps = nullptr, *pool_hf = nullptr, *pool_rf = nullptr;
     int pool_N = 0, pool_D = 0;
     long long pool_R = 0;
-    int* pool_cols = nullptr;
-    size_t pool_cols_cap = 0;
+    DevBuf<int> pool_cols;
     // resampled (weekly) return rows: see bp_set_resampled
     double *lr_w = nullptr, *rf_w = nullptr, *mcm_w = nullptr;
     int* rs_idx = nullptr;
@@ -101,50 +105,35 @@ struct bp_handle {
     long long seg_end[MAX_SEG] = {0};          // return rows < seg_end[s] are valid once ev_seg[s] has fired
     cudaEvent_t ev_seg[MAX_SEG] = {nullptr};
     CUtensorMap map_d, map_hf;
-    // window descriptors on the device: day_row, span, row0, hf_row0, hf_m
-    int* desc = nullptr;
-    int* desc_host = nullptr;          // page-locked staging of the descriptors (read zero-copy by a kernel)
-    size_t desc_cap = 0;               // capacity in ints
-    // two descriptor slots used alternately: planning the next batch on the host never waits for the GPU to
-    // have fetched (or finished using) the previous one, only for the batch before that
-    int* desc_slot[2] = {nullptr, nullptr};
-    int* desc_host_slot[2] = {nullptr, nullptr};
-    size_t desc_cap_slot[2] = {0, 0};
+    // descriptor images (batch_plan.h) on the device and their page-locked staging (read zero-copy by a kernel), in
+    // two slots used alternately: planning the next batch on the host never waits for the GPU to have fetched (or
+    // finished using) the previous one, only for the batch before that
+    DevBuf<int> desc_slot[2];
+    DevBuf<int> desc_host_slot[2] = {{nullptr, 0, true}, {nullptr, 0, true}};
     cudaEvent_t ev_desc[2] = {nullptr, nullptr};
     bool ev_desc_armed[2] = {false, false};
     int desc_turn = 0;
     bool async_outputs = false;        // host outputs are complete only after bp_synchronize (see bp_set_async_outputs)
     // block tile stores of the Gram kernel (window-overlap reuse) and the smallest batch that uses them
-    double* store[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};      // [phase][level]
-    size_t store_cap[2][2] = {{0, 0}, {0, 0}};                           // capacity in doubles
-    double* rstore[2] = {nullptr, nullptr};                              // phase-B range-sum stores [level]
-    size_t rstore_cap[2] = {0, 0};
-    double* fstore = nullptr;                                            // phase-B combined runs (coarse + fine + fine)
-    size_t fstore_cap = 0;
+    DevBuf<double> store[2][2];        // [phase][level]
+    DevBuf<double> rstore[2];          // phase-B range-sum stores [level]
+    DevBuf<double> fstore;             // phase-B combined runs (coarse + fine + fine)
     int reuse_min_windows = 32;
     // pre-summed intraday day blocks (long HF look-backs): windows with at least this many trading days add <= 3 scanned
     // tiles instead of one tile per day (0 disables); vector store [3 nb][ld] of the scanned per-day column sums
     int presum_min_days = 8;
-    double* vstore = nullptr;
-    size_t vstore_cap = 0;
-    double work_scan_tiles = 0;
+    DevBuf<double> vstore;
     // work counters of the Gram stage since the last bp_get_gram_work (bench.py's roofline accounting)
     double work_k_rows = 0, work_add_blocks = 0, work_pre_rows = 0, work_full_rows = 0;
     // Jeffreys windows of consecutive trade dates: only every chain_group-th window is factorised, the others are
     // solved relative to it (jeffreys_chain.cu); < 2 disables.  Work counters for bench.py's roofline accounting.
     int chain_group = 8;
-    int work_stride = 1;               // upload_batch counts the Gram work of every work_stride-th window only
     double work_factored = 0, work_chained = 0;
-    double* prior_n = nullptr;
-    int prior_n_cap = 0;
+    DevBuf<double> prior_n;
     // banded-GEMM daily pass (band_prep.cu): risk-free weights [W][band_ld] and their sums [W][2]
-    double *band_aw = nullptr, *band_stats = nullptr;
-    size_t band_aw_cap = 0, band_stats_cap = 0;
+    DevBuf<double> band_aw, band_stats;
     // workspace
-    unsigned char* ws = nullptr;
-    size_t ws_bytes = 0;
-    unsigned char* stage = nullptr;
-    size_t stage_bytes = 0;
+    DevBuf<unsigned char> ws, stage;
     bool need_sync = false;
     PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
     // optional per-stage CUDA-event timing (bench.py's roofline numbers)
@@ -271,26 +260,16 @@ int make_solve_map(bp_handle* h, CUtensorMap* map, const double* base, long long
     return BP_OK;
 }
 
-int ensure_ws(bp_handle* h, size_t bytes) {
-    if (bytes <= h->ws_bytes) return BP_OK;
-    if (h->ws) cudaFree(h->ws);
-    h->ws = nullptr;
-    h->ws_bytes = 0;
-    CU_TRY(cudaMalloc(&h->ws, bytes));
-    h->ws_bytes = bytes;
-    return BP_OK;
-}
-
-int ensure_stage(bp_handle* h, size_t bytes) {
-    if (bytes <= h->stage_bytes) return BP_OK;
-    if (h->stage) {
-        CU_TRY(cudaStreamSynchronize(h->stream));
-        cudaFree(h->stage);
-    }
-    h->stage = nullptr;
-    h->stage_bytes = 0;
-    CU_TRY(cudaMalloc(&h->stage, bytes));
-    h->stage_bytes = bytes;
+// Grows buf to at least n elements, without keeping its contents; waits for the stream first, which may still read the
+// old buffer.
+template <class T>
+int grow(bp_handle* h, DevBuf<T>& buf, size_t n) {
+    if (n <= buf.cap) return BP_OK;
+    if (buf.p) CU_TRY(cudaStreamSynchronize(h->stream));
+    free_buf(buf);
+    if (buf.pinned) CU_TRY(cudaHostAlloc(&buf.p, sizeof(T) * n, cudaHostAllocDefault));
+    else CU_TRY(cudaMalloc(&buf.p, sizeof(T) * n));
+    buf.cap = n;
     return BP_OK;
 }
 
@@ -355,524 +334,89 @@ Chunk chunk_at(const Chunk& c, const Layout& L, int k) {
     return o;
 }
 
-// validated, device-resident description of one batch
+// validated, planned batch and its descriptor image on the device
 struct Batch {
-    int W = 0, n = 0, max_m = 0;
-    bool has_hf = false;
-    const int *day_row = nullptr, *span = nullptr, *row0 = nullptr, *hf_row0 = nullptr, *hf_m = nullptr;
-    const double* prior_n = nullptr;
-    int mcm_rows = 0;
-    bool resampled = false;
+    BatchPlan plan;
+    const int *day_row = nullptr, *span = nullptr, *hf_row0 = nullptr, *hf_m = nullptr;
     const int *extra_row = nullptr, *caps_row = nullptr;
     const int* gdesc = nullptr;        // [W][GRAM_DESC_INTS] Gram job descriptors
     const int* bdesc[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // block precompute launches [phase][level]
-    int nblocks[2][2] = {{0, 0}, {0, 0}};
     const int* rdesc[2] = {nullptr, nullptr};      // phase B: [lo, hi) block ranges to pre-sum, per level
-    int nranges[2] = {0, 0};
     const int* fdesc = nullptr;                    // phase B: [coarse, fineA, fineB] run ids to combine
-    int nfull = 0;
-    bool band_ok = false;              // consecutive trade dates: the daily pass runs as a banded GEMM
-    // intraday block grid (for the pipelined upload): block k of level l ends at return row hf_off + (hf_bmin[l]+k+1)*hf_blk[l]
-    int hf_off = 0, hf_bmin[2] = {0, 0}, hf_blk[2] = {0, 0};
-    bool hf_inner = false;             // day blocks without their overnight return + gathered overnight rows (PhasePlan::inner)
-    int hf_nb0 = 0;
-    std::vector<int> hf_starts;        // inner: price row where day block k starts (nb + 1 entries), host copy
-    const int* hf_starts_dev = nullptr;
-    bool presum = false;               // windows add <= 3 scanned tiles (PhasePlan::chunk)
-    int presum_chunk = 0;
+    const int* hf_starts = nullptr;    // inner day blocks: price row where block k starts (nb + 1 entries)
     const int* hf_vids = nullptr;      // [W][3] scanned-vector ids of each window
+    const double* prior_n = nullptr;
 };
 
-// Block grids of one phase, two levels (0 = coarse, 1 = fine; the fine size divides the coarse size): block b of
-// level l covers return rows [off + b*blk[l], off + (b+1)*blk[l]); blk[l] == 0: level unused
-struct PhasePlan {
-    int blk[2] = {0, 0};
-    int off = 0;
-    int bmin[2] = {0, 0}, nb[2] = {0, 0};
-    // "inner" day blocks: every hf_lo / hf_hi of the batch is a block boundary (the HF look-back always covers whole
-    // days, :310-312, whatever the bar calendar), block b = return rows starts[b]+1 .. starts[b+1]-1, i.e. a trading
-    // day WITHOUT its first (overnight) return; the overnight rows are gathered into a compact row range behind the
-    // intraday matrix, so a window is [its days' inner blocks] + [one short run of overnight rows]
-    bool inner = false;
-    std::vector<int> starts;
-    // pre-summed runs (long look-backs): chunk > 0 -> a window adds suffix'[first day] + prefix[...] tiles (<= 3)
-    int chunk = 0;
-};
-
-inline long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
-
-// Split of the row range [row0, row0+rows) of a window: head rows, fine blocks, coarse blocks, fine blocks, tail rows
-struct Split {
-    long long k0_row = 0, k0_n = 0, k1_row = 0, k1_n = 0;     // rows contracted on the tensor cores
-    long long c_lo = 0, c_hi = 0;                             // coarse blocks [c_lo, c_hi)
-    long long fa_lo = 0, fa_hi = 0, fb_lo = 0, fb_hi = 0;     // fine blocks on the head / tail side
-};
-
-Split split_rows(int row0, int rows, const PhasePlan& P) {
-    Split s;
-    s.k0_row = row0;
-    s.k0_n = rows;
-    if (rows <= 0 || (P.blk[0] <= 0 && P.blk[1] <= 0)) return s;
-    const long long r0 = (long long)row0 - P.off, r1 = r0 + rows;
-    long long head_end = r1, tail_begin = r1;      // relative rows; head = [r0, head_end), tail = [tail_begin, r1)
-    if (P.blk[0] > 0) {
-        const long long B = P.blk[0];
-        const long long lo = floor_div(r0 + B - 1, B), hi = floor_div(r1, B);
-        if (hi > lo) {
-            s.c_lo = lo;
-            s.c_hi = hi;
-            head_end = lo * B;
-            tail_begin = hi * B;
-        }
-    }
-    if (P.blk[1] > 0) {
-        const long long F = P.blk[1];
-        if (s.c_hi > s.c_lo) {
-            const long long f_lo = floor_div(r0 + F - 1, F), f_hi = floor_div(r1, F);
-            s.fa_lo = f_lo;  s.fa_hi = head_end / F;          // head_end is a multiple of the coarse (hence fine) size
-            s.fb_lo = tail_begin / F;  s.fb_hi = f_hi;
-            s.k0_n = f_lo * F - r0;
-            s.k1_row = P.off + f_hi * F;
-            s.k1_n = r1 - f_hi * F;
-        } else {
-            const long long f_lo = floor_div(r0 + F - 1, F), f_hi = floor_div(r1, F);
-            if (f_hi > f_lo) {
-                s.fa_lo = f_lo;  s.fa_hi = f_hi;
-                s.k0_n = f_lo * F - r0;
-                s.k1_row = P.off + f_hi * F;
-                s.k1_n = r1 - f_hi * F;
-            }
-        }
-    } else if (s.c_hi > s.c_lo) {
-        s.k0_n = head_end - r0;
-        s.k1_row = P.off + tail_begin;
-        s.k1_n = r1 - tail_begin;
-    }
-    return s;
+PlanCtx plan_ctx(const bp_handle* h, int stride) {
+    PlanCtx c;
+    c.has_market = h->has_market;
+    c.N = h->N; c.ld = h->ld; c.D = h->D; c.Rw = h->Rw; c.n_mcm = h->n_mcm;
+    c.R = h->R;
+    c.hf_extra_rows = h->hf_extra_rows;
+    c.has_caps = h->has_caps;
+    c.has_mcm_w = h->mcm_w != nullptr;
+    c.ws_limit = h->ws_limit;
+    c.reuse_min_windows = h->reuse_min_windows;
+    c.presum_min_days = h->presum_min_days;
+    c.stride = stride;
+    return c;
 }
 
-// descriptor ints of one phase (GRAM_PHASE_INTS) from a split, block indices relative to the stores
-void write_phase_desc(const Split& s, const PhasePlan& P, int* d) {
-    d[0] = (int)s.k0_row; d[1] = (int)s.k0_n; d[2] = (int)s.k1_row; d[3] = (int)s.k1_n;
-    d[4] = (int)(s.c_lo - P.bmin[0]);  d[5] = (int)(s.c_hi - s.c_lo);
-    d[6] = (int)(s.fa_lo - P.bmin[1]); d[7] = (int)(s.fa_hi - s.fa_lo);
-    d[8] = (int)(s.fb_lo - P.bmin[1]); d[9] = (int)(s.fb_hi - s.fb_lo);
-    if (d[5] == 0) d[4] = 0;
-    if (d[7] == 0) d[6] = 0;
-    if (d[9] == 0) d[8] = 0;
-}
-
-int upload_batch(bp_handle* h, const bp_window_batch* b, bool need_hf, Batch* out) {
+// stride: the chain path runs only every stride-th window through the Gram kernel
+int upload_batch(bp_handle* h, const bp_window_batch* b, bool need_hf, int stride, Batch* out) {
     if (!h || !b) return fail(BP_ERR_INVALID, "null handle or batch");
-    if (!h->has_market) return fail(BP_ERR_STATE, "no market uploaded: call bp_upload_market first");
-    const int W = b->n_windows, n = b->rolling_window;
-    if (W <= 0) return fail(BP_ERR_INVALID, "n_windows must be positive");
-    if (n < 3) return fail(BP_ERR_INVALID, "rolling_window must be >= 3");
-    if (!b->day_row || !b->span_days) return fail(BP_ERR_INVALID, "day_row / span_days missing");
-    if (need_hf) {
-        if (!b->hf_lo || !b->hf_hi) return fail(BP_ERR_INVALID, "hf_lo / hf_hi missing");
-        if (h->R <= 0) return fail(BP_ERR_STATE, "the uploaded market has no intraday prices");
-        if (b->resampled && !b->prior_n && !h->mcm_w) return fail(BP_ERR_STATE, "bp_set_resampled was given no MCM rows");
-        if (!b->prior_n && (b->mcm_index < 0 || b->mcm_index >= h->n_mcm))
-            return fail(BP_ERR_INVALID, "mcm_index %d out of range", b->mcm_index);
-        if (b->mcm_rows < 0 || b->mcm_rows > n) return fail(BP_ERR_INVALID, "mcm_rows must be in [0, rolling_window]");
-        if (b->prior_weights == 0 && !h->has_caps) return fail(BP_ERR_STATE, "value-weighted prior needs market caps");
-    }
-    const bool rs = b->resampled != 0;
-    if (rs) {
-        if (h->Rw <= 0) return fail(BP_ERR_STATE, "resampled windows need bp_set_resampled first");
-        if (!b->extra_row || !b->caps_row) return fail(BP_ERR_INVALID, "resampled windows need extra_row and caps_row");
-    }
-    // ---- block grids for the window-overlap reuse of the Gram kernel
-    const int npairs_t = ((h->N + GRAM_TILE - 1) / GRAM_TILE) * ((h->N + GRAM_TILE - 1) / GRAM_TILE + 1) / 2;
-    PhasePlan plan[2];
-    if (W >= h->reuse_min_windows) {
-        const int K = n - 1;
-        if (!rs) {          // resampled windows: shared weekly rows + one per-date row, no block reuse
-            // Block sizes were tuned on the bench workload (N = 500): coarse/fine 128/32 for the 1007-row Jeffreys
-            // window and 64/16 for the 251-row conjugate window gave 18.6 ms for the Gram stage, 512/64 + 128/32
-            // 19.4 ms, a single level (128 / 64) 21.9 ms; neither the DMMA pipe (40-50 %) nor L2 (26-32 %) is
-            // saturated then, the stage is bound by per-item latencies.
-            if (K >= 512) { plan[1].blk[0] = 128; plan[1].blk[1] = 32; }
-            else if (K >= 128) { plan[1].blk[0] = 64; plan[1].blk[1] = 16; }
-        }
-        if (need_hf) {
-            // Day blocks: the HF look-back of every window covers whole days, so the sorted set of all hf_lo / hf_hi
-            // values cuts the bars into blocks of which every window is a run -- whatever the bar calendar (half
-            // days, holidays).  Worth it when the windows overlap (each block serves >= 2 windows on average).
-            static const bool no_inner = getenv("BP_NO_INNER_BLOCKS") != nullptr;
-            std::vector<int>& st = plan[0].starts;
-            st.reserve(2 * (size_t)W);
-            for (int w = 0; w < W; ++w) { st.push_back(b->hf_lo[w]); st.push_back(b->hf_hi[w]); }
-            std::sort(st.begin(), st.end());
-            st.erase(std::unique(st.begin(), st.end()), st.end());
-            if (st.size() >= 3) {
-                // stretches no window starts or ends in (the look-back of the first windows of a short batch) would be
-                // single giant blocks contracted by one CTA per tile pair: cut them to the typical block length (a
-                // window contains such a stretch entirely or not at all, so any cut inside it is a valid boundary)
-                std::vector<int> gaps(st.size() - 1);
-                for (size_t k = 0; k + 1 < st.size(); ++k) gaps[k] = st[k + 1] - st[k];
-                std::nth_element(gaps.begin(), gaps.begin() + gaps.size() / 2, gaps.end());
-                const int typical = std::max(8, gaps[gaps.size() / 2]);
-                std::vector<int> cut;
-                cut.reserve(st.size());
-                for (size_t k = 0; k + 1 < st.size(); ++k) {
-                    cut.push_back(st[k]);
-                    const int gap = st[k + 1] - st[k];
-                    if (gap > 2 * typical) {
-                        const int pieces = gap / typical;
-                        for (int q = 1; q < pieces; ++q) cut.push_back(st[k] + (int)((long long)gap * q / pieces));
-                    }
-                }
-                cut.push_back(st.back());
-                st.swap(cut);
-            }
-            const long long nb = (long long)st.size() - 1;
-            long long sumD = 0;
-            int minD = 1 << 30, maxD = 0, min_rows = 1 << 30;
-            for (int w = 0; w < W; ++w) {
-                const int D = (int)(std::lower_bound(st.begin(), st.end(), b->hf_hi[w]) - std::lower_bound(st.begin(), st.end(), b->hf_lo[w]));
-                sumD += D; minD = std::min(minD, D); maxD = std::max(maxD, D);
-            }
-            for (long long k = 0; k < nb; ++k) min_rows = std::min(min_rows, st[k + 1] - st[k]);
-            const bool day_blocks = !no_inner && nb >= 2 && minD >= 2 && min_rows >= 8 && sumD >= 2 * nb && nb <= h->hf_extra_rows;
-            if (day_blocks) {
-                plan[0].inner = true;
-                plan[0].blk[0] = 1;                 // level 0 in use (block sizes vary: see starts)
-                const int minL = minD - 1, maxL = maxD - 1;       // full days (overnight return included) per window
-                static const bool no_presum = getenv("BP_NO_PRESUM") != nullptr;
-                if (!no_presum && h->presum_min_days > 0 && minD >= h->presum_min_days && maxL <= 2 * minL &&
-                    3 * (size_t)nb * npairs_t * GRAM_BLOCK_TILE_DOUBLES * sizeof(double) <= h->ws_limit)
-                    plan[0].chunk = minL;
-            } else {
-                st.clear();
-                const int H0 = b->hf_hi[0] - b->hf_lo[0];
-                if (H0 >= 3 * 64) {
-                    plan[0].blk[0] = 64;
-                    plan[0].blk[1] = 16;
-                }
-            }
-        }
-    }
-    auto phase_rows = [&](int ph, int w, int& row0, int& rows) {
-        row0 = ph == 0 ? b->hf_lo[w] + 1 : b->day_row[w] - n + 2;
-        rows = ph == 0 ? b->hf_hi[w] - b->hf_lo[w] - 1 : n - 1;
-    };
-    // split of window w's rows in phase ph; inner-block plans take every day of the window as a whole block
-    auto split_of = [&](int ph, int w) {
-        int row0, rows;
-        phase_rows(ph, w, row0, rows);
-        if (ph == 0 && plan[0].inner) {
-            const std::vector<int>& st = plan[0].starts;
-            Split sp;
-            sp.c_lo = std::lower_bound(st.begin(), st.end(), b->hf_lo[w]) - st.begin();
-            sp.c_hi = std::lower_bound(st.begin(), st.end(), b->hf_hi[w]) - st.begin();
-            return sp;
-        }
-        return split_rows(row0, rows, plan[ph]);
-    };
-    // phase B (daily rows): the run of whole blocks inside a window is the same for many consecutive windows, so
-    // each distinct run [lo, hi) is summed once (range_sum_kernel) and a window adds one tile per run
-    std::map<std::pair<long long, long long>, int> range_id[2];
-    // ... and the (coarse, fine, fine) run triple of a window is combined once per distinct triple (combine_runs_kernel)
-    typedef std::array<long long, 6> RunKey;
-    std::map<RunKey, int> full_id;
-    // first pass: block ranges touched by the windows, per level
-    for (int ph = 0; ph < 2; ++ph) {
-        if (plan[ph].blk[0] <= 0 && plan[ph].blk[1] <= 0) continue;
-        if (ph == 0 && !need_hf) { plan[ph] = PhasePlan(); continue; }
-        long long lo[2] = {1LL << 40, 1LL << 40}, hi[2] = {-(1LL << 40), -(1LL << 40)};
-        for (int w = 0; w < W; ++w) {
-            if (w % h->work_stride != 0) continue;      // chain path: only the base windows go through the Gram kernel
-            const Split sp = split_of(ph, w);
-            if (sp.c_hi > sp.c_lo) { lo[0] = std::min(lo[0], sp.c_lo); hi[0] = std::max(hi[0], sp.c_hi); }
-            if (sp.fa_hi > sp.fa_lo) { lo[1] = std::min(lo[1], sp.fa_lo); hi[1] = std::max(hi[1], sp.fa_hi); }
-            if (sp.fb_hi > sp.fb_lo) { lo[1] = std::min(lo[1], sp.fb_lo); hi[1] = std::max(hi[1], sp.fb_hi); }
-            if (ph == 1) {
-                if (sp.c_hi > sp.c_lo) range_id[0].emplace(std::make_pair(sp.c_lo, sp.c_hi), 0);
-                if (sp.fa_hi > sp.fa_lo) range_id[1].emplace(std::make_pair(sp.fa_lo, sp.fa_hi), 0);
-                if (sp.fb_hi > sp.fb_lo) range_id[1].emplace(std::make_pair(sp.fb_lo, sp.fb_hi), 0);
-                if (sp.c_hi > sp.c_lo || sp.fa_hi > sp.fa_lo || sp.fb_hi > sp.fb_lo)
-                    full_id.emplace(RunKey{sp.c_lo, sp.c_hi, sp.fa_lo, sp.fa_hi, sp.fb_lo, sp.fb_hi}, 0);
-            }
-        }
-        for (int l = 0; l < 2; ++l) {
-            if (hi[l] <= lo[l]) { plan[ph].blk[l] = 0; plan[ph].nb[l] = 0; continue; }
-            plan[ph].bmin[l] = (int)lo[l];
-            plan[ph].nb[l] = (int)(hi[l] - lo[l]);
-            size_t need = (size_t)plan[ph].nb[l] * npairs_t * GRAM_BLOCK_TILE_DOUBLES;
-            if (need * sizeof(double) > h->ws_limit / 2) {      // too big: give up the reuse of this phase
-                plan[ph] = PhasePlan();
-                break;
-            }
-            if (ph == 0 && l == 0 && plan[0].chunk > 0) need *= 3;      // + suffix' and prefix tiles of every block
-            if (need > h->store_cap[ph][l]) {
-                CU_TRY(cudaStreamSynchronize(h->stream));
-                cudaFree(h->store[ph][l]);
-                h->store[ph][l] = nullptr;
-                h->store_cap[ph][l] = 0;
-                CU_TRY(cudaMalloc(&h->store[ph][l], need * sizeof(double)));
-                h->store_cap[ph][l] = need;
-            }
-        }
-    }
-    if (plan[0].inner && plan[0].nb[0] != (int)plan[0].starts.size() - 1)
-        return fail(BP_ERR_STATE, "internal: day-block plan out of step with its boundaries");
-    const bool presum = plan[0].inner && plan[0].chunk > 0;
-    const int nb0 = plan[0].inner ? plan[0].nb[0] : 0;
-    if (presum) {
-        const size_t need = 3 * (size_t)nb0 * h->ld;
-        if (need > h->vstore_cap) {
-            CU_TRY(cudaStreamSynchronize(h->stream));
-            cudaFree(h->vstore);
-            h->vstore = nullptr;
-            h->vstore_cap = 0;
-            CU_TRY(cudaMalloc(&h->vstore, need * sizeof(double)));
-            h->vstore_cap = need;
-        }
-    }
-    int nranges[2] = {0, 0};
-    for (int l = 0; l < 2; ++l) {
-        if (plan[1].blk[l] <= 0) { range_id[l].clear(); continue; }
-        for (auto& kv : range_id[l]) kv.second = nranges[l]++;
-        const size_t need = (size_t)nranges[l] * npairs_t * GRAM_BLOCK_TILE_DOUBLES;
-        if (need > h->rstore_cap[l]) {
-            CU_TRY(cudaStreamSynchronize(h->stream));
-            cudaFree(h->rstore[l]);
-            h->rstore[l] = nullptr;
-            h->rstore_cap[l] = 0;
-            CU_TRY(cudaMalloc(&h->rstore[l], need * sizeof(double)));
-            h->rstore_cap[l] = need;
-        }
-    }
-    int nfull = 0;
-    if (plan[1].blk[0] <= 0 && plan[1].blk[1] <= 0) full_id.clear();
-    for (auto& kv : full_id) kv.second = nfull++;
-    {
-        const size_t need = (size_t)nfull * npairs_t * GRAM_BLOCK_TILE_DOUBLES;
-        if (need > h->fstore_cap) {
-            CU_TRY(cudaStreamSynchronize(h->stream));
-            cudaFree(h->fstore);
-            h->fstore = nullptr;
-            h->fstore_cap = 0;
-            CU_TRY(cudaMalloc(&h->fstore, need * sizeof(double)));
-            h->fstore_cap = need;
-        }
-    }
-    const int nb_total = plan[0].nb[0] + plan[0].nb[1] + plan[1].nb[0] + plan[1].nb[1];
-    const size_t ints_needed = (size_t)(7 + GRAM_DESC_INTS) * W + (size_t)GRAM_DESC_INTS * nb_total +
-                               2 * (size_t)(nranges[0] + nranges[1]) + 3 * (size_t)nfull +
-                               (plan[0].inner ? (size_t)nb0 + 1 : 0) + (presum ? 3 * (size_t)W : 0);
+    const PlanCtx ctx = plan_ctx(h, stride);
+    int rc = check_batch(ctx, b, need_hf, &g_err);
+    if (!rc) rc = plan_batch(ctx, b, need_hf, &out->plan, &g_err);
+    if (rc) return rc;
+    const BatchPlan& P = out->plan;
+    const int W = P.W;
+    for (int ph = 0; ph < 2; ++ph)
+        for (int l = 0; l < 2; ++l)
+            if ((rc = grow(h, h->store[ph][l], P.store[ph][l]))) return rc;
+    for (int l = 0; l < 2; ++l)
+        if ((rc = grow(h, h->rstore[l], P.rstore[l]))) return rc;
+    if ((rc = grow(h, h->fstore, P.fstore)) || (rc = grow(h, h->vstore, P.vstore))) return rc;
     const int slot = h->desc_turn ^= 1;
     if (h->ev_desc_armed[slot]) {
         CU_TRY(cudaEventSynchronize(h->ev_desc[slot]));      // its staging buffer has been fetched
         h->ev_desc_armed[slot] = false;
     }
-    if (ints_needed > h->desc_cap_slot[slot]) {
-        if (h->desc_slot[slot]) {
-            CU_TRY(cudaStreamSynchronize(h->stream));
-            cudaFree(h->desc_slot[slot]);
-            cudaFreeHost(h->desc_host_slot[slot]);
-        }
-        h->desc_slot[slot] = nullptr;
-        h->desc_host_slot[slot] = nullptr;
-        h->desc_cap_slot[slot] = 0;
-        CU_TRY(cudaMalloc(&h->desc_slot[slot], sizeof(int) * ints_needed));
-        CU_TRY(cudaHostAlloc(&h->desc_host_slot[slot], sizeof(int) * ints_needed, cudaHostAllocDefault));
-        h->desc_cap_slot[slot] = ints_needed;
-    }
-    h->desc = h->desc_slot[slot];
-    h->desc_host = h->desc_host_slot[slot];
-    h->desc_cap = h->desc_cap_slot[slot];
-    int* host = h->desc_host;
-    memset(host, 0, sizeof(int) * ints_needed);
-    int* gd = host + (size_t)7 * W;                  // Gram job descriptors
-    int max_m = 0;
-    for (int w = 0; w < W; ++w) {
-        const int dr = b->day_row[w];
-        if (rs) {
-            // shared weekly rows dr-(n-2)+1 .. dr (row 0 is the zero row of the first week) + one per-date row
-            if (dr - (n - 2) + 1 < 1 || dr >= h->Rw)
-                return fail(BP_ERR_INVALID, "window %d: resampled day_row %d needs %d prior rows inside [1,%d)", w, dr, n - 2, h->Rw);
-            if (b->extra_row[w] < 0 || b->extra_row[w] >= h->Rw || b->caps_row[w] < 0 || b->caps_row[w] >= h->D)
-                return fail(BP_ERR_INVALID, "window %d: extra_row / caps_row out of range", w);
-            host[(size_t)5 * W + w] = b->extra_row[w];
-            host[(size_t)6 * W + w] = b->caps_row[w];
-        } else {
-            if (dr < n - 1 || dr >= h->D)
-                return fail(BP_ERR_INVALID, "window %d: day_row %d needs %d prior price rows inside [0,%d)", w, dr, n - 1, h->D);
-            host[(size_t)5 * W + w] = -1;
-            host[(size_t)6 * W + w] = dr;
-        }
-        if (need_hf && !b->prior_n && dr < (b->mcm_rows ? b->mcm_rows : n) - 1 - (rs ? 1 : 0))
-            return fail(BP_ERR_INVALID, "window %d: not enough MCM observations before day_row %d", w, dr);
-        if (b->span_days[w] <= 0) return fail(BP_ERR_INVALID, "window %d: span_days must be positive", w);
-        host[w] = dr;
-        host[(size_t)W + w] = b->span_days[w];
-        host[(size_t)2 * W + w] = rs ? dr - (n - 2) + 1 : dr - n + 2;   // first RETURN row (F2: n prices -> n-1 returns)
-        if (need_hf) {
-            const int lo = b->hf_lo[w], hi = b->hf_hi[w];
-            const int m = hi - lo - 1;
-            if (lo < 0 || (long long)hi > h->R || m < 2)
-                return fail(BP_ERR_INVALID, "window %d: intraday rows [%d,%d) give %d returns (need >= 2, rows < %lld)", w, lo, hi, m, h->R);
-            host[(size_t)3 * W + w] = lo + 1;        // first HF return row: the window's first bar has no return (F5)
-            host[(size_t)4 * W + w] = m;
-            max_m = std::max(max_m, m);
-            int* dA = gd + (size_t)w * GRAM_DESC_INTS;
-            write_phase_desc(split_of(0, w), plan[0], dA);
-            if (presum) {
-                // suffix'[first day] (+ one whole chunk) (+ prefix[last day]): explicit tile ids into the unified store
-                // [inner | suffix' | prefix]; the same ids address the scanned column sums (hf_vids)
-                const int C = plan[0].chunk, c_lo = dA[4], last = dA[4] + dA[5] - 1;
-                const int qa = c_lo / C, s_next = std::min((qa + 1) * C, nb0);
-                int ids[3] = {nb0 + c_lo, -1, -1};
-                if (s_next <= last) {
-                    const int ql = last / C;
-                    if (ql > qa + 2) return fail(BP_ERR_STATE, "internal: pre-summed run spans more than three chunks");
-                    if (ql == qa + 2) ids[1] = 2 * nb0 + (qa + 2) * C - 1;
-                    ids[2] = 2 * nb0 + last;
-                }
-                dA[0] = dA[1] = dA[2] = dA[3] = 0;
-                for (int k = 0; k < 3; ++k) { dA[4 + 2 * k] = ids[k] >= 0 ? ids[k] : 0; dA[5 + 2 * k] = ids[k] >= 0 ? 1 : 0; }
-                int* vid = host + ((size_t)(7 + GRAM_DESC_INTS) * W + (size_t)GRAM_DESC_INTS * nb_total +
-                                   2 * (size_t)(nranges[0] + nranges[1]) + 3 * (size_t)nfull + (size_t)nb0 + 1) + 3 * (size_t)w;
-                vid[0] = ids[0]; vid[1] = ids[1]; vid[2] = ids[2];
-            } else if (plan[0].inner) {
-                // overnight returns of days 2..last of the window: a run of dA[5]-1 gathered rows behind the matrix
-                dA[0] = (int)(h->R + dA[4] + 1);
-                dA[1] = dA[5] - 1;
-            }
-        }
-        if (rs) {
-            int* dB = gd + (size_t)w * GRAM_DESC_INTS + GRAM_PHASE_INTS;
-            dB[0] = dr - (n - 2) + 1; dB[1] = n - 2;       // shared weekly rows
-            dB[2] = b->extra_row[w];  dB[3] = 1;           // the trade date's own row
-        } else if (w % h->work_stride == 0) {
-            const Split sp = split_rows(dr - n + 2, n - 1, plan[1]);
-            int* dB = gd + (size_t)w * GRAM_DESC_INTS + GRAM_PHASE_INTS;
-            write_phase_desc(sp, plan[1], dB);
-            // one pre-summed tile per run of whole blocks
-            // ... combined into one tile per distinct (coarse, fine, fine) triple: the coarse slot points into fstore
-            if (dB[5] > 0 || dB[7] > 0 || dB[9] > 0) {
-                dB[4] = full_id[RunKey{sp.c_lo, sp.c_hi, sp.fa_lo, sp.fa_hi, sp.fb_lo, sp.fb_hi}];
-                dB[5] = 1;
-                dB[6] = dB[7] = dB[8] = dB[9] = 0;
-            }
-        }
-        const int* d = gd + (size_t)w * GRAM_DESC_INTS;
-        auto r8 = [](int r) { return (r + 7) / 8 * 8; };
-        for (int ph = 0; ph < 2 && w % h->work_stride == 0; ++ph) {
-            const int* dp = d + ph * GRAM_PHASE_INTS;
-            h->work_k_rows += r8(dp[1]) + r8(dp[3]);
-            h->work_add_blocks += dp[5] + dp[7] + dp[9];
-        }
-        h->work_full_rows += (need_hf ? b->hf_hi[w] - b->hf_lo[w] - 1 : 0) + (n - 1);
-    }
-    for (int ph = 0; ph < 2; ++ph)
-        for (int l = 0; l < 2; ++l) {
-            if (ph == 0 && l == 0 && plan[0].inner) {
-                for (int k = 0; k < nb0; ++k) h->work_pre_rows += (plan[0].starts[k + 1] - plan[0].starts[k] - 1 + 7) / 8 * 8;
-                continue;
-            }
-            h->work_pre_rows += (double)plan[ph].nb[l] * ((plan[ph].blk[l] + 7) / 8 * 8);
-        }
-    if (presum) h->work_scan_tiles += (double)nb0;
-    // descriptors of the block precompute launches: one pseudo-window per block, rows of that block only
-    int* bd = gd + (size_t)W * GRAM_DESC_INTS;
-    for (int ph = 0; ph < 2; ++ph)
-        for (int l = 0; l < 2; ++l) {
-            for (int k = 0; k < plan[ph].nb[l]; ++k) {
-                int* d = bd + (size_t)k * GRAM_DESC_INTS + GRAM_PHASE_INTS * ph;
-                if (plan[ph].inner) {           // the day without its overnight return
-                    d[0] = plan[ph].starts[k] + 1;
-                    d[1] = plan[ph].starts[k + 1] - plan[ph].starts[k] - 1;
-                } else {
-                    d[0] = plan[ph].off + (plan[ph].bmin[l] + k) * plan[ph].blk[l];
-                    d[1] = plan[ph].blk[l];
-                }
-            }
-            out->bdesc[ph][l] = plan[ph].nb[l] ? h->desc + (bd - host) : nullptr;
-            out->nblocks[ph][l] = plan[ph].nb[l];
-            bd += (size_t)plan[ph].nb[l] * GRAM_DESC_INTS;
-        }
-    // block runs to pre-sum (store-relative block indices)
-    for (int l = 0; l < 2; ++l) {
-        for (const auto& kv : range_id[l]) {
-            bd[2 * kv.second] = (int)(kv.first.first - plan[1].bmin[l]);
-            bd[2 * kv.second + 1] = (int)(kv.first.second - plan[1].bmin[l]);
-        }
-        out->rdesc[l] = nranges[l] ? h->desc + (bd - host) : nullptr;
-        out->nranges[l] = nranges[l];
-        bd += 2 * (size_t)nranges[l];
-    }
-    for (const auto& kv : full_id) {
-        const RunKey& k = kv.first;
-        int* d = bd + 3 * (size_t)kv.second;
-        d[0] = k[1] > k[0] ? range_id[0][std::make_pair(k[0], k[1])] : -1;
-        d[1] = k[3] > k[2] ? range_id[1][std::make_pair(k[2], k[3])] : -1;
-        d[2] = k[5] > k[4] ? range_id[1][std::make_pair(k[4], k[5])] : -1;
-    }
-    out->fdesc = nfull ? h->desc + (bd - host) : nullptr;
-    out->nfull = nfull;
-    bd += 3 * (size_t)nfull;
-    if (plan[0].inner) {
-        for (int k = 0; k <= nb0; ++k) bd[k] = plan[0].starts[k];
-        out->hf_starts_dev = h->desc + (bd - host);
-        out->hf_starts = plan[0].starts;
-        bd += (size_t)nb0 + 1;
-        if (presum) {
-            out->hf_vids = h->desc + (bd - host);       // filled per window above
-            bd += 3 * (size_t)W;
-        }
-    }
-    out->presum = presum;
-    out->presum_chunk = plan[0].chunk;
-    out->gdesc = h->desc + (size_t)7 * W;
-    {
-        // banded-GEMM daily pass: worth it when 32 consecutive windows share almost all of their rows
-        static const bool no_band = getenv("BP_NO_BAND") != nullptr;
-        bool ok = !no_band && !rs && W >= 32 && n >= 16;
-        for (int w = 1; ok && w < W; ++w) ok = b->day_row[w] >= b->day_row[w - 1];
-        if (ok) ok = (long long)b->day_row[W - 1] - b->day_row[0] <= 2LL * W;
-        out->band_ok = ok;
-    }
-    out->hf_off = plan[0].off;
-    for (int l = 0; l < 2; ++l) { out->hf_bmin[l] = plan[0].bmin[l]; out->hf_blk[l] = plan[0].blk[l]; }
-    out->hf_inner = plan[0].inner;
-    out->hf_nb0 = plan[0].nb[0];
-    out->resampled = rs;
-    out->extra_row = rs ? h->desc + 5 * (size_t)W : nullptr;
-    out->caps_row = h->desc + 6 * (size_t)W;
+    if ((rc = grow(h, h->desc_slot[slot], P.ints)) || (rc = grow(h, h->desc_host_slot[slot], P.ints))) return rc;
+    int* dev = h->desc_slot[slot].p;
+    write_batch(P, b, h->desc_host_slot[slot].p);
     // zero-copy fetch by a kernel on the compute stream (not the copy engine, see fetch_ints_kernel); the
     // staging buffer of this slot is rewritten two batches later, after this event
-    launch_fetch_ints(host, h->desc, (long long)ints_needed, h->stream);
+    launch_fetch_ints(h->desc_host_slot[slot].p, dev, (long long)P.ints, h->stream);
     h->launches++;
     CU_TRY(cudaGetLastError());
     if (!h->ev_desc[slot]) CU_TRY(cudaEventCreateWithFlags(&h->ev_desc[slot], cudaEventDisableTiming));
     CU_TRY(cudaEventRecord(h->ev_desc[slot], h->stream));
     h->ev_desc_armed[slot] = true;
     if (need_hf && b->prior_n) {
-        if (W > h->prior_n_cap) {
-            cudaFree(h->prior_n);
-            h->prior_n = nullptr;
-            h->prior_n_cap = 0;
-            CU_TRY(cudaMalloc(&h->prior_n, sizeof(double) * (size_t)W));
-            h->prior_n_cap = W;
-        }
-        CU_TRY(cudaMemcpyAsync(h->prior_n, b->prior_n, sizeof(double) * (size_t)W, cudaMemcpyHostToDevice, h->stream));
+        if ((rc = grow(h, h->prior_n, (size_t)W))) return rc;
+        CU_TRY(cudaMemcpyAsync(h->prior_n.p, b->prior_n, sizeof(double) * (size_t)W, cudaMemcpyHostToDevice, h->stream));
         CU_TRY(cudaStreamSynchronize(h->stream));
-        out->prior_n = h->prior_n;
+        out->prior_n = h->prior_n.p;
     }
-    out->mcm_rows = b->mcm_rows ? b->mcm_rows : n;
-    out->W = W;
-    out->n = n;
-    out->max_m = max_m;
-    out->has_hf = need_hf;
-    out->day_row = h->desc;
-    out->span = h->desc + W;
-    out->row0 = h->desc + 2 * (size_t)W;
-    out->hf_row0 = h->desc + 3 * (size_t)W;
-    out->hf_m = h->desc + 4 * (size_t)W;
+    out->day_row = dev;
+    out->span = dev + W;
+    out->hf_row0 = dev + 3 * (size_t)W;
+    out->hf_m = dev + 4 * (size_t)W;
+    out->extra_row = P.resampled ? dev + 5 * (size_t)W : nullptr;
+    out->caps_row = dev + 6 * (size_t)W;
+    out->gdesc = dev + P.off_gram;
+    for (int ph = 0; ph < 2; ++ph)
+        for (int l = 0; l < 2; ++l) out->bdesc[ph][l] = P.phase[ph].nb[l] ? dev + P.off_blocks[ph][l] : nullptr;
+    for (int l = 0; l < 2; ++l) out->rdesc[l] = P.nranges[l] ? dev + P.off_ranges[l] : nullptr;
+    out->fdesc = P.nfull ? dev + P.off_triples : nullptr;
+    out->hf_starts = P.phase[0].inner ? dev + P.off_starts : nullptr;
+    out->hf_vids = P.presum ? dev + P.off_vids : nullptr;
+    h->work_k_rows += P.work_k_rows;
+    h->work_add_blocks += P.work_add_blocks;
+    h->work_pre_rows += P.work_pre_rows;
+    h->work_full_rows += P.work_full_rows;
     return BP_OK;
 }
 
@@ -886,11 +430,11 @@ int emit_vec(bp_handle* h, const double* src, const Layout& L, int Wc, double* d
         const size_t bytes = sizeof(double) * (size_t)Wc * L.N;
         // the single staging buffer is reused: drain the previous D2H copy before overwriting it
         if (h->need_sync) CU_TRY(cudaStreamSynchronize(h->stream));
-        int rc = ensure_stage(h, bytes);
+        int rc = grow(h, h->stage, bytes);
         if (rc) return rc;
-        launch_unpack_vec(src, L.ldv, L.N, Wc, reinterpret_cast<double*>(h->stage), h->stream);
+        launch_unpack_vec(src, L.ldv, L.N, Wc, reinterpret_cast<double*>(h->stage.p), h->stream);
         h->launches++;
-        CU_TRY(cudaMemcpyAsync(dst, h->stage, bytes, cudaMemcpyDeviceToHost, h->stream));
+        CU_TRY(cudaMemcpyAsync(dst, h->stage.p, bytes, cudaMemcpyDeviceToHost, h->stream));
         h->need_sync = true;
     }
     return BP_OK;
@@ -904,11 +448,11 @@ int emit_sym(bp_handle* h, const double* S, const Layout& L, int Wc, double* dst
     } else {
         const size_t bytes = sizeof(double) * (size_t)Wc * L.N * L.N;
         if (h->need_sync) CU_TRY(cudaStreamSynchronize(h->stream));
-        int rc = ensure_stage(h, bytes);
+        int rc = grow(h, h->stage, bytes);
         if (rc) return rc;
-        launch_unpack_sym(S, L.win_stride, L.ldS, L.N, Wc, reinterpret_cast<double*>(h->stage), h->stream);
+        launch_unpack_sym(S, L.win_stride, L.ldS, L.N, Wc, reinterpret_cast<double*>(h->stage.p), h->stream);
         h->launches++;
-        CU_TRY(cudaMemcpyAsync(dst, h->stage, bytes, cudaMemcpyDeviceToHost, h->stream));
+        CU_TRY(cudaMemcpyAsync(dst, h->stage.p, bytes, cudaMemcpyDeviceToHost, h->stream));
         h->need_sync = true;
     }
     return BP_OK;
@@ -927,20 +471,20 @@ PrepParams prep_params(const bp_handle* h, const bp_window_batch* b, const Batch
     PrepParams p{};
     p.mode = mode;
     p.n_assets = h->N;
-    p.n_window = B.n;
+    p.n_window = B.plan.n;
     p.ld = h->ld;
     p.ldv = L.ldv;
     p.prior_kind = b->prior_weights == 0 ? BP_PRIOR_VW : BP_PRIOR_EW;
     p.mcm_scaling = b->mcm_scaling;
-    p.lr_daily = B.resampled ? h->lr_w : h->lr_d;
+    p.lr_daily = B.plan.resampled ? h->lr_w : h->lr_d;
     p.lr_hf = h->lr_hf;
     p.caps = h->has_caps ? h->caps : nullptr;
     p.ld_caps = h->N;
     p.mcm = (mode == BP_MODE_CONJUGATE && h->mcm) ? h->mcm + (size_t)b->mcm_index * h->D : nullptr;
-    if (B.resampled) p.mcm = (mode == BP_MODE_CONJUGATE && h->mcm_w) ? h->mcm_w + (size_t)b->mcm_index * h->Rw : nullptr;
-    p.mcm_rows = B.mcm_rows;
+    if (B.plan.resampled) p.mcm = (mode == BP_MODE_CONJUGATE && h->mcm_w) ? h->mcm_w + (size_t)b->mcm_index * h->Rw : nullptr;
+    p.mcm_rows = B.plan.mcm_rows;
     p.prior_n = B.prior_n ? B.prior_n + w0 : nullptr;
-    p.rf_row = B.resampled ? h->rf_w : h->rf_row;
+    p.rf_row = B.plan.resampled ? h->rf_w : h->rf_row;
     p.day_row = B.day_row + w0;
     p.extra_row = B.extra_row ? B.extra_row + w0 : nullptr;
     p.caps_row = B.caps_row ? B.caps_row + w0 : nullptr;
@@ -951,13 +495,13 @@ PrepParams prep_params(const bp_handle* h, const bp_window_batch* b, const Batch
     p.scal = c.scal;
     p.y_ws = c.y;
     p.y_stride = L.y_stride;
-    p.hf_presum = (mode == BP_MODE_CONJUGATE && B.presum) ? 1 : 0;
-    p.hf_vsum = h->vstore;
+    p.hf_presum = (mode == BP_MODE_CONJUGATE && B.plan.presum) ? 1 : 0;
+    p.hf_vsum = h->vstore.p;
     p.hf_vids = B.hf_vids ? B.hf_vids + 3 * (size_t)w0 : nullptr;
-    p.use_band = B.band_ok ? 1 : 0;
-    p.band_ld = round_up(B.n - 1, 2);
-    p.band_aw = B.band_ok ? h->band_aw + (size_t)w0 * p.band_ld : nullptr;
-    p.band_stats = B.band_ok ? h->band_stats + 2 * (size_t)w0 : nullptr;
+    p.use_band = B.plan.band_ok ? 1 : 0;
+    p.band_ld = round_up(B.plan.n - 1, 2);
+    p.band_aw = B.plan.band_ok ? h->band_aw.p + (size_t)w0 * p.band_ld : nullptr;
+    p.band_stats = B.plan.band_ok ? h->band_stats.p + 2 * (size_t)w0 : nullptr;
     return p;
 }
 
@@ -975,13 +519,13 @@ GramParams gram_params(const bp_handle* h, const Batch& B, const Layout& L, cons
     g.out = c.S;
     g.desc = B.gdesc + (size_t)w0 * GRAM_DESC_INTS;
     for (int l = 0; l < 2; ++l) {
-        g.store[0][l] = h->store[0][l];          // intraday: one tile per whole block
-        g.store[1][l] = l == 0 ? h->fstore : h->rstore[l];      // daily: ONE combined tile per window (runs of whole blocks, pre-summed)
+        g.store[0][l] = h->store[0][l].p;        // intraday: one tile per whole block
+        g.store[1][l] = l == 0 ? h->fstore.p : h->rstore[l].p;      // daily: ONE combined tile per window (runs of whole blocks, pre-summed)
     }
     const bool hf = kind == GRAM_S0 || kind == GRAM_S1;
     const bool daily = kind != GRAM_S0;
-    if (B.presum) {
-        g.store[0][1] = h->store[0][0];          // explicit tile ids into the unified [inner | suffix' | prefix] store
+    if (B.plan.presum) {
+        g.store[0][1] = h->store[0][0].p;          // explicit tile ids into the unified [inner | suffix' | prefix] store
         if (hf) {
             g.mv_part = c.mv;
             g.mv_w0 = c.w0;
@@ -1008,7 +552,7 @@ int run_block_precompute(bp_handle* h, const Batch& B, int ph, const int* k0 = n
     const int nt = (h->N + GRAM_TILE - 1) / GRAM_TILE;
     const size_t tile_doubles = (size_t)(nt * (nt + 1) / 2) * GRAM_BLOCK_TILE_DOUBLES;
     for (int l = 0; l < 2; ++l) {
-        const int b0 = k0 ? k0[l] : 0, b1 = k1 ? k1[l] : B.nblocks[ph][l];
+        const int b0 = k0 ? k0[l] : 0, b1 = k1 ? k1[l] : B.plan.phase[ph].nb[l];
         if (b1 <= b0) continue;
         GramParams g{};
         g.n_windows = b1 - b0;
@@ -1017,19 +561,19 @@ int run_block_precompute(bp_handle* h, const Batch& B, int ph, const int* k0 = n
         g.use_phaseA = ph == 0;
         g.use_phaseB = ph == 1;
         g.tile_store_out = 1;
-        g.out = h->store[ph][l] + (size_t)b0 * tile_doubles;
+        g.out = h->store[ph][l].p + (size_t)b0 * tile_doubles;
         StageTimer tm(h, BP_STAGE_GRAM);
         CU_TRY(launch_gram(g, h->map_hf, h->map_d, h->sm_count, h->stream));
         h->launches++;
-        if (ph == 1 && B.nranges[l] > 0) {
-            launch_range_sum(h->store[1][l], B.rdesc[l], B.nranges[l], nt * (nt + 1) / 2, h->rstore[l], h->stream);
+        if (ph == 1 && B.plan.nranges[l] > 0) {
+            launch_range_sum(h->store[1][l].p, B.rdesc[l], B.plan.nranges[l], nt * (nt + 1) / 2, h->rstore[l].p, h->stream);
             h->launches++;
             CU_TRY(cudaGetLastError());
         }
     }
-    if (ph == 1 && !k0 && B.nfull > 0) {
+    if (ph == 1 && !k0 && B.plan.nfull > 0) {
         StageTimer tm(h, BP_STAGE_GRAM);
-        launch_combine_runs(h->rstore[0], h->rstore[1], B.fdesc, B.nfull, nt * (nt + 1) / 2, h->fstore, h->stream);
+        launch_combine_runs(h->rstore[0].p, h->rstore[1].p, B.fdesc, B.plan.nfull, nt * (nt + 1) / 2, h->fstore.p, h->stream);
         h->launches++;
         CU_TRY(cudaGetLastError());
     }
@@ -1073,62 +617,51 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
         // closer to the rank limit every window is factorised on its own (the path the parity tests pin).
         if (G >= 2 && b->rolling_window - 1 < h->N + 2 * G + 8) G = 0;
     }
-    if (h) h->work_stride = G >= 2 ? G : 1;
-    int rc = upload_batch(h, b, mode == BP_MODE_CONJUGATE, &B);
-    if (h) h->work_stride = 1;
+    int rc = upload_batch(h, b, mode == BP_MODE_CONJUGATE, G >= 2 ? G : 1, &B);
     if (rc) return rc;
-    const Layout L = make_layout(h, B.presum ? 0 : B.max_m, B.presum);
-    int Wc = (int)std::min<size_t>((size_t)B.W, std::max<size_t>(1, h->ws_limit / L.per_window));
+    const BatchPlan& P = B.plan;
+    const PhasePlan& A = P.phase[0];
+    const Layout L = make_layout(h, P.presum ? 0 : P.max_m, P.presum);
+    int Wc = (int)std::min<size_t>((size_t)P.W, std::max<size_t>(1, h->ws_limit / L.per_window));
     // (the descriptors were planned for the base windows only: the chain path must not be abandoned after upload_batch;
     // the check above uses the same layout, so this cannot trigger unless the two are changed apart)
-    if (Wc < B.W && G >= 2) return fail(BP_ERR_STATE, "internal: chained batch does not fit one workspace chunk");
+    if (Wc < P.W && G >= 2) return fail(BP_ERR_STATE, "internal: chained batch does not fit one workspace chunk");
     // Pipelined against a segmented asynchronous intraday upload: prep + Gram of the windows whose bars have
     // arrived run while the rest is still being copied; the solve follows for all windows at once.
     const bool pipelined = mode == BP_MODE_CONJUGATE && h->hf_pending && h->n_seg > 1 && h->seg_waited < h->n_seg &&
-                           solve && !out->T && !out->S0 && Wc >= B.W && !B.presum;
+                           solve && !out->T && !out->S0 && Wc >= P.W && !P.presum;
     if (mode == BP_MODE_CONJUGATE && !pipelined) {
         long long need = 0;                   // intraday price rows this batch reads
-        for (int w = 0; w < B.W; ++w) need = std::max<long long>(need, b->hf_hi[w]);
+        for (int w = 0; w < P.W; ++w) need = std::max<long long>(need, b->hf_hi[w]);
         if ((rc = wait_hf_rows(h, need))) return rc;
     }
-    rc = ensure_ws(h, (size_t)Wc * L.per_window + 256);
+    rc = grow(h, h->ws, (size_t)Wc * L.per_window + 256);
     if (rc) return rc;
-    const Chunk c = carve(h->ws, L, Wc);
+    const Chunk c = carve(h->ws.p, L, Wc);
     const int N = h->N;
-    if (B.band_ok) {
-        const size_t need_aw = (size_t)B.W * round_up(B.n - 1, 2), need_st = 2 * (size_t)B.W;
-        if (need_aw > h->band_aw_cap || need_st > h->band_stats_cap) {
-            CU_TRY(cudaStreamSynchronize(h->stream));
-            cudaFree(h->band_aw);
-            cudaFree(h->band_stats);
-            h->band_aw = h->band_stats = nullptr;
-            h->band_aw_cap = h->band_stats_cap = 0;
-            CU_TRY(cudaMalloc(&h->band_aw, sizeof(double) * need_aw));
-            CU_TRY(cudaMalloc(&h->band_stats, sizeof(double) * need_st));
-            h->band_aw_cap = need_aw;
-            h->band_stats_cap = need_st;
-        }
-    }
+    if (P.band_ok && ((rc = grow(h, h->band_aw, (size_t)P.W * round_up(P.n - 1, 2))) ||
+                      (rc = grow(h, h->band_stats, 2 * (size_t)P.W))))
+        return rc;
     if (solve && (mode == BP_MODE_CONJUGATE || estimator != BP_EST_NONE) && !(b->risk_aversion != 0.0))
         return fail(BP_ERR_INVALID, "risk_aversion must be non-zero");
-    if (estimator == BP_EST_JORION && B.n - 1 - N - 2 <= 0)
+    if (estimator == BP_EST_JORION && P.n - 1 - N - 2 <= 0)
         return fail(BP_ERR_INVALID, "Jorion needs T - N - 2 > 0 (T = rolling_window - 1 returns, :879)");
 
     const bool any_gram = out->T || out->S0 || out->S1 || solve;
     if (any_gram && !pipelined) {
-        if (mode == BP_MODE_CONJUGATE && B.hf_inner && !B.presum) {
-            launch_gather_rows_indexed(h->lr_hf, h->ld, B.hf_starts_dev, h->R, 0, B.hf_nb0, h->stream);
+        if (mode == BP_MODE_CONJUGATE && A.inner && !P.presum) {
+            launch_gather_rows_indexed(h->lr_hf, h->ld, B.hf_starts, h->R, 0, A.nb[0], h->stream);
             h->launches++;
             CU_TRY(cudaGetLastError());
         }
-        if (mode == BP_MODE_CONJUGATE && (out->S0 || out->S1 || solve || B.presum) && (rc = run_block_precompute(h, B, 0))) return rc;
-        if (mode == BP_MODE_CONJUGATE && B.presum) {
+        if (mode == BP_MODE_CONJUGATE && (out->S0 || out->S1 || solve || P.presum) && (rc = run_block_precompute(h, B, 0))) return rc;
+        if (mode == BP_MODE_CONJUGATE && P.presum) {
             // scans of the day blocks: column sums (vectors) and Gram tiles, suffix' and prefix per chunk
             StageTimer tm(h, BP_STAGE_GRAM);
             const int nt = (N + GRAM_TILE - 1) / GRAM_TILE;
-            launch_block_col_sums(h->lr_hf, h->ld, B.hf_starts_dev, 0, B.hf_nb0, h->vstore, h->stream);
-            launch_vec_scan(h->vstore, h->ld, h->lr_hf, B.hf_starts_dev, B.hf_nb0, B.presum_chunk, h->stream);
-            launch_tile_scan(h->store[0][0], nt * (nt + 1) / 2, nt, h->lr_hf, h->ld, B.hf_starts_dev, B.hf_nb0, B.presum_chunk, h->stream);
+            launch_block_col_sums(h->lr_hf, h->ld, B.hf_starts, 0, A.nb[0], h->vstore.p, h->stream);
+            launch_vec_scan(h->vstore.p, h->ld, h->lr_hf, B.hf_starts, A.nb[0], A.chunk, h->stream);
+            launch_tile_scan(h->store[0][0].p, nt * (nt + 1) / 2, nt, h->lr_hf, h->ld, B.hf_starts, A.nb[0], A.chunk, h->stream);
             h->launches += 3;
             CU_TRY(cudaGetLastError());
         }
@@ -1147,7 +680,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
         sp.ldv = L.ldv;
         sp.mode = mode;
         sp.estimator = estimator;
-        sp.n_returns = B.n - 1;
+        sp.n_returns = P.n - 1;
         sp.inv_gamma = 1.0 / b->risk_aversion;         // the reference evaluates (1/gamma) * nu (:836,:849)
         sp.S = cs.S;
         sp.rhs = cs.rhs;
@@ -1181,19 +714,19 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
             h->lr_hf_done = r_end;
             int k_ready[2];
             for (int l = 0; l < 2; ++l) {
-                k_ready[l] = B.nblocks[0][l];
-                if (!last && l == 0 && B.hf_inner) {
+                k_ready[l] = A.nb[l];
+                if (!last && l == 0 && A.inner) {
                     // day block k is complete once the bars below starts[k+1] have arrived
-                    const long long k = std::upper_bound(B.hf_starts.begin() + 1, B.hf_starts.end(), (int)std::min<long long>(r_end, 0x7fffffff)) -
-                                        (B.hf_starts.begin() + 1);
-                    k_ready[l] = (int)std::min<long long>(B.nblocks[0][l], std::max<long long>(k, k_done[l]));
-                } else if (!last && B.hf_blk[l] > 0) {
-                    const long long k = floor_div(r_end - B.hf_off, B.hf_blk[l]) - B.hf_bmin[l];
-                    k_ready[l] = (int)std::min<long long>(B.nblocks[0][l], std::max<long long>(k, k_done[l]));
+                    const long long k = std::upper_bound(A.starts.begin() + 1, A.starts.end(), (int)std::min<long long>(r_end, 0x7fffffff)) -
+                                        (A.starts.begin() + 1);
+                    k_ready[l] = (int)std::min<long long>(A.nb[l], std::max<long long>(k, k_done[l]));
+                } else if (!last && A.blk[l] > 0) {
+                    const long long k = floor_div(r_end, A.blk[l]) - A.bmin[l];
+                    k_ready[l] = (int)std::min<long long>(A.nb[l], std::max<long long>(k, k_done[l]));
                 }
             }
-            if (B.hf_inner) {
-                launch_gather_rows_indexed(h->lr_hf, h->ld, B.hf_starts_dev, h->R, k_done[0], k_ready[0], h->stream);
+            if (A.inner) {
+                launch_gather_rows_indexed(h->lr_hf, h->ld, B.hf_starts, h->R, k_done[0], k_ready[0], h->stream);
                 h->launches++;
                 CU_TRY(cudaGetLastError());
             }
@@ -1201,8 +734,8 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
             k_done[0] = k_ready[0];
             k_done[1] = k_ready[1];
             int w_end = w_done;
-            if (last) w_end = B.W;
-            else while (w_end < B.W && (long long)b->hf_hi[w_end] <= r_end) ++w_end;
+            if (last) w_end = P.W;
+            else while (w_end < P.W && (long long)b->hf_hi[w_end] <= r_end) ++w_end;
             if (w_end > w_done) {
                 const Chunk cw = chunk_at(c, L, w_done);
                 PrepParams pp = prep_params(h, b, B, L, cw, w_done, mode);
@@ -1212,7 +745,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
                     h->launches += pp.use_band ? 2 : 0;
                 }
                 h->launches++;
-                if ((rc = run_gram(h, gram_params(h, B, L, cw, w_done, w_end - w_done, GRAM_S1), B.resampled))) return rc;
+                if ((rc = run_gram(h, gram_params(h, B, L, cw, w_done, w_end - w_done, GRAM_S1), P.resampled))) return rc;
                 w_done = w_end;
             }
             // Solve the full waves of windows that are ready: the compute stream would otherwise idle until the next
@@ -1236,12 +769,12 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
         h->seg_waited = h->n_seg;
         h->hf_pending = false;
     }
-    for (int w0 = 0; w0 < B.W; w0 += Wc) {
-        const int wc = std::min(Wc, B.W - w0);
+    for (int w0 = 0; w0 < P.W; w0 += Wc) {
+        const int wc = std::min(Wc, P.W - w0);
         const size_t ov = (size_t)w0 * N, om = (size_t)w0 * N * N;
         if (!pipelined) {
             PrepParams pp = prep_params(h, b, B, L, c, w0, mode);
-            if (estimator != BP_EST_NONE) pp.beta_den = B.n - 1;       // sample covariance: centre with 1/m, m = n-1 returns
+            if (estimator != BP_EST_NONE) pp.beta_den = P.n - 1;       // sample covariance: centre with 1/m, m = n-1 returns
             {
                 StageTimer tm(h, BP_STAGE_PREP);
                 CU_TRY(launch_window_prep(pp, wc, h->stream, h->D));
@@ -1250,14 +783,14 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
             h->launches++;
         }
         if (out->T) {
-            rc = run_gram(h, gram_params(h, B, L, c, w0, wc, GRAM_T), B.resampled);
+            rc = run_gram(h, gram_params(h, B, L, c, w0, wc, GRAM_T), P.resampled);
             if (rc) return rc;
             rc = emit_sym(h, c.S, L, wc, out->T + om);
             if (rc) return rc;
         }
         // pre-summed day blocks: S0 w0, v0, c and rhs are finished from the G w0 partials of the first Gram launch
         // that contracts the intraday phase (it must precede the solve and every emit of rhs / scalars)
-        bool post_pending = mode == BP_MODE_CONJUGATE && B.presum;
+        bool post_pending = mode == BP_MODE_CONJUGATE && P.presum;
         auto run_post = [&]() -> int {
             if (!post_pending) return BP_OK;
             post_pending = false;
@@ -1278,7 +811,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
             return BP_OK;
         };
         if ((out->S0 || (post_pending && !solve && !out->S1)) && mode == BP_MODE_CONJUGATE) {
-            rc = run_gram(h, gram_params(h, B, L, c, w0, wc, GRAM_S0), B.resampled);
+            rc = run_gram(h, gram_params(h, B, L, c, w0, wc, GRAM_S0), P.resampled);
             if (rc) return rc;
             if ((rc = run_post())) return rc;
             rc = emit_sym(h, c.S, L, wc, out->S0 ? out->S0 + om : nullptr);
@@ -1291,7 +824,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
                     gp.w_stride = G;
                     gp.n_windows = (wc + G - 1) / G;
                 }
-                rc = run_gram(h, gp, B.resampled);
+                rc = run_gram(h, gp, P.resampled);
                 if (rc) return rc;
                 if ((rc = run_post())) return rc;
             }
@@ -1300,13 +833,13 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
                 ShrinkParams q{};
                 q.n_windows = wc;
                 q.n_assets = N;
-                q.n_window = B.n;
+                q.n_window = P.n;
                 q.ld = h->ld;
                 q.ldv = L.ldv;
                 q.ldS = L.ldS;
                 q.win_stride = L.win_stride;
-                q.lr_daily = B.resampled ? h->lr_w : h->lr_d;
-                q.rf_row = B.resampled ? h->rf_w : h->rf_row;
+                q.lr_daily = P.resampled ? h->lr_w : h->lr_d;
+                q.rf_row = P.resampled ? h->rf_w : h->rf_row;
                 q.day_row = B.day_row + w0;
                 q.extra_row = B.extra_row ? B.extra_row + w0 : nullptr;
                 q.span_days = B.span + w0;
@@ -1328,7 +861,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
             cp.n_windows = wc;
             cp.group = G;
             cp.n_assets = N;
-            cp.n_window = B.n;
+            cp.n_window = P.n;
             cp.estimator = estimator;
             cp.ld = h->ld;
             cp.ldv = L.ldv;
@@ -1367,7 +900,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
         if ((rc = emit_raw(h, c.scal, sizeof(double) * (size_t)wc * BP_NSCAL,
                            out->scalars ? out->scalars + (size_t)w0 * BP_NSCAL : nullptr))) return rc;
         // the workspace is reused by the next chunk: host-bound copies must have drained
-        if (w0 + wc < B.W && h->need_sync) {
+        if (w0 + wc < P.W && h->need_sync) {
             CU_TRY(cudaStreamSynchronize(h->stream));
             h->need_sync = false;
         }
@@ -1424,28 +957,28 @@ int bp_destroy(bp_handle* h) {
     cudaStreamSynchronize(h->copy_stream);
     free_market(h);
     free_pool(h);
-    cudaFree(h->pool_cols);
+    free_buf(h->pool_cols);
     cudaStreamDestroy(h->copy_stream);
     cudaEventDestroy(h->ev_main);
     cudaEventDestroy(h->ev_hf);
     for (cudaEvent_t e : h->ev_seg)
         if (e) cudaEventDestroy(e);
     for (int k = 0; k < 2; ++k) {
-        cudaFree(h->desc_slot[k]);
-        cudaFreeHost(h->desc_host_slot[k]);
+        free_buf(h->desc_slot[k]);
+        free_buf(h->desc_host_slot[k]);
         if (h->ev_desc[k]) cudaEventDestroy(h->ev_desc[k]);
     }
     for (int a = 0; a < 2; ++a)
-        for (int l = 0; l < 2; ++l) cudaFree(h->store[a][l]);
-    cudaFree(h->rstore[0]);
-    cudaFree(h->rstore[1]);
-    cudaFree(h->fstore);
-    cudaFree(h->vstore);
-    cudaFree(h->prior_n);
-    cudaFree(h->band_aw);
-    cudaFree(h->band_stats);
-    cudaFree(h->ws);
-    cudaFree(h->stage);
+        for (int l = 0; l < 2; ++l) free_buf(h->store[a][l]);
+    free_buf(h->rstore[0]);
+    free_buf(h->rstore[1]);
+    free_buf(h->fstore);
+    free_buf(h->vstore);
+    free_buf(h->prior_n);
+    free_buf(h->band_aw);
+    free_buf(h->band_stats);
+    free_buf(h->ws);
+    free_buf(h->stage);
     for (cudaEvent_t e : h->ev_pool) cudaEventDestroy(e);
     if (h->ev_t0) cudaEventDestroy(h->ev_t0);
     delete h;
@@ -1766,9 +1299,9 @@ int bp_path_metrics(bp_handle* h, int n_paths, int n_obs, const double* returns,
     if (!(years > 0.0)) return fail(BP_ERR_INVALID, "years must be positive");
     CU_TRY(cudaSetDevice(h->device));
     const size_t n = (size_t)n_paths * n_obs;
-    int rc = ensure_stage(h, sizeof(double) * (2 * n + (size_t)n_paths * BP_PM_COUNT));
+    int rc = grow(h, h->stage, sizeof(double) * (2 * n + (size_t)n_paths * BP_PM_COUNT));
     if (rc) return rc;
-    double* d = reinterpret_cast<double*>(h->stage);
+    double* d = reinterpret_cast<double*>(h->stage.p);
     cudaStream_t st = h->stream;
     CU_TRY(cudaMemcpyAsync(d, returns, sizeof(double) * n, cudaMemcpyHostToDevice, st));
     CU_TRY(cudaMemcpyAsync(d + n, excess, sizeof(double) * n, cudaMemcpyHostToDevice, st));
@@ -1830,27 +1363,20 @@ int bp_select_market(bp_handle* h, const bp_pool_select* s) {
     if ((rc = begin_market(h, N, D, R, 0))) return rc;
     h->has_caps = h->pool_caps != nullptr;
     cudaStream_t st = h->stream;
-    if ((size_t)N > h->pool_cols_cap) {
-        CU_TRY(cudaStreamSynchronize(st));
-        cudaFree(h->pool_cols);
-        h->pool_cols = nullptr;
-        h->pool_cols_cap = 0;
-        CU_TRY(cudaMalloc(&h->pool_cols, sizeof(int) * (size_t)N));
-        h->pool_cols_cap = (size_t)N;
-    }
+    if ((rc = grow(h, h->pool_cols, (size_t)N))) return rc;
     // (pageable host memory: the copy is staged before the call returns, so the caller's array may go away; stream
     // order keeps earlier gathers, which read the previous column list, ahead of it)
-    CU_TRY(cudaMemcpyAsync(h->pool_cols, s->cols, sizeof(int) * (size_t)N, cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(h->pool_cols.p, s->cols, sizeof(int) * (size_t)N, cudaMemcpyHostToDevice, st));
     const long long pN = h->pool_N;
-    launch_gather_cols(h->pool_prices + (size_t)s->day_lo * pN, pN, h->prices, N, D, h->pool_cols, h->sm_count, st);
+    launch_gather_cols(h->pool_prices + (size_t)s->day_lo * pN, pN, h->prices, N, D, h->pool_cols.p, h->sm_count, st);
     h->launches++;
     if (h->pool_caps) {
-        launch_gather_cols(h->pool_caps + (size_t)s->day_lo * pN, pN, h->caps, N, D, h->pool_cols, h->sm_count, st);
+        launch_gather_cols(h->pool_caps + (size_t)s->day_lo * pN, pN, h->caps, N, D, h->pool_cols.p, h->sm_count, st);
         h->launches++;
     }
     CU_TRY(cudaMemcpyAsync(h->rf_row, h->pool_rf + s->day_lo, sizeof(double) * (size_t)D, cudaMemcpyDeviceToDevice, st));
     if (R > 0) {
-        launch_gather_cols(h->pool_hf + (size_t)s->hf_lo * pN, pN, h->hf_prices, N, R, h->pool_cols, h->sm_count, st);
+        launch_gather_cols(h->pool_hf + (size_t)s->hf_lo * pN, pN, h->hf_prices, N, R, h->pool_cols.p, h->sm_count, st);
         h->launches++;
         CU_TRY(cudaEventRecord(h->ev_hf, st));
         h->hf_pending = true;            // the first consumer computes the intraday log returns (wait_hf)
@@ -1970,9 +1496,9 @@ int bp_backtest_batched(bp_handle* h, const bp_backtest_desc* d) {
     const size_t b_w = al(sizeof(double) * (size_t)R * N), b_m = al((size_t)R * N), b_r = al(sizeof(int) * (size_t)R);
     const size_t b_ret = al(sizeof(double) * (size_t)std::max(T, 1)), b_to = al(sizeof(double) * (size_t)std::max(R - 1, 1));
     const size_t b_met = al(sizeof(double) * (size_t)R * 5);
-    int rc = ensure_ws(h, b_w + b_m + b_r + b_ret + b_to + b_met + 256);
+    int rc = grow(h, h->ws, b_w + b_m + b_r + b_ret + b_to + b_met + 256);
     if (rc) return rc;
-    unsigned char* base = h->ws;
+    unsigned char* base = h->ws.p;
     double* dw = reinterpret_cast<double*>(base);                    base += b_w;
     unsigned char* dm = base;                                          base += b_m;
     int* dr = reinterpret_cast<int*>(base);                           base += b_r;
@@ -2009,17 +1535,16 @@ int bp_backtest_batched(bp_handle* h, const bp_backtest_desc* d) {
 int bp_excess_returns(bp_handle* h, const bp_window_batch* b, double* X) {
     if (!h || !b || !X) return fail(BP_ERR_INVALID, "null argument");
     if (b->n_windows != 1) return fail(BP_ERR_INVALID, "bp_excess_returns handles one window per call");
-    Batch B;
-    CU_TRY(cudaSetDevice(h->device));
-    int rc = upload_batch(h, b, false, &B);
+    int rc = check_batch(plan_ctx(h, 1), b, false, &g_err);
     if (rc) return rc;
+    CU_TRY(cudaSetDevice(h->device));
     const int K = b->rolling_window - 1;
     const size_t bytes = sizeof(double) * (size_t)K * h->N;
     const bool dev = is_device_ptr(X);
     double* dst = X;
     if (!dev) {
-        if ((rc = ensure_stage(h, bytes))) return rc;
-        dst = reinterpret_cast<double*>(h->stage);
+        if ((rc = grow(h, h->stage, bytes))) return rc;
+        dst = reinterpret_cast<double*>(h->stage.p);
     }
     launch_excess_returns(h->lr_d, h->ld, h->rf_row, b->day_row[0], b->span_days[0], b->rolling_window, h->N, dst, h->stream);
     h->launches++;
@@ -2035,9 +1560,9 @@ int bp_quadratic_form(bp_handle* h, int n, const double* w, const double* S, dou
     if (!h || !w || !S || !out || n <= 0) return fail(BP_ERR_INVALID, "bad argument");
     CU_TRY(cudaSetDevice(h->device));
     const size_t need = sizeof(double) * ((size_t)n * n + n + 8);
-    int rc = ensure_stage(h, need);
+    int rc = grow(h, h->stage, need);
     if (rc) return rc;
-    double* dS = reinterpret_cast<double*>(h->stage);
+    double* dS = reinterpret_cast<double*>(h->stage.p);
     double* dw = dS + (size_t)n * n;
     double* dv = dw + n;
     CU_TRY(cudaMemcpyAsync(dS, S, sizeof(double) * (size_t)n * n, cudaMemcpyHostToDevice, h->stream));
@@ -2062,9 +1587,9 @@ int bp_dense_posterior(bp_handle* h, const bp_dense_problem* in, const bp_dense_
     const size_t NN = (size_t)N * N;
     auto al = [](size_t x) { return (x + 3) & ~(size_t)3; };      // keep every carve 32-byte aligned
     const size_t doubles = 3 * al(NN) + 4 * al(N) + 4 * al(ldv) + (size_t)rowsS * ldS + al(BP_NSCAL) + 8;
-    int rc = ensure_ws(h, sizeof(double) * doubles + 64);
+    int rc = grow(h, h->ws, sizeof(double) * doubles + 64);
     if (rc) return rc;
-    double* p = reinterpret_cast<double*>(h->ws);
+    double* p = reinterpret_cast<double*>(h->ws.p);
     double* dT = p;            p += al(NN);
     double* dS0 = p;           p += al(NN);
     double* dS1in = p;         p += al(NN);

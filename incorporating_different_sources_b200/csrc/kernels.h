@@ -218,8 +218,6 @@ cudaError_t launch_path_metrics(const PathMetricsParams& p, cudaStream_t st);
 void launch_gather_log_returns(const double* P, int ld_in, const int* num, const int* den, double* out, int ld_out,
                                int rows, int n_assets, cudaStream_t st);
 void launch_range_sum(const double* store, const int* ranges, int n_ranges, int npairs, double* out, cudaStream_t st);
-void launch_gather_strided_rows(double* M, int ld, long long src_row0, int stride, long long dst_row0, int k0, int k1,
-                                cudaStream_t st);
 void launch_combine_runs(const double* rs_coarse, const double* rs_fine, const int* triples, int n, int npairs,
                          double* out, cudaStream_t st);
 void launch_fetch_ints(const int* src_host, int* dst, long long n, cudaStream_t st);

@@ -506,23 +506,6 @@ void launch_range_sum(const double* store, const int* ranges, int n_ranges, int 
     range_sum_kernel<<<grid, 256, 0, st>>>(store, ranges, npairs, out);
 }
 
-// dst row (dst_row0 + k) = src row (src_row0 + k * stride), k in [k0, k1): the overnight returns of the trading
-// days, gathered behind the intraday matrix so that a window reads them as one contiguous run (PhasePlan::inner)
-__global__ void gather_strided_rows_kernel(double* __restrict__ M, int ld, long long src_row0, int stride,
-                                           long long dst_row0, int k0, int k1) {
-    const int k = k0 + blockIdx.x;
-    if (k >= k1) return;
-    const double2* src = reinterpret_cast<const double2*>(M + (src_row0 + (long long)k * stride) * ld);
-    double2* dst = reinterpret_cast<double2*>(M + (dst_row0 + k) * ld);
-    for (int c = threadIdx.x; c < ld / 2; c += blockDim.x) dst[c] = src[c];
-}
-
-void launch_gather_strided_rows(double* M, int ld, long long src_row0, int stride, long long dst_row0, int k0, int k1,
-                                cudaStream_t st) {
-    if (k1 <= k0) return;
-    gather_strided_rows_kernel<<<k1 - k0, 128, 0, st>>>(M, ld, src_row0, stride, dst_row0, k0, k1);
-}
-
 // dst[r][j] = src[r][cols[j]]: a column subset (any order) of a row-major matrix, dense output.  HBM bound; the reads
 // of a row are scattered over its 128-byte lines, the writes are coalesced.
 __global__ void gather_cols_kernel(const double* __restrict__ src, long long ld_src, double* __restrict__ dst, int n,
@@ -542,7 +525,8 @@ void launch_gather_cols(const double* src, long long ld_src, double* dst, int n,
     gather_cols_kernel<<<grid, n >= 256 ? 256 : 128, 0, st>>>(src, ld_src, dst, n, rows, cols);
 }
 
-// dst row (dst_row0 + k) = src row src_rows[k], k in [k0, k1): the overnight returns of arbitrary day blocks
+// dst row (dst_row0 + k) = src row src_rows[k], k in [k0, k1): the overnight returns of arbitrary day blocks, gathered
+// behind the intraday matrix so that a window reads them as one contiguous run (PhasePlan::inner)
 __global__ void gather_rows_indexed_kernel(double* __restrict__ M, int ld, const int* __restrict__ src_rows,
                                            long long dst_row0, int k0, int k1) {
     const int k = k0 + blockIdx.x;
