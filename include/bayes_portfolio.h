@@ -326,6 +326,24 @@ typedef struct {
 
 int bp_dense_posterior(bp_handle* h, const bp_dense_problem* in, const bp_dense_result* out);
 
+/* The solve stage alone on caller-supplied matrices, W windows at once: the batched form of the injected-moment calls
+ * calculate_conjugate_posterior_w / calculate_mean_conjugate_posterior_nu with conjugate_posterior_S_df= (:485-489,
+ * :572-575), calculate_mean_jeffreys_posterior_nu (:600-606) and Jorion from C and t (:851-895).  No market is needed.
+ * Outputs honoured: weights, nu, w1, scalars (v1 in BP_SCAL_V1, n1 in BP_SCAL_N1; Jorion: BP_SCAL_JORION_*) and
+ * status; asking for T, S0, S1, t, w0 or rhs is an error.  The solver accepts N <= 3072 (Jorion: N <= 1536). */
+typedef struct {
+    int n_windows, n_assets;    /* W, N                                                              */
+    int jeffreys;               /* 0: nu = (n1 + N + 2) w1 / (n1 - w1' S w1); 1: nu = w1             */
+    int estimator;              /* 0, or BP_ESTIMATOR_JORION: S = C, rhs = t, and a right-hand side of
+                                   ones rides along (jeffreys and n1 are then ignored)               */
+    int n_returns;              /* Jorion's m, must exceed N + 2                                     */
+    double risk_aversion;
+    const double* S;            /* [W][N][N] host; only the lower triangle is read                   */
+    const double* rhs;          /* [W][N] host                                                       */
+    const double* n1;           /* [W] host, conjugate scaling only                                  */
+} bp_solve_desc;
+int bp_solve_batched(bp_handle* h, const bp_solve_desc* d, const bp_outputs* out);
+
 #ifdef __cplusplus
 }
 #endif

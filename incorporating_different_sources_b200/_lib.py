@@ -29,6 +29,7 @@ EXPORTED = [
     "bp_upload_market_async", "bp_backtest_batched", "bp_get_gram_work", "bp_set_reuse_min_windows", "bp_set_upload_pipeline", "bp_set_async_outputs",
     "bp_set_resampled", "bp_estimator_batched", "bp_set_jeffreys_chain", "bp_get_solve_work",
     "bp_set_upload_fractions", "bp_solve_wave_windows", "bp_set_hf_presum_min_days", "bp_wait_upload", "bp_upload_pool", "bp_select_market", "bp_path_metrics",
+    "bp_solve_batched",
 ]
 BP_NSTAGE = 8
 STAGES = ("logret", "prep", "gram", "solve", "chain")
@@ -75,6 +76,14 @@ class DenseProblem(C.Structure):
 
 class DenseResult(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("scalars", "S1", "w1", "nu", "weights", "status")]
+
+
+class SolveDesc(C.Structure):
+    _fields_ = [
+        ("n_windows", C.c_int), ("n_assets", C.c_int), ("jeffreys", C.c_int), ("estimator", C.c_int),
+        ("n_returns", C.c_int), ("risk_aversion", C.c_double), ("S", C.c_void_p), ("rhs", C.c_void_p),
+        ("n1", C.c_void_p),
+    ]
 
 
 class BacktestDesc(C.Structure):
@@ -147,6 +156,7 @@ def load():
     lib.bp_excess_returns.argtypes = [C.c_void_p, C.POINTER(WindowBatchDesc), C.c_void_p]
     lib.bp_quadratic_form.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.bp_dense_posterior.argtypes = [C.c_void_p, C.POINTER(DenseProblem), C.POINTER(DenseResult)]
+    lib.bp_solve_batched.argtypes = [C.c_void_p, C.POINTER(SolveDesc), C.POINTER(Outputs)]
     for name in EXPORTED:
         getattr(lib, name)          # every declared entry point must be exported
     _lib = lib

@@ -57,6 +57,10 @@ __global__ void __launch_bounds__(128) rf_weights_kernel(PrepParams p, int K) {
             scal[BP_S_V0] = 0.0;
             scal[BP_S_M] = 0.0;
             scal[BP_S_SUMA] = sa;
+            // first writer of the record in the never-cleared workspace (see window_prep_kernel): no stale slot
+            scal[BP_S_MCM_AVG] = 0.0;
+            scal[BP_S_V1] = 0.0;
+            for (int k = BP_S_MCM_AVG + 1; k < BP_S_COUNT; ++k) scal[k] = 0.0;
         }
     }
 }

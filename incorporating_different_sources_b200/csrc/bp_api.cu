@@ -595,10 +595,59 @@ int finish(bp_handle* h) {
     return BP_OK;
 }
 
+// The solver's size limit, checked before anything is uploaded or launched
+int check_solver_size(int N, int estimator) {
+    const int nrhs = estimator == BP_EST_JORION ? 2 : 1;
+    const int max_n = chol_max_assets(nrhs);
+    if (N > max_n)
+        return fail(BP_ERR_INVALID, "the Cholesky solver supports at most %d assets with %d right-hand side%s; got %d", max_n,
+                    nrhs, nrhs > 1 ? "s" : "", N);
+    return BP_OK;
+}
+
+// Cholesky + solves of wn windows of the workspace, starting at c: CTA job q factorises window q * stride.  Shared by
+// run_batches, bp_dense_posterior and bp_solve_batched.  c.scal must hold n1 for conjugate windows.
+int solve_windows(bp_handle* h, const Chunk& c, const Layout& L, int wn, int stride, int mode, int estimator, int n_returns,
+                  double inv_gamma) {
+    if (wn <= 0) return BP_OK;
+    SolveParams sp{};
+    sp.n_windows = wn;
+    sp.w_stride = stride;
+    sp.n_assets = L.N;
+    sp.ldS = L.ldS;
+    sp.win_stride = L.win_stride;
+    sp.ldv = L.ldv;
+    sp.mode = mode;
+    sp.estimator = estimator;
+    sp.n_returns = n_returns;
+    sp.inv_gamma = inv_gamma;
+    sp.S = c.S;
+    sp.rhs = c.rhs;
+    sp.scal = c.scal;
+    sp.w1 = c.w1;
+    sp.nu = c.nu;
+    sp.weights = c.weights;
+    sp.status = c.status;
+    CUtensorMap smap;
+    int rc = make_solve_map(h, &smap, c.S, ((long long)(wn - 1) * stride + 1) * L.rowsS, L.ldS);
+    if (rc) return rc;
+    {
+        StageTimer tm(h, BP_STAGE_SOLVE);
+        CU_TRY(launch_chol_solve(sp, smap, h->sm_count, h->stream));
+    }
+    h->launches++;
+    h->work_factored += wn;
+    return BP_OK;
+}
+
 // shared driver of bp_conjugate_batched / bp_jeffreys_batched / bp_stats_batched / bp_hf_cov_batched
 int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, int mode, bool solve, int estimator = BP_EST_NONE) {
     Batch B;
     if (!h || !b) return fail(BP_ERR_INVALID, "null handle or batch");
+    if (solve && h->has_market) {
+        const int rcl = check_solver_size(h->N, estimator);
+        if (rcl) return rcl;
+    }
     // every allocation / launch below (upload_batch included) must land on the handle's device, whatever the
     // calling thread's current device is (two handles on two GPUs in one thread, or torch having switched)
     CU_TRY(cudaSetDevice(h->device));
@@ -667,38 +716,9 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
         }
         if ((out->T || out->S1 || solve) && (rc = run_block_precompute(h, B, 1))) return rc;
     }
-    // Cholesky + solves of the windows [ws, ws+wn) of the workspace
+    // Cholesky + solves of the windows [ws, ws+wn) of the workspace; the reference evaluates (1/gamma) * nu (:836,:849)
     auto solve_range = [&](int ws, int wn, int stride = 1) -> int {
-        if (wn <= 0) return BP_OK;
-        const Chunk cs = chunk_at(c, L, ws % Wc);
-        SolveParams sp{};
-        sp.n_windows = wn;
-        sp.w_stride = stride;
-        sp.n_assets = N;
-        sp.ldS = L.ldS;
-        sp.win_stride = L.win_stride;
-        sp.ldv = L.ldv;
-        sp.mode = mode;
-        sp.estimator = estimator;
-        sp.n_returns = P.n - 1;
-        sp.inv_gamma = 1.0 / b->risk_aversion;         // the reference evaluates (1/gamma) * nu (:836,:849)
-        sp.S = cs.S;
-        sp.rhs = cs.rhs;
-        sp.scal = cs.scal;
-        sp.w1 = cs.w1;
-        sp.nu = cs.nu;
-        sp.weights = cs.weights;
-        sp.status = cs.status;
-        CUtensorMap smap;
-        int rcs = make_solve_map(h, &smap, cs.S, ((long long)(wn - 1) * stride + 1) * L.rowsS, L.ldS);
-        if (rcs) return rcs;
-        {
-            StageTimer tm(h, BP_STAGE_SOLVE);
-            CU_TRY(launch_chol_solve(sp, smap, h->sm_count, h->stream));
-        }
-        h->launches++;
-        h->work_factored += wn;
-        return BP_OK;
+        return solve_windows(h, chunk_at(c, L, ws % Wc), L, wn, stride, mode, estimator, P.n - 1, 1.0 / b->risk_aversion);
     };
     int w_solved = 0;          // windows already solved by the pipelined path (full waves, between the upload segments)
     if (pipelined) {
@@ -1582,12 +1602,15 @@ int bp_dense_posterior(bp_handle* h, const bp_dense_problem* in, const bp_dense_
     if (N <= 0 || (!c_only && (!in->T || !in->t))) return fail(BP_ERR_INVALID, "T and t are required");
     if (!in->jeffreys && (!in->S0 || !in->w0)) return fail(BP_ERR_INVALID, "conjugate posterior needs S0 and w0");
     if (!(in->risk_aversion != 0.0)) return fail(BP_ERR_INVALID, "risk_aversion must be non-zero");
+    const bool solves = !c_only && (in->jeffreys || !in->w1);      // an injected posterior w skips the solver
+    int rc = BP_OK;
+    if (solves && (rc = check_solver_size(N, BP_EST_NONE))) return rc;
     CU_TRY(cudaSetDevice(h->device));
     const int ldS = round_up(N, 32), rowsS = ldS + 8, ldv = round_up(N, 16);
     const size_t NN = (size_t)N * N;
     auto al = [](size_t x) { return (x + 3) & ~(size_t)3; };      // keep every carve 32-byte aligned
     const size_t doubles = 3 * al(NN) + 4 * al(N) + 4 * al(ldv) + (size_t)rowsS * ldS + al(BP_NSCAL) + 8;
-    int rc = grow(h, h->ws, sizeof(double) * doubles + 64);
+    rc = grow(h, h->ws, sizeof(double) * doubles + 64);
     if (rc) return rc;
     double* p = reinterpret_cast<double*>(h->ws.p);
     double* dT = p;            p += al(NN);
@@ -1643,15 +1666,11 @@ int bp_dense_posterior(bp_handle* h, const bp_dense_problem* in, const bp_dense_
         h->launches++;
         CU_TRY(cudaMemcpyAsync(dw1, dw1in, sizeof(double) * N, cudaMemcpyDeviceToDevice, st));
     } else {
-        SolveParams sp{};
-        sp.n_windows = 1; sp.n_assets = N; sp.ldS = ldS; sp.win_stride = (long long)rowsS * ldS; sp.ldv = ldv;
-        sp.mode = in->jeffreys ? BP_MODE_JEFFREYS : BP_MODE_CONJUGATE;
-        sp.inv_gamma = inv_gamma;
-        sp.S = dS; sp.rhs = drhs; sp.scal = dscal; sp.w1 = dw1; sp.nu = dnu; sp.weights = dwts; sp.status = dstatus;
-        CUtensorMap smap;
-        if ((rc = make_solve_map(h, &smap, dS, rowsS, ldS))) return rc;
-        CU_TRY(launch_chol_solve(sp, smap, h->sm_count, st));
-        h->launches++;
+        const Layout L{N, ldv, ldS, rowsS, (long long)rowsS * ldS, 2, 0};
+        Chunk c{};
+        c.S = dS; c.rhs = drhs; c.scal = dscal; c.w1 = dw1; c.nu = dnu; c.weights = dwts; c.status = dstatus;
+        if ((rc = solve_windows(h, c, L, 1, 1, in->jeffreys ? BP_MODE_JEFFREYS : BP_MODE_CONJUGATE, BP_EST_NONE, 0, inv_gamma)))
+            return rc;
     }
     CU_TRY(cudaGetLastError());
     if (out->scalars) CU_TRY(cudaMemcpyAsync(out->scalars, dscal, sizeof(double) * BP_NSCAL, cudaMemcpyDeviceToHost, st));
@@ -1661,6 +1680,67 @@ int bp_dense_posterior(bp_handle* h, const bp_dense_problem* in, const bp_dense_
     if (out->status) CU_TRY(cudaMemcpyAsync(out->status, dstatus, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     return BP_OK;
+}
+
+int bp_solve_batched(bp_handle* h, const bp_solve_desc* d, const bp_outputs* out) {
+    if (!h || !d || !out) return fail(BP_ERR_INVALID, "null argument");
+    const int W = d->n_windows, N = d->n_assets;
+    if (W <= 0 || N <= 0) return fail(BP_ERR_INVALID, "need n_windows > 0 and n_assets > 0");
+    if (!d->S || !d->rhs) return fail(BP_ERR_INVALID, "S and rhs are required");
+    if (d->estimator != BP_EST_NONE && d->estimator != BP_EST_JORION)
+        return fail(BP_ERR_INVALID, "estimator must be 0 or BP_ESTIMATOR_JORION");
+    const bool jorion = d->estimator == BP_EST_JORION;
+    const int mode = (d->jeffreys || jorion) ? BP_MODE_JEFFREYS : BP_MODE_CONJUGATE;
+    if (mode == BP_MODE_CONJUGATE && !d->n1) return fail(BP_ERR_INVALID, "the conjugate scaling needs n1");
+    if (jorion && d->n_returns - N - 2 <= 0) return fail(BP_ERR_INVALID, "Jorion needs n_returns - N - 2 > 0 (:879)");
+    if (!(d->risk_aversion != 0.0)) return fail(BP_ERR_INVALID, "risk_aversion must be non-zero");
+    if (out->T || out->S0 || out->S1 || out->t || out->w0 || out->rhs)
+        return fail(BP_ERR_INVALID, "bp_solve_batched returns w1, nu, weights, scalars and status only");
+    int rc = check_solver_size(N, d->estimator);
+    if (rc) return rc;
+    CU_TRY(cudaSetDevice(h->device));
+    // the layout of bp_dense_posterior for W windows
+    Layout L{};
+    L.N = N;
+    L.ldv = round_up(N, 16);
+    L.ldS = round_up(N, 32);
+    L.rowsS = L.ldS + 8;
+    L.win_stride = (long long)L.rowsS * L.ldS;
+    L.y_stride = 2;
+    L.mv_stride = 0;
+    L.per_window = sizeof(double) * ((size_t)L.win_stride + 9 * (size_t)L.ldv + BP_NSCAL + (size_t)L.y_stride) + 16;
+    const int Wc = (int)std::min<size_t>((size_t)W, std::max<size_t>(1, h->ws_limit / L.per_window));
+    if ((rc = grow(h, h->ws, (size_t)Wc * L.per_window + 256))) return rc;
+    const Chunk c = carve(h->ws.p, L, Wc);
+    cudaStream_t st = h->stream;
+    for (int w0 = 0; w0 < W; w0 += Wc) {
+        const int wc = std::min(Wc, W - w0);
+        const size_t NN = (size_t)N * N;
+        // only the N x N entries of each window: the padding rows and columns keep whatever the workspace held
+        for (int k = 0; k < wc; ++k)
+            CU_TRY(cudaMemcpy2DAsync(c.S + (size_t)k * L.win_stride, sizeof(double) * L.ldS, d->S + (size_t)(w0 + k) * NN,
+                                     sizeof(double) * N, sizeof(double) * N, N, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpy2DAsync(c.rhs, sizeof(double) * L.ldv, d->rhs + (size_t)w0 * N, sizeof(double) * N,
+                                 sizeof(double) * N, wc, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemsetAsync(c.scal, 0, sizeof(double) * BP_NSCAL * (size_t)wc, st));
+        if (mode == BP_MODE_CONJUGATE)
+            CU_TRY(cudaMemcpy2DAsync(c.scal + BP_SCAL_N1, sizeof(double) * BP_NSCAL, d->n1 + w0, sizeof(double), sizeof(double),
+                                     wc, cudaMemcpyHostToDevice, st));
+        if ((rc = solve_windows(h, c, L, wc, 1, mode, d->estimator, d->n_returns, 1.0 / d->risk_aversion))) return rc;
+        const size_t ov = (size_t)w0 * N;
+        if ((rc = emit_vec(h, c.weights, L, wc, out->weights ? out->weights + ov : nullptr))) return rc;
+        if ((rc = emit_vec(h, c.nu, L, wc, out->nu ? out->nu + ov : nullptr))) return rc;
+        if ((rc = emit_vec(h, c.w1, L, wc, out->w1 ? out->w1 + ov : nullptr))) return rc;
+        if ((rc = emit_raw(h, c.status, sizeof(int) * (size_t)wc, out->status ? out->status + w0 : nullptr))) return rc;
+        if ((rc = emit_raw(h, c.scal, sizeof(double) * (size_t)wc * BP_NSCAL,
+                           out->scalars ? out->scalars + (size_t)w0 * BP_NSCAL : nullptr))) return rc;
+        // the workspace is reused by the next chunk: host-bound copies must have drained
+        if (w0 + wc < W && h->need_sync) {
+            CU_TRY(cudaStreamSynchronize(st));
+            h->need_sync = false;
+        }
+    }
+    return finish(h);
 }
 
 }  // extern "C"

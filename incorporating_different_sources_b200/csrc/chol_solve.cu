@@ -533,6 +533,10 @@ size_t chol_smem_bytes(int n_assets, int nrhs) {
     return (size_t)CH_TMA_SMEM + sizeof(double) * (size_t)(NB * LDQ + 40);
 }
 
+int chol_max_assets(int nrhs) {
+    return (int)((size_t)CH_STAGES * CH_STAGE_BYTES / (sizeof(double) * (size_t)nrhs)) / NB * NB;
+}
+
 cudaError_t launch_chol_solve(const SolveParams& p, const CUtensorMap& smap, int sm_count, cudaStream_t st) {
     if (p.n_windows <= 0) return cudaSuccess;
     static const bool profile = getenv("BP_CHOL_PROFILE") != nullptr;

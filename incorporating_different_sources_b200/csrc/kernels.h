@@ -281,6 +281,12 @@ int chain_max_group();
 cudaError_t launch_jeffreys_chain(const ChainParams& p, cudaStream_t st);
 cudaError_t launch_chol_solve(const SolveParams& p, const CUtensorMap& smap, int sm_count, cudaStream_t st);
 int chol_wave_windows(int sm_count);
+// dynamic shared memory of chol_solve_kernel for N assets and nrhs right-hand sides; 0 if N is too large for the
+// back-substitution vectors, which alias the TMA stage ring
+size_t chol_smem_bytes(int n_assets, int nrhs);
+// largest N the solver accepts with nrhs right-hand sides (3072 for one, 1536 for Jorion's two): the callers check it
+// before any upload or launch
+int chol_max_assets(int nrhs);
 // chol_cluster.cu: one thread-block cluster of K CTAs per window for launches of fewer than cta_slots / 2 windows (K =
 // 8, 4 or 2, the largest with n_windows * K <= cta_slots); cudaErrorNotSupported otherwise (and when N is too large for
 // the aliased back-substitution vectors, or with BP_CHOL_CLUSTER=0): the caller then runs chol_solve_kernel

@@ -165,6 +165,13 @@ __device__ __forceinline__ double2 reduce_cols(const double2 (&part)[NCH], doubl
     return s;
 }
 
+// The prep kernel is the first writer of a window's scalar record, which lives in the shared, never-cleared workspace:
+// it zeroes v1 (written by the solver, if one follows) and the unused slots, so that no call returns stale values
+__device__ __forceinline__ void clear_later_slots(double* scal) {
+    scal[BP_S_V1] = 0.0;
+    for (int k = BP_S_MCM_AVG + 1; k < BP_S_COUNT; ++k) scal[k] = 0.0;
+}
+
 __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams p) {
     extern __shared__ double smem[];
     const int K = p.n_window - 1;                 // daily returns per window (F2)
@@ -239,6 +246,8 @@ __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams
             scal[BP_S_V0] = 0.0;
             scal[BP_S_M] = 0.0;
             scal[BP_S_SUMA] = sa;
+            scal[BP_S_MCM_AVG] = 0.0;
+            clear_later_slots(scal);
         }
         return;
     }
@@ -306,6 +315,7 @@ __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams
             scal[BP_S_M] = (double)m;
             scal[BP_S_SUMA] = sa;
             scal[BP_S_MCM_AVG] = avg;
+            clear_later_slots(scal);
         }
         return;
     }
@@ -390,6 +400,7 @@ __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams
         scal[BP_S_M] = (double)m;
         scal[BP_S_SUMA] = sa;
         scal[BP_S_MCM_AVG] = avg;
+        clear_later_slots(scal);
     }
 }
 

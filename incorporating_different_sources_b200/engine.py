@@ -372,8 +372,9 @@ class BayesEngine:
             d.prior_n = pn.ctypes.data
         return d, keep
 
-    def _alloc_outputs(self, W: int, names: Iterable[str], device_out: bool, into: Optional[dict]):
-        N = self.n_assets
+    def _alloc_outputs(self, W: int, names: Iterable[str], device_out: bool, into: Optional[dict],
+                       n_assets: Optional[int] = None):
+        N = self.n_assets if n_assets is None else n_assets
         o = Outputs()
         res = {}
         for f, _ in Outputs._fields_:
@@ -593,6 +594,39 @@ class BayesEngine:
         for k, v in res.items():
             setattr(out, k, v.ctypes.data)
         rc = self._lib.bp_dense_posterior(self._h, C.byref(pr), C.byref(out))
+        del keep
+        if rc:
+            _raise(rc)
+        return res
+
+    def solve(self, S, rhs, *, jeffreys: bool = True, n1=None, jorion: bool = False, n_returns: int = 0,
+              risk_aversion: float = 1.0, outputs: Sequence[str] = ("weights", "nu", "w1", "scalars", "status"),
+              ) -> Dict[str, np.ndarray]:
+        """The solve stage alone on caller-supplied matrices ``S`` [W][N][N] (lower triangle read) and ``rhs`` [W][N]:
+        ``w1 = S^-1 rhs``, ``v1 = w1'S w1`` and the epilogue of the conjugate (``n1`` [W], :485-489, :572-575), Jeffreys
+        (:600-606) or, with ``jorion=True``, Jorion (``S`` = C, ``rhs`` = t, ``n_returns`` = m, :851-895) path."""
+        S = _c64(S)
+        rhs = _c64(rhs)
+        if S.ndim != 3 or S.shape[1] != S.shape[2]:
+            raise ValueError("S must be [W][N][N]")
+        W, N = S.shape[0], S.shape[1]
+        if rhs.shape != (W, N):
+            raise ValueError(f"rhs has shape {rhs.shape}, expected {(W, N)}")
+        d = _lib.SolveDesc()
+        d.n_windows, d.n_assets = W, N
+        d.jeffreys, d.estimator = int(bool(jeffreys)), _lib.EST_JORION if jorion else 0
+        d.n_returns, d.risk_aversion = int(n_returns), float(risk_aversion)
+        d.S, d.rhs = S.ctypes.data, rhs.ctypes.data
+        keep = [S, rhs]
+        d.n1 = None
+        if n1 is not None:
+            n1 = _c64(n1)
+            if n1.shape != (W,):
+                raise ValueError("n1 must have one entry per window")
+            keep.append(n1)
+            d.n1 = n1.ctypes.data
+        o, res = self._alloc_outputs(W, outputs, False, None, n_assets=N)
+        rc = self._lib.bp_solve_batched(self._h, C.byref(d), C.byref(o))
         del keep
         if rc:
             _raise(rc)
