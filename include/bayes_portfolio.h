@@ -36,11 +36,11 @@ extern "C" {
 /* indices into the per-window scalar record */
 #define BP_SCAL_N0 0          /* conjugate prior n0            portfolio_calculations.py:247-267     */
 #define BP_SCAL_N1 1          /* posterior n1 = n0 + n         :269-282                              */
-#define BP_SCAL_ALPHA 2       /* n0 * m/(m-1)                  :317-318,:333                         */
+#define BP_SCAL_ALPHA 2       /* n0 * m/(m-1); NaN when m < 2  :317-318,:333                         */
 #define BP_SCAL_BETA 3        /* rank-1 coefficient used by the Gram epilogue                       */
 #define BP_SCAL_C 4           /* conjugate c                   :382-430                              */
 #define BP_SCAL_V0 5          /* w0' S0 w0                     :64-88                                */
-#define BP_SCAL_M 6           /* number of HF returns m        :314                                  */
+#define BP_SCAL_M 6           /* HF returns m kept by dropna   :314 (of the hf_hi - hf_lo - 1 spanned) */
 #define BP_SCAL_SUMA 7        /* sum of risk-free adjustments  :48                                   */
 #define BP_SCAL_V1 8          /* w1' S1 w1                     :574                                  */
 #define BP_SCAL_MCM_AVG 9     /* average MCM over the window   :112                                  */
@@ -64,6 +64,12 @@ typedef struct {
     const double* prices;       /* [D][N] daily close           -> k_stock_prices_df                 */
     const double* caps;         /* [D][N] market caps           -> k_stock_market_caps_df (may be NULL) */
     const double* hf_prices;    /* [R][N] intraday prices       -> k_stock_intraday_prices_df        */
+                                /* May hold NaN (missing bars).  As the reference's dropna (:314), intraday
+                                   return row r (log of price row r over row r-1) is dropped when any of its
+                                   N returns is NaN: a NaN bar in row r-1 or r of ANY column drops it.  The
+                                   decision does not depend on the window; a window uses the kept rows among
+                                   its own, m of them (BP_SCAL_M), and a window with m < 2 gets NaN S0, S1
+                                   and weights and a non-zero status, as the reference's all-NaN cov does. */
     const double* mcm;          /* [n_mcm][D] VIX / EPU ...     -> mcm_prices_df (may be NULL)       */
     int n_mcm;
     const double* rf_row;       /* [D] annualised risk-free rate forward-filled onto the daily rows

@@ -17,6 +17,7 @@ from typing import Callable, Dict, List, Optional
 import numpy as np
 import pandas as pd
 
+from ._lib import SCAL
 from .windows import HF_LOOKBACK_DAYS, ffill_rows, mcm_prior_n, plan_daily_windows, plan_weekly_windows
 
 # ``data_handling.extract_unique_tickers(d, d)`` of the reference reads the S&P-500 constituents of a date
@@ -66,8 +67,9 @@ def select_universes(stock_market_caps_df, stock_prices_df, stock_intraday_price
     date — membership AND order identical to the per-date function (tests/test_host_vs_reference.py).
 
     Also returns ``nan_bars`` [T][C] (bool, in candidate order) = the stock has a NaN bar inside the date's intraday
-    LOOK-BACK of ``lookback_days`` calendar days (default: the eligibility range's own length), and the candidate list:
-    the reference would drop such bars (``dropna``, :314); the batched path raises."""
+    LOOK-BACK of ``lookback_days`` calendar days (default: the eligibility range's own length), and the candidate list.
+    Such bars do not exclude a stock: the conjugate windows drop the returns next to them, as the reference's
+    ``dropna`` does (:314)."""
     if rolling_window_frequency not in HF_LOOKBACK_DAYS:
         raise RuntimeError("Unknown rolling window frequency.")                                   # :637
     days = HF_LOOKBACK_DAYS[rolling_window_frequency]
@@ -295,7 +297,13 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
                 batch = plan_daily_windows(portfolio_spec, dates_ns, d_idx, hf_ts, hf_lookback_days=hf_lookback_days,
                                            row_offset=day_lo, hf_row_offset=hf_lo)
             batch.prior_n = np.ascontiguousarray(prior_n_all[rows])
-            res = engine.conjugate(batch, outputs=("weights", "status"))
+            res = engine.conjugate(batch, outputs=("weights", "scalars", "status"))
+            few = np.nonzero(res["scalars"][:, SCAL["m"]] < 2)[0]
+            if len(few):
+                # fewer than 2 intraday returns left after dropna: the reference's S0 is all NaN (:317) and so is w1
+                raise ValueError(f"conjugate_posterior_w_df contains NaN values.  ({dates_all[d_idx[few[0]]].date()}: "
+                                 f"{int(res['scalars'][few[0], SCAL['m']])} intraday returns left after dropping the "
+                                 f"missing bars)")                                            # :492-494
             _raise_on_status(res["status"], dates_all, d_idx)
             w = res["weights"]
         elif strat in ("jeffreys", "jorion", "shrinkage"):
@@ -343,20 +351,12 @@ def backtest_portfolio(portfolio_spec, ts_start_date, ts_end_date, market_data, 
     flags = rebalance_flags(bt_dates, portfolio_spec["rebalancing_frequency"])
     reb_pos = in_range[flags]
     t1 = time.perf_counter()
-    universes, nan_bars, cand = select_universes(market_data["stock_market_caps_df"], prices_df,
+    universes, _, _ = select_universes(market_data["stock_market_caps_df"], prices_df,
                                                  market_data["stock_intraday_prices_df"], dates_all[reb_pos],
                                                  portfolio_spec["size"], get_window_trading_days(portfolio_spec),
                                                  portfolio_spec["rebalancing_frequency"],      # sic (:960)
                                                  lookback_days=hf_lookback_days if hf_lookback_days is not None else
                                                  HF_LOOKBACK_DAYS.get(portfolio_spec["rolling_window_frequency"]))
-    if nan_bars is not None and portfolio_spec["weighting_strategy"].startswith("conjugate"):
-        pos_of = {s: j for j, s in enumerate(cand)}
-        for r, names in enumerate(universes):
-            hit = [s for s in names if nan_bars[r, pos_of[s]]]
-            if hit:
-                raise ValueError(f"NaN intraday bar inside the look-back of {hit[0]} at {dates_all[reb_pos[r]].date()}: the "
-                                 f"reference drops such bars (dropna, :314); the batched CUDA path does not -- clean the "
-                                 f"intraday frame or exclude the stock")
     t2 = time.perf_counter()
     W, member = _batched_weights(eng, portfolio_spec, market_data, dates_all, list(reb_pos), universes, hf_lookback_days)
     t3 = time.perf_counter()

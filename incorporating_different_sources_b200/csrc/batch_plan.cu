@@ -368,7 +368,7 @@ void write_batch(const BatchPlan& P, const bp_window_batch* b, int* dst) {
         dst[(size_t)2 * W + w] = P.resampled ? dr - (n - 2) + 1 : dr - n + 2;   // first RETURN row (F2: n prices -> n-1 returns)
         if (P.need_hf) {
             dst[(size_t)3 * W + w] = b->hf_lo[w] + 1;       // first HF return row: the window's first bar has no return (F5)
-            dst[(size_t)4 * W + w] = b->hf_hi[w] - b->hf_lo[w] - 1;
+            dst[(size_t)4 * W + w] = b->hf_hi[w] - b->hf_lo[w] - 1;   // span; the prep kernel counts the kept rows m in it
         }
         dst[(size_t)5 * W + w] = P.resampled ? b->extra_row[w] : -1;
         dst[(size_t)6 * W + w] = P.resampled ? b->caps_row[w] : dr;

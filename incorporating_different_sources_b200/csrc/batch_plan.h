@@ -58,7 +58,7 @@ struct BatchPlan {
     std::map<std::pair<long long, long long>, int> range_id[2];
     std::map<RunKey, int> full_id;
     int nranges[2] = {0, 0}, nfull = 0;
-    // descriptor image, offsets in ints: 7 columns [W] (day_row, span, row0, hf_row0, hf_m, extra_row, caps_row),
+    // descriptor image, offsets in ints: 7 columns [W] (day_row, span, row0, hf_row0, hf_span, extra_row, caps_row),
     // Gram jobs [W][GRAM_DESC_INTS], block jobs [phase][level][nb][GRAM_DESC_INTS], ranges [level][n][2],
     // triples [nfull][3], day-block starts [nb + 1] (inner), scanned-vector ids [W][3] (presum)
     size_t off_gram = 0, off_blocks[2][2] = {{0, 0}, {0, 0}}, off_ranges[2] = {0, 0}, off_triples = 0,

@@ -99,6 +99,7 @@ struct bp_handle {
     int n_frac = 0;                            // > 0: explicit cumulative row fractions of the segments (bp_set_upload_fractions)
     double frac[MAX_SEG] = {0};
     long long lr_hf_done = 0;                  // intraday return rows < lr_hf_done have been computed
+    DevBuf<unsigned char> hf_keep;             // [R] 1 = intraday return row kept, 0 = dropped (hf_returns)
     long long hf_extra_rows = 0;               // rows allocated behind lr_hf for gathered overnight returns
     int lr_hf_ld_cap = 1;
     long long lr_hf_rows_cap = 0;              // rows allocated for lr_hf (at the leading dimension it was allocated with)
@@ -195,15 +196,23 @@ void free_market(bp_handle* h) {
     h->has_market = false;
 }
 
+// Intraday return rows [row_begin, row_end) and their keep flags: every intraday log return goes through here, so that
+// lr_hf and hf_keep always describe the same rows.  Price rows arrive in row order, so row row_begin - 1, which the first
+// return row reads, is already resident.
+int hf_returns(bp_handle* h, long long row_begin, long long row_end) {
+    launch_hf_log_returns(h->hf_prices, h->N, h->lr_hf, h->ld, h->hf_keep.p, row_begin, row_end, h->N, h->sm_count, h->stream);
+    h->launches++;
+    CU_TRY(cudaGetLastError());
+    return BP_OK;
+}
+
 // Conjugate stages read lr_hf.  The intraday prices arrive on the copy stream; their log returns are computed
 // on the COMPUTE stream once the copy event has fired (a kernel on the copy stream would have to wait for
 // free SMs behind the persistent Gram / solve kernels, and the next segment's copy would queue behind it).
 int wait_hf(bp_handle* h) {
     if (h->hf_pending) {
         CU_TRY(cudaStreamWaitEvent(h->stream, h->ev_hf, 0));
-        launch_log_returns(h->hf_prices, h->N, h->lr_hf, h->ld, h->R, h->N, h->sm_count, h->stream, h->lr_hf_done);
-        h->launches++;
-        CU_TRY(cudaGetLastError());
+        if (int rc = hf_returns(h, h->lr_hf_done, h->R)) return rc;
         h->lr_hf_done = h->R;
         h->hf_pending = false;
         h->seg_waited = h->n_seg;
@@ -221,9 +230,7 @@ int wait_hf_rows(bp_handle* h, long long rows_needed) {
     while (h->seg_waited < h->n_seg && h->lr_hf_done < rows_needed) {
         const int s = h->seg_waited;
         CU_TRY(cudaStreamWaitEvent(h->stream, h->ev_seg[s], 0));
-        launch_log_returns(h->hf_prices, h->N, h->lr_hf, h->ld, h->seg_end[s], h->N, h->sm_count, h->stream, h->lr_hf_done);
-        h->launches++;
-        CU_TRY(cudaGetLastError());
+        if (int rc = hf_returns(h, h->lr_hf_done, h->seg_end[s])) return rc;
         h->lr_hf_done = h->seg_end[s];
         h->seg_waited = s + 1;
     }
@@ -337,7 +344,7 @@ Chunk chunk_at(const Chunk& c, const Layout& L, int k) {
 // validated, planned batch and its descriptor image on the device
 struct Batch {
     BatchPlan plan;
-    const int *day_row = nullptr, *span = nullptr, *hf_row0 = nullptr, *hf_m = nullptr;
+    const int *day_row = nullptr, *span = nullptr, *hf_row0 = nullptr, *hf_span = nullptr;
     const int *extra_row = nullptr, *caps_row = nullptr;
     const int* gdesc = nullptr;        // [W][GRAM_DESC_INTS] Gram job descriptors
     const int* bdesc[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // block precompute launches [phase][level]
@@ -403,7 +410,7 @@ int upload_batch(bp_handle* h, const bp_window_batch* b, bool need_hf, int strid
     out->day_row = dev;
     out->span = dev + W;
     out->hf_row0 = dev + 3 * (size_t)W;
-    out->hf_m = dev + 4 * (size_t)W;
+    out->hf_span = dev + 4 * (size_t)W;
     out->extra_row = P.resampled ? dev + 5 * (size_t)W : nullptr;
     out->caps_row = dev + 6 * (size_t)W;
     out->gdesc = dev + P.off_gram;
@@ -478,6 +485,7 @@ PrepParams prep_params(const bp_handle* h, const bp_window_batch* b, const Batch
     p.mcm_scaling = b->mcm_scaling;
     p.lr_daily = B.plan.resampled ? h->lr_w : h->lr_d;
     p.lr_hf = h->lr_hf;
+    p.hf_keep = h->hf_keep.p;
     p.caps = h->has_caps ? h->caps : nullptr;
     p.ld_caps = h->N;
     p.mcm = (mode == BP_MODE_CONJUGATE && h->mcm) ? h->mcm + (size_t)b->mcm_index * h->D : nullptr;
@@ -490,7 +498,7 @@ PrepParams prep_params(const bp_handle* h, const bp_window_batch* b, const Batch
     p.caps_row = B.caps_row ? B.caps_row + w0 : nullptr;
     p.span_days = B.span + w0;
     p.hf_row0 = B.hf_row0 + w0;
-    p.hf_m = B.hf_m + w0;
+    p.hf_span = B.hf_span + w0;
     p.t = c.t; p.pvec = c.pvec; p.gvec = c.gvec; p.rhs = c.rhs; p.w0 = c.w0; p.s0w0 = c.s0w0;
     p.scal = c.scal;
     p.y_ws = c.y;
@@ -728,9 +736,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
             CU_TRY(cudaStreamWaitEvent(h->stream, h->ev_seg[s], 0));
             const bool last = s == h->n_seg - 1;
             const long long r_end = h->seg_end[s];
-            launch_log_returns(h->hf_prices, h->N, h->lr_hf, h->ld, r_end, h->N, h->sm_count, h->stream, h->lr_hf_done);
-            h->launches++;
-            CU_TRY(cudaGetLastError());
+            if ((rc = hf_returns(h, h->lr_hf_done, r_end))) return rc;
             h->lr_hf_done = r_end;
             int k_ready[2];
             for (int l = 0; l < 2; ++l) {
@@ -978,6 +984,7 @@ int bp_destroy(bp_handle* h) {
     free_market(h);
     free_pool(h);
     free_buf(h->pool_cols);
+    free_buf(h->hf_keep);
     cudaStreamDestroy(h->copy_stream);
     cudaEventDestroy(h->ev_main);
     cudaEventDestroy(h->ev_hf);
@@ -1174,10 +1181,7 @@ int bp_prepare_market(bp_handle* h) {
         StageTimer tm(h, BP_STAGE_LOGRET);
         launch_log_returns(h->prices, h->N, h->lr_d, h->ld, h->D, h->N, h->sm_count, h->stream);
         h->launches++;
-        if (h->R > 0) {
-            launch_log_returns(h->hf_prices, h->N, h->lr_hf, h->ld, h->R, h->N, h->sm_count, h->stream);
-            h->launches++;
-        }
+        if (h->R > 0 && (rc = hf_returns(h, 0, h->R))) return rc;
     }
     CU_TRY(cudaGetLastError());
     return BP_OK;
@@ -1219,6 +1223,7 @@ static int begin_market(bp_handle* h, int N, int D, long long R, int n_mcm) {
         CU_TRY(cudaStreamSynchronize(h->stream));
         free_resampled(h);
     }
+    if (int rc = grow(h, h->hf_keep, (size_t)R)) return rc;
     h->N = N; h->D = D; h->ld = ld; h->R = R; h->n_mcm = n_mcm;
     if (h->timing) {
         if (!h->ev_t0) CU_TRY(cudaEventCreate(&h->ev_t0));

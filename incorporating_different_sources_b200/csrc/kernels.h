@@ -47,7 +47,8 @@ struct PrepParams {
     int prior_kind;      // BP_PRIOR_*
     double mcm_scaling;
     const double* lr_daily;   // [D][ld] daily log returns (row r = log(P_r / P_{r-1}))
-    const double* lr_hf;      // [R][ld] intraday log returns
+    const double* lr_hf;      // [R][ld] intraday log returns (dropped rows are zero rows)
+    const unsigned char* hf_keep;   // [R] 1 = the return row is kept (dropna, :314), 0 = dropped
     const double* caps;       // [D][ld_caps] (dense upload layout)
     int ld_caps;
     const double* mcm;        // [D]
@@ -59,7 +60,7 @@ struct PrepParams {
     const int* caps_row;      // [W] row of the trade date in the caps matrix, or nullptr (= day_row)
     const int* span_days;     // [W]
     const int* hf_row0;       // [W] first intraday RETURN row of the HF window (= first price row + 1)
-    const int* hf_m;          // [W] number of HF returns m
+    const int* hf_span;       // [W] HF return rows the window spans; m = the kept rows among them
     double* t;                // [W][ldv]
     double* pvec;             // [W][ldv]  u - a'a/2
     double* gvec;             // [W][ldv]  hbar (conjugate) or t (Jeffreys)
@@ -228,6 +229,9 @@ void launch_quadform(const double* S, int ldS, const double* w, int N, double* v
                      double* nu, double* weights, cudaStream_t st);
 void launch_log_returns(const double* P, int ld_in, double* out, int ld_out, long long rows, int n_assets,
                         int sm_count, cudaStream_t st, long long row_begin = 0);
+// intraday rows [row_begin, rows): returns with the reference's dropna, keep[r] = 1 for a kept row (stream_kernels.cu)
+void launch_hf_log_returns(const double* P, int ld_in, double* out, int ld_out, unsigned char* keep, long long row_begin,
+                           long long rows, int n_assets, int sm_count, cudaStream_t st);
 size_t prep_smem_bytes(int n_window, int ldv);
 cudaError_t launch_window_prep(const PrepParams& p, int n_windows, cudaStream_t st, long long n_daily_rows = 0);
 cudaError_t launch_daily_band(const PrepParams& p, int n_windows, long long n_rows, cudaStream_t st);

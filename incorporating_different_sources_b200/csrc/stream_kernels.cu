@@ -1,6 +1,7 @@
 // Streaming (HBM / L2 bound) stages of the path.
 //
 //  * log_returns_kernel        : prices -> log(P_i / P_{i-1})           (portfolio_calculations.py:37, :314)
+//  * hf_log_returns_kernel     : the same for the intraday rows, with the dropna of :314 (keep mask per row)
 //  * window_prep_kernel        : per rebalance window, everything that is O(N*K):
 //      a_k, t, u            (:40-57, :222)        excess-return column sums via the rank-2 form
 //      n0, n1               (:90-114, :247-282)   MCM (VIX/EPU) scaling of the prior
@@ -63,6 +64,56 @@ void launch_log_returns(const double* P, int ld_in, double* out, int ld_out, lon
         log_returns_kernel<true><<<grid, threads, 0, st>>>(P, ld_in, out, ld_out, row_begin, rows, n_assets);
     else
         log_returns_kernel<false><<<grid, threads, 0, st>>>(P, ld_in, out, ld_out, row_begin, rows, n_assets);
+}
+
+// Intraday returns with the reference's dropna (:314): a return row with a NaN in ANY column -- a NaN bar in price
+// row r-1 or r, or a 0/0 or inf/inf quotient -- is dropped.  A dropped row is written as zeros, which add nothing to any
+// sum the later stages form, and keep[r] = 0; a kept row is exactly log_returns_kernel's row.  One warp per row: the
+// keep decision is a warp vote, so no block barrier holds the other rows back.  Row 0 has no return (keep[0] = 0).
+template <bool VEC>
+__global__ void __launch_bounds__(256, 6) hf_log_returns_kernel(const double* __restrict__ P, int ld_in, double* __restrict__ out,
+                                                                int ld_out, unsigned char* __restrict__ keep, long long row_begin, long long rows, int n_assets) {
+    const int lane = threadIdx.x & 31;
+    const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
+    for (long long r = row_begin + blockIdx.x * (long long)(blockDim.x >> 5) + (threadIdx.x >> 5); r < rows; r += warps) {
+        double* o_row = out + r * ld_out;
+        bool nan = r == 0;
+#pragma unroll 4
+        for (int c = lane * 2; c < ld_out; c += 64) {
+            double2 o = make_double2(0.0, 0.0);
+            if (r > 0 && c < n_assets) {
+                const double* cur = P + r * ld_in + c;
+                const double* prv = cur - ld_in;
+                if (VEC && c + 1 < n_assets) {
+                    const double2 p = *reinterpret_cast<const double2*>(cur);
+                    const double2 q = *reinterpret_cast<const double2*>(prv);
+                    o.x = log(p.x / q.x);
+                    o.y = log(p.y / q.y);
+                } else {
+                    o.x = log(cur[0] / prv[0]);
+                    if (c + 1 < n_assets) o.y = log(cur[1] / prv[1]);
+                }
+            }
+            nan |= isnan(o.x) || isnan(o.y);
+            *reinterpret_cast<double2*>(o_row + c) = o;
+        }
+        const bool drop = __any_sync(0xffffffffu, nan);
+        if (drop)
+            for (int c = lane * 2; c < ld_out; c += 64) *reinterpret_cast<double2*>(o_row + c) = make_double2(0.0, 0.0);
+        if (lane == 0) keep[r] = drop ? 0 : 1;
+    }
+}
+
+void launch_hf_log_returns(const double* P, int ld_in, double* out, int ld_out, unsigned char* keep, long long row_begin,
+                           long long rows, int n_assets, int sm_count, cudaStream_t st) {
+    if (rows <= row_begin) return;
+    const int threads = 256, rows_per_block = threads / 32;
+    long long blocks = (rows - row_begin + rows_per_block - 1) / rows_per_block;
+    if (blocks > (long long)sm_count * 6) blocks = (long long)sm_count * 6;     // one wave at the launch bounds
+    if ((ld_in & 1) == 0)
+        hf_log_returns_kernel<true><<<(unsigned)blocks, threads, 0, st>>>(P, ld_in, out, ld_out, keep, row_begin, rows, n_assets);
+    else
+        hf_log_returns_kernel<false><<<(unsigned)blocks, threads, 0, st>>>(P, ld_in, out, ld_out, keep, row_begin, rows, n_assets);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -163,6 +214,31 @@ __device__ __forceinline__ double2 reduce_cols(const double2 (&part)[NCH], doubl
         s.y += v.y;
     }
     return s;
+}
+
+// block_sum of both components at once (each summed in block_sum's order); scratch holds >= 34 doubles
+__device__ __forceinline__ double2 block_sum2(double2 v, double* scratch) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
+    v.x = warp_sum(v.x);
+    v.y = warp_sum(v.y);
+    __syncthreads();
+    if (lane == 0) {
+        scratch[warp] = v.x;
+        scratch[16 + warp] = v.y;
+    }
+    __syncthreads();
+    if (warp == 0) {
+        double sx = lane < nw ? scratch[lane] : 0.0;
+        double sy = lane < nw ? scratch[16 + lane] : 0.0;
+        sx = warp_sum(sx);
+        sy = warp_sum(sy);
+        if (lane == 0) {
+            scratch[32] = sx;
+            scratch[33] = sy;
+        }
+    }
+    __syncthreads();
+    return make_double2(scratch[32], scratch[33]);
 }
 
 // The prep kernel is the first writer of a window's scalar record, which lives in the shared, never-cleared workspace:
@@ -286,8 +362,21 @@ __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams
     }
     __syncthreads();
 
-    const int m = p.hf_m[w];                                // HF returns in the window
+    // HF returns of the window: m = the kept rows of the span (dropna, :314).  A dropped row is a zero row of lr_hf, so
+    // every sum below may run over the whole span; only the mean divides by m and only kept rows are centred.
+    const int span = p.hf_span[w];
+    const long long h0 = (long long)p.hf_row0[w];           // first HF return row (first bar dropped, F5)
+    const unsigned char* keep = p.hf_keep + h0;
+    auto count_kept = [&]() {
+        double kept = 0.0;
+        for (int k = tid; k < span; k += PREP_THREADS) kept += (double)keep[k];
+        return (int)block_sum(kept, scratch);
+    };
+    // m < 2: pandas' cov is all NaN (:317), so S0 and everything derived from it is NaN and the solve reports a pivot
+    auto alpha_of = [&](int m) { return m >= 2 ? n0 * ((double)m / (double)(m - 1)) : nan(""); };   // S0 = n0 * cov * m  (:317-318, :333)
     if (p.hf_presum) {
+        const int m = count_kept();
+        const double alpha = alpha_of(m);
         // pre-summed day blocks: the window's column sums are <= 3 scanned vectors (suffix' + whole chunk + prefix);
         // S0 w0, v0, c and rhs follow the Gram launch (conj_post_kernel)
         const int* ids = p.hf_vids + 3 * (long long)w;
@@ -305,7 +394,6 @@ __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams
             *reinterpret_cast<double2*>(p.gvec + (long long)w * p.ldv + c) = hb;
         }
         if (tid == 0) {
-            const double alpha = n0 * ((double)m / (double)(m - 1));   // S0 = n0 * cov * m  (:317-318, :333)
             scal[BP_S_N0] = n0;
             scal[BP_S_N1] = n1;
             scal[BP_S_ALPHA] = alpha;
@@ -321,22 +409,17 @@ __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams
     }
 
     // ---- HF pass 1: column means hbar and row dots y_k = h_k . w0   (:314-318)
-    const long long h0 = (long long)p.hf_row0[w];           // first HF return row (first bar dropped, F5)
     double* y = p.y_ws + (long long)w * p.y_stride;
     const bool one_pass = p.ldv <= 512;
+    int m = one_pass ? 0 : count_kept();     // one pass: counted with the sum of y below (one reduction fewer)
     double2 hs1 = make_double2(0.0, 0.0), q1 = make_double2(0.0, 0.0);
     if (one_pass) {
-        hf_single_pass(p.lr_hf, p.ld, h0, m, w0_s, y, sum, wsum);
+        hf_single_pass(p.lr_hf, p.ld, h0, span, w0_s, y, sum, wsum);
         hs1 = reduce_cols(sum, red);
         q1 = reduce_cols(wsum, red);
-        const int c = tid * 2;
-        if (c < p.ldv) {
-            double2 hb = make_double2(c < N ? hs1.x / (double)m : 0.0, c + 1 < N ? hs1.y / (double)m : 0.0);
-            *reinterpret_cast<double2*>(p.gvec + (long long)w * p.ldv + c) = hb;
-        }
     } else {
         for (int col0 = 0; col0 < p.ldv; col0 += 512) {
-            col_accumulate<true>(p.lr_hf, p.ld, h0, m, col0, nullptr, w0_s, y, col0 > 0, sum, wsum);
+            col_accumulate<true>(p.lr_hf, p.ld, h0, span, col0, nullptr, w0_s, y, col0 > 0, sum, wsum);
             const double2 hs = reduce_cols(sum, red);
             const int c = col0 + tid * 2;
             if (c < p.ldv) {
@@ -346,20 +429,35 @@ __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams
         }
     }
     __syncthreads();
-    // centre y:  y_c = y - mean(y)   (sum_k y_c = 0 => S0 w0 = alpha * H' y_c, v0 = alpha * |y_c|^2)
-    double ys = 0.0;
-    for (int k = tid; k < m; k += PREP_THREADS) ys += y[k];
-    ys = block_sum(ys, scratch);
+    // centre y over the kept rows:  y_c = y - mean(y)   (sum_k y_c = 0 => S0 w0 = alpha * H' y_c, v0 = alpha * |y_c|^2).
+    // A dropped row has y = 0 and stays 0, so it enters neither the mean nor |y_c|^2 (and H' y_c, its H row being 0).
+    double ys = 0.0, kept = 0.0;
+    for (int k = tid; k < span; k += PREP_THREADS) {
+        ys += y[k];
+        kept += (double)keep[k];
+    }
+    if (one_pass) {
+        const double2 s2 = block_sum2(make_double2(ys, kept), scratch);
+        ys = s2.x;
+        m = (int)s2.y;
+        const int c = tid * 2;
+        if (c < p.ldv) {
+            double2 hb = make_double2(c < N ? hs1.x / (double)m : 0.0, c + 1 < N ? hs1.y / (double)m : 0.0);
+            *reinterpret_cast<double2*>(p.gvec + (long long)w * p.ldv + c) = hb;
+        }
+    } else {
+        ys = block_sum(ys, scratch);
+    }
+    const double alpha = alpha_of(m);
     const double ybar = ys / (double)m;
     double yy = 0.0;
-    for (int k = tid; k < m; k += PREP_THREADS) {
-        const double v = y[k] - ybar;
+    for (int k = tid; k < span; k += PREP_THREADS) {
+        const double v = keep[k] ? y[k] - ybar : 0.0;
         if (!one_pass) y[k] = v;
         yy = fma(v, v, yy);
     }
     yy = block_sum(yy, scratch);      // block_sum's barriers also publish the centred y to the block
 
-    const double alpha = n0 * ((double)m / (double)(m - 1));   // S0 = n0 * cov * m  (:317-318, :333)
     const double v0 = alpha * yy;
     const double kk = n0 + (double)N + 2.0;
     const double cc = (2.0 * n0) / (kk + sqrt(kk * kk + 4.0 * n0 * v0));   // :415-418
@@ -378,7 +476,7 @@ __global__ void __launch_bounds__(PREP_THREADS, 2) window_prep_kernel(PrepParams
     } else {
         // HF pass 2
         for (int col0 = 0; col0 < p.ldv; col0 += 512) {
-            col_accumulate<false>(p.lr_hf, p.ld, h0, m, col0, y, nullptr, nullptr, false, sum, wsum);
+            col_accumulate<false>(p.lr_hf, p.ld, h0, span, col0, y, nullptr, nullptr, false, sum, wsum);
             const double2 qs = reduce_cols(wsum, red);
             const int c = col0 + tid * 2;
             if (c < p.ldv) {

@@ -204,7 +204,11 @@ class BayesEngine:
         """Host arrays -> HBM.  With ``async_copy=True`` the arrays must be page-locked and are kept
         alive by the engine until :meth:`synchronize`; the intraday block then overlaps with stages that
         do not read it (Jeffreys, daily statistics).  ``prices`` [D][N], ``rf_row`` [D] (risk-free rate forward-filled onto
-        the daily rows), ``caps`` [D][N], ``hf_prices`` [R][N], ``mcm`` [n_mcm][D] (row 0 VIX, row 1 EPU)."""
+        the daily rows), ``caps`` [D][N], ``hf_prices`` [R][N], ``mcm`` [n_mcm][D] (row 0 VIX, row 1 EPU).
+
+        ``hf_prices`` may hold NaN (missing bars).  As the reference's ``dropna`` (:314), an intraday return row with a
+        NaN in any column is dropped: a NaN bar removes the returns on both sides of it.  A conjugate window uses the
+        m returns it keeps (scalar ``m``); with m < 2 its S0 and weights are NaN and its status is non-zero."""
         prices = _c64(prices)
         rf_row = _c64(rf_row)
         D, N = prices.shape
@@ -253,7 +257,9 @@ class BayesEngine:
 
     def upload_pool(self, prices, rf_row, caps=None, hf_prices=None):
         """The FULL market (every candidate column, every row) into a resident pool; :meth:`select_market` then builds
-        the working market of a batch on the device.  ``upload_pool(None, None)`` releases the pool."""
+        the working market of a batch on the device.  ``upload_pool(None, None)`` releases the pool.  ``hf_prices`` may
+        hold NaN as in :meth:`upload_market`; the rows to drop are decided on the selected columns only, so holes in
+        columns a working market does not select change nothing."""
         if prices is None:
             rc = self._lib.bp_upload_pool(self._h, None)
             if rc:

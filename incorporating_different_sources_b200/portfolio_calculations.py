@@ -11,12 +11,16 @@ Per-window calls upload a minimal market (the window's own rows) and are meant f
 for tests; whole backtests should use :class:`~.engine.BayesEngine` / :func:`backtest_portfolio`,
 which evaluate all rebalance windows in one launch sequence.
 
+Missing intraday bars are handled as the reference's ``dropna`` (:314-318): a NaN bar in any column of the
+window drops the return rows on both sides of it (no return bridges the gap), and the realised covariance
+uses the m returns that are left.  With m < 2 the prior is all NaN, as pandas' ``cov`` is, and the posterior
+and portfolio functions raise the reference's ``ValueError`` (:492-494).
+
 Deviations from the reference (documented, all raise instead of silently differing):
 * ``rolling_window_frequency == "monthly"`` raises ``NotImplementedError`` (the reference itself
   fails under pandas >= 2.2, SURVEY F10);
 * a window with fewer than ``rolling_window`` price rows raises ``ValueError`` (the reference would
   silently use the shorter window);
-* NaNs inside the selected intraday window raise ``ValueError`` (the reference drops those rows);
 * a non-positive Cholesky pivot raises ``numpy.linalg.LinAlgError`` where ``np.linalg.inv`` would
   return garbage for a numerically singular matrix (SURVEY F6).
 """
@@ -113,7 +117,8 @@ def _window_arrays(portfolio_spec, price_window_df, risk_free_rate_df, full_wind
 
 
 def _hf_window(portfolio_spec, trading_date_ts, intraday_df, columns):
-    """Rows of the intraday frame inside the HF look-back (:299-312), in ``columns`` order."""
+    """Rows of the intraday frame inside the HF look-back (:299-312), in ``columns`` order.  NaN bars stay: the
+    device drops the returns next to them (dropna, :314)."""
     freq = portfolio_spec["rolling_window_frequency"]
     if freq not in HF_LOOKBACK_DAYS:
         raise RuntimeError("Unknown rolling window frequency.")                       # :308
@@ -124,8 +129,6 @@ def _hf_window(portfolio_spec, trading_date_ts, intraday_df, columns):
     if set(sel.columns) != set(columns):
         raise ValueError("intraday and daily price frames must hold the same stocks")
     H = np.ascontiguousarray(sel[list(columns)].to_numpy(dtype=np.float64))
-    if np.isnan(H).any():
-        raise ValueError("NaN in the intraday window: not supported on the CUDA path")
     if H.shape[0] < 3:
         raise ValueError("the intraday window needs at least 3 price rows")
     return H
@@ -204,6 +207,11 @@ def _weight_frame(values, index, index_name=None):
     df = pd.DataFrame({"Weight": np.asarray(values, dtype=np.float64)}, index=index)
     df.index.name = index_name
     return df
+
+
+def _raise_no_hf_returns():
+    # fewer than 2 intraday returns survive dropna: S0 is all NaN and so is w1 (:317, :492-494)
+    raise ValueError("conjugate_posterior_w_df contains NaN values.")
 
 
 def _check_status(status):
@@ -370,7 +378,9 @@ def _conj_fused(portfolio_spec, trading_date_ts, k_stock_prices_df, k_stock_mark
     eng, batch, cols = _upload_window(portfolio_spec, trading_date_ts, k_stock_prices_df, risk_free_rate_df,
                                       k_stock_market_caps_df, k_stock_intraday_prices_df, mcm_prices_df)
     if solve:
-        res = eng.conjugate(batch, outputs=tuple(outputs) + ("status",))
+        res = eng.conjugate(batch, outputs=tuple(outputs) + ("scalars", "status"))
+        if res["scalars"][0][SCAL["m"]] < 2:
+            _raise_no_hf_returns()
         _check_status(res["status"][0])
     else:
         res = eng.moments(batch, outputs=tuple(outputs))
@@ -466,6 +476,8 @@ def _dense_conjugate(portfolio_spec, trading_date_ts, k_stock_prices_df, k_stock
     gamma = portfolio_spec["risk_aversion"] if portfolio_spec.get("risk_aversion") is not None else 1.0
     res = eng.dense_posterior(jeffreys=False, rolling_window=portfolio_spec["rolling_window"], risk_aversion=gamma, **kw)
     if conjugate_posterior_w_df is None:
+        if np.isnan(kw["S0"]).any():
+            _raise_no_hf_returns()
         _check_status(res["status"][0])
     return res, S1_order
 
