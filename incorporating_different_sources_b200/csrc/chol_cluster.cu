@@ -3,7 +3,8 @@
 // Same mathematics and the same panel kernels as chol_solve.cu (left-looking, 32-column panels, TMA-fed DMMA panel
 // update with the panel solve fused into its epilogue, register-level 32x32 diagonal block; w1 = inv(S1)(c S0 w0 + t)
 // :485-489, nu :572-575, Jeffreys :600-606, weights = (1/gamma) nu :836,:849), but the rows of a window are spread
-// over the K CTAs of a cluster instead of one CTA doing everything.
+// over the K CTAs of a cluster instead of one CTA doing everything.  The right-hand side(s) ride along as rows R, R+1
+// of the factorisation with R = chol_rhs_row(N), exactly as there, so that both kernels give the same bits.
 //
 // Why: (1) latency -- a launch of a few windows (one façade call, the 65 Jeffreys base windows of a date-range shard on
 // 8 GPUs) leaves most SMs idle with one 4-warp CTA per window; K CTAs per window finish it roughly K times sooner.
@@ -138,7 +139,9 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
     const int g = lane >> 2, tig = lane & 3;
     const int N = p.n_assets;
     const int ld = p.ldS;
-    const int Nr = (N + NB - 1) / NB * NB;     // row index of the right-hand side
+    const int Nr = (N + NB - 1) / NB * NB;
+    const int R = chol_rhs_row(N);             // row index of the right-hand side (see chol_solve.cu)
+    const int rows_end = max(Nr, R + 8);       // the panels cover rows j0 .. rows_end-1
     const int rowsS = (int)(p.win_stride / ld);
     const int stride = max(p.w_stride, 1);
     // back substitution vectors alias the TMA stages (idle after the last panel): running rhs and solution
@@ -169,7 +172,7 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
         __syncthreads();
 
         for (int j0 = 0, pi = 0; j0 < N; j0 += NB, ++pi) {
-            const int mt_total = (Nr + 8 - j0) / 8;        // m-tiles covering rows j0 .. Nr+7
+            const int mt_total = (rows_end - j0) / 8;      // m-tiles covering rows j0 .. rows_end-1
             const int ng = (mt_total + 3) >> 2;            // 32-row groups
             const int nchunks = j0 / 16;
             const bool diag_owner = rank == pi % K;
@@ -200,15 +203,15 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
 #pragma unroll
                 for (int i = 0; i < TPW; ++i) {
                     const int row = j0 + 32 * (q0 + i * K) + 8 * warp + g;
-                    const bool real = i < ni && (row < N || (row >= Nr && row < Nr + NRHS));
+                    const bool real = i < ni && (row < N || (row >= R && row < R + NRHS));
 #pragma unroll
                     for (int nt = 0; nt < 4; ++nt) {
                         const int col = j0 + 8 * nt + 2 * tig;
                         double2 sv = make_double2(0.0, 0.0);
                         if (real && col < N) {
                             if (row < N) sv = *reinterpret_cast<const double2*>(S + (long long)row * ld + col);
-                            else if (NRHS == 2 && row == Nr + 1) sv = make_double2(1.0, 1.0);
-                            else sv = *reinterpret_cast<const double2*>(rhs + col);     // the right-hand side rides along as row Nr
+                            else if (NRHS == 2 && row == R + 1) sv = make_double2(1.0, 1.0);
+                            else sv = *reinterpret_cast<const double2*>(rhs + col);     // the right-hand side rides along as row R
                         }
                         if (real) {
                             acc[i][nt][0] = -sv.x;
@@ -245,23 +248,19 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
                     if (tid == 0 && c + CC_STAGES < nchunks) issue(c + CC_STAGES, it + CC_STAGES);
                 }
 
-                // padding: rows N..Nr-1 and columns >= N of the workspace hold no data; whatever the update
-                // accumulated there is replaced by the identity (rows) / zero (columns)
+                // padding: rows N..rows_end-1 other than the right-hand sides, and columns >= N, hold no data;
+                // whatever the update accumulated there is replaced by the identity (zero for the rows of S, a unit
+                // diagonal for a right-hand-side row R < Nr in the diagonal block of the last panel)
                 if (j0 + 32 * (q0 + (nboxes - 1) * K) + 32 > N || j0 + NB > N) {
 #pragma unroll
                     for (int i = 0; i < TPW; ++i) {
                         const int row = j0 + 32 * (q0 + i * K) + 8 * warp + g;
-                        const bool real = row < N || (row >= Nr && row < Nr + NRHS);
+                        const bool real = row < N || (row >= R && row < R + NRHS);
 #pragma unroll
                         for (int nt = 0; nt < 4; ++nt) {
                             const int col = j0 + 8 * nt + 2 * tig;
-                            if (!real) {
-                                acc[i][nt][0] = row == col ? -1.0 : 0.0;
-                                acc[i][nt][1] = row == col + 1 ? -1.0 : 0.0;
-                            } else {
-                                if (col >= N) acc[i][nt][0] = 0.0;
-                                if (col + 1 >= N) acc[i][nt][1] = 0.0;
-                            }
+                            if (!real || col >= N) acc[i][nt][0] = row == col ? -1.0 : 0.0;
+                            if (!real || col + 1 >= N) acc[i][nt][1] = row == col + 1 ? -1.0 : 0.0;
                         }
                     }
                 }
@@ -273,7 +272,8 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
                         if (warp == cb) {
                             double d0 = -acc[0][cb][0], d1 = -acc[0][cb][1], y0, y1;
                             const int f = potrf8_inv8(d0, d1, y0, y1, g, tig, lane);
-                            if (lane == 0 && f != 0 && fail_s == 0) fail_s = j0 + 8 * cb + f;
+                            // tiles from row N on: padding and right-hand sides, no pivots of S (see chol_solve.cu)
+                            if (lane == 0 && f != 0 && fail_s == 0 && j0 + 8 * cb < N) fail_s = j0 + 8 * cb + f;
                             double* row = P + (8 * cb + g) * LDQ + 8 * cb + 2 * tig;
                             if (2 * tig <= g) row[0] = d0;
                             if (2 * tig + 1 <= g) row[1] = d1;
@@ -307,7 +307,8 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
                                 }
                         }
                     }
-                    // push the packed block to the peers, then barrier A; write L_d back (lower part, real rows only)
+                    // push the packed block to the peers, then barrier A; write L_d back (lower part, real rows only:
+                    // in the last panel z of a right-hand side R < Nr)
                     for (int peer = 0; peer < K; ++peer) {
                         if (peer == rank) continue;
                         double* dst = cluster.map_shared_rank(P, peer);
@@ -316,7 +317,8 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
                     cluster_arrive();
                     for (int i = warp; i < NB; i += CC_WARPS) {
                         const int row = j0 + i, col = j0 + lane;
-                        if (row < N && col < N && lane <= i) S[(long long)row * ld + col] = P[i * LDQ + lane];
+                        if ((row < N || (row >= R && row < R + NRHS)) && col < N && lane <= i)
+                            S[(long long)row * ld + col] = P[i * LDQ + lane];
                     }
                 }
                 if (!waitedA) {
@@ -329,7 +331,7 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
                     const int q = q0 + i * K;                     // group index within the panel
                     if (i >= ni || q == 0) continue;
                     const int row = j0 + 32 * q + 8 * warp + g;
-                    const bool real = row < N || (row >= Nr && row < Nr + NRHS);
+                    const bool real = row < N || (row >= R && row < R + NRHS);
 #pragma unroll
                     for (int cb = 0; cb < NB / 8; ++cb) {
                         double x0 = 0.0, x1 = 0.0;
@@ -354,13 +356,13 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
             fence_proxy_async_all();
         }
 
-        // ---------------- z = L^-1 b sits in row Nr (+r);  v1 = z'z = w1' S1 w1   (:574)
+        // ---------------- z = L^-1 b sits in row R (+r);  v1 = z'z = w1' S1 w1   (:574)
         double zz = 0.0;
         for (int j = tid; j < Nr; j += CC_THREADS) {
-            const double z = j < N ? S[(long long)Nr * ld + j] : 0.0;
+            const double z = j < N ? S[(long long)R * ld + j] : 0.0;
             zs[j] = z;
             zz = fma(z, z, zz);
-            if constexpr (NRHS == 2) zs[Nr + j] = j < N ? S[(long long)(Nr + 1) * ld + j] : 0.0;
+            if constexpr (NRHS == 2) zs[Nr + j] = j < N ? S[(long long)(R + 1) * ld + j] : 0.0;
         }
         const double v1 = block_sum(zz, scratch);
 

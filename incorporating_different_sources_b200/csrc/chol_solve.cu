@@ -28,9 +28,13 @@
 //                     traffic per window and 15% of the kernel.)
 // The factor is written with generic stores and re-read by TMA in later panels, so every panel ends
 // with fence.proxy.async + a block barrier.  The right-hand side rides along as one extra row
-// (row Nr = roundup(N,32)) of the matrix, so the forward substitution L z = b is a by-product of
-// the factorisation.  The back substitution then walks the panels in reverse with coalesced row
-// reads and a warp-level triangular solve.
+// (row R = chol_rhs_row(N), kernels.h) of the matrix, so the forward substitution L z = b is a by-product
+// of the factorisation.  R is the first 8-row tile after the data: for N mod 32 in 1..24 it lies in the
+// padding rows below Nr = roundup(N,32), so the panels stop at row Nr - 1 instead of paying a whole slab
+// (every chunk of the factored columns through the TMA ring) for one m-tile at row Nr; in the last panel
+// the right-hand-side row then sits in the diagonal block, where it is solved by F and keeps an
+// identity entry in its own padding column.  The back substitution then walks the panels in reverse
+// with coalesced row reads and a warp-level triangular solve.
 //
 // k-permutation: inside a 16-column chunk, DMMA step q contracts columns {2q, 2q+1, 8+2q, 9+2q}
 // over the four tig lanes.  With the 128-byte swizzle (16-byte unit index XOR row&7) the 16 lanes of
@@ -136,7 +140,7 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const void* tmap, in
 __device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 
 // NRHS = 1: the posterior solves of the conjugate / Jeffreys path.  NRHS = 2 (Jorion, :851-895): a second
-// right-hand side (the vector of ones) rides along as row Nr+1, so that both C^-1 t and C^-1 1 come out of ONE
+// right-hand side (the vector of ones) rides along as row R+1, so that both C^-1 t and C^-1 1 come out of ONE
 // factorisation; the Bayes-Stein combination is the epilogue of this kernel.
 template <int NRHS>
 __global__ void __launch_bounds__(CH_THREADS, NRHS == 1 ? CH_OCC : 4)
@@ -156,7 +160,9 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
     const int g = lane >> 2, tig = lane & 3;
     const int N = p.n_assets;
     const int ld = p.ldS;
-    const int Nr = (N + NB - 1) / NB * NB;     // row index of the right-hand side
+    const int Nr = (N + NB - 1) / NB * NB;
+    const int R = chol_rhs_row(N);             // row index of the right-hand side
+    const int rows_end = max(Nr, R + 8);       // the panels cover rows j0 .. rows_end-1
     const int rowsS = (int)(p.win_stride / ld);
 
     if (tid == 0) {
@@ -191,14 +197,14 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
         const double* rhs = p.rhs + (long long)w * p.ldv;
         const int grow0 = w * rowsS;           // first row of this window in the tensor map
         if (tid == 0) fail_s = 0;
-        for (int j = tid; j < ld; j += CH_THREADS) S[(long long)Nr * ld + j] = j < N ? rhs[j] : 0.0;
+        for (int j = tid; j < ld; j += CH_THREADS) S[(long long)R * ld + j] = j < N ? rhs[j] : 0.0;
         if constexpr (NRHS == 2)
-            for (int j = tid; j < ld; j += CH_THREADS) S[(long long)(Nr + 1) * ld + j] = j < N ? 1.0 : 0.0;
+            for (int j = tid; j < ld; j += CH_THREADS) S[(long long)(R + 1) * ld + j] = j < N ? 1.0 : 0.0;
         fence_proxy_async_all();
         __syncthreads();
 
         for (int j0 = 0; j0 < N; j0 += NB) {
-            const int mt_total = (Nr + 8 - j0) / 8;        // m-tiles covering rows j0 .. Nr+7
+            const int mt_total = (rows_end - j0) / 8;      // m-tiles covering rows j0 .. rows_end-1
             const int nchunks = j0 / 16;
             // ---------------- U (+F after the first slab) + fused T, one slab of SLAB_TILES m-tiles per pass
             for (int slab0 = 0; slab0 < mt_total; slab0 += SLAB_TILES) {
@@ -227,7 +233,7 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
 #pragma unroll
                 for (int i = 0; i < TPW; ++i) {
                     const int row = j0 + 8 * (slab0 + warp + CH_WARPS * i) + g;
-                    const bool real = i < ni && (row < N || (row >= Nr && row < Nr + NRHS));
+                    const bool real = i < ni && (row < N || (row >= R && row < R + NRHS));
 #pragma unroll
                     for (int nt = 0; nt < 4; ++nt) {
                         const int col = j0 + 8 * nt + 2 * tig;
@@ -290,23 +296,20 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
                     if (tid == 0 && c + CH_STAGES < nchunks) issue(c + CH_STAGES, it + CH_STAGES);
                 }
 
-                // padding: rows N..Nr-1 and columns >= N of the workspace hold no data; whatever the update
-                // accumulated there is replaced by the identity (rows) / zero (columns)
+                // padding: rows N..rows_end-1 other than the right-hand sides, and columns >= N, hold no data;
+                // whatever the update accumulated there is replaced by the identity.  In a padding column that is
+                // zero for the rows of S and a unit diagonal for a right-hand-side row R < Nr, which sits in the
+                // diagonal block of the last panel: its pivot must not be zero
                 if (slab_row + 8 * slab_tiles > N || j0 + NB > N) {
 #pragma unroll
                     for (int i = 0; i < TPW; ++i) {
                         const int row = j0 + 8 * (slab0 + warp + CH_WARPS * i) + g;
-                        const bool real = row < N || (row >= Nr && row < Nr + NRHS);
+                        const bool real = row < N || (row >= R && row < R + NRHS);
 #pragma unroll
                         for (int nt = 0; nt < 4; ++nt) {
                             const int col = j0 + 8 * nt + 2 * tig;
-                            if (!real) {
-                                acc[i][nt][0] = row == col ? -1.0 : 0.0;
-                                acc[i][nt][1] = row == col + 1 ? -1.0 : 0.0;
-                            } else {
-                                if (col >= N) acc[i][nt][0] = 0.0;
-                                if (col + 1 >= N) acc[i][nt][1] = 0.0;
-                            }
+                            if (!real || col >= N) acc[i][nt][0] = row == col ? -1.0 : 0.0;
+                            if (!real || col + 1 >= N) acc[i][nt][1] = row == col + 1 ? -1.0 : 0.0;
                         }
                     }
                 }
@@ -322,7 +325,9 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
                         if (warp == cb) {
                             double d0 = -acc[0][cb][0], d1 = -acc[0][cb][1], y0, y1;
                             const int f = potrf8_inv8(d0, d1, y0, y1, g, tig, lane);
-                            if (lane == 0 && f != 0 && fail_s == 0) fail_s = j0 + 8 * cb + f;
+                            // a tile from row N on holds padding and right-hand sides, whose pivots are none of S's
+                            // (a right-hand side's is 1 - |its z in this panel|^2 and may be negative)
+                            if (lane == 0 && f != 0 && fail_s == 0 && j0 + 8 * cb < N) fail_s = j0 + 8 * cb + f;
                             double* row = P + (8 * cb + g) * LDQ + 8 * cb + 2 * tig;
                             if (2 * tig <= g) row[0] = d0;
                             if (2 * tig + 1 <= g) row[1] = d1;
@@ -357,10 +362,11 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
                         }
                     }
                     PROF(1)
-                    // write L_d back (lower part, real rows only)
+                    // write L_d back (lower part, real rows only: in the last panel z of a right-hand side R < Nr)
                     for (int i = warp; i < NB; i += CH_WARPS) {
                         const int row = j0 + i, col = j0 + lane;
-                        if (row < N && col < N && lane <= i) S[(long long)row * ld + col] = P[i * LDQ + lane];
+                        if ((row < N || (row >= R && row < R + NRHS)) && col < N && lane <= i)
+                            S[(long long)row * ld + col] = P[i * LDQ + lane];
                     }
                 }
                 // ---------------- T: X = C inv(L_d)' straight from the accumulators, by block forward substitution
@@ -371,7 +377,7 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
                     const int q = slab0 + warp + CH_WARPS * i;     // m-tile index within the panel
                     if (i >= ni || q < NB / 8) continue;
                     const int row = j0 + 8 * q + g;
-                    const bool real = row < N || (row >= Nr && row < Nr + NRHS);
+                    const bool real = row < N || (row >= R && row < R + NRHS);
 #pragma unroll
                     for (int cb = 0; cb < NB / 8; ++cb) {
                         double x0 = 0.0, x1 = 0.0;
@@ -394,13 +400,13 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
             PROF(2)
         }
 
-        // ---------------- z = L^-1 b sits in row Nr (+r);  v1 = z'z = w1' S1 w1   (:574)
+        // ---------------- z = L^-1 b sits in row R (+r);  v1 = z'z = w1' S1 w1   (:574)
         double zz = 0.0;
         for (int j = tid; j < Nr; j += CH_THREADS) {
-            const double z = j < N ? S[(long long)Nr * ld + j] : 0.0;
+            const double z = j < N ? S[(long long)R * ld + j] : 0.0;
             xs[j] = z;
             zz = fma(z, z, zz);
-            if constexpr (NRHS == 2) xs[Nr + j] = j < N ? S[(long long)(Nr + 1) * ld + j] : 0.0;
+            if constexpr (NRHS == 2) xs[Nr + j] = j < N ? S[(long long)(R + 1) * ld + j] : 0.0;
         }
         const double v1 = block_sum(zz, scratch);
 

@@ -170,6 +170,12 @@ struct SolveParams {
     long long* debug;        // optional phase-cycle counters (BP_CHOL_PROFILE), normally nullptr
 };
 
+// Row R of the solver workspace at which the right-hand side(s) ride along through the factorisation (rows R .. R+nrhs-1,
+// so that L z = b comes out as row R of the factor).  R = roundup(N, 8): for N mod 32 in 1..24 that is a padding row at
+// most Nr - 8 (Nr = roundup(N, 32)), so up to 8 right-hand sides fit below Nr and the panels end at row Nr - 1;
+// otherwise R = Nr and the panels cover the extra m-tile Nr .. Nr+7 (the workspace has ldS + 8 rows for it).
+__host__ __device__ constexpr int chol_rhs_row(int n_assets) { return (n_assets + 7) / 8 * 8; }
+
 struct DenseParams {
     int n_assets, ldS, ldv, n_window;
     double n0, n1, c_in;
