@@ -1,10 +1,10 @@
 // Batched blocked Cholesky + triangular solves + posterior scalars, ONE THREAD-BLOCK CLUSTER PER WINDOW.
 //
-// Same mathematics and the same panel kernels as chol_solve.cu (left-looking, 32-column panels, TMA-fed DMMA panel
-// update with the panel solve fused into its epilogue, register-level 32x32 diagonal block; w1 = inv(S1)(c S0 w0 + t)
-// :485-489, nu :572-575, Jeffreys :600-606, weights = (1/gamma) nu :836,:849), but the rows of a window are spread
-// over the K CTAs of a cluster instead of one CTA doing everything.  The right-hand side(s) ride along as rows R, R+1
-// of the factorisation with R = chol_rhs_row(N), exactly as there, so that both kernels give the same bits.
+// The factorisation of chol_solve_kernel (left-looking, 32-column panels, TMA-fed DMMA panel update with the panel
+// solve fused into its epilogue, register-level 32x32 diagonal block, right-hand side(s) riding along as rows R, R+1;
+// w1 = inv(S1)(c S0 w0 + t) :485-489, nu :572-575, Jeffreys :600-606, weights = (1/gamma) nu :836,:849), but the rows
+// of a window are spread over the K CTAs of a cluster instead of one CTA doing everything.  All arithmetic is the
+// shared code of chol_panel.cuh, so that both kernels give the same bits; this file holds the cluster's schedule.
 //
 // Why: (1) latency -- a launch of a few windows (one façade call, the 65 Jeffreys base windows of a date-range shard on
 // 8 GPUs) leaves most SMs idle with one 4-warp CTA per window; K CTAs per window finish it roughly K times sooner.
@@ -34,85 +34,28 @@
 #include <cstdio>
 #include <cstdlib>
 
-#include "common.cuh"
-#include "jorion_math.cuh"
-#include "kernels.h"
+#include "chol_panel.cuh"
 
 namespace cg = cooperative_groups;
 
 namespace bp {
 
+using namespace chol;
+
 namespace {
 
-constexpr int NB = 32;
 constexpr int CC_WARPS = 4;
 constexpr int CC_THREADS = CC_WARPS * 32;
 #ifndef CC_CTAS_PER_SM
 #define CC_CTAS_PER_SM 6
 #endif
 constexpr int CC_OCC = CC_CTAS_PER_SM;
-constexpr int LDQ = 34;                              // row stride of the packed diagonal-block array
 constexpr int TPW = 2;                               // groups (A boxes) per pass = m-tiles per warp and pass
 constexpr int CC_STAGES = 2;
-constexpr int BOX_BYTES = 32 * 16 * 8;               // one TMA box: 32 rows x 16 columns of doubles
 constexpr int CC_STAGE_BYTES = (TPW + 1) * BOX_BYTES;   // A boxes + 1 B box
 constexpr int CC_TMA_SMEM = CC_STAGES * CC_STAGE_BYTES + 1024;
 constexpr int CC_MAX_CLUSTER = 8;
 
-// Cholesky factor AND inverse of one 8x8 diagonal tile by one warp in registers (see chol_solve.cu: potrf8_inv8).
-// The tile is in DMMA accumulator layout; on return d0/d1 hold L, y0/y1 inv(L).  Returns the 1-based index of the
-// first non-positive pivot, or 0.
-__device__ __forceinline__ int potrf8_inv8(double& d0, double& d1, double& y0, double& y1, int g, int tig, int lane) {
-    constexpr unsigned FULL = 0xffffffffu;
-    int fail = 0;
-    double u0 = 2 * tig == g ? 1.0 : 0.0, u1 = 2 * tig + 1 == g ? 1.0 : 0.0;
-    double invrow = 0.0;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        const double dk = (k & 1) ? d1 : d0;
-        const int sq = k >> 1;
-        const double piv = __shfl_sync(FULL, dk, 4 * k + sq);               // D[k][k]
-        const double colg = __shfl_sync(FULL, dk, (lane & ~3) | sq);        // D[g][k]
-        const double colj0 = __shfl_sync(FULL, dk, 8 * tig + sq);           // D[2tig][k]
-        const double colj1 = __shfl_sync(FULL, dk, 8 * tig + 4 + sq);       // D[2tig+1][k]
-        const double yk0 = __shfl_sync(FULL, u0, 4 * k + tig);              // Y[k][2tig]
-        const double yk1 = __shfl_sync(FULL, u1, 4 * k + tig);              // Y[k][2tig+1]
-        if (!(piv > 0.0) && fail == 0) fail = k + 1;
-        const double inv = rsqrt(piv);
-        const double lg = colg * inv;
-        const double mg = lg * inv;
-        if (g == k) invrow = inv;
-        if (g > k) {
-            if (2 * tig > k) d0 = fma(-lg, colj0 * inv, d0);
-            if (2 * tig + 1 > k) d1 = fma(-lg, colj1 * inv, d1);
-            if (2 * tig <= k) u0 = fma(-mg, yk0, u0);
-            if (2 * tig + 1 <= k) u1 = fma(-mg, yk1, u1);
-        }
-        if (sq == tig) {
-            if (k & 1) d1 = g >= k ? lg : 0.0;
-            else d0 = g >= k ? lg : 0.0;
-        }
-    }
-    y0 = u0 * invrow;
-    y1 = u1 * invrow;
-    return fail;
-}
-
-// B fragment of the panel solve from the packed block P (L below the diagonal, W' = L with inverted diagonal tiles,
-// transposed and shifted by one column, above it); conflict free, see chol_solve.cu
-__device__ __forceinline__ double wfrag(const double* P, int kb, int nb, int h, int g, int tig) {
-    const double v = P[(8 * kb + 2 * tig + h) * LDQ + 8 * nb + g + 1];
-    return (nb == kb && 2 * tig + h > g) ? 0.0 : v;
-}
-
-__device__ __forceinline__ void tma_load_2d(void* smem_dst, const void* tmap, int c0, int c1, uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1), "r"(smem_u32(bar))
-        : "memory");
-}
-// generic-proxy global writes (the factor) must be visible to later async-proxy (TMA) reads, here and in the peers
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 __device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release;" ::: "memory"); }
 __device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire;" ::: "memory"); }
 
@@ -140,7 +83,7 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
     const int N = p.n_assets;
     const int ld = p.ldS;
     const int Nr = (N + NB - 1) / NB * NB;
-    const int R = chol_rhs_row(N);             // row index of the right-hand side (see chol_solve.cu)
+    const int R = chol_rhs_row(N);             // row index of the right-hand side
     const int rows_end = max(Nr, R + 8);       // the panels cover rows j0 .. rows_end-1
     const int rowsS = (int)(p.win_stride / ld);
     const int stride = max(p.w_stride, 1);
@@ -148,15 +91,7 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
     double* zs = reinterpret_cast<double*>(stage_mem);   // [NRHS][Nr]
     double* xsol = zs + NRHS * Nr;                        // [NRHS][Nr]
 
-    if (tid == 0) {
-        tma_prefetch_desc(&smap);
-        for (int s = 0; s < CC_STAGES; ++s) {
-            mbar_init(&full_bar[s], 1);
-            mbar_init(&empty_bar[s], CC_WARPS);
-        }
-        fence_barrier_init();
-        fence_proxy_async();
-    }
+    if (tid == 0) init_tma_ring<CC_STAGES, CC_WARPS>(&smap, full_bar, empty_bar);
     __syncthreads();
     int foff[4];
 #pragma unroll
@@ -198,30 +133,10 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
                 if (tid == 0)
                     for (int c = 0; c < CC_STAGES && c < nchunks; ++c) issue(c, it + c);
 
-                // accumulators start as -S (identity rows for the padding), collect +L L': acc = -C
-                double acc[TPW][4][2];
+                double acc[TPW][4][2];     // m-tile i of this warp: row j0 + 32 (q0 + i K) + 8 warp + g
 #pragma unroll
-                for (int i = 0; i < TPW; ++i) {
-                    const int row = j0 + 32 * (q0 + i * K) + 8 * warp + g;
-                    const bool real = i < ni && (row < N || (row >= R && row < R + NRHS));
-#pragma unroll
-                    for (int nt = 0; nt < 4; ++nt) {
-                        const int col = j0 + 8 * nt + 2 * tig;
-                        double2 sv = make_double2(0.0, 0.0);
-                        if (real && col < N) {
-                            if (row < N) sv = *reinterpret_cast<const double2*>(S + (long long)row * ld + col);
-                            else if (NRHS == 2 && row == R + 1) sv = make_double2(1.0, 1.0);
-                            else sv = *reinterpret_cast<const double2*>(rhs + col);     // the right-hand side rides along as row R
-                        }
-                        if (real) {
-                            acc[i][nt][0] = -sv.x;
-                            acc[i][nt][1] = col + 1 < N ? -sv.y : 0.0;
-                        } else {
-                            acc[i][nt][0] = row == col ? -1.0 : 0.0;
-                            acc[i][nt][1] = row == col + 1 ? -1.0 : 0.0;
-                        }
-                    }
-                }
+                for (int i = 0; i < TPW; ++i)
+                    tile_start<NRHS, false>(acc[i], j0 + 32 * (q0 + i * K) + 8 * warp + g, i < ni, S, ld, rhs, N, R, j0, tig);
 
                 for (int c = 0; c < nchunks; ++c, ++it) {
                     const int stage = it % CC_STAGES;
@@ -248,105 +163,33 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
                     if (tid == 0 && c + CC_STAGES < nchunks) issue(c + CC_STAGES, it + CC_STAGES);
                 }
 
-                // padding: rows N..rows_end-1 other than the right-hand sides, and columns >= N, hold no data;
-                // whatever the update accumulated there is replaced by the identity (zero for the rows of S, a unit
-                // diagonal for a right-hand-side row R < Nr in the diagonal block of the last panel)
                 if (j0 + 32 * (q0 + (nboxes - 1) * K) + 32 > N || j0 + NB > N) {
 #pragma unroll
-                    for (int i = 0; i < TPW; ++i) {
-                        const int row = j0 + 32 * (q0 + i * K) + 8 * warp + g;
-                        const bool real = row < N || (row >= R && row < R + NRHS);
-#pragma unroll
-                        for (int nt = 0; nt < 4; ++nt) {
-                            const int col = j0 + 8 * nt + 2 * tig;
-                            if (!real || col >= N) acc[i][nt][0] = row == col ? -1.0 : 0.0;
-                            if (!real || col + 1 >= N) acc[i][nt][1] = row == col + 1 ? -1.0 : 0.0;
-                        }
-                    }
+                    for (int i = 0; i < TPW; ++i)
+                        tile_fix_padding<NRHS>(acc[i], j0 + 32 * (q0 + i * K) + 8 * warp + g, N, R, j0, tig);
                 }
 
                 if (q0 == 0) {
-                    // ---------------- F: 32x32 diagonal block in fragment space (this CTA owns the diagonal group)
-#pragma unroll
-                    for (int cb = 0; cb < NB / 8; ++cb) {
-                        if (warp == cb) {
-                            double d0 = -acc[0][cb][0], d1 = -acc[0][cb][1], y0, y1;
-                            const int f = potrf8_inv8(d0, d1, y0, y1, g, tig, lane);
-                            // tiles from row N on: padding and right-hand sides, no pivots of S (see chol_solve.cu)
-                            if (lane == 0 && f != 0 && fail_s == 0 && j0 + 8 * cb < N) fail_s = j0 + 8 * cb + f;
-                            double* row = P + (8 * cb + g) * LDQ + 8 * cb + 2 * tig;
-                            if (2 * tig <= g) row[0] = d0;
-                            if (2 * tig + 1 <= g) row[1] = d1;
-                            if (2 * tig <= g) P[(8 * cb + 2 * tig) * LDQ + 8 * cb + g + 1] = y0;
-                            if (2 * tig + 1 <= g) P[(8 * cb + 2 * tig + 1) * LDQ + 8 * cb + g + 1] = y1;
-                        }
-                        __syncthreads();
-                        if (cb == NB / 8 - 1) break;
-                        if (warp > cb && warp < NB / 8) {
-                            double x0 = 0.0, x1 = 0.0;
-#pragma unroll
-                            for (int h = 0; h < 2; ++h) dmma884(x0, x1, acc[0][cb][h], wfrag(P, cb, cb, h, g, tig));
-                            x0 = -x0;
-                            x1 = -x1;
-                            acc[0][cb][0] = x0;      // this tile now holds +L
-                            acc[0][cb][1] = x1;
-                            double* row = P + (8 * warp + g) * LDQ + 8 * cb + 2 * tig;
-                            row[0] = x0;
-                            row[1] = x1;
-                            P[(8 * cb + 2 * tig) * LDQ + 8 * warp + g + 1] = x0;
-                            P[(8 * cb + 2 * tig + 1) * LDQ + 8 * warp + g + 1] = x1;
-                        }
-                        __syncthreads();
-                        if (warp > cb && warp < NB / 8) {
-#pragma unroll
-                            for (int nb = cb + 1; nb < NB / 8; ++nb)
-                                if (nb <= warp) {
-#pragma unroll
-                                    for (int h = 0; h < 2; ++h)
-                                        dmma884(acc[0][nb][0], acc[0][nb][1], acc[0][cb][h], wfrag(P, cb, nb, h, g, tig));
-                                }
-                        }
-                    }
-                    // push the packed block to the peers, then barrier A; write L_d back (lower part, real rows only:
-                    // in the last panel z of a right-hand side R < Nr)
+                    // ---------------- F (this CTA owns the diagonal group), packed block pushed to the peers, barrier A
+                    factor_diag_block(acc[0], P, fail_s, j0, N, warp, lane);
                     for (int peer = 0; peer < K; ++peer) {
                         if (peer == rank) continue;
                         double* dst = cluster.map_shared_rank(P, peer);
                         for (int e = tid; e < NB * LDQ; e += CC_THREADS) dst[e] = P[e];
                     }
                     cluster_arrive();
-                    for (int i = warp; i < NB; i += CC_WARPS) {
-                        const int row = j0 + i, col = j0 + lane;
-                        if ((row < N || (row >= R && row < R + NRHS)) && col < N && lane <= i)
-                            S[(long long)row * ld + col] = P[i * LDQ + lane];
-                    }
+                    store_diag_block<NRHS, CC_WARPS>(S, ld, P, j0, N, R, warp, lane);
                 }
                 if (!waitedA) {
                     cluster_wait();
                     waitedA = true;
                 }
-                // ---------------- T: X = C inv(L_d)' straight from the accumulators (block forward substitution)
+                // ---------------- T: the groups below the diagonal one
 #pragma unroll
                 for (int i = 0; i < TPW; ++i) {
                     const int q = q0 + i * K;                     // group index within the panel
                     if (i >= ni || q == 0) continue;
-                    const int row = j0 + 32 * q + 8 * warp + g;
-                    const bool real = row < N || (row >= R && row < R + NRHS);
-#pragma unroll
-                    for (int cb = 0; cb < NB / 8; ++cb) {
-                        double x0 = 0.0, x1 = 0.0;
-#pragma unroll
-                        for (int h = 0; h < 2; ++h) dmma884(x0, x1, acc[i][cb][h], wfrag(P, cb, cb, h, g, tig));
-                        x0 = -x0;
-                        x1 = -x1;
-                        const int col = j0 + 8 * cb + 2 * tig;
-                        if (real && col < N) *reinterpret_cast<double2*>(S + (long long)row * ld + col) = make_double2(x0, x1);
-#pragma unroll
-                        for (int nb = cb + 1; nb < NB / 8; ++nb) {
-                            dmma884(acc[i][nb][0], acc[i][nb][1], x0, wfrag(P, cb, nb, 0, g, tig));
-                            dmma884(acc[i][nb][0], acc[i][nb][1], x1, wfrag(P, cb, nb, 1, g, tig));
-                        }
-                    }
+                    tile_solve<NRHS>(acc[i], P, S, ld, j0 + 32 * q + 8 * warp + g, N, R, j0, g, tig);
                 }
             }
             if (!waitedA) cluster_wait();       // a CTA without groups in this panel
@@ -356,73 +199,26 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
             fence_proxy_async_all();
         }
 
-        // ---------------- z = L^-1 b sits in row R (+r);  v1 = z'z = w1' S1 w1   (:574)
-        double zz = 0.0;
-        for (int j = tid; j < Nr; j += CC_THREADS) {
-            const double z = j < N ? S[(long long)R * ld + j] : 0.0;
-            zs[j] = z;
-            zz = fma(z, z, zz);
-            if constexpr (NRHS == 2) zs[Nr + j] = j < N ? S[(long long)(R + 1) * ld + j] : 0.0;
-        }
-        const double v1 = block_sum(zz, scratch);
+        const double v1 = load_z<NRHS, CC_THREADS>(zs, S, ld, N, Nr, R, scratch);
 
-        // ---------------- back substitution L' x = z, right-looking over 32-column blocks (block b: CTA b mod K)
+        // ---------------- back substitution, right-looking over 32-column blocks (block b: CTA b mod K)
         const int nblk = Nr / NB;
-        auto load_diag = [&](int b) {
-            const int j0 = NB * b;
-            for (int i = warp; i < NB; i += CC_WARPS) {
-                const int row = j0 + i, col = j0 + lane;
-                double v;
-                if (row < N && col < N) v = lane <= i ? S[(long long)row * ld + col] : 0.0;
-                else v = i == lane ? 1.0 : 0.0;
-                P[i * LDQ + lane] = v;
-            }
-        };
-        if (rank == (nblk - 1) % K) load_diag(nblk - 1);
+        if (rank == (nblk - 1) % K) load_diag_block<CC_WARPS>(P, S, ld, nblk - 1, N, warp, lane);
         for (int b = nblk - 1; b >= 0; --b) {
             const int j0 = NB * b;
             if (rank == b % K) {
                 __syncthreads();                              // P and the running right-hand side are complete
                 if (warp < NRHS) {
-                    double r = zs[warp * Nr + j0 + lane];
-                    const double rd = 1.0 / P[lane * LDQ + lane];
-#pragma unroll
-                    for (int k = NB - 1; k >= 0; --k) {
-                        const double xk = __shfl_sync(0xffffffffu, r * rd, k);
-                        if (lane == k) r = xk;
-                        if (lane < k) r = fma(-P[k * LDQ + lane], xk, r);
-                    }
+                    const double r = solve_diag_block(zs[warp * Nr + j0 + lane], P, lane);
                     for (int peer = 0; peer < K; ++peer) cluster.map_shared_rank(xsol, peer)[warp * Nr + j0 + lane] = r;
                 }
                 if (K == 1) __syncthreads();                  // the same CTA refills P below
             }
-            if (b > 0 && rank == (b - 1) % K) load_diag(b - 1);     // ahead of the barrier: independent of x_b
+            if (b > 0 && rank == (b - 1) % K) load_diag_block<CC_WARPS>(P, S, ld, b - 1, N, warp, lane);   // ahead of the barrier: independent of x_b
             cluster_arrive();
             cluster_wait();
-            // my blocks bb < b: z_bb -= L[rows of b, columns of bb]' x_b, one warp per block
-            for (int bb = rank + K * warp; bb < b; bb += K * CC_WARPS) {
-                const int col = NB * bb + lane;
-                double a0[NRHS], a1[NRHS];
-#pragma unroll
-                for (int r = 0; r < NRHS; ++r) a0[r] = a1[r] = 0.0;
-                const int rows = min(NB, N - j0);
-#pragma unroll 4
-                for (int i = 0; i + 1 < rows; i += 2) {
-                    const double l0 = S[(long long)(j0 + i) * ld + col], l1 = S[(long long)(j0 + i + 1) * ld + col];
-#pragma unroll
-                    for (int r = 0; r < NRHS; ++r) {
-                        a0[r] = fma(l0, xsol[r * Nr + j0 + i], a0[r]);
-                        a1[r] = fma(l1, xsol[r * Nr + j0 + i + 1], a1[r]);
-                    }
-                }
-                if (rows & 1) {
-                    const double l0 = S[(long long)(j0 + rows - 1) * ld + col];
-#pragma unroll
-                    for (int r = 0; r < NRHS; ++r) a0[r] = fma(l0, xsol[r * Nr + j0 + rows - 1], a0[r]);
-                }
-#pragma unroll
-                for (int r = 0; r < NRHS; ++r) zs[r * Nr + col] -= a0[r] + a1[r];
-            }
+            // my blocks bb < b, one warp per block
+            for (int bb = rank + K * warp; bb < b; bb += K * CC_WARPS) reduce_block<NRHS>(zs, xsol, S, ld, Nr, N, b, NB * bb + lane);
         }
         // every CTA reports its first failing pivot to rank 0
         if (tid == 0) cluster.map_shared_rank(fail_all, 0)[rank] = fail_s;
@@ -431,59 +227,11 @@ chol_cluster_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams 
 
         // ---------------- posterior scalars and weights (rank 0; its xsol holds the whole solution)
         if (rank == 0) {
-            double* scal = p.scal + (long long)w * BP_S_COUNT;
-            if constexpr (NRHS == 2) {
-                // Jorion's Bayes-Stein estimator (:851-895) from y = C^-1 t and z = C^-1 1: see jorion_math.cuh
-                const double* y = xsol;
-                const double* z = xsol + Nr;
-                double sy = 0.0, sz = 0.0, ty = 0.0;
-                for (int j = tid; j < N; j += CC_THREADS) {
-                    sy += y[j];
-                    sz += z[j];
-                    ty = fma(rhs[j], y[j], ty);
-                }
-                sy = block_sum(sy, scratch);
-                sz = block_sum(sz, scratch);
-                ty = block_sum(ty, scratch);
-                const JorionCoef jc = jorion_coefficients(sy, sz, ty, (double)p.n_returns, (double)N);
-                for (int j = tid; j < p.ldv; j += CC_THREADS) {
-                    double yj = 0.0, nu = 0.0;
-                    if (j < N) {
-                        yj = y[j];
-                        nu = jc.c_y * yj + jc.c_z * z[j];
-                    }
-                    p.w1[(long long)w * p.ldv + j] = yj;
-                    p.nu[(long long)w * p.ldv + j] = nu;
-                    p.weights[(long long)w * p.ldv + j] = p.inv_gamma * nu;
-                }
-                if (tid == 0) {
-                    scal[BP_S_JORION_MU_G] = jc.mu_g;
-                    scal[BP_S_JORION_LAMBDA] = jc.lambda;
-                    scal[BP_S_JORION_V] = jc.v;
-                    scal[BP_S_JORION_Q] = jc.q;
-                    scal[BP_S_JORION_ONE_VINV_ONE] = jc.one_vinv_one;
-                }
-            } else {
-                double mult = 1.0;
-                if (p.mode == BP_MODE_CONJUGATE) {
-                    const double n1 = scal[BP_S_N1];
-                    mult = (n1 + (double)N + 2.0) / (n1 - v1);
-                }
-                for (int j = tid; j < p.ldv; j += CC_THREADS) {
-                    const double wv = j < N ? xsol[j] : 0.0;
-                    const double nu = p.mode == BP_MODE_CONJUGATE ? (wv * mult) : wv;
-                    p.w1[(long long)w * p.ldv + j] = wv;
-                    p.nu[(long long)w * p.ldv + j] = nu;
-                    p.weights[(long long)w * p.ldv + j] = p.inv_gamma * nu;
-                }
-            }
-            if (tid == 0) {
-                int f = 0;
+            int f = 0;       // the window's status: the first failing pivot over the ranks (written by thread 0)
+            if (tid == 0)
                 for (int r = 0; r < K; ++r)
                     if (fail_all[r] != 0 && (f == 0 || fail_all[r] < f)) f = fail_all[r];
-                scal[BP_S_V1] = v1;
-                p.status[w] = f;
-            }
+            write_outputs<NRHS, CC_THREADS>(p, w, xsol, Nr, v1, f, scratch);
         }
         __syncthreads();       // zs / xsol / fail_s are reused by the next window
     }

@@ -35,6 +35,8 @@
 // the right-hand-side row then sits in the diagonal block, where it is solved by F and keeps an
 // identity entry in its own padding column.  The back substitution then walks the panels in reverse
 // with coalesced row reads and a warp-level triangular solve.
+// The arithmetic of U's start and padding, F, T, the back substitution and the epilogue is the shared code of
+// chol_panel.cuh, so that chol_cluster_kernel gives the same bits; this file holds the slab schedule.
 //
 // k-permutation: inside a 16-column chunk, DMMA step q contracts columns {2q, 2q+1, 8+2q, 9+2q}
 // over the four tig lanes.  With the 128-byte swizzle (16-byte unit index XOR row&7) the 16 lanes of
@@ -43,13 +45,11 @@
 #include <cstdio>
 #include <cstdlib>
 
-#include "common.cuh"
-#include "jorion_math.cuh"
-#include "kernels.h"
+#include "chol_panel.cuh"
 
 namespace bp {
 
-constexpr int NB = 32;
+using namespace chol;
 
 #ifndef CH_NWARPS
 #define CH_NWARPS 4
@@ -61,61 +61,6 @@ constexpr int CH_WARPS = CH_NWARPS;                 // warps per window (CTA)
 constexpr int CH_OCC = CH_CTAS_PER_SM;              // resident CTAs (windows) per SM
 constexpr int CH_THREADS = CH_WARPS * 32;
 
-constexpr int LDQ = 34;    // row stride of the packed diagonal-block array
-
-// Cholesky factor AND inverse of one 8x8 diagonal tile, by one warp, entirely in registers.
-// The tile is in DMMA accumulator layout: lane (g,tig) holds D[g][2tig], D[g][2tig+1] (lower part valid).
-// On return d0/d1 hold L (zero above the diagonal) and y0/y1 inv(L), same layout.  Eight steps, each one
-// round of shuffles (pivot, own-row and own-column entries of column k, row k of the inverse) and a
-// handful of FMAs -- the 32-step shared-memory loop this replaces cost 170 instructions per warp and step
-// and was a third of the kernel.  Inverse: with Y[i][j] = inv(L)[i][j] L[i][i], Y[i][j] -= (D[i][k]/piv) Y[k][j]
-// for j <= k < i; the row scaling is applied at the end.  Returns the 1-based index of the first
-// non-positive pivot, or 0.
-__device__ __forceinline__ int potrf8_inv8(double& d0, double& d1, double& y0, double& y1, int g, int tig, int lane) {
-    constexpr unsigned FULL = 0xffffffffu;
-    int fail = 0;
-    double u0 = 2 * tig == g ? 1.0 : 0.0, u1 = 2 * tig + 1 == g ? 1.0 : 0.0;
-    double invrow = 0.0;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        const double dk = (k & 1) ? d1 : d0;
-        const int sq = k >> 1;
-        const double piv = __shfl_sync(FULL, dk, 4 * k + sq);               // D[k][k]
-        const double colg = __shfl_sync(FULL, dk, (lane & ~3) | sq);        // D[g][k]
-        const double colj0 = __shfl_sync(FULL, dk, 8 * tig + sq);           // D[2tig][k]
-        const double colj1 = __shfl_sync(FULL, dk, 8 * tig + 4 + sq);       // D[2tig+1][k]
-        const double yk0 = __shfl_sync(FULL, u0, 4 * k + tig);              // Y[k][2tig]
-        const double yk1 = __shfl_sync(FULL, u1, 4 * k + tig);              // Y[k][2tig+1]
-        if (!(piv > 0.0) && fail == 0) fail = k + 1;
-        const double inv = rsqrt(piv);
-        const double lg = colg * inv;
-        const double mg = lg * inv;
-        if (g == k) invrow = inv;
-        if (g > k) {
-            if (2 * tig > k) d0 = fma(-lg, colj0 * inv, d0);
-            if (2 * tig + 1 > k) d1 = fma(-lg, colj1 * inv, d1);
-            if (2 * tig <= k) u0 = fma(-mg, yk0, u0);
-            if (2 * tig + 1 <= k) u1 = fma(-mg, yk1, u1);
-        }
-        if (sq == tig) {
-            if (k & 1) d1 = g >= k ? lg : 0.0;
-            else d0 = g >= k ? lg : 0.0;
-        }
-    }
-    y0 = u0 * invrow;
-    y1 = u1 * invrow;
-    return fail;
-}
-
-// B fragment of the panel solve: with W = L_d whose 8x8 diagonal tiles are replaced by their inverses,
-// W[8nb+n][8kb+k] sits TRANSPOSED and shifted by one column in the strictly upper part of P, at
-// P[(8kb+k)*LDQ + 8nb+n+1]; lanes (g,tig) read 8-byte bank (4 tig + g + const) mod 16: conflict free.
-// Inside a diagonal tile the entries above the diagonal (k > n) are zero (that spot holds L itself).
-__device__ __forceinline__ double wfrag(const double* P, int kb, int nb, int h, int g, int tig) {
-    const double v = P[(8 * kb + 2 * tig + h) * LDQ + 8 * nb + g + 1];
-    return (nb == kb && 2 * tig + h > g) ? 0.0 : v;
-}
-
 #ifndef CH_TPW
 #define CH_TPW 2                                     // m-tiles per warp and slab
 #endif
@@ -126,18 +71,8 @@ constexpr int TPW = CH_TPW;
 constexpr int SLAB_TILES = CH_WARPS * TPW;           // m-tiles per slab (one pass of the panel update)
 constexpr int ABOXES = SLAB_TILES / 4;               // 32-row TMA boxes per slab
 constexpr int CH_STAGES = CH_NSTAGES;
-constexpr int BOX_BYTES = 32 * 16 * 8;               // one TMA box: 32 rows x 16 columns of doubles
 constexpr int CH_STAGE_BYTES = (ABOXES + 1) * BOX_BYTES;   // A slab + 1 B box
 constexpr int CH_TMA_SMEM = CH_STAGES * CH_STAGE_BYTES + 1024;
-
-__device__ __forceinline__ void tma_load_2d(void* smem_dst, const void* tmap, int c0, int c1, uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(c0), "r"(c1), "r"(smem_u32(bar))
-        : "memory");
-}
-// generic-proxy global writes (the factor) must be visible to later async-proxy (TMA) reads
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 
 // NRHS = 1: the posterior solves of the conjugate / Jeffreys path.  NRHS = 2 (Jorion, :851-895): a second
 // right-hand side (the vector of ones) rides along as row R+1, so that both C^-1 t and C^-1 1 come out of ONE
@@ -165,15 +100,7 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
     const int rows_end = max(Nr, R + 8);       // the panels cover rows j0 .. rows_end-1
     const int rowsS = (int)(p.win_stride / ld);
 
-    if (tid == 0) {
-        tma_prefetch_desc(&smap);
-        for (int s = 0; s < CH_STAGES; ++s) {
-            mbar_init(&full_bar[s], 1);
-            mbar_init(&empty_bar[s], CH_WARPS);
-        }
-        fence_barrier_init();
-        fence_proxy_async();
-    }
+    if (tid == 0) init_tma_ring<CH_STAGES, CH_WARPS>(&smap, full_bar, empty_bar);
     __syncthreads();
     // per-lane fragment offsets inside a [32][16] swizzled box: row r = 8*t + g, DMMA step q reads column
     // c = 2q + (tig&1) + 8*(tig>>1): 16-byte unit (q + 4*(tig>>1)) ^ g, 8-byte half tig&1
@@ -197,6 +124,7 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
         const double* rhs = p.rhs + (long long)w * p.ldv;
         const int grow0 = w * rowsS;           // first row of this window in the tensor map
         if (tid == 0) fail_s = 0;
+        // the right-hand side(s) ride along as rows R (, R+1) of S
         for (int j = tid; j < ld; j += CH_THREADS) S[(long long)R * ld + j] = j < N ? rhs[j] : 0.0;
         if constexpr (NRHS == 2)
             for (int j = tid; j < ld; j += CH_THREADS) S[(long long)(R + 1) * ld + j] = j < N ? 1.0 : 0.0;
@@ -228,26 +156,10 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
                 if (tid == 0)
                     for (int c = 0; c < CH_STAGES && c < nchunks; ++c) issue(c, it + c);
 
-                // accumulators start as -S (identity rows for the padding), collect +L L': acc = -C
-                double acc[TPW][4][2];
+                double acc[TPW][4][2];     // m-tile i of this warp: row j0 + 8 (slab0 + warp + CH_WARPS i) + g
 #pragma unroll
-                for (int i = 0; i < TPW; ++i) {
-                    const int row = j0 + 8 * (slab0 + warp + CH_WARPS * i) + g;
-                    const bool real = i < ni && (row < N || (row >= R && row < R + NRHS));
-#pragma unroll
-                    for (int nt = 0; nt < 4; ++nt) {
-                        const int col = j0 + 8 * nt + 2 * tig;
-                        double2 sv = make_double2(0.0, 0.0);
-                        if (real && col < N) sv = *reinterpret_cast<const double2*>(S + (long long)row * ld + col);
-                        if (real) {
-                            acc[i][nt][0] = -sv.x;
-                            acc[i][nt][1] = col + 1 < N ? -sv.y : 0.0;
-                        } else {
-                            acc[i][nt][0] = row == col ? -1.0 : 0.0;
-                            acc[i][nt][1] = row == col + 1 ? -1.0 : 0.0;
-                        }
-                    }
-                }
+                for (int i = 0; i < TPW; ++i)
+                    tile_start<NRHS, true>(acc[i], j0 + 8 * (slab0 + warp + CH_WARPS * i) + g, i < ni, S, ld, rhs, N, R, j0, tig);
 
                 for (int c = 0; c < nchunks; ++c, ++it) {
                     const int stage = it % CH_STAGES;
@@ -296,103 +208,25 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
                     if (tid == 0 && c + CH_STAGES < nchunks) issue(c + CH_STAGES, it + CH_STAGES);
                 }
 
-                // padding: rows N..rows_end-1 other than the right-hand sides, and columns >= N, hold no data;
-                // whatever the update accumulated there is replaced by the identity.  In a padding column that is
-                // zero for the rows of S and a unit diagonal for a right-hand-side row R < Nr, which sits in the
-                // diagonal block of the last panel: its pivot must not be zero
                 if (slab_row + 8 * slab_tiles > N || j0 + NB > N) {
 #pragma unroll
-                    for (int i = 0; i < TPW; ++i) {
-                        const int row = j0 + 8 * (slab0 + warp + CH_WARPS * i) + g;
-                        const bool real = row < N || (row >= R && row < R + NRHS);
-#pragma unroll
-                        for (int nt = 0; nt < 4; ++nt) {
-                            const int col = j0 + 8 * nt + 2 * tig;
-                            if (!real || col >= N) acc[i][nt][0] = row == col ? -1.0 : 0.0;
-                            if (!real || col + 1 >= N) acc[i][nt][1] = row == col + 1 ? -1.0 : 0.0;
-                        }
-                    }
+                    for (int i = 0; i < TPW; ++i)
+                        tile_fix_padding<NRHS>(acc[i], j0 + 8 * (slab0 + warp + CH_WARPS * i) + g, N, R, j0, tig);
                 }
 
                 if (slab0 == 0) {
-                    // ---------------- F: 32x32 diagonal block, blocked by 8 in fragment space.  Warp q < 4 holds
-                    // row block q (acc[0][0..3] = -C).  Column block cb: warp cb factors and inverts its 8x8
-                    // tile in registers; the warps below solve their tile against it (2 DMMAs) and update their
-                    // remaining tiles (2 DMMAs each); L goes to the lower part of P, W' to the upper part.
+                    // ---------------- F: warp q < 4 holds row block q of the diagonal block in acc[0]
                     PROF(0)
-#pragma unroll
-                    for (int cb = 0; cb < NB / 8; ++cb) {
-                        if (warp == cb) {
-                            double d0 = -acc[0][cb][0], d1 = -acc[0][cb][1], y0, y1;
-                            const int f = potrf8_inv8(d0, d1, y0, y1, g, tig, lane);
-                            // a tile from row N on holds padding and right-hand sides, whose pivots are none of S's
-                            // (a right-hand side's is 1 - |its z in this panel|^2 and may be negative)
-                            if (lane == 0 && f != 0 && fail_s == 0 && j0 + 8 * cb < N) fail_s = j0 + 8 * cb + f;
-                            double* row = P + (8 * cb + g) * LDQ + 8 * cb + 2 * tig;
-                            if (2 * tig <= g) row[0] = d0;
-                            if (2 * tig + 1 <= g) row[1] = d1;
-                            if (2 * tig <= g) P[(8 * cb + 2 * tig) * LDQ + 8 * cb + g + 1] = y0;
-                            if (2 * tig + 1 <= g) P[(8 * cb + 2 * tig + 1) * LDQ + 8 * cb + g + 1] = y1;
-                        }
-                        __syncthreads();
-                        if (cb == NB / 8 - 1) break;
-                        if (warp > cb && warp < NB / 8) {
-                            double x0 = 0.0, x1 = 0.0;
-#pragma unroll
-                            for (int h = 0; h < 2; ++h) dmma884(x0, x1, acc[0][cb][h], wfrag(P, cb, cb, h, g, tig));
-                            x0 = -x0;
-                            x1 = -x1;
-                            acc[0][cb][0] = x0;      // this tile now holds +L
-                            acc[0][cb][1] = x1;
-                            double* row = P + (8 * warp + g) * LDQ + 8 * cb + 2 * tig;
-                            row[0] = x0;
-                            row[1] = x1;
-                            P[(8 * cb + 2 * tig) * LDQ + 8 * warp + g + 1] = x0;
-                            P[(8 * cb + 2 * tig + 1) * LDQ + 8 * warp + g + 1] = x1;
-                        }
-                        __syncthreads();
-                        if (warp > cb && warp < NB / 8) {
-#pragma unroll
-                            for (int nb = cb + 1; nb < NB / 8; ++nb)
-                                if (nb <= warp) {
-#pragma unroll
-                                    for (int h = 0; h < 2; ++h)
-                                        dmma884(acc[0][nb][0], acc[0][nb][1], acc[0][cb][h], wfrag(P, cb, nb, h, g, tig));
-                                }
-                        }
-                    }
+                    factor_diag_block(acc[0], P, fail_s, j0, N, warp, lane);
                     PROF(1)
-                    // write L_d back (lower part, real rows only: in the last panel z of a right-hand side R < Nr)
-                    for (int i = warp; i < NB; i += CH_WARPS) {
-                        const int row = j0 + i, col = j0 + lane;
-                        if ((row < N || (row >= R && row < R + NRHS)) && col < N && lane <= i)
-                            S[(long long)row * ld + col] = P[i * LDQ + lane];
-                    }
+                    store_diag_block<NRHS, CH_WARPS>(S, ld, P, j0, N, R, warp, lane);
                 }
-                // ---------------- T: X = C inv(L_d)' straight from the accumulators, by block forward substitution
-                // with W: X_cb = C_cb inv(L_cb,cb)', C_nb -= X_cb L_nb,cb' (nb > cb).  DMMA step h contracts the
-                // columns 8cb+2tig+h the lanes already hold, so the accumulators are used as A fragments as they are.
+                // ---------------- T: the m-tiles below the diagonal block
 #pragma unroll
                 for (int i = 0; i < TPW; ++i) {
                     const int q = slab0 + warp + CH_WARPS * i;     // m-tile index within the panel
                     if (i >= ni || q < NB / 8) continue;
-                    const int row = j0 + 8 * q + g;
-                    const bool real = row < N || (row >= R && row < R + NRHS);
-#pragma unroll
-                    for (int cb = 0; cb < NB / 8; ++cb) {
-                        double x0 = 0.0, x1 = 0.0;
-#pragma unroll
-                        for (int h = 0; h < 2; ++h) dmma884(x0, x1, acc[i][cb][h], wfrag(P, cb, cb, h, g, tig));
-                        x0 = -x0;
-                        x1 = -x1;
-                        const int col = j0 + 8 * cb + 2 * tig;
-                        if (real && col < N) *reinterpret_cast<double2*>(S + (long long)row * ld + col) = make_double2(x0, x1);
-#pragma unroll
-                        for (int nb = cb + 1; nb < NB / 8; ++nb) {
-                            dmma884(acc[i][nb][0], acc[i][nb][1], x0, wfrag(P, cb, nb, 0, g, tig));
-                            dmma884(acc[i][nb][0], acc[i][nb][1], x1, wfrag(P, cb, nb, 1, g, tig));
-                        }
-                    }
+                    tile_solve<NRHS>(acc[i], P, S, ld, j0 + 8 * q + g, N, R, j0, g, tig);
                 }
             }
             fence_proxy_async_all();        // the factor written above is read by TMA in the next panels
@@ -400,120 +234,23 @@ chol_solve_kernel(const __grid_constant__ CUtensorMap smap, const SolveParams p)
             PROF(2)
         }
 
-        // ---------------- z = L^-1 b sits in row R (+r);  v1 = z'z = w1' S1 w1   (:574)
-        double zz = 0.0;
-        for (int j = tid; j < Nr; j += CH_THREADS) {
-            const double z = j < N ? S[(long long)R * ld + j] : 0.0;
-            xs[j] = z;
-            zz = fma(z, z, zz);
-            if constexpr (NRHS == 2) xs[Nr + j] = j < N ? S[(long long)(R + 1) * ld + j] : 0.0;
-        }
-        const double v1 = block_sum(zz, scratch);
+        const double v1 = load_z<NRHS, CH_THREADS>(xs, S, ld, N, Nr, R, scratch);
 
-        // ---------------- back substitution  L' x = z, right-looking over 32-column blocks, in place in xs: block b is
-        // solved (warp r finishes right-hand side r), then every block bb < b is reduced by L[rows of b, columns of bb]' x_b
-        // (one warp per block, coalesced rows).  Operation for operation the arithmetic of chol_cluster.cu, so that a
-        // batch gives bit-identical weights however its windows are split over launches and kernels.
+        // ---------------- back substitution, in place in xs
         for (int b = Nr / NB - 1; b >= 0; --b) {
-            const int j0 = NB * b;
-            for (int i = warp; i < NB; i += CH_WARPS) {
-                const int row = j0 + i, col = j0 + lane;
-                double v;
-                if (row < N && col < N) v = lane <= i ? S[(long long)row * ld + col] : 0.0;
-                else v = i == lane ? 1.0 : 0.0;
-                P[i * LDQ + lane] = v;
-            }
+            load_diag_block<CH_WARPS>(P, S, ld, b, N, warp, lane);
             __syncthreads();
             if (warp < NRHS) {
-                double r = xs[warp * Nr + j0 + lane];
-                const double rd = 1.0 / P[lane * LDQ + lane];      // all 32 reciprocals in parallel
-#pragma unroll
-                for (int k = NB - 1; k >= 0; --k) {
-                    const double xk = __shfl_sync(0xffffffffu, r * rd, k);
-                    if (lane == k) r = xk;
-                    if (lane < k) r = fma(-P[k * LDQ + lane], xk, r);
-                }
-                xs[warp * Nr + j0 + lane] = r;
+                double* x = xs + warp * Nr + NB * b + lane;
+                *x = solve_diag_block(*x, P, lane);
             }
             __syncthreads();
-            const int rows = min(NB, N - j0);
-            for (int bb = warp; bb < b; bb += CH_WARPS) {
-                const int col = NB * bb + lane;
-                double a0[NRHS], a1[NRHS];
-#pragma unroll
-                for (int r = 0; r < NRHS; ++r) a0[r] = a1[r] = 0.0;
-#pragma unroll 4
-                for (int i = 0; i + 1 < rows; i += 2) {
-                    const double l0 = S[(long long)(j0 + i) * ld + col], l1 = S[(long long)(j0 + i + 1) * ld + col];
-#pragma unroll
-                    for (int r = 0; r < NRHS; ++r) {
-                        a0[r] = fma(l0, xs[r * Nr + j0 + i], a0[r]);
-                        a1[r] = fma(l1, xs[r * Nr + j0 + i + 1], a1[r]);
-                    }
-                }
-                if (rows & 1) {
-                    const double l0 = S[(long long)(j0 + rows - 1) * ld + col];
-#pragma unroll
-                    for (int r = 0; r < NRHS; ++r) a0[r] = fma(l0, xs[r * Nr + j0 + rows - 1], a0[r]);
-                }
-#pragma unroll
-                for (int r = 0; r < NRHS; ++r) xs[r * Nr + col] -= a0[r] + a1[r];
-            }
+            for (int bb = warp; bb < b; bb += CH_WARPS) reduce_block<NRHS>(xs, xs, S, ld, Nr, N, b, NB * bb + lane);
         }
         __syncthreads();
 
         PROF(3)
-        // ---------------- posterior scalars and weights
-        double* scal = p.scal + (long long)w * BP_S_COUNT;
-        if constexpr (NRHS == 2) {
-            // Jorion's Bayes-Stein estimator (:851-895) from y = C^-1 t and z = C^-1 1: see jorion_math.cuh
-            const double* y = xs;
-            const double* z = xs + Nr;
-            double sy = 0.0, sz = 0.0, ty = 0.0;
-            for (int j = tid; j < N; j += CH_THREADS) {
-                sy += y[j];
-                sz += z[j];
-                ty = fma(rhs[j], y[j], ty);
-            }
-            sy = block_sum(sy, scratch);
-            sz = block_sum(sz, scratch);
-            ty = block_sum(ty, scratch);
-            const JorionCoef jc = jorion_coefficients(sy, sz, ty, (double)p.n_returns, (double)N);
-            for (int j = tid; j < p.ldv; j += CH_THREADS) {
-                double yj = 0.0, nu = 0.0;
-                if (j < N) {
-                    yj = y[j];
-                    nu = jc.c_y * yj + jc.c_z * z[j];
-                }
-                p.w1[(long long)w * p.ldv + j] = yj;
-                p.nu[(long long)w * p.ldv + j] = nu;
-                p.weights[(long long)w * p.ldv + j] = p.inv_gamma * nu;
-            }
-            if (tid == 0) {
-                scal[BP_S_JORION_MU_G] = jc.mu_g;
-                scal[BP_S_JORION_LAMBDA] = jc.lambda;
-                scal[BP_S_JORION_V] = jc.v;
-                scal[BP_S_JORION_Q] = jc.q;
-                scal[BP_S_JORION_ONE_VINV_ONE] = jc.one_vinv_one;
-            }
-        } else {
-        double mult = 1.0;
-        if (p.mode == BP_MODE_CONJUGATE) {
-            const double n1 = scal[BP_S_N1];
-            mult = (n1 + (double)N + 2.0) / (n1 - v1);
-        }
-        for (int j = tid; j < p.ldv; j += CH_THREADS) {
-            const double wv = j < N ? xs[j] : 0.0;
-            const double nu = p.mode == BP_MODE_CONJUGATE ? (wv * mult) : wv;
-            p.w1[(long long)w * p.ldv + j] = wv;
-            p.nu[(long long)w * p.ldv + j] = nu;
-            p.weights[(long long)w * p.ldv + j] = p.inv_gamma * nu;
-        }
-        }
-        if (tid == 0) {
-            scal[BP_S_V1] = v1;
-            p.status[w] = fail_s;
-        }
+        write_outputs<NRHS, CH_THREADS>(p, w, xs, Nr, v1, fail_s, scratch);
         __syncthreads();
         PROF(4)
     }
