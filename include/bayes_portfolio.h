@@ -44,6 +44,18 @@ extern "C" {
 #define BP_SCAL_SUMA 7        /* sum of risk-free adjustments  :48                                   */
 #define BP_SCAL_V1 8          /* w1' S1 w1                     :574                                  */
 #define BP_SCAL_MCM_AVG 9     /* average MCM over the window   :112                                  */
+/* Condition estimate (bp_set_condition_estimate; the solver writes neither slot while it is off), for every window the solver
+ * factorises.  A is the symmetric matrix of the lower triangle the solver factorises: S1 (conjugate), J (Jeffreys),
+ * C (Jorion), C + rho I (shrinkage, after the Ledoit-Wolf rewrite), the caller's S (bp_solve_batched), S1
+ * (bp_dense_posterior).  Windows solved relative to a base window (bp_set_jeffreys_chain) are not factorised: while
+ * the estimate is on, every window is.                                                                           */
+#define BP_SCAL_ANORM1 10     /* max_j sum_i |A_ij|, read before the factorisation overwrites A                   */
+#define BP_SCAL_RCOND 11      /* (1 / est) / anorm1, est = dlacn2's estimate of ||A^-1||_1 (Hager-Higham, ITMAX 5,
+                                 x >= 0 -> +1, first-index idamax) with A^-1 v through the window's own factor L L':
+                                 what LAPACK's dpocon returns.  0 when the status is non-zero (incomplete factor),
+                                 when anorm1 is 0 (or not a positive number), and when a solve has a non-finite
+                                 1-norm (dpocon's overflow exit); N = 1 gives 1 / (|A^-1| anorm1).  est is a lower
+                                 bound of ||A^-1||_1 up to the rounding of the solves, so rcond >= 1/cond_1.        */
 
 /* stages reported by bp_get_stage_times */
 #define BP_NSTAGE 8
@@ -52,6 +64,7 @@ extern "C" {
 #define BP_STAGE_GRAM 2       /* batched Gram / covariance (DMMA)       :180-182, :317-318, :358, :600 */
 #define BP_STAGE_SOLVE 3      /* Cholesky + solves + weights            :485-489, :572-575, :602-606  */
 #define BP_STAGE_CHAIN 4      /* Jeffreys windows solved relative to a factorised base window :600-606 */
+#define BP_STAGE_COND 5       /* condition estimate: anorm1 before, rcond after each factorisation      */
 
 typedef struct bp_handle bp_handle;
 
@@ -182,6 +195,10 @@ int bp_set_jeffreys_chain(bp_handle* h, int group);
 /* Solve-stage work since the previous call (then reset): out2[0] windows factorised, out2[1] windows solved
  * relative to a base window. */
 int bp_get_solve_work(bp_handle* h, double* out2);
+/* enable != 0: every window the solver factorises also gets BP_SCAL_ANORM1 and BP_SCAL_RCOND (two more kernels per
+ * solve launch, timed as BP_STAGE_COND), and the Jeffreys chain is not used (every window is factorised).  Weights,
+ * nu, w1, status and scalar slots 0-9 are the same bits as with it off.  Default 0. */
+int bp_set_condition_estimate(bp_handle* h, int enable);
 
 /* Pipelining of bp_upload_market_async against bp_conjugate_batched: an intraday block of at least min_bytes
  * is copied in `segments` pieces (1..8; 1 disables; geometric: 1/2, 1/4, ... of the rows), and the conjugate

@@ -16,7 +16,7 @@ BP_NSCAL = 12
 EST_JORION, EST_SHRINKAGE = 1, 2
 SCAL_JORION = dict(mu_g=0, lambda_hat=1, v_hat=2, q=4, one_vinv_one=5)
 SCAL_LW = dict(shrinkage=0, mu=1, beta=2, delta=4)
-SCAL = dict(n0=0, n1=1, alpha=2, beta=3, c=4, v0=5, m=6, sum_a=7, v1=8, mcm_avg=9)
+SCAL = dict(n0=0, n1=1, alpha=2, beta=3, c=4, v0=5, m=6, sum_a=7, v1=8, mcm_avg=9, anorm1=10, rcond=11)
 
 BP_OK, BP_ERR_INVALID, BP_ERR_CUDA, BP_ERR_NO_DEVICE, BP_ERR_STATE = 0, 1, 2, 3, 4
 
@@ -29,10 +29,10 @@ EXPORTED = [
     "bp_upload_market_async", "bp_backtest_batched", "bp_get_gram_work", "bp_set_reuse_min_windows", "bp_set_upload_pipeline", "bp_set_async_outputs",
     "bp_set_resampled", "bp_estimator_batched", "bp_set_jeffreys_chain", "bp_get_solve_work",
     "bp_set_upload_fractions", "bp_solve_wave_windows", "bp_set_hf_presum_min_days", "bp_wait_upload", "bp_upload_pool", "bp_select_market", "bp_path_metrics",
-    "bp_solve_batched",
+    "bp_solve_batched", "bp_set_condition_estimate",
 ]
 BP_NSTAGE = 8
-STAGES = ("logret", "prep", "gram", "solve", "chain")
+STAGES = ("logret", "prep", "gram", "solve", "chain", "cond")
 
 c_double_p = C.POINTER(C.c_double)
 c_int_p = C.POINTER(C.c_int)
@@ -150,6 +150,7 @@ def load():
     lib.bp_solve_wave_windows.argtypes = [C.c_void_p]
     lib.bp_set_jeffreys_chain.argtypes = [C.c_void_p, C.c_int]
     lib.bp_get_solve_work.argtypes = [C.c_void_p, c_double_p]
+    lib.bp_set_condition_estimate.argtypes = [C.c_void_p, C.c_int]
     lib.bp_set_upload_pipeline.argtypes = [C.c_void_p, C.c_int, C.c_longlong]
     lib.bp_set_async_outputs.argtypes = [C.c_void_p, C.c_int]
     lib.bp_backtest_batched.argtypes = [C.c_void_p, C.POINTER(BacktestDesc)]

@@ -213,10 +213,13 @@ def calculate_portfolio_weights(trading_date_ts, portfolio_spec, market_data):
     raise ValueError("Unknown weights spec.")                                                     # :1050
 
 
-def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, universes, hf_lookback_days=None):
+def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, universes, hf_lookback_days=None,
+                     rcond=None):
     """Weights [R][N_all] (0 outside each date's universe) for every rebalance date.  The full market is resident in
     the engine's pool (ONE upload per backtest); per distinct asset set the working market -- its columns, the daily
-    rows its windows read and their intraday look-backs -- is gathered on the device and one batched call follows."""
+    rows its windows read and their intraday look-backs -- is gathered on the device and one batched call follows.
+    With the engine's condition estimate on, ``rcond`` [R] (if given) receives each window's estimate; vw / ew windows,
+    which solve nothing, are left as they are."""
     from . import portfolio_calculations as pc
     prices_df = market_data["stock_prices_df"]
     caps_df = market_data["stock_market_caps_df"]
@@ -229,6 +232,7 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
     R = len(reb_pos)
     W = np.zeros((R, N_all))
     member = np.zeros((R, N_all), dtype=np.uint8)
+    estimate = engine.condition_estimate and rcond is not None
     groups: Dict[tuple, List[int]] = {}
     for r, names in enumerate(universes):
         idx = tuple(sorted(col_pos[n] for n in names))
@@ -306,6 +310,8 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
                                  f"missing bars)")                                            # :492-494
             _raise_on_status(res["status"], dates_all, d_idx)
             w = res["weights"]
+            if estimate:
+                rcond[rows] = res["scalars"][:, SCAL["rcond"]]
         elif strat in ("jeffreys", "jorion", "shrinkage"):
             if weekly:
                 rows_w, batch = plan_weekly_windows(portfolio_spec, dates_ns, d_idx, rf_dates, rf_vals, None, need_hf=False)
@@ -313,9 +319,11 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
             else:
                 batch = plan_daily_windows(portfolio_spec, dates_ns, d_idx, need_hf=False, row_offset=day_lo)
             run = {"jeffreys": engine.jeffreys, "jorion": engine.jorion, "shrinkage": engine.shrinkage}[strat]
-            res = run(batch, outputs=("weights", "status"))
+            res = run(batch, outputs=("weights", "status") + (("scalars",) if estimate else ()))
             _raise_on_status(res["status"], dates_all, d_idx)
             w = res["weights"]
+            if estimate:
+                rcond[rows] = res["scalars"][:, SCAL["rcond"]]
             if strat == "shrinkage":
                 w = pc.clean_weights(w)                        # the reference returns clean_weights() (:743)
         else:
@@ -333,15 +341,45 @@ def _raise_on_status(status, dates_all, d_idx):
 
 
 def backtest_portfolio(portfolio_spec, ts_start_date, ts_end_date, market_data, engine=None, hf_lookback_days=None,
-                       timings: Optional[dict] = None):
+                       timings: Optional[dict] = None, min_rcond: Optional[float] = None,
+                       diagnostics: Optional[dict] = None):
     """:1221-1238 — same signature and the same three output containers.  Extensions (keyword only in spirit):
     ``engine`` (reuse a CUDA context), ``hf_lookback_days`` (the intraday look-back the reference reaches through
-    ``conjugate_prior_S_df=``, e.g. 7 or 366 calendar days where its own 1-day window is rank deficient, F6) and
-    ``timings`` (a dict that receives the wall-clock seconds of the host / device phases)."""
+    ``conjugate_prior_S_df=``, e.g. 7 or 366 calendar days where its own 1-day window is rank deficient, F6),
+    ``timings`` (a dict that receives the wall-clock seconds of the host / device phases), and the condition of the
+    windows: a positive-definite window with cond = 1e13 passes the pivot check and returns weights with hardly a
+    correct digit.  With ``min_rcond`` or ``diagnostics`` given, every window's reciprocal 1-norm condition estimate
+    (LAPACK dpocon's, from the window's own Cholesky factor, ``BayesEngine.set_condition_estimate``) is computed for
+    this backtest; ``diagnostics["rcond"]`` receives it as a Series over the rebalance dates (NaN for vw / ew, which
+    solve nothing), and a window below ``min_rcond`` raises ``np.linalg.LinAlgError`` naming the first such date."""
     import time
     from . import portfolio_calculations as pc
     t0 = time.perf_counter()
     eng = engine or pc._engine()
+    estimate = min_rcond is not None or diagnostics is not None
+    was_on = eng.condition_estimate
+    if estimate:
+        eng.set_condition_estimate(True)
+    try:
+        out, rcond = _backtest(eng, portfolio_spec, ts_start_date, ts_end_date, market_data, hf_lookback_days, timings, t0)
+    finally:
+        if estimate:
+            eng.set_condition_estimate(was_on)
+    if diagnostics is not None:
+        diagnostics["rcond"] = rcond
+    if min_rcond is not None:
+        low = np.nonzero(rcond.to_numpy() < min_rcond)[0]
+        if len(low):
+            raise np.linalg.LinAlgError(
+                f"ill-conditioned posterior matrix at {rcond.index[low[0]].date()} ({len(low)} of {len(rcond)} windows "
+                f"with rcond below {min_rcond:g}, smallest {np.nanmin(rcond.to_numpy()):.3e}): the weights keep hardly "
+                f"any correct digits")
+    return out
+
+
+def _backtest(eng, portfolio_spec, ts_start_date, ts_end_date, market_data, hf_lookback_days, timings, t0):
+    """The body of backtest_portfolio: its three output containers and the windows' rcond Series."""
+    import time
     prices_df = market_data["stock_prices_df"]
     dates_all = prices_df.index
     in_range = np.nonzero((dates_all >= ts_start_date) & (dates_all <= ts_end_date))[0]
@@ -358,7 +396,9 @@ def backtest_portfolio(portfolio_spec, ts_start_date, ts_end_date, market_data, 
                                                  lookback_days=hf_lookback_days if hf_lookback_days is not None else
                                                  HF_LOOKBACK_DAYS.get(portfolio_spec["rolling_window_frequency"]))
     t2 = time.perf_counter()
-    W, member = _batched_weights(eng, portfolio_spec, market_data, dates_all, list(reb_pos), universes, hf_lookback_days)
+    rcond = np.full(len(reb_pos), np.nan)
+    W, member = _batched_weights(eng, portfolio_spec, market_data, dates_all, list(reb_pos), universes, hf_lookback_days,
+                                 rcond)
     t3 = time.perf_counter()
     # loop body on the full column set: gathered from the resident pool, no second upload
     eng.select_market(np.arange(len(prices_df.columns)), 0, len(dates_all), 0, 0)
@@ -377,6 +417,7 @@ def backtest_portfolio(portfolio_spec, ts_start_date, ts_end_date, market_data, 
         t4 = time.perf_counter()
         timings.update(calendar_s=t1 - t0, universe_selection_s=t2 - t1, weights_s=t3 - t2, loop_body_s=t4 - t3, total_s=t4 - t0,
                        rebalances=int(len(reb_pos)), asset_sets=int(len({tuple(sorted(u)) for u in universes})))
-    return {"portfolio_simple_returns_series": returns_series,
-            "portfolio_turnover_series": turnover_series,
-            "portfolio_weights_metrics_df": metrics_df}
+    out = {"portfolio_simple_returns_series": returns_series,
+           "portfolio_turnover_series": turnover_series,
+           "portfolio_weights_metrics_df": metrics_df}
+    return out, pd.Series(rcond, index=reb_dates, dtype="float64", name=name)

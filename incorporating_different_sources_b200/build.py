@@ -16,7 +16,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbayes_portfolio.so")
-SOURCES = ["bp_api.cu", "batch_plan.cu", "stream_kernels.cu", "gram_dmma.cu", "chol_solve.cu", "chol_cluster.cu", "loop_kernels.cu", "eval_kernels.cu", "band_prep.cu", "estimators.cu", "jeffreys_chain.cu"]
+SOURCES = ["bp_api.cu", "batch_plan.cu", "stream_kernels.cu", "gram_dmma.cu", "chol_solve.cu", "chol_cluster.cu", "chol_rcond.cu", "loop_kernels.cu", "eval_kernels.cu", "band_prep.cu", "estimators.cu", "jeffreys_chain.cu"]
 HEADERS = ["batch_plan.h", "chol_panel.cuh", "common.cuh", "jorion_math.cuh", "kernels.h", os.path.join("..", "..", "include", "bayes_portfolio.h")]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

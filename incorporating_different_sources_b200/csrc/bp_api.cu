@@ -130,6 +130,8 @@ struct bp_handle {
     // solved relative to it (jeffreys_chain.cu); < 2 disables.  Work counters for bench.py's roofline accounting.
     int chain_group = 8;
     double work_factored = 0, work_chained = 0;
+    // reciprocal condition estimate of every factorised window (bp_set_condition_estimate)
+    bool cond_estimate = false;
     DevBuf<double> prior_n;
     // banded-GEMM daily pass (band_prep.cu): risk-free weights [W][band_ld] and their sums [W][2]
     DevBuf<double> band_aw, band_stats;
@@ -639,11 +641,22 @@ int solve_windows(bp_handle* h, const Chunk& c, const Layout& L, int wn, int str
     CUtensorMap smap;
     int rc = make_solve_map(h, &smap, c.S, ((long long)(wn - 1) * stride + 1) * L.rowsS, L.ldS);
     if (rc) return rc;
+    if (h->cond_estimate) {
+        // anorm1 of the matrix the factorisation is about to overwrite
+        StageTimer tm(h, BP_STAGE_COND);
+        CU_TRY(launch_sym_norm1(sp, h->stream));
+        h->launches++;
+    }
     {
         StageTimer tm(h, BP_STAGE_SOLVE);
         CU_TRY(launch_chol_solve(sp, smap, h->sm_count, h->stream));
     }
     h->launches++;
+    if (h->cond_estimate) {
+        StageTimer tm(h, BP_STAGE_COND);
+        CU_TRY(launch_chol_rcond(sp, h->stream));
+        h->launches++;
+    }
     h->work_factored += wn;
     return BP_OK;
 }
@@ -659,9 +672,10 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
     // every allocation / launch below (upload_batch included) must land on the handle's device, whatever the
     // calling thread's current device is (two handles on two GPUs in one thread, or torch having switched)
     CU_TRY(cudaSetDevice(h->device));
-    // Jeffreys batches of consecutive trade dates: factorise every G-th window only (jeffreys_chain.cu)
+    // Jeffreys batches of consecutive trade dates: factorise every G-th window only (jeffreys_chain.cu).  Not with the
+    // condition estimate on: a chained window's matrix is never factorised, so there is no factor to estimate from.
     int G = 0;
-    if (h && b && out && mode == BP_MODE_JEFFREYS && (estimator == BP_EST_NONE || estimator == BP_EST_JORION) && solve && !out->T && !out->S0 && !out->S1 &&
+    if (h && b && out && !h->cond_estimate && mode == BP_MODE_JEFFREYS && (estimator == BP_EST_NONE || estimator == BP_EST_JORION) && solve && !out->T && !out->S0 && !out->S1 &&
         !b->resampled && h->chain_group >= 2 && b->n_windows >= 2 * h->chain_group && b->day_row && h->has_market &&
         chain_smem_bytes(h->N) <= (size_t)227 * 1024) {
         bool consecutive = true;
@@ -1083,6 +1097,12 @@ int bp_set_jeffreys_chain(bp_handle* h, int group) {
     if (!h) return fail(BP_ERR_INVALID, "null handle");
     if (group < 0 || group > chain_max_group()) return fail(BP_ERR_INVALID, "group must be in [0, %d]", chain_max_group());
     h->chain_group = group;
+    return BP_OK;
+}
+
+int bp_set_condition_estimate(bp_handle* h, int enable) {
+    if (!h) return fail(BP_ERR_INVALID, "null handle");
+    h->cond_estimate = enable != 0;
     return BP_OK;
 }
 

@@ -2,6 +2,7 @@
 // chol_cluster_kernel (chol_cluster.cu, one thread-block cluster per window).  A batch's weights must not depend on
 // how its windows are split over launches, so both kernels run exactly these operations in exactly this order;
 // only the schedule (which CTA, warp and accumulator slot handles which m-tile) and the synchronisation differ.
+// The condition estimate (chol_rcond.cu) solves with the factor through the same diagonal-block and substitution code.
 //
 // Fragment layout: lane (g, tig) of a warp (g = lane / 4, tig = lane % 4) holds, for the 8-row m-tile that starts at
 // row `row - g` of the window, acc[nt][h] = entry (row, j0 + 8 nt + 2 tig + h) of the 32-column panel j0.  Rows below
@@ -296,6 +297,61 @@ __device__ __forceinline__ void reduce_block(double* z, const double* x, const d
     }
 #pragma unroll
     for (int r = 0; r < NRHS; ++r) z[r * Nr + col] -= a0[r] + a1[r];
+}
+
+// Forward substitution L y = b in the same 32-block form, left-looking over the blocks b = 0 .. Nr/32-1 (the
+// factorisation itself only forward-substitutes through its right-hand-side rows; chol_rcond.cu needs it for any
+// vector).  Per block: the rows of b are reduced by L[rows of b, columns < 32 b] y (forward_reduce_block), then warp r
+// solves the block's triangle for right-hand side r (solve_diag_block_lower, P from load_diag_block).
+
+// One warp solves L_d y = r for the 32 entries r (lane k holds entry k) of one block; returns y the same way
+__device__ __forceinline__ double solve_diag_block_lower(double r, const double* P, int lane) {
+    const double rd = 1.0 / P[lane * LDQ + lane];
+#pragma unroll
+    for (int k = 0; k < NB; ++k) {
+        const double yk = __shfl_sync(0xffffffffu, r * rd, k);
+        if (lane == k) r = yk;
+        if (lane > k) r = fma(-P[lane * LDQ + k], yk, r);
+    }
+    return r;
+}
+
+// z[r][row] -= sum_{j < j0} L[row][j] y[r][j] for the data rows row = j0 + i of block b (j0 = 32 b), i = warp, warp +
+// NWARPS, ...: the lanes stride along the row (coalesced), then one warp sum per row.  z and y are [NRHS][Nr] and may be
+// the same array.
+template <int NRHS, int NWARPS>
+__device__ __forceinline__ void forward_reduce_block(double* z, const double* y, const double* S, int ld, int Nr, int N,
+                                                     int b, int warp, int lane) {
+    constexpr int RPW = NB / NWARPS;
+    const int j0 = NB * b;
+    double acc[RPW][NRHS];
+#pragma unroll
+    for (int q = 0; q < RPW; ++q)
+#pragma unroll
+        for (int r = 0; r < NRHS; ++r) acc[q][r] = 0.0;
+    for (int j = lane; j < j0; j += 32) {
+        double yv[NRHS];
+#pragma unroll
+        for (int r = 0; r < NRHS; ++r) yv[r] = y[r * Nr + j];
+#pragma unroll
+        for (int q = 0; q < RPW; ++q) {
+            const int row = j0 + warp + NWARPS * q;
+            if (row < N) {
+                const double l = S[(long long)row * ld + j];
+#pragma unroll
+                for (int r = 0; r < NRHS; ++r) acc[q][r] = fma(l, yv[r], acc[q][r]);
+            }
+        }
+    }
+#pragma unroll
+    for (int q = 0; q < RPW; ++q) {
+        const int row = j0 + warp + NWARPS * q;
+#pragma unroll
+        for (int r = 0; r < NRHS; ++r) {
+            const double s = warp_sum(acc[q][r]);
+            if (lane == 0 && row < N) z[r * Nr + row] -= s;
+        }
+    }
 }
 
 // Posterior scalars and weights of window w from the solution x[NRHS][Nr], v1 and the window's pivot status

@@ -25,6 +25,8 @@ enum {
     BP_S_SUMA = 7,   // sum_k a_k
     BP_S_V1 = 8,     // w1' S1 w1                    (:574)
     BP_S_MCM_AVG = 9,  // average MCM over the window (:112)
+    BP_S_ANORM1 = 10,  // 1-norm of the factorised matrix (condition estimate on, chol_rcond.cu)
+    BP_S_RCOND = 11,   // dpocon's reciprocal 1-norm condition estimate (condition estimate on, chol_rcond.cu)
     BP_S_COUNT = 12,
     // estimator batches reuse the slots the Jeffreys path leaves at zero (slot 3 stays the Gram's beta)
     BP_S_JORION_MU_G = 0,          // grand mean mu_g                     (:882)
@@ -301,5 +303,10 @@ int chol_max_assets(int nrhs);
 // 8, 4 or 2, the largest with n_windows * K <= cta_slots); cudaErrorNotSupported otherwise (and when N is too large for
 // the aliased back-substitution vectors, or with BP_CHOL_CLUSTER=0): the caller then runs chol_solve_kernel
 cudaError_t launch_chol_cluster(const SolveParams& p, const CUtensorMap& smap, int cta_slots, cudaStream_t st);
+// chol_rcond.cu, the condition estimate of the windows of a solve launch (same n_windows, w_stride, S, scal, status):
+// launch_sym_norm1 before the factorisation writes anorm1 of the lower triangle of S to scal[BP_S_ANORM1];
+// launch_chol_rcond after it reads the factor, the status and anorm1 and writes scal[BP_S_RCOND]
+cudaError_t launch_sym_norm1(const SolveParams& p, cudaStream_t st);
+cudaError_t launch_chol_rcond(const SolveParams& p, cudaStream_t st);
 
 }  // namespace bp

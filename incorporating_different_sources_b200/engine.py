@@ -57,6 +57,7 @@ class BayesEngine:
         self.n_assets = 0
         self.n_days = 0
         self.n_hf_rows = 0
+        self.condition_estimate = False
         self._torch = None
         self._stream = stream        # a torch.cuda.Stream of this engine's own (two engines then overlap on one GPU)
         if use_torch_stream or stream is not None:
@@ -138,6 +139,16 @@ class BayesEngine:
         rc = self._lib.bp_set_jeffreys_chain(self._h, int(group))
         if rc:
             _raise(rc)
+
+    def set_condition_estimate(self, enable: bool):
+        """Every window the solver factorises also gets ``scalars[:, SCAL["anorm1"]]`` (1-norm of the factorised
+        matrix) and ``scalars[:, SCAL["rcond"]]``, LAPACK ``dpocon``'s reciprocal 1-norm condition estimate from the
+        window's own Cholesky factor (0 for a window with a non-zero status).  While it is on, the Jeffreys chain is
+        not used (every window is factorised); every other output is unchanged.  Off by default."""
+        rc = self._lib.bp_set_condition_estimate(self._h, int(bool(enable)))
+        if rc:
+            _raise(rc)
+        self.condition_estimate = bool(enable)
 
     def solve_work(self) -> Dict[str, float]:
         """Windows factorised / solved relative to a base window since the last call."""
