@@ -746,6 +746,23 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
     if (pipelined) {
         if ((rc = run_block_precompute(h, B, 1))) return rc;          // daily blocks do not wait for the bars
         int w_done = 0, k_done[2] = {0, 0};
+        // S1 has to leave every segment's windows before the full waves below factorise them in place.  A device S1 is
+        // unpacked straight into the output; a host S1 into the staging buffer (grown once, here), which is copied out
+        // after the last segment, so that no segment waits for the host.
+        double* s1_dev = nullptr;
+        const size_t s1_bytes = sizeof(double) * (size_t)P.W * N * N;
+        if (out->S1) {
+            if (is_device_ptr(out->S1)) {
+                s1_dev = out->S1;
+            } else {
+                if (h->need_sync) {
+                    CU_TRY(cudaStreamSynchronize(h->stream));
+                    h->need_sync = false;
+                }
+                if ((rc = grow(h, h->stage, s1_bytes))) return rc;
+                s1_dev = reinterpret_cast<double*>(h->stage.p);
+            }
+        }
         for (int s = h->seg_waited; s < h->n_seg; ++s) {
             CU_TRY(cudaStreamWaitEvent(h->stream, h->ev_seg[s], 0));
             const bool last = s == h->n_seg - 1;
@@ -786,6 +803,11 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
                 }
                 h->launches++;
                 if ((rc = run_gram(h, gram_params(h, B, L, cw, w_done, w_end - w_done, GRAM_S1), P.resampled))) return rc;
+                if (s1_dev) {
+                    launch_unpack_sym(cw.S, L.win_stride, L.ldS, N, w_end - w_done, s1_dev + (size_t)w_done * N * N, h->stream);
+                    h->launches++;
+                    CU_TRY(cudaGetLastError());
+                }
                 w_done = w_end;
             }
             // Solve the full waves of windows that are ready: the compute stream would otherwise idle until the next
@@ -805,6 +827,10 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
                     w_solved += wn;
                 }
             }
+        }
+        if (s1_dev && s1_dev != out->S1) {
+            CU_TRY(cudaMemcpyAsync(out->S1, s1_dev, s1_bytes, cudaMemcpyDeviceToHost, h->stream));
+            h->need_sync = true;
         }
         h->seg_waited = h->n_seg;
         h->hf_pending = false;
@@ -891,7 +917,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
                 CU_TRY(launch_lw_shrink(q, h->stream));
                 h->launches++;
             }
-            rc = emit_sym(h, c.S, L, wc, out->S1 ? out->S1 + om : nullptr);
+            rc = emit_sym(h, c.S, L, wc, out->S1 && !pipelined ? out->S1 + om : nullptr);
             if (rc) return rc;
         }
         if (solve && G >= 2) {
