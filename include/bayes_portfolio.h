@@ -235,6 +235,30 @@ typedef struct bp_pool_select {
     long long hf_lo, hf_hi; /* intraday rows [hf_lo, hf_hi) (equal: none) */
 } bp_pool_select;
 int bp_select_market(bp_handle* h, const bp_pool_select* s);
+/* A STACKED working market: windows whose universes differ, evaluated in one batch.  Window w gets its own contiguous
+ * block of rows -- daily pool rows [day_lo[w], day_hi[w]) (prices, caps, risk-free rate) and intraday pool rows
+ * [hf_lo[w], hf_hi[w]) -- holding its own pool columns cols[w][0..n_cols), in that order.  The blocks follow one
+ * another: block w starts at stack row day_off[w] (intraday: hf_off[w]), with day_off[0] = 0 and
+ * day_off[w+1] = day_off[w] + day_hi[w] - day_lo[w] (the host's prefix sums; anything else is BP_ERR_INVALID, as is a
+ * column or row range outside the pool).  A batch that follows names stack rows: a window must read its own block
+ * only, which a block holding exactly the rows a bp_select_market slice would give that window guarantees (its rows
+ * then sit at the same relative positions, and every kernel gives the same bits).
+ * Windows of a stacked market share no rows, so the routes that share work between windows -- the Gram kernel's block
+ * reuse and pre-summed day blocks, the banded daily pass, the Jeffreys chain -- are off for every batch on it, whatever
+ * bp_set_reuse_min_windows / bp_set_jeffreys_chain say; the next bp_select_market / bp_upload_market restores them.
+ * Weekly windows: bp_set_resampled then names rows of the stack (one set of shared weekly rows per window). */
+typedef struct bp_window_select {
+    int n_windows;                  /* W                                                                  */
+    int n_cols;                     /* N: columns of every block                                          */
+    const int* cols;                /* [W][N] pool columns of each window                                 */
+    const int* day_lo;              /* [W] daily pool rows [day_lo, day_hi) of each block                 */
+    const int* day_hi;
+    const int* day_off;             /* [W] first stack row of each daily block                            */
+    const long long* hf_lo;         /* [W] intraday pool rows [hf_lo, hf_hi) (equal: none); all three     */
+    const long long* hf_hi;         /*     intraday arrays NULL: a stack without intraday rows           */
+    const long long* hf_off;        /* [W] first stack row of each intraday block (< 2^31 rows in all)    */
+} bp_window_select;
+int bp_select_windows(bp_handle* h, const bp_window_select* s);
 /* Re-run the log-return stage on the resident prices (device-only timing of the whole path). */
 int bp_prepare_market(bp_handle* h);
 

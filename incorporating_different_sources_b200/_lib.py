@@ -29,6 +29,7 @@ EXPORTED = [
     "bp_upload_market_async", "bp_backtest_batched", "bp_get_gram_work", "bp_set_reuse_min_windows", "bp_set_upload_pipeline", "bp_set_async_outputs",
     "bp_set_resampled", "bp_estimator_batched", "bp_set_jeffreys_chain", "bp_get_solve_work",
     "bp_set_upload_fractions", "bp_solve_wave_windows", "bp_set_hf_presum_min_days", "bp_wait_upload", "bp_upload_pool", "bp_select_market", "bp_path_metrics",
+    "bp_select_windows",
     "bp_solve_batched", "bp_set_condition_estimate",
 ]
 BP_NSTAGE = 8
@@ -107,6 +108,12 @@ class PoolSelect(C.Structure):
                 ("hf_lo", C.c_longlong), ("hf_hi", C.c_longlong)]
 
 
+class WindowSelect(C.Structure):
+    _fields_ = [("n_windows", C.c_int), ("n_cols", C.c_int), ("cols", C.c_void_p), ("day_lo", C.c_void_p),
+                ("day_hi", C.c_void_p), ("day_off", C.c_void_p), ("hf_lo", C.c_void_p), ("hf_hi", C.c_void_p),
+                ("hf_off", C.c_void_p)]
+
+
 def load():
     """Load the shared library (building is the job of ``__graft_entry__.build()``)."""
     global _lib
@@ -126,6 +133,7 @@ def load():
     lib.bp_wait_upload.argtypes = [C.c_void_p]
     lib.bp_upload_pool.argtypes = [C.c_void_p, C.POINTER(MarketDesc)]
     lib.bp_select_market.argtypes = [C.c_void_p, C.POINTER(PoolSelect)]
+    lib.bp_select_windows.argtypes = [C.c_void_p, C.POINTER(WindowSelect)]
     lib.bp_path_metrics.argtypes = [C.c_void_p, C.c_int, C.c_int, c_double_p, c_double_p, C.c_double, c_double_p]
     lib.bp_set_workspace_limit.argtypes = [C.c_void_p, C.c_size_t]
     lib.bp_device_info.argtypes = [C.c_void_p, c_int_p, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]

@@ -18,7 +18,8 @@ import numpy as np
 import pandas as pd
 
 from ._lib import SCAL
-from .windows import HF_LOOKBACK_DAYS, ffill_rows, mcm_prior_n, plan_daily_windows, plan_weekly_windows
+from .windows import (HF_LOOKBACK_DAYS, ffill_rows, mcm_prior_n, plan_daily_windows, plan_weekly_windows, slice_batch,
+                      stack_batches, stack_windows)
 
 # ``data_handling.extract_unique_tickers(d, d)`` of the reference reads the S&P-500 constituents of a date
 # from a CSV (:619); offline there is no such file, so the universe provider is pluggable.  Default: every
@@ -213,14 +214,22 @@ def calculate_portfolio_weights(trading_date_ts, portfolio_spec, market_data):
     raise ValueError("Unknown weights spec.")                                                     # :1050
 
 
+# HBM a stacked batch may fill: its working market (daily prices, caps and returns, intraday prices and returns) and the
+# solver workspace of its windows.  The shipped spec's 178 weekly windows of 50 stocks take about 0.3 GB.
+STACK_BUDGET_BYTES = 2 << 30
+
+
 def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, universes, hf_lookback_days=None,
-                     rcond=None):
+                     rcond=None, counts: Optional[dict] = None):
     """Weights [R][N_all] (0 outside each date's universe) for every rebalance date.  The full market is resident in
-    the engine's pool (ONE upload per backtest); per distinct asset set the working market -- its columns, the daily
-    rows its windows read and their intraday look-backs -- is gathered on the device and one batched call follows.
-    With the engine's condition estimate on, ``rcond`` [R] (if given) receives each window's estimate; vw / ew windows,
-    which solve nothing, are left as they are."""
-    from . import portfolio_calculations as pc
+    the engine's pool (ONE upload per backtest).  An asset set with more windows than ``engine.stack_max_windows`` gets
+    its own working market -- its columns, the daily rows its windows read and their intraday look-backs, gathered on
+    the device -- and one batched call.  The windows of all smaller sets (the top-k universes that change with nearly
+    every rebalance date) are evaluated together instead: one stacked working market per batch of windows with the same
+    number of stocks, each window in a block of its own rows and columns (``select_windows``), with the same bits as
+    the per-set calls.  With the engine's condition estimate on, ``rcond`` [R] (if given) receives each window's
+    estimate; vw / ew windows, which solve nothing, are left as they are.  ``counts`` (if given) receives the number
+    of stacked windows and stacked calls."""
     prices_df = market_data["stock_prices_df"]
     caps_df = market_data["stock_market_caps_df"]
     intr_df = market_data["stock_intraday_prices_df"]
@@ -243,7 +252,6 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
     hf_ts = intr_df.index.values.astype("datetime64[ns]")
     conj = strat.startswith("conjugate")
     needs_hf = conj or strat in ("vw", "ew")
-    weekly = portfolio_spec["rolling_window_frequency"] == "weekly" and strat not in ("vw", "ew")
     if portfolio_spec["rolling_window_frequency"] not in ("daily", "weekly") and strat not in ("vw", "ew"):
         raise NotImplementedError("monthly windows: resample('M') was removed from pandas (SURVEY F10)")
     rf_dates = rf_df.index.values.astype("datetime64[ns]")
@@ -264,72 +272,192 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
     engine.upload_pool(prices=prices_df.to_numpy(dtype=np.float64), rf_row=rf_row,
                        caps=caps_df.reindex(index=dates_all, columns=all_cols).to_numpy(dtype=np.float64), hf_prices=hf_all)
     del hf_all
-    day = np.timedelta64(1, "D")
+    if strat in ("vw", "ew"):
+        spec = dict(portfolio_spec, weighting_strategy="conjugate_hf_vix_" + strat, mcm_scaling=1,
+                    rolling_window=3, rolling_window_frequency="daily", risk_aversion=1)
+    else:
+        spec = portfolio_spec
+    stack_max = engine.stack_max_windows
+    # every set's results, or the exception its planning or evaluation raised: the checks then run set by set in the
+    # order of first appearance, stacked or not, so that the first failing set raises exactly as it did one by one
+    outcome: Dict[tuple, object] = {}
+    small = []
     for idx, rows in groups.items():
-        cols = list(idx)
-        d_idx = np.asarray([reb_pos[r] for r in rows], dtype=np.int64)
-        if strat in ("vw", "ew"):
-            spec = dict(portfolio_spec, weighting_strategy="conjugate_hf_vix_" + strat, mcm_scaling=1,
-                        rolling_window=3, rolling_window_frequency="daily", risk_aversion=1)
-        else:
-            spec = portfolio_spec
-        if weekly:
-            day_lo, hf_lo, hf_hi = 0, 0, (len(hf_ts) if needs_hf else 0)       # weekly closes: the whole history stays addressable
-            day_hi = len(dates_ns)
-        else:
-            n = int(spec["rolling_window"])
-            day_lo, day_hi = int(d_idx.min()) - (n - 1), int(d_idx.max()) + 1
-            if day_lo < 0:
-                raise ValueError(f"a window of {n} prices needs {n - 1} rows before the trade date")
-            hf_lo = hf_hi = 0
-            if needs_hf:
-                Dd = hf_lookback_days if (hf_lookback_days is not None and conj) else HF_LOOKBACK_DAYS[spec["rolling_window_frequency"]]
-                hf_lo = int(np.searchsorted(hf_ts, dates_ns[int(d_idx.min())] - Dd * day + day, side="right"))
-                hf_hi = int(np.searchsorted(hf_ts, dates_ns[int(d_idx.max())] + day, side="right"))
-                hf_lo = max(hf_lo - 1, 0)          # keep one row in front: an empty selection is not a market
-        engine.select_market(cols, day_lo, day_hi, hf_lo, hf_hi)
-        if strat in ("vw", "ew"):
-            batch = plan_daily_windows(spec, dates_ns, d_idx, hf_ts, row_offset=day_lo, hf_row_offset=hf_lo)
-            batch.prior_n = np.ones(len(d_idx))                 # w0 does not depend on the MCM series
-            w = engine.moments(batch, outputs=("w0",))["w0"]
-        elif conj:
-            if weekly:
-                rows_w, batch = plan_weekly_windows(portfolio_spec, dates_ns, d_idx, rf_dates, rf_vals, None, hf_ts,
-                                                    hf_lookback_days=hf_lookback_days)
-                engine.set_resampled(rows_w)
-            else:
-                batch = plan_daily_windows(portfolio_spec, dates_ns, d_idx, hf_ts, hf_lookback_days=hf_lookback_days,
-                                           row_offset=day_lo, hf_row_offset=hf_lo)
-            batch.prior_n = np.ascontiguousarray(prior_n_all[rows])
-            res = engine.conjugate(batch, outputs=("weights", "scalars", "status"))
-            few = np.nonzero(res["scalars"][:, SCAL["m"]] < 2)[0]
-            if len(few):
-                # fewer than 2 intraday returns left after dropna: the reference's S0 is all NaN (:317) and so is w1
-                raise ValueError(f"conjugate_posterior_w_df contains NaN values.  ({dates_all[d_idx[few[0]]].date()}: "
-                                 f"{int(res['scalars'][few[0], SCAL['m']])} intraday returns left after dropping the "
-                                 f"missing bars)")                                            # :492-494
-            _raise_on_status(res["status"], dates_all, d_idx)
-            w = res["weights"]
-            if estimate:
-                rcond[rows] = res["scalars"][:, SCAL["rcond"]]
-        elif strat in ("jeffreys", "jorion", "shrinkage"):
-            if weekly:
-                rows_w, batch = plan_weekly_windows(portfolio_spec, dates_ns, d_idx, rf_dates, rf_vals, None, need_hf=False)
-                engine.set_resampled(rows_w)
-            else:
-                batch = plan_daily_windows(portfolio_spec, dates_ns, d_idx, need_hf=False, row_offset=day_lo)
-            run = {"jeffreys": engine.jeffreys, "jorion": engine.jorion, "shrinkage": engine.shrinkage}[strat]
-            res = run(batch, outputs=("weights", "status") + (("scalars",) if estimate else ()))
-            _raise_on_status(res["status"], dates_all, d_idx)
-            w = res["weights"]
-            if estimate:
-                rcond[rows] = res["scalars"][:, SCAL["rcond"]]
-            if strat == "shrinkage":
-                w = pc.clean_weights(w)                        # the reference returns clean_weights() (:743)
-        else:
-            raise ValueError("Unknown weights spec.")
-        W[np.ix_(rows, cols)] = w
+        if len(rows) <= stack_max:
+            small.append((idx, rows))
+            continue
+        try:
+            outcome[idx] = _per_set(engine, portfolio_spec, spec, strat, idx, rows, dates_ns, reb_pos, hf_ts, rf_dates,
+                                    rf_vals, prior_n_all, hf_lookback_days, estimate)
+        except Exception as e:          # raised below, in its set's turn
+            outcome[idx] = e
+    n_calls = 0
+    if small:
+        n_calls = _stacked_weights(engine, spec, strat, small, dates_ns, reb_pos, hf_ts, rf_dates, rf_vals, prior_n_all,
+                                   hf_lookback_days, estimate, outcome)
+    for idx, rows in groups.items():
+        res = outcome[idx]
+        if isinstance(res, Exception):
+            raise res
+        _store_set(strat, res, rows, list(idx), dates_all, np.asarray([reb_pos[r] for r in rows], dtype=np.int64), W,
+                   rcond, estimate)
+    if counts is not None:
+        counts.update(stacked_windows=sum(len(rows) for _, rows in small), stacked_calls=n_calls)
     return W, member
+
+
+def _per_set(engine, portfolio_spec, spec, strat, idx, rows, dates_ns, reb_pos, hf_ts, rf_dates, rf_vals, prior_n_all,
+             hf_lookback_days, estimate):
+    """One asset set on a working market of its own: its columns, the daily rows its windows read and their intraday
+    look-backs, gathered from the pool; one batched call."""
+    conj = strat.startswith("conjugate")
+    needs_hf = conj or strat in ("vw", "ew")
+    weekly = portfolio_spec["rolling_window_frequency"] == "weekly" and strat not in ("vw", "ew")
+    day = np.timedelta64(1, "D")
+    cols = list(idx)
+    d_idx = np.asarray([reb_pos[r] for r in rows], dtype=np.int64)
+    if weekly:
+        day_lo, hf_lo, hf_hi = 0, 0, (len(hf_ts) if needs_hf else 0)       # weekly closes: the whole history stays addressable
+        day_hi = len(dates_ns)
+    else:
+        n = int(spec["rolling_window"])
+        day_lo, day_hi = int(d_idx.min()) - (n - 1), int(d_idx.max()) + 1
+        if day_lo < 0:
+            raise ValueError(f"a window of {n} prices needs {n - 1} rows before the trade date")
+        hf_lo = hf_hi = 0
+        if needs_hf:
+            Dd = hf_lookback_days if (hf_lookback_days is not None and conj) else HF_LOOKBACK_DAYS[spec["rolling_window_frequency"]]
+            hf_lo = int(np.searchsorted(hf_ts, dates_ns[int(d_idx.min())] - Dd * day + day, side="right"))
+            hf_hi = int(np.searchsorted(hf_ts, dates_ns[int(d_idx.max())] + day, side="right"))
+            hf_lo = max(hf_lo - 1, 0)          # keep one row in front: an empty selection is not a market
+    engine.select_market(cols, day_lo, day_hi, hf_lo, hf_hi)
+    if strat in ("vw", "ew"):
+        batch = plan_daily_windows(spec, dates_ns, d_idx, hf_ts, row_offset=day_lo, hf_row_offset=hf_lo)
+    elif conj:
+        if weekly:
+            rows_w, batch = plan_weekly_windows(portfolio_spec, dates_ns, d_idx, rf_dates, rf_vals, None, hf_ts,
+                                                hf_lookback_days=hf_lookback_days)
+            engine.set_resampled(rows_w)
+        else:
+            batch = plan_daily_windows(portfolio_spec, dates_ns, d_idx, hf_ts, hf_lookback_days=hf_lookback_days,
+                                       row_offset=day_lo, hf_row_offset=hf_lo)
+    elif strat in ("jeffreys", "jorion", "shrinkage"):
+        if weekly:
+            rows_w, batch = plan_weekly_windows(portfolio_spec, dates_ns, d_idx, rf_dates, rf_vals, None, need_hf=False)
+            engine.set_resampled(rows_w)
+        else:
+            batch = plan_daily_windows(portfolio_spec, dates_ns, d_idx, need_hf=False, row_offset=day_lo)
+    else:
+        raise ValueError("Unknown weights spec.")
+    return _evaluate(engine, strat, batch, prior_n_all, rows, estimate)
+
+
+def _evaluate(engine, strat, batch, prior_n_all, rows, estimate):
+    """One batched call of the strategy on the engine's working market."""
+    if strat in ("vw", "ew"):
+        batch.prior_n = np.ones(batch.n_windows)                 # w0 does not depend on the MCM series
+        return engine.moments(batch, outputs=("w0",))
+    if strat.startswith("conjugate"):
+        batch.prior_n = np.ascontiguousarray(prior_n_all[rows])
+        return engine.conjugate(batch, outputs=("weights", "scalars", "status"))
+    run = getattr(engine, strat)                  # jeffreys / jorion / shrinkage
+    return run(batch, outputs=("weights", "status") + (("scalars",) if estimate else ()))
+
+
+def _store_set(strat, res, rows, cols, dates_all, d_idx, W, rcond, estimate):
+    """The checks of one asset set's windows, in the reference's order, then their weights into ``W``."""
+    from . import portfolio_calculations as pc
+    if strat in ("vw", "ew"):
+        W[np.ix_(rows, cols)] = res["w0"]
+        return
+    if strat.startswith("conjugate"):
+        few = np.nonzero(res["scalars"][:, SCAL["m"]] < 2)[0]
+        if len(few):
+            # fewer than 2 intraday returns left after dropna: the reference's S0 is all NaN (:317) and so is w1
+            raise ValueError(f"conjugate_posterior_w_df contains NaN values.  ({dates_all[d_idx[few[0]]].date()}: "
+                             f"{int(res['scalars'][few[0], SCAL['m']])} intraday returns left after dropping the "
+                             f"missing bars)")                                            # :492-494
+    _raise_on_status(res["status"], dates_all, d_idx)
+    w = res["weights"]
+    if estimate:
+        rcond[rows] = res["scalars"][:, SCAL["rcond"]]
+    if strat == "shrinkage":
+        w = pc.clean_weights(w)                        # the reference returns clean_weights() (:743)
+    W[np.ix_(rows, cols)] = w
+
+
+def _stacked_weights(engine, spec, strat, sets, dates_ns, reb_pos, hf_ts, rf_dates, rf_vals, prior_n_all,
+                     hf_lookback_days, estimate, outcome):
+    """The windows of the asset sets ``sets`` [(columns, rebalance indices)], planned on the full calendar exactly as
+    the per-set route plans them, relocated into stacked working markets (``stack_windows``) of one N each and
+    evaluated per batch.  ``outcome[columns]`` receives each set's results, row for row as its own call would return
+    them, or the exception its planning or its batch raised.  Returns the number of batched calls."""
+    weekly = spec["rolling_window_frequency"] == "weekly" and strat not in ("vw", "ew")
+    need_hf = strat in ("vw", "ew") or strat.startswith("conjugate")
+    look = hf_lookback_days if strat.startswith("conjugate") else None
+    if strat not in ("vw", "ew", "jeffreys", "jorion", "shrinkage") and not strat.startswith("conjugate"):
+        for idx, _ in sets:
+            outcome[idx] = ValueError("Unknown weights spec.")
+        return 0
+
+    def plan(d):
+        if weekly:
+            return plan_weekly_windows(spec, dates_ns, d, rf_dates, rf_vals, None, hf_ts if need_hf else None,
+                                       hf_lookback_days=look, need_hf=need_hf)
+        return None, plan_daily_windows(spec, dates_ns, d, hf_ts if need_hf else None, hf_lookback_days=look, need_hf=need_hf)
+
+    d_of = lambda rows: np.asarray(reb_pos, dtype=np.int64)[np.asarray(rows, dtype=np.int64)]
+    sets = sorted(sets, key=lambda s: len(s[0]))                          # windows of one N next to each other
+    try:
+        rows_w, whole = plan(np.concatenate([d_of(rows) for _, rows in sets]))
+    except Exception:
+        # some set cannot be planned: find which (each raises in its turn), stack the others
+        ok = []
+        for idx, rows in sets:
+            try:
+                plan(d_of(rows))
+                ok.append((idx, rows))
+            except Exception as e:
+                outcome[idx] = e
+        sets = ok
+        if not sets:
+            return 0
+        rows_w, whole = plan(np.concatenate([d_of(rows) for _, rows in sets]))
+    win_set = np.asarray([k for k, (_, rows) in enumerate(sets) for _ in rows], dtype=np.int64)
+    win_r = np.asarray([r for _, rows in sets for r in rows], dtype=np.int64)
+    # HBM of each window in a stack: daily blocks x (prices, caps, returns), intraday blocks x (prices, returns), solver
+    stk = stack_windows(whole, rows_w)
+    n_cols = np.asarray([len(sets[k][0]) for k in win_set], dtype=np.int64)
+    ld, ldS = (n_cols + 15) // 16 * 16, (n_cols + 31) // 32 * 32
+    hf_rows = 0 if stk.hf_lo is None else stk.hf_hi - stk.hf_lo
+    nbytes = 8 * ((stk.day_hi - stk.day_lo) * 3 * ld + hf_rows * 2 * ld + (ldS + 8) * ldS + 16 * ld)
+    per_window: Dict[str, list] = {}             # output name -> one row per window (the N differs between batches)
+    failed: Dict[int, Exception] = {}
+    n_calls = 0
+    for pos in stack_batches(n_cols, nbytes, STACK_BUDGET_BYTES):
+        i0, i1 = int(pos[0]), int(pos[-1]) + 1
+        try:
+            part = stack_windows(slice_batch(whole, i0, i1), rows_w)
+            cols = np.asarray([sets[k][0] for k in win_set[i0:i1]], dtype=np.int32)
+            hf = None if part.hf_lo is None else np.stack([part.hf_lo, part.hf_hi], axis=1)
+            engine.select_windows(cols, np.stack([part.day_lo, part.day_hi], axis=1), hf)
+            if part.resampled is not None:
+                engine.set_resampled(part.resampled)
+            res = _evaluate(engine, strat, part.batch, prior_n_all, win_r[i0:i1], estimate)
+        except Exception as e:                  # every set with a window in this batch raises it in its turn
+            for k in np.unique(win_set[i0:i1]):
+                failed.setdefault(int(k), e)
+            continue
+        n_calls += 1
+        for name, a in res.items():
+            per_window.setdefault(name, [None] * len(win_r))[i0:i1] = list(a)
+    for k, (idx, _) in enumerate(sets):
+        if k in failed:
+            outcome[idx] = failed[k]
+            continue
+        sel = np.nonzero(win_set == k)[0]
+        outcome[idx] = {name: np.stack([rows_[i] for i in sel]) for name, rows_ in per_window.items()}
+    return n_calls
 
 
 def _raise_on_status(status, dates_all, d_idx):
@@ -346,7 +474,8 @@ def backtest_portfolio(portfolio_spec, ts_start_date, ts_end_date, market_data, 
     """:1221-1238 — same signature and the same three output containers.  Extensions (keyword only in spirit):
     ``engine`` (reuse a CUDA context), ``hf_lookback_days`` (the intraday look-back the reference reaches through
     ``conjugate_prior_S_df=``, e.g. 7 or 366 calendar days where its own 1-day window is rank deficient, F6),
-    ``timings`` (a dict that receives the wall-clock seconds of the host / device phases), and the condition of the
+    ``timings`` (a dict that receives the wall-clock seconds of the host / device phases, and how many windows were
+    evaluated in stacked batches and in how many calls), and the condition of the
     windows: a positive-definite window with cond = 1e13 passes the pivot check and returns weights with hardly a
     correct digit.  With ``min_rcond`` or ``diagnostics`` given, every window's reciprocal 1-norm condition estimate
     (LAPACK dpocon's, from the window's own Cholesky factor, ``BayesEngine.set_condition_estimate``) is computed for
@@ -397,8 +526,9 @@ def _backtest(eng, portfolio_spec, ts_start_date, ts_end_date, market_data, hf_l
                                                  HF_LOOKBACK_DAYS.get(portfolio_spec["rolling_window_frequency"]))
     t2 = time.perf_counter()
     rcond = np.full(len(reb_pos), np.nan)
+    counts: dict = {}
     W, member = _batched_weights(eng, portfolio_spec, market_data, dates_all, list(reb_pos), universes, hf_lookback_days,
-                                 rcond)
+                                 rcond, counts)
     t3 = time.perf_counter()
     # loop body on the full column set: gathered from the resident pool, no second upload
     eng.select_market(np.arange(len(prices_df.columns)), 0, len(dates_all), 0, 0)
@@ -416,7 +546,7 @@ def _backtest(eng, portfolio_spec, ts_start_date, ts_end_date, market_data, hf_l
     if timings is not None:
         t4 = time.perf_counter()
         timings.update(calendar_s=t1 - t0, universe_selection_s=t2 - t1, weights_s=t3 - t2, loop_body_s=t4 - t3, total_s=t4 - t0,
-                       rebalances=int(len(reb_pos)), asset_sets=int(len({tuple(sorted(u)) for u in universes})))
+                       rebalances=int(len(reb_pos)), asset_sets=int(len({tuple(sorted(u)) for u in universes})), **counts)
     out = {"portfolio_simple_returns_series": returns_series,
            "portfolio_turnover_series": turnover_series,
            "portfolio_weights_metrics_df": metrics_df}

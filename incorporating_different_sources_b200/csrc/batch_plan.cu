@@ -218,6 +218,33 @@ int check_batch(const PlanCtx& ctx, const bp_window_batch* b, bool need_hf, std:
                 return fail_to(err, BP_ERR_INVALID, "window %d: intraday rows [%d,%d) give %d returns (need >= 2, rows < %lld)", w, lo, hi, m, ctx.R);
         }
     }
+    if (ctx.n_blocks > 0) {
+        // stacked market: every row a window reads (prices, caps, resampled rows' prices, intraday bars) lies in ONE
+        // window's block, the same block for the daily and the intraday rows
+        auto block_of = [&ctx](const long long* start, long long row) {
+            return (int)(std::upper_bound(start, start + ctx.n_blocks, row) - start) - 1;
+        };
+        for (int w = 0; w < W; ++w) {
+            const int dr = b->day_row[w];
+            int blk;
+            bool ok = true;
+            if (rs) {
+                blk = block_of(ctx.day_block, b->caps_row[w]);
+                ok = ctx.rs_num && ctx.rs_den;
+                for (int i = dr - (n - 2) + 1; ok && i <= dr + 1; ++i) {
+                    const int row = i <= dr ? i : b->extra_row[w];
+                    ok = block_of(ctx.day_block, ctx.rs_num[row]) == blk && block_of(ctx.day_block, ctx.rs_den[row]) == blk;
+                }
+            } else {
+                blk = block_of(ctx.day_block, dr - n + 1);
+                ok = block_of(ctx.day_block, dr) == blk;
+            }
+            if (ok && need_hf)
+                ok = ctx.hf_block && block_of(ctx.hf_block, b->hf_lo[w]) == blk && block_of(ctx.hf_block, b->hf_hi[w] - 1) == blk;
+            if (!ok)
+                return fail_to(err, BP_ERR_INVALID, "window %d reads stack rows outside one window's block (bp_select_windows)", w);
+        }
+    }
     return BP_OK;
 }
 
@@ -237,7 +264,7 @@ int plan_batch(const PlanCtx& ctx, const bp_window_batch* b, bool need_hf, Batch
     // ---- block grids for the window-overlap reuse of the Gram kernel
     const int npairs_t = ((ctx.N + GRAM_TILE - 1) / GRAM_TILE) * ((ctx.N + GRAM_TILE - 1) / GRAM_TILE + 1) / 2;
     const size_t tiles = (size_t)npairs_t * GRAM_BLOCK_TILE_DOUBLES;      // doubles per block
-    if (W >= ctx.reuse_min_windows) {
+    if (W >= ctx.reuse_min_windows && !ctx.stacked) {
         const int K = n - 1;
         if (!rs) {          // resampled windows: shared weekly rows + one per-date row, no block reuse
             // Block sizes were tuned on the bench workload (N = 500): coarse/fine 128/32 for the 1007-row Jeffreys
@@ -352,7 +379,7 @@ int plan_batch(const PlanCtx& ctx, const bp_window_batch* b, bool need_hf, Batch
             P.work_pre_rows += (double)plan[ph].nb[l] * r8(plan[ph].blk[l]);
         }
     // banded-GEMM daily pass: worth it when 32 consecutive windows share almost all of their rows
-    bool ok = !rs && W >= 32 && n >= 16;
+    bool ok = !rs && !ctx.stacked && W >= 32 && n >= 16;
     for (int w = 1; ok && w < W; ++w) ok = b->day_row[w] >= b->day_row[w - 1];
     P.band_ok = ok && (long long)b->day_row[W - 1] - b->day_row[0] <= 2LL * W;
     return BP_OK;

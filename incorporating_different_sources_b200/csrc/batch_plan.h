@@ -25,6 +25,14 @@ struct PlanCtx {
     int reuse_min_windows = 32;
     int presum_min_days = 8;
     int stride = 1;                    // chain path: only every stride-th window goes through the Gram kernel
+    bool stacked = false;              // stacked market (bp_select_windows): windows share no rows, no block reuse / band
+    // stacked market: first stack row of every block (daily; intraday or nullptr) and the price rows of the resampled
+    // rows (bp_set_resampled, or nullptr), so that each window of a batch is held to one block
+    int n_blocks = 0;
+    const long long* day_block = nullptr;
+    const long long* hf_block = nullptr;
+    const int* rs_num = nullptr;
+    const int* rs_den = nullptr;
 };
 
 inline long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }

@@ -81,6 +81,12 @@ struct bp_handle {
     int pool_N = 0, pool_D = 0;
     long long pool_R = 0;
     DevBuf<int> pool_cols;
+    // stacked working market (bp_select_windows): one block of rows per window, no rows shared between windows, so no
+    // route that shares work between windows may run; the per-window (first pool row, first stack row, rows) table
+    bool stacked = false;
+    DevBuf<long long> stack_rows;
+    std::vector<long long> stack_day_start, stack_hf_start;     // first stack row of each block (check_batch)
+    std::vector<int> rs_num_host, rs_den_host;                  // stacked market: price rows of the resampled rows
     // resampled (weekly) return rows: see bp_set_resampled
     double *lr_w = nullptr, *rf_w = nullptr, *mcm_w = nullptr;
     int* rs_idx = nullptr;
@@ -180,6 +186,8 @@ void free_resampled(bp_handle* h) {
     h->lr_w = h->rf_w = h->mcm_w = nullptr;
     h->rs_idx = nullptr;
     h->Rw = 0;
+    h->rs_num_host.clear();
+    h->rs_den_host.clear();
 }
 
 void free_pool(bp_handle* h) {
@@ -368,6 +376,14 @@ PlanCtx plan_ctx(const bp_handle* h, int stride) {
     c.ws_limit = h->ws_limit;
     c.reuse_min_windows = h->reuse_min_windows;
     c.presum_min_days = h->presum_min_days;
+    c.stacked = h->stacked;
+    if (h->stacked) {
+        c.n_blocks = (int)h->stack_day_start.size();
+        c.day_block = h->stack_day_start.data();
+        c.hf_block = h->stack_hf_start.empty() ? nullptr : h->stack_hf_start.data();
+        c.rs_num = h->rs_num_host.empty() ? nullptr : h->rs_num_host.data();
+        c.rs_den = h->rs_den_host.empty() ? nullptr : h->rs_den_host.data();
+    }
     c.stride = stride;
     return c;
 }
@@ -676,7 +692,7 @@ int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, i
     // condition estimate on: a chained window's matrix is never factorised, so there is no factor to estimate from.
     int G = 0;
     if (h && b && out && !h->cond_estimate && mode == BP_MODE_JEFFREYS && (estimator == BP_EST_NONE || estimator == BP_EST_JORION) && solve && !out->T && !out->S0 && !out->S1 &&
-        !b->resampled && h->chain_group >= 2 && b->n_windows >= 2 * h->chain_group && b->day_row && h->has_market &&
+        !b->resampled && !h->stacked && h->chain_group >= 2 && b->n_windows >= 2 * h->chain_group && b->day_row && h->has_market &&
         chain_smem_bytes(h->N) <= (size_t)227 * 1024) {
         bool consecutive = true;
         for (int w = 1; consecutive && w < b->n_windows; ++w) consecutive = b->day_row[w] == b->day_row[0] + w;
@@ -1043,6 +1059,7 @@ int bp_destroy(bp_handle* h) {
     free_buf(h->vstore);
     free_buf(h->prior_n);
     free_buf(h->band_aw);
+    free_buf(h->stack_rows);
     free_buf(h->band_stats);
     free_buf(h->ws);
     free_buf(h->stage);
@@ -1280,6 +1297,9 @@ static int begin_market(bp_handle* h, int N, int D, long long R, int n_mcm) {
     h->seg_waited = 0;
     h->lr_hf_done = 0;
     h->hf_pending = false;
+    h->stacked = false;
+    h->stack_day_start.clear();
+    h->stack_hf_start.clear();
     return BP_OK;
 }
 
@@ -1456,6 +1476,89 @@ int bp_select_market(bp_handle* h, const bp_pool_select* s) {
     return finish_market(h);
 }
 
+int bp_select_windows(bp_handle* h, const bp_window_select* s) {
+    if (!h || !s) return fail(BP_ERR_INVALID, "null handle or selection");
+    if (!h->pool_prices) return fail(BP_ERR_STATE, "no pool resident: call bp_upload_pool first");
+    const int W = s->n_windows, N = s->n_cols;
+    if (W <= 0 || N <= 0 || !s->cols || !s->day_lo || !s->day_hi || !s->day_off)
+        return fail(BP_ERR_INVALID, "selection needs windows, columns and daily row ranges with their offsets");
+    const bool with_hf = s->hf_lo || s->hf_hi || s->hf_off;
+    if (with_hf && (!s->hf_lo || !s->hf_hi || !s->hf_off))
+        return fail(BP_ERR_INVALID, "intraday row ranges need hf_lo, hf_hi and hf_off");
+    if (N > h->pool_N || N > 12288)      // (the gather keeps a window's column list in 48 KB of shared memory)
+        return fail(BP_ERR_INVALID, "%d columns per window: the pool has %d, a stack takes at most 12288", N, h->pool_N);
+    // [W][3] daily blocks, then [W][3] intraday blocks: (first pool row, first stack row, rows)
+    std::vector<long long> tab(6 * (size_t)W, 0);
+    long long D = 0, R = 0, max_d = 0, max_r = 0;
+    for (int w = 0; w < W; ++w) {
+        const int* c = s->cols + (size_t)w * N;
+        for (int j = 0; j < N; ++j)
+            if (c[j] < 0 || c[j] >= h->pool_N)
+                return fail(BP_ERR_INVALID, "window %d: column %d outside the pool's %d columns", w, c[j], h->pool_N);
+        const int lo = s->day_lo[w], hi = s->day_hi[w];
+        if (lo < 0 || hi > h->pool_D || hi <= lo)
+            return fail(BP_ERR_INVALID, "window %d: daily row range [%d, %d) outside the pool's %d rows (or empty)", w, lo, hi, h->pool_D);
+        if (s->day_off[w] != D)
+            return fail(BP_ERR_INVALID, "window %d: daily block starts at stack row %d, the blocks before it end at %lld: the blocks must tile the stack",
+                        w, s->day_off[w], D);
+        tab[3 * (size_t)w] = lo;
+        tab[3 * (size_t)w + 1] = D;
+        tab[3 * (size_t)w + 2] = hi - lo;
+        D += hi - lo;
+        max_d = std::max<long long>(max_d, hi - lo);
+        if (D > 0x7fffffffLL) return fail(BP_ERR_INVALID, "too many daily rows in the stack for int32 row indices");
+        if (!with_hf) continue;
+        const long long hlo = s->hf_lo[w], hhi = s->hf_hi[w];
+        if (hlo < 0 || hhi < hlo || hhi > h->pool_R)
+            return fail(BP_ERR_INVALID, "window %d: intraday row range [%lld, %lld) outside the pool's %lld rows", w, hlo, hhi, h->pool_R);
+        if (s->hf_off[w] != R)
+            return fail(BP_ERR_INVALID, "window %d: intraday block starts at stack row %lld, the blocks before it end at %lld: the blocks must tile the stack",
+                        w, s->hf_off[w], R);
+        tab[3 * ((size_t)W + w)] = hlo;
+        tab[3 * ((size_t)W + w) + 1] = R;
+        tab[3 * ((size_t)W + w) + 2] = hhi - hlo;
+        R += hhi - hlo;
+        max_r = std::max(max_r, hhi - hlo);
+        if (R > 0x7fffffffLL) return fail(BP_ERR_INVALID, "too many intraday rows in the stack for int32 row indices");
+    }
+    if (D < 2) return fail(BP_ERR_INVALID, "the stack needs at least 2 daily rows");
+    CU_TRY(cudaSetDevice(h->device));
+    int rc;
+    if ((rc = begin_market(h, N, (int)D, R, 0))) return rc;
+    h->has_caps = h->pool_caps != nullptr;
+    cudaStream_t st = h->stream;
+    if ((rc = grow(h, h->pool_cols, (size_t)W * N)) || (rc = grow(h, h->stack_rows, tab.size()))) return rc;
+    // (pageable host memory: staged before the call returns, as in bp_select_market)
+    CU_TRY(cudaMemcpyAsync(h->pool_cols.p, s->cols, sizeof(int) * (size_t)W * N, cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(h->stack_rows.p, tab.data(), sizeof(long long) * tab.size(), cudaMemcpyHostToDevice, st));
+    const long long pN = h->pool_N;
+    const long long* day_tab = h->stack_rows.p;
+    launch_gather_window_blocks(h->pool_prices, pN, h->prices, N, W, h->pool_cols.p, day_tab, max_d, st);
+    h->launches++;
+    if (h->pool_caps) {
+        launch_gather_window_blocks(h->pool_caps, pN, h->caps, N, W, h->pool_cols.p, day_tab, max_d, st);
+        h->launches++;
+    }
+    launch_gather_window_blocks(h->pool_rf, 1, h->rf_row, 1, W, nullptr, day_tab, max_d, st);
+    h->launches++;
+    if (R > 0) {
+        launch_gather_window_blocks(h->pool_hf, pN, h->hf_prices, N, W, h->pool_cols.p, day_tab + 3 * (size_t)W, max_r, st);
+        h->launches++;
+        CU_TRY(cudaEventRecord(h->ev_hf, st));
+        h->hf_pending = true;            // the first consumer computes the intraday log returns (wait_hf)
+    }
+    CU_TRY(cudaGetLastError());
+    if ((rc = finish_market(h))) return rc;
+    h->stacked = true;
+    h->stack_day_start.resize(W);
+    h->stack_hf_start.resize(with_hf ? W : 0);
+    for (int w = 0; w < W; ++w) {
+        h->stack_day_start[w] = tab[3 * (size_t)w + 1];
+        if (with_hf) h->stack_hf_start[w] = tab[3 * ((size_t)W + w) + 1];
+    }
+    return BP_OK;
+}
+
 int bp_upload_market(bp_handle* h, const bp_market_desc* m) { return upload_market_impl(h, m, true); }
 
 int bp_upload_market_async(bp_handle* h, const bp_market_desc* m) { return upload_market_impl(h, m, false); }
@@ -1485,6 +1588,10 @@ int bp_set_resampled(bp_handle* h, const bp_resampled_desc* r) {
     h->launches++;
     CU_TRY(cudaGetLastError());
     h->Rw = Rw;
+    if (h->stacked) {
+        h->rs_num_host.assign(r->num_row, r->num_row + Rw);
+        h->rs_den_host.assign(r->den_row, r->den_row + Rw);
+    }
     int rc = make_map(h, &h->map_w, h->lr_w, Rw, h->ld);
     if (rc) return rc;
     CU_TRY(cudaStreamSynchronize(h->stream));     // host index arrays may be freed after return

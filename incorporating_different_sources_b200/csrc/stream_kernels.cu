@@ -634,6 +634,44 @@ void launch_gather_cols(const double* src, long long ld_src, double* dst, int n,
     gather_cols_kernel<<<grid, n >= 256 ? 256 : 128, 0, st>>>(src, ld_src, dst, n, rows, cols);
 }
 
+// Stacked working market (bp_select_windows): block w = pool rows [rows[3w], rows[3w] + rows[3w+2]) of its own columns
+// cols[w][0..n) (cols == nullptr: columns 0..n-1), written densely from stack row rows[3w+1] on.  One CTA per (window,
+// slice of rows); the window's column list sits in shared memory.  A thread keeps one column (and, for n below the
+// CTA size, one of the blockDim / n rows handled per step), so the loop has no index division, and each step stores
+// a contiguous run of the output.
+__global__ void gather_window_blocks_kernel(const double* __restrict__ src, long long ld_src, double* __restrict__ dst,
+                                            int n, const int* __restrict__ cols, const long long* __restrict__ rows,
+                                            int slice_rows) {
+    extern __shared__ int wcols[];
+    const int w = blockIdx.x;
+    for (int j = threadIdx.x; j < n; j += blockDim.x) wcols[j] = cols ? cols[(long long)w * n + j] : j;
+    __syncthreads();
+    const long long s0 = rows[3 * (long long)w], d0 = rows[3 * (long long)w + 1], nr = rows[3 * (long long)w + 2];
+    const bool wide = n >= (int)blockDim.x;
+    const int per_step = wide ? 1 : blockDim.x / n;          // rows per step
+    const int tr = wide ? 0 : threadIdx.x / n;               // this thread's row within a step
+    const int tc = wide ? threadIdx.x : threadIdx.x % n;     // and its first column
+    const int cstep = wide ? blockDim.x : n;
+    if (tr >= per_step) return;
+    for (long long r0 = (long long)blockIdx.y * slice_rows; r0 < nr; r0 += (long long)gridDim.y * slice_rows) {
+        const long long r1 = nr - r0 < slice_rows ? nr : r0 + slice_rows;
+        for (long long r = r0 + tr; r < r1; r += per_step) {
+            const double* s = src + (s0 + r) * ld_src;
+            double* d = dst + (d0 + r) * n;
+            for (int j = tc; j < n; j += cstep) d[j] = s[wcols[j]];
+        }
+    }
+}
+
+void launch_gather_window_blocks(const double* src, long long ld_src, double* dst, int n, int n_windows, const int* cols,
+                                 const long long* rows, long long max_rows, cudaStream_t st) {
+    if (n_windows <= 0 || n <= 0 || max_rows <= 0) return;
+    const int slice_rows = n >= 2048 ? 1 : 2048 / n;
+    const long long slices = (max_rows + slice_rows - 1) / slice_rows;
+    const dim3 grid(n_windows, (unsigned)(slices < 65535 ? slices : 65535));
+    gather_window_blocks_kernel<<<grid, 256, sizeof(int) * (size_t)n, st>>>(src, ld_src, dst, n, cols, rows, slice_rows);
+}
+
 // dst row (dst_row0 + k) = src row src_rows[k], k in [k0, k1): the overnight returns of arbitrary day blocks, gathered
 // behind the intraday matrix so that a window reads them as one contiguous run (PhasePlan::inner)
 __global__ void gather_rows_indexed_kernel(double* __restrict__ M, int ld, const int* __restrict__ src_rows,

@@ -58,6 +58,9 @@ class BayesEngine:
         self.n_days = 0
         self.n_hf_rows = 0
         self.condition_estimate = False
+        self.reuse_min_windows = 32      # library defaults (bp_set_reuse_min_windows / bp_set_jeffreys_chain)
+        self.jeffreys_chain = 8
+        self._stack_max = 15
         self._torch = None
         self._stream = stream        # a torch.cuda.Stream of this engine's own (two engines then overlap on one GPU)
         if use_torch_stream or stream is not None:
@@ -139,6 +142,7 @@ class BayesEngine:
         rc = self._lib.bp_set_jeffreys_chain(self._h, int(group))
         if rc:
             _raise(rc)
+        self.jeffreys_chain = int(group)
 
     def set_condition_estimate(self, enable: bool):
         """Every window the solver factorises also gets ``scalars[:, SCAL["anorm1"]]`` (1-norm of the factorised
@@ -163,6 +167,26 @@ class BayesEngine:
         rc = self._lib.bp_set_reuse_min_windows(self._h, int(n))
         if rc:
             _raise(rc)
+        self.reuse_min_windows = int(n)
+
+    def set_stack_max_windows(self, n: int = 15):
+        """Backtests evaluate the windows of every asset set with at most ``n`` windows together, in stacked batches
+        (:meth:`select_windows`), instead of one working market and one batched call per set; 0 never stacks.  The
+        results are the same bits either way.  Sets large enough for a route that shares work between windows keep
+        their own call: :attr:`stack_max_windows` stays below the engine's block-reuse minimum and below the 2 x
+        group windows of the Jeffreys chain."""
+        if int(n) < 0:
+            raise ValueError("n must be >= 0")
+        self._stack_max = int(n)
+
+    @property
+    def stack_max_windows(self) -> int:
+        """The largest asset set (in windows) that a backtest stacks: :meth:`set_stack_max_windows` capped by the
+        routes that share work between the windows of one set."""
+        cap = min(self._stack_max, self.reuse_min_windows - 1)
+        if self.jeffreys_chain >= 2:
+            cap = min(cap, 2 * self.jeffreys_chain - 1)
+        return max(cap, 0)
 
     def set_hf_presum_min_days(self, min_days: int = 8):
         """Windows whose intraday look-back covers at least ``min_days`` trading days add at most three pre-summed
@@ -324,6 +348,42 @@ class BayesEngine:
         if rc:
             _raise(rc)
         self.n_assets, self.n_days, self.n_hf_rows = int(cols.shape[0]), sel.day_hi - sel.day_lo, int(sel.hf_hi - sel.hf_lo)
+
+    def select_windows(self, cols_per_window, day_ranges, hf_ranges=None):
+        """Stacked working market: window w gets its own block of pool rows -- daily rows ``day_ranges[w]`` = (lo, hi)
+        and intraday rows ``hf_ranges[w]`` -- in its own pool columns ``cols_per_window[w]`` (one N for all), the
+        blocks one after the other in window order.  A following batch names stack rows and each window must read its
+        own block only (:func:`~.windows.stack_windows` plans both).  Every window is then evaluated exactly as on a
+        :meth:`select_market` slice of its own; the routes that share work between windows are off until the next
+        ``select_market`` / ``upload_market``.  Returns the blocks' first stack rows (daily, intraday)."""
+        cols = np.ascontiguousarray(cols_per_window, dtype=np.int32)
+        if cols.ndim != 2:
+            raise ValueError("cols_per_window must be [W][N]")
+        W = cols.shape[0]
+        days = np.ascontiguousarray(day_ranges, dtype=np.int64).reshape(-1, 2)
+        if days.shape[0] != W:
+            raise ValueError("day_ranges must have one (lo, hi) per window")
+        day_lo, day_hi = np.ascontiguousarray(days[:, 0], dtype=np.int32), np.ascontiguousarray(days[:, 1], dtype=np.int32)
+        day_off = np.ascontiguousarray(np.r_[0, np.cumsum(days[:, 1] - days[:, 0])[:-1]], dtype=np.int32)
+        sel = _lib.WindowSelect()
+        sel.n_windows, sel.n_cols = W, int(cols.shape[1])
+        sel.cols, sel.day_lo, sel.day_hi, sel.day_off = cols.ctypes.data, day_lo.ctypes.data, day_hi.ctypes.data, day_off.ctypes.data
+        sel.hf_lo = sel.hf_hi = sel.hf_off = None
+        hf_off = None
+        n_hf = 0
+        if hf_ranges is not None:
+            hf = np.ascontiguousarray(hf_ranges, dtype=np.int64).reshape(-1, 2)
+            if hf.shape[0] != W:
+                raise ValueError("hf_ranges must have one (lo, hi) per window")
+            hf_lo, hf_hi = np.ascontiguousarray(hf[:, 0]), np.ascontiguousarray(hf[:, 1])
+            hf_off = np.ascontiguousarray(np.r_[0, np.cumsum(hf_hi - hf_lo)[:-1]], dtype=np.int64)
+            sel.hf_lo, sel.hf_hi, sel.hf_off = hf_lo.ctypes.data, hf_hi.ctypes.data, hf_off.ctypes.data
+            n_hf = int((hf_hi - hf_lo).sum())
+        rc = self._lib.bp_select_windows(self._h, C.byref(sel))
+        if rc:
+            _raise(rc)
+        self.n_assets, self.n_days, self.n_hf_rows = int(cols.shape[1]), int((days[:, 1] - days[:, 0]).sum()), n_hf
+        return day_off.astype(np.int64), hf_off
 
     def set_resampled(self, rows):
         """Build the weekly return rows (:class:`~.windows.ResampledRows`) on the device from the resident prices."""

@@ -259,6 +259,98 @@ def plan_weekly_windows(spec, dates: np.ndarray, d_indices: Sequence[int], rf_da
     return rows, batch
 
 
+@dataclass
+class StackedWindows:
+    """Windows laid out in one stacked working market (``BayesEngine.select_windows``): window w owns the daily pool
+    rows [day_lo[w], day_hi[w]), which start at stack row day_off[w], and the intraday pool rows [hf_lo[w], hf_hi[w]) at
+    stack row hf_off[w] (``None``: no intraday rows).  ``batch`` and, for weekly windows, ``resampled`` name stack rows."""
+    batch: WindowBatch
+    resampled: Optional[ResampledRows]
+    day_lo: np.ndarray
+    day_hi: np.ndarray
+    day_off: np.ndarray
+    hf_lo: Optional[np.ndarray]
+    hf_hi: Optional[np.ndarray]
+    hf_off: Optional[np.ndarray]
+
+
+def _block_offsets(lengths: np.ndarray) -> np.ndarray:
+    return np.r_[0, np.cumsum(lengths)[:-1]].astype(np.int64)
+
+
+def stack_windows(batch: WindowBatch, rows: Optional[ResampledRows] = None) -> StackedWindows:
+    """Relocate windows planned on the full calendar (``plan_daily_windows`` without row offsets, or
+    ``plan_weekly_windows`` and its ``rows``) into one block each of a stacked market, in batch order.
+
+    A block holds the rows a ``select_market`` slice gives the window, at the same positions relative to the window:
+    daily windows the n prices up to the trade date; weekly windows the daily rows from the first week close their
+    returns read up to the trade date (its caps row); intraday rows from one row in front of the window's first bar
+    (``hf_lo - 1``, as the per-set slices keep it) to its last.  Weekly windows get their own copy of the resampled
+    rows they read -- n-2 week rows then the trade date's row, each with its ``rf_row`` value (the partial week's
+    look-ahead label included) and ``num_row`` / ``den_row`` moved into the block -- behind one unused row 0.  Nothing
+    is re-derived, so every descriptor equals the plan's up to the block offsets."""
+    W, n = batch.n_windows, int(batch.rolling_window)
+    dr = batch.day_row.astype(np.int64)
+    res = None
+    if batch.resampled:
+        if rows is None:
+            raise ValueError("weekly windows need the ResampledRows of their plan")
+        # resampled rows of every window: its n-2 shared week rows, then its own trade-date row
+        sel = np.concatenate([dr[:, None] + np.arange(-(n - 3), 1)[None, :], batch.extra_row.astype(np.int64)[:, None]], axis=1)
+        num, den = rows.num_row[sel].astype(np.int64), rows.den_row[sel].astype(np.int64)
+        caps = batch.caps_row.astype(np.int64)
+        day_lo = np.minimum(np.minimum(num.min(axis=1), den.min(axis=1)), caps)
+        day_hi = np.maximum(np.maximum(num.max(axis=1), den.max(axis=1)), caps) + 1
+        day_off = _block_offsets(day_hi - day_lo)
+        shift = (day_off - day_lo)[:, None]
+        mcm = None
+        if rows.mcm is not None:
+            mcm = np.concatenate([np.zeros((rows.mcm.shape[0], 1)), rows.mcm[:, sel.ravel()]], axis=1)
+        res = ResampledRows(num_row=np.r_[0, (num + shift).ravel()].astype(np.int32),
+                            den_row=np.r_[0, (den + shift).ravel()].astype(np.int32),
+                            rf_row=np.r_[0.0, rows.rf_row[sel.ravel()]].astype(np.float64), mcm=mcm,
+                            n_weeks=1 + W * (n - 1))
+        first = 1 + np.arange(W, dtype=np.int64) * (n - 1)
+        day_row, extra_row, caps_row = first + n - 3, first + n - 2, caps - day_lo + day_off
+    else:
+        day_lo, day_hi = dr - (n - 1), dr + 1
+        if day_lo.min() < 0:
+            raise ValueError(f"a window of {n} prices needs {n - 1} rows before the trade date")
+        day_off = _block_offsets(day_hi - day_lo)
+        day_row, extra_row = dr - day_lo + day_off, batch.extra_row
+        caps_row = None if batch.caps_row is None else batch.caps_row - day_lo + day_off
+    hf_lo = hf_hi = hf_off = new_lo = new_hi = None
+    if batch.hf_lo is not None:
+        lo, hf_hi = batch.hf_lo.astype(np.int64), batch.hf_hi.astype(np.int64)
+        hf_lo = np.maximum(lo - 1, 0)
+        hf_off = _block_offsets(hf_hi - hf_lo)
+        new_lo, new_hi = lo - hf_lo + hf_off, hf_hi - hf_lo + hf_off
+    i32 = lambda a: None if a is None else np.asarray(a).astype(np.int32)
+    import dataclasses
+    stacked = dataclasses.replace(batch, day_row=i32(day_row), hf_lo=i32(new_lo), hf_hi=i32(new_hi),
+                                  extra_row=i32(extra_row), caps_row=i32(caps_row))
+    return StackedWindows(stacked, res, day_lo, day_hi, day_off, hf_lo, hf_hi, hf_off)
+
+
+def stack_batches(n_cols: Sequence[int], window_bytes: Sequence[int], budget: int):
+    """Positions of the windows of each stacked batch: windows with the same number of columns (a stacked market has
+    one N), in their given order, cut so that a batch's ``window_bytes`` stay within ``budget`` (a window larger than
+    the budget forms a batch of its own)."""
+    n_cols = np.asarray(n_cols, dtype=np.int64)
+    out = []
+    for N in dict.fromkeys(n_cols.tolist()):
+        pos = np.nonzero(n_cols == N)[0]
+        start, acc = 0, 0
+        for k, i in enumerate(pos):
+            b = int(window_bytes[i])
+            if k > start and acc + b > budget:
+                out.append(pos[start:k])
+                start, acc = k, 0
+            acc += b
+        out.append(pos[start:])
+    return out
+
+
 def mcm_prior_n(spec, mcm_dates: np.ndarray, mcm_values: np.ndarray, trade_dates: np.ndarray) -> np.ndarray:
     """``calculate_conjugate_prior_n`` (:247-267) for many trade dates, on the MCM series' OWN calendar.
 
