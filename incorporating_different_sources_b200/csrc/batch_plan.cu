@@ -248,6 +248,67 @@ int check_batch(const PlanCtx& ctx, const bp_window_batch* b, bool need_hf, std:
     return BP_OK;
 }
 
+int check_call(const PlanCtx& ctx, const bp_window_batch* b, const CallDesc& call, std::string* err) {
+    if (call.solve && (call.mode == BP_MODE_CONJUGATE || call.estimator != BP_EST_NONE) && !(b->risk_aversion != 0.0))
+        return fail_to(err, BP_ERR_INVALID, "risk_aversion must be non-zero");
+    if (call.estimator == BP_EST_JORION && b->rolling_window - 1 - ctx.N - 2 <= 0)
+        return fail_to(err, BP_ERR_INVALID, "Jorion needs T - N - 2 > 0 (T = rolling_window - 1 returns, :879)");
+    return BP_OK;
+}
+
+Layout make_layout(int N, int ld, int max_m, bool with_mv) {
+    Layout L;
+    L.N = N;
+    L.ldv = ld;
+    L.ldS = round_up(N, 32);
+    L.rowsS = L.ldS + 8;
+    L.win_stride = (long long)L.rowsS * L.ldS;
+    L.y_stride = round_up(std::max(max_m, 2), 2);
+    const int nt = (N + GRAM_TILE - 1) / GRAM_TILE;
+    L.mv_stride = with_mv ? (long long)(nt * (nt + 1) / 2) * 2 * GRAM_TILE : 0;
+    L.per_window = sizeof(double) * ((size_t)L.win_stride + 9 * (size_t)L.ldv + BP_NSCAL + (size_t)L.y_stride + (size_t)L.mv_stride) + 16;
+    return L;
+}
+
+int plan_chain_group(const PlanCtx& ctx, const bp_window_batch* b, const CallDesc& call) {
+    // Jeffreys batches of consecutive trade dates.  Not with the condition estimate on: a chained window's matrix is
+    // never factorised, so there is no factor to estimate from.
+    if (ctx.cond_estimate || call.mode != BP_MODE_JEFFREYS || (call.estimator != BP_EST_NONE && call.estimator != BP_EST_JORION) ||
+        !call.solve || call.T || call.S0 || call.S1 || b->resampled || ctx.stacked || ctx.chain_group < 2 ||
+        b->n_windows < 2 * ctx.chain_group || !ctx.chain_smem_fits)
+        return 0;
+    for (int w = 1; w < b->n_windows; ++w)
+        if (b->day_row[w] != b->day_row[0] + w) return 0;
+    // the whole batch in one workspace chunk: the descriptors are planned for the base windows only
+    if ((size_t)b->n_windows * make_layout(ctx.N, ctx.ld, 0, false).per_window > ctx.ws_limit) return 0;
+    const int G = std::min(ctx.chain_group, ctx.chain_max);
+    // Conditioning guard: window b+k is the base with k rows removed and k rows added; the down-dated matrix
+    // has rank n-1-k, and its Woodbury pivots -1 + l'J_b^-1 l tend to 0 as n-1-k approaches N (leverage 1),
+    // where the small system loses digits while no pivot is exactly zero.  Chain only with a margin of rows;
+    // closer to the rank limit every window is factorised on its own (the path the parity tests pin).
+    if (G >= 2 && b->rolling_window - 1 < ctx.N + 2 * G + 8) return 0;
+    return G;
+}
+
+int plan_route(const PlanCtx& ctx, const BatchPlan& P, const bp_window_batch* b, const CallDesc& call, int G, Route* out,
+               std::string* err) {
+    Route& r = *out;
+    r = Route();
+    r.G = G;
+    r.L = make_layout(ctx.N, ctx.ld, P.presum ? 0 : P.max_m, P.presum);
+    r.Wc = (int)std::min<size_t>((size_t)P.W, std::max<size_t>(1, ctx.ws_limit / r.L.per_window));
+    // (plan_chain_group checks the same layout for a chained batch, so this cannot trigger unless the two are changed
+    // apart)
+    if (r.Wc < P.W && G >= 2) return fail_to(err, BP_ERR_STATE, "internal: chained batch does not fit one workspace chunk");
+    // Pipelined against a segmented asynchronous intraday upload: prep + Gram of the windows whose bars have
+    // arrived run while the rest is still being copied; the solve follows for all windows at once.
+    r.pipelined = call.mode == BP_MODE_CONJUGATE && ctx.hf_pending && ctx.n_seg > 1 && ctx.seg_waited < ctx.n_seg &&
+                  call.solve && !call.T && !call.S0 && r.Wc >= P.W && !P.presum;
+    if (call.mode == BP_MODE_CONJUGATE && !r.pipelined)
+        for (int w = 0; w < P.W; ++w) r.hf_wait_rows = std::max<long long>(r.hf_wait_rows, b->hf_hi[w]);
+    return BP_OK;
+}
+
 int plan_batch(const PlanCtx& ctx, const bp_window_batch* b, bool need_hf, BatchPlan* out, std::string* err) {
     BatchPlan& P = *out;
     P = BatchPlan();

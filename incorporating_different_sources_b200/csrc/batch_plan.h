@@ -33,9 +33,35 @@ struct PlanCtx {
     const long long* hf_block = nullptr;
     const int* rs_num = nullptr;
     const int* rs_den = nullptr;
+    // route choice (plan_chain_group, plan_route)
+    bool cond_estimate = false;        // bp_set_condition_estimate: every window must be factorised
+    int chain_group = 0;               // bp_set_jeffreys_chain
+    int chain_max = 0;                 // chain_max_group()
+    bool chain_smem_fits = false;      // chain_smem_bytes(N) <= 227 KB
+    bool hf_pending = false;           // an asynchronous intraday upload is still in flight ...
+    int n_seg = 0, seg_waited = 0;     // ... in n_seg segments, of which seg_waited have been waited for
+};
+
+// What a batched call computes: the route decisions depend on it
+struct CallDesc {
+    int mode = BP_MODE_CONJUGATE;
+    bool solve = false;
+    int estimator = BP_EST_NONE;
+    bool T = false, S0 = false, S1 = false;        // these outputs are requested
 };
 
 inline long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
+
+// Workspace layout of one window: the solver matrix (ldS columns, rowsS rows) and the vectors (ldv doubles each)
+struct Layout {
+    int N, ldv, ldS, rowsS;
+    long long win_stride, y_stride, mv_stride;
+    size_t per_window;
+};
+
+// max_m: longest intraday window (scratch of the row dots); with_mv: room for the Gram kernel's G w0 partials
+Layout make_layout(int N, int ld, int max_m, bool with_mv);
 
 // Block grids of one phase, two levels (0 = coarse, 1 = fine; the fine size divides the coarse size): block b of
 // level l covers return rows [b*blk[l], (b+1)*blk[l]); blk[l] == 0: level unused
@@ -81,9 +107,27 @@ struct BatchPlan {
 int fail_to(std::string* err, int code, const char* fmt, ...);
 // Every validation of a batch against the resident market; BP_OK or a BP_ERR_* code with the message in *err.
 int check_batch(const PlanCtx& ctx, const bp_window_batch* b, bool need_hf, std::string* err);
+// The call's own arguments (risk aversion, Jorion's T - N - 2 > 0) for a batch check_batch accepted.
+int check_call(const PlanCtx& ctx, const bp_window_batch* b, const CallDesc& call, std::string* err);
+// Chain group G of a batch check_batch accepted: >= 2 factorises only every G-th window and solves the others
+// relative to it (jeffreys_chain.cu); plan_batch takes it as its stride.
+int plan_chain_group(const PlanCtx& ctx, const bp_window_batch* b, const CallDesc& call);
 // Plans a batch that check_batch accepted.  Fails only when the plan is internally inconsistent.
 int plan_batch(const PlanCtx& ctx, const bp_window_batch* b, bool need_hf, BatchPlan* plan, std::string* err);
 // Writes the descriptor image (plan.ints ints) to dst.
 void write_batch(const BatchPlan& plan, const bp_window_batch* b, int* dst);
+
+// How the driver runs a planned batch
+struct Route {
+    int G = 0;                         // chain group (plan_chain_group)
+    // prep + Gram of the windows whose intraday bars have arrived run between the segments of an asynchronous upload
+    bool pipelined = false;
+    int Wc = 0;                        // windows per workspace chunk
+    long long hf_wait_rows = 0;        // > 0: wait for the intraday price rows below this before the batch
+    Layout L{};
+};
+// Route of a batch plan_batch planned with stride G.  Fails only when the route is internally inconsistent.
+int plan_route(const PlanCtx& ctx, const BatchPlan& plan, const bp_window_batch* b, const CallDesc& call, int G,
+               Route* route, std::string* err);
 
 }  // namespace bp

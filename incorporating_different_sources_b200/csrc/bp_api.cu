@@ -32,8 +32,6 @@ thread_local std::string g_err;      // bp_last_error
             return fail(BP_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__); \
     } while (0)
 
-inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
-
 bool is_device_ptr(const void* p) {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
@@ -296,27 +294,6 @@ struct Chunk {
     int* status;
 };
 
-struct Layout {
-    int N, ldv, ldS, rowsS;
-    long long win_stride, y_stride, mv_stride;
-    size_t per_window;
-};
-
-// max_m: longest intraday window (scratch of the row dots); with_mv: room for the Gram kernel's G w0 partials
-Layout make_layout(const bp_handle* h, int max_m, bool with_mv = false) {
-    Layout L;
-    L.N = h->N;
-    L.ldv = h->ld;
-    L.ldS = round_up(h->N, 32);
-    L.rowsS = L.ldS + 8;
-    L.win_stride = (long long)L.rowsS * L.ldS;
-    L.y_stride = round_up(std::max(max_m, 2), 2);
-    const int nt = (h->N + GRAM_TILE - 1) / GRAM_TILE;
-    L.mv_stride = with_mv ? (long long)(nt * (nt + 1) / 2) * 2 * GRAM_TILE : 0;
-    L.per_window = sizeof(double) * ((size_t)L.win_stride + 9 * (size_t)L.ldv + BP_NSCAL + (size_t)L.y_stride + (size_t)L.mv_stride) + 16;
-    return L;
-}
-
 Chunk carve(unsigned char* ws, const Layout& L, int Wc) {
     Chunk c;
     double* p = reinterpret_cast<double*>(ws);
@@ -365,7 +342,7 @@ struct Batch {
     const double* prior_n = nullptr;
 };
 
-PlanCtx plan_ctx(const bp_handle* h, int stride) {
+PlanCtx plan_ctx(const bp_handle* h) {
     PlanCtx c;
     c.has_market = h->has_market;
     c.N = h->N; c.ld = h->ld; c.D = h->D; c.Rw = h->Rw; c.n_mcm = h->n_mcm;
@@ -384,19 +361,21 @@ PlanCtx plan_ctx(const bp_handle* h, int stride) {
         c.rs_num = h->rs_num_host.empty() ? nullptr : h->rs_num_host.data();
         c.rs_den = h->rs_den_host.empty() ? nullptr : h->rs_den_host.data();
     }
-    c.stride = stride;
+    c.cond_estimate = h->cond_estimate;
+    c.chain_group = h->chain_group;
+    c.chain_max = chain_max_group();
+    c.chain_smem_fits = chain_smem_bytes(h->N) <= (size_t)227 * 1024;
+    c.hf_pending = h->hf_pending;
+    c.n_seg = h->n_seg;
+    c.seg_waited = h->seg_waited;
     return c;
 }
 
-// stride: the chain path runs only every stride-th window through the Gram kernel
-int upload_batch(bp_handle* h, const bp_window_batch* b, bool need_hf, int stride, Batch* out) {
-    if (!h || !b) return fail(BP_ERR_INVALID, "null handle or batch");
-    const PlanCtx ctx = plan_ctx(h, stride);
-    int rc = check_batch(ctx, b, need_hf, &g_err);
-    if (!rc) rc = plan_batch(ctx, b, need_hf, &out->plan, &g_err);
-    if (rc) return rc;
+// The descriptor image of the batch planned in out->plan, on the device
+int upload_batch(bp_handle* h, const bp_window_batch* b, Batch* out) {
     const BatchPlan& P = out->plan;
     const int W = P.W;
+    int rc;
     for (int ph = 0; ph < 2; ++ph)
         for (int l = 0; l < 2; ++l)
             if ((rc = grow(h, h->store[ph][l], P.store[ph][l]))) return rc;
@@ -419,7 +398,7 @@ int upload_batch(bp_handle* h, const bp_window_batch* b, bool need_hf, int strid
     if (!h->ev_desc[slot]) CU_TRY(cudaEventCreateWithFlags(&h->ev_desc[slot], cudaEventDisableTiming));
     CU_TRY(cudaEventRecord(h->ev_desc[slot], h->stream));
     h->ev_desc_armed[slot] = true;
-    if (need_hf && b->prior_n) {
+    if (P.need_hf && b->prior_n) {
         if ((rc = grow(h, h->prior_n, (size_t)W))) return rc;
         CU_TRY(cudaMemcpyAsync(h->prior_n.p, b->prior_n, sizeof(double) * (size_t)W, cudaMemcpyHostToDevice, h->stream));
         CU_TRY(cudaStreamSynchronize(h->stream));
@@ -445,41 +424,40 @@ int upload_batch(bp_handle* h, const bp_window_batch* b, bool need_hf, int strid
     return BP_OK;
 }
 
-// dense [Wc][N] copy of a strided device vector to a host or device destination
-int emit_vec(bp_handle* h, const double* src, const Layout& L, int Wc, double* dst) {
-    if (!dst) return BP_OK;
-    if (is_device_ptr(dst)) {
-        launch_unpack_vec(src, L.ldv, L.N, Wc, dst, h->stream);
-        h->launches++;
-    } else {
-        const size_t bytes = sizeof(double) * (size_t)Wc * L.N;
-        // the single staging buffer is reused: drain the previous D2H copy before overwriting it
-        if (h->need_sync) CU_TRY(cudaStreamSynchronize(h->stream));
-        int rc = grow(h, h->stage, bytes);
-        if (rc) return rc;
-        launch_unpack_vec(src, L.ldv, L.N, Wc, reinterpret_cast<double*>(h->stage.p), h->stream);
-        h->launches++;
-        CU_TRY(cudaMemcpyAsync(dst, h->stage.p, bytes, cudaMemcpyDeviceToHost, h->stream));
-        h->need_sync = true;
+// The page-locked staging buffer of host-bound outputs, grown to `bytes`.  There is one: the previous copy out of it
+// is drained first.
+int host_stage(bp_handle* h, size_t bytes, double** p) {
+    if (h->need_sync) {
+        CU_TRY(cudaStreamSynchronize(h->stream));
+        h->need_sync = false;
     }
+    int rc = grow(h, h->stage, bytes);
+    if (rc) return rc;
+    *p = reinterpret_cast<double*>(h->stage.p);
     return BP_OK;
 }
 
-int emit_sym(bp_handle* h, const double* S, const Layout& L, int Wc, double* dst) {
+// dense copy of Wc windows' strided vectors ([Wc][N]) or symmetric matrices (sym: [Wc][N][N]) to dst, on the device
+void unpack(bp_handle* h, const double* src, const Layout& L, int Wc, bool sym, double* dst) {
+    if (sym) launch_unpack_sym(src, L.win_stride, L.ldS, L.N, Wc, dst, h->stream);
+    else launch_unpack_vec(src, L.ldv, L.N, Wc, dst, h->stream);
+    h->launches++;
+}
+
+// the same to a host or device destination; a host destination is reached through the staging buffer
+int emit_dense(bp_handle* h, const double* src, const Layout& L, int Wc, bool sym, double* dst) {
     if (!dst) return BP_OK;
     if (is_device_ptr(dst)) {
-        launch_unpack_sym(S, L.win_stride, L.ldS, L.N, Wc, dst, h->stream);
-        h->launches++;
-    } else {
-        const size_t bytes = sizeof(double) * (size_t)Wc * L.N * L.N;
-        if (h->need_sync) CU_TRY(cudaStreamSynchronize(h->stream));
-        int rc = grow(h, h->stage, bytes);
-        if (rc) return rc;
-        launch_unpack_sym(S, L.win_stride, L.ldS, L.N, Wc, reinterpret_cast<double*>(h->stage.p), h->stream);
-        h->launches++;
-        CU_TRY(cudaMemcpyAsync(dst, h->stage.p, bytes, cudaMemcpyDeviceToHost, h->stream));
-        h->need_sync = true;
+        unpack(h, src, L, Wc, sym, dst);
+        return BP_OK;
     }
+    const size_t bytes = sizeof(double) * (size_t)Wc * L.N * (sym ? L.N : 1);
+    double* stage = nullptr;
+    int rc = host_stage(h, bytes, &stage);
+    if (rc) return rc;
+    unpack(h, src, L, Wc, sym, stage);
+    CU_TRY(cudaMemcpyAsync(dst, stage, bytes, cudaMemcpyDeviceToHost, h->stream));
+    h->need_sync = true;
     return BP_OK;
 }
 
@@ -677,315 +655,323 @@ int solve_windows(bp_handle* h, const Chunk& c, const Layout& L, int wn, int str
     return BP_OK;
 }
 
-// shared driver of bp_conjugate_batched / bp_jeffreys_batched / bp_stats_batched / bp_hf_cov_batched
-int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, int mode, bool solve, int estimator = BP_EST_NONE) {
-    Batch B;
-    if (!h || !b) return fail(BP_ERR_INVALID, "null handle or batch");
-    if (solve && h->has_market) {
-        const int rcl = check_solver_size(h->N, estimator);
-        if (rcl) return rcl;
+// Cholesky + solves of wn windows of a batched call, from window k of the chunk at c; the reference evaluates
+// (1/gamma) * nu (:836,:849)
+int solve_batch_windows(bp_handle* h, const bp_window_batch* b, const Layout& L, const Chunk& c, const CallDesc& call, int k,
+                        int wn, int stride = 1) {
+    return solve_windows(h, chunk_at(c, L, k), L, wn, stride, call.mode, call.estimator, b->rolling_window - 1,
+                         1.0 / b->risk_aversion);
+}
+
+// Outputs of the chunk's windows [w0, w0 + wc) of a batch of W windows, in one order: the solution when solved
+// (weights, nu, w1, status), then t, w0 (with_w0), rhs and the scalars.  Shared by run_batches and bp_solve_batched.
+int emit_chunk(bp_handle* h, const Chunk& c, const Layout& L, const bp_outputs* out, int w0, int wc, int W, bool solved,
+               bool with_w0) {
+    const size_t ov = (size_t)w0 * L.N;
+    auto at = [ov](double* p) { return p ? p + ov : nullptr; };
+    int rc;
+    if (solved) {
+        if ((rc = emit_dense(h, c.weights, L, wc, false, at(out->weights)))) return rc;
+        if ((rc = emit_dense(h, c.nu, L, wc, false, at(out->nu)))) return rc;
+        if ((rc = emit_dense(h, c.w1, L, wc, false, at(out->w1)))) return rc;
+        if ((rc = emit_raw(h, c.status, sizeof(int) * (size_t)wc, out->status ? out->status + w0 : nullptr))) return rc;
     }
-    // every allocation / launch below (upload_batch included) must land on the handle's device, whatever the
-    // calling thread's current device is (two handles on two GPUs in one thread, or torch having switched)
-    CU_TRY(cudaSetDevice(h->device));
-    // Jeffreys batches of consecutive trade dates: factorise every G-th window only (jeffreys_chain.cu).  Not with the
-    // condition estimate on: a chained window's matrix is never factorised, so there is no factor to estimate from.
-    int G = 0;
-    if (h && b && out && !h->cond_estimate && mode == BP_MODE_JEFFREYS && (estimator == BP_EST_NONE || estimator == BP_EST_JORION) && solve && !out->T && !out->S0 && !out->S1 &&
-        !b->resampled && !h->stacked && h->chain_group >= 2 && b->n_windows >= 2 * h->chain_group && b->day_row && h->has_market &&
-        chain_smem_bytes(h->N) <= (size_t)227 * 1024) {
-        bool consecutive = true;
-        for (int w = 1; consecutive && w < b->n_windows; ++w) consecutive = b->day_row[w] == b->day_row[0] + w;
-        const Layout L0 = make_layout(h, 0);
-        if (consecutive && (size_t)b->n_windows * L0.per_window <= h->ws_limit) G = std::min(h->chain_group, chain_max_group());
-        // Conditioning guard: window b+k is the base with k rows removed and k rows added; the down-dated matrix
-        // has rank n-1-k, and its Woodbury pivots -1 + l'J_b^-1 l tend to 0 as n-1-k approaches N (leverage 1),
-        // where the small system loses digits while no pivot is exactly zero.  Chain only with a margin of rows;
-        // closer to the rank limit every window is factorised on its own (the path the parity tests pin).
-        if (G >= 2 && b->rolling_window - 1 < h->N + 2 * G + 8) G = 0;
+    if ((rc = emit_dense(h, c.t, L, wc, false, at(out->t)))) return rc;
+    if (with_w0 && (rc = emit_dense(h, c.w0, L, wc, false, at(out->w0)))) return rc;
+    if ((rc = emit_dense(h, c.rhs, L, wc, false, at(out->rhs)))) return rc;
+    if ((rc = emit_raw(h, c.scal, sizeof(double) * (size_t)wc * BP_NSCAL,
+                       out->scalars ? out->scalars + (size_t)w0 * BP_NSCAL : nullptr))) return rc;
+    // the workspace is reused by the next chunk: host-bound copies must have drained
+    if (w0 + wc < W && h->need_sync) {
+        CU_TRY(cudaStreamSynchronize(h->stream));
+        h->need_sync = false;
     }
-    int rc = upload_batch(h, b, mode == BP_MODE_CONJUGATE, G >= 2 ? G : 1, &B);
-    if (rc) return rc;
+    return BP_OK;
+}
+
+// Block precompute before the chunk loop: the gathered overnight returns and the intraday blocks (with their scans on
+// the pre-summed path) of a conjugate batch, then the daily blocks
+int run_blocks(bp_handle* h, const Batch& B, const CallDesc& call) {
     const BatchPlan& P = B.plan;
     const PhasePlan& A = P.phase[0];
-    const Layout L = make_layout(h, P.presum ? 0 : P.max_m, P.presum);
-    int Wc = (int)std::min<size_t>((size_t)P.W, std::max<size_t>(1, h->ws_limit / L.per_window));
-    // (the descriptors were planned for the base windows only: the chain path must not be abandoned after upload_batch;
-    // the check above uses the same layout, so this cannot trigger unless the two are changed apart)
-    if (Wc < P.W && G >= 2) return fail(BP_ERR_STATE, "internal: chained batch does not fit one workspace chunk");
-    // Pipelined against a segmented asynchronous intraday upload: prep + Gram of the windows whose bars have
-    // arrived run while the rest is still being copied; the solve follows for all windows at once.
-    const bool pipelined = mode == BP_MODE_CONJUGATE && h->hf_pending && h->n_seg > 1 && h->seg_waited < h->n_seg &&
-                           solve && !out->T && !out->S0 && Wc >= P.W && !P.presum;
-    if (mode == BP_MODE_CONJUGATE && !pipelined) {
-        long long need = 0;                   // intraday price rows this batch reads
-        for (int w = 0; w < P.W; ++w) need = std::max<long long>(need, b->hf_hi[w]);
-        if ((rc = wait_hf_rows(h, need))) return rc;
+    const bool conj = call.mode == BP_MODE_CONJUGATE;
+    int rc;
+    if (conj && A.inner && !P.presum) {
+        launch_gather_rows_indexed(h->lr_hf, h->ld, B.hf_starts, h->R, 0, A.nb[0], h->stream);
+        h->launches++;
+        CU_TRY(cudaGetLastError());
     }
-    rc = grow(h, h->ws, (size_t)Wc * L.per_window + 256);
+    if (conj && (call.S0 || call.S1 || call.solve || P.presum) && (rc = run_block_precompute(h, B, 0))) return rc;
+    if (conj && P.presum) {
+        // scans of the day blocks: column sums (vectors) and Gram tiles, suffix' and prefix per chunk
+        StageTimer tm(h, BP_STAGE_GRAM);
+        const int nt = (h->N + GRAM_TILE - 1) / GRAM_TILE;
+        launch_block_col_sums(h->lr_hf, h->ld, B.hf_starts, 0, A.nb[0], h->vstore.p, h->stream);
+        launch_vec_scan(h->vstore.p, h->ld, h->lr_hf, B.hf_starts, A.nb[0], A.chunk, h->stream);
+        launch_tile_scan(h->store[0][0].p, nt * (nt + 1) / 2, nt, h->lr_hf, h->ld, B.hf_starts, A.nb[0], A.chunk, h->stream);
+        h->launches += 3;
+        CU_TRY(cudaGetLastError());
+    }
+    if ((call.T || call.S1 || call.solve) && (rc = run_block_precompute(h, B, 1))) return rc;
+    return BP_OK;
+}
+
+// Window prep of the windows [w0, w0 + wc) of the batch; c: the workspace of window w0
+int run_prep(bp_handle* h, const bp_window_batch* b, const Batch& B, const Layout& L, const Chunk& c, int w0, int wc,
+             const CallDesc& call) {
+    PrepParams pp = prep_params(h, b, B, L, c, w0, call.mode);
+    if (call.estimator != BP_EST_NONE) pp.beta_den = B.plan.n - 1;       // sample covariance: centre with 1/m, m = n-1 returns
+    {
+        StageTimer tm(h, BP_STAGE_PREP);
+        CU_TRY(launch_window_prep(pp, wc, h->stream, h->D));
+        h->launches += pp.use_band ? (call.mode == BP_MODE_JEFFREYS ? 1 : 2) : 0;
+    }
+    h->launches++;
+    return BP_OK;
+}
+
+// Pre-summed day blocks: S0 w0, v0, c and rhs are finished from the G w0 partials of the first Gram launch that
+// contracts the intraday phase (it must precede the solve and every emit of rhs / scalars)
+int run_post(bp_handle* h, const Layout& L, const Chunk& c, int wc) {
+    PostParams q{};
+    q.n_windows = wc;
+    q.n_assets = L.N;
+    q.ldv = L.ldv;
+    q.mv_part = c.mv;
+    q.w0 = c.w0;
+    q.gvec = c.gvec;
+    q.t = c.t;
+    q.s0w0 = c.s0w0;
+    q.rhs = c.rhs;
+    q.scal = c.scal;
+    StageTimer tm(h, BP_STAGE_PREP);
+    CU_TRY(launch_conj_post(q, h->stream));
+    h->launches++;
+    return BP_OK;
+}
+
+// C = X_c'X_c  ->  m Sigma_LW / (1 - shrinkage) = C + rho I, rhs = t / (1 - shrinkage), in place (:727-729)
+int run_shrink(bp_handle* h, const Batch& B, const Layout& L, const Chunk& c, int w0, int wc) {
+    const BatchPlan& P = B.plan;
+    ShrinkParams q{};
+    q.n_windows = wc;
+    q.n_assets = L.N;
+    q.n_window = P.n;
+    q.ld = h->ld;
+    q.ldv = L.ldv;
+    q.ldS = L.ldS;
+    q.win_stride = L.win_stride;
+    q.lr_daily = P.resampled ? h->lr_w : h->lr_d;
+    q.rf_row = P.resampled ? h->rf_w : h->rf_row;
+    q.day_row = B.day_row + w0;
+    q.extra_row = B.extra_row ? B.extra_row + w0 : nullptr;
+    q.span_days = B.span + w0;
+    q.t = c.t;
+    q.S = c.S;
+    q.rhs = c.rhs;
+    q.scal = c.scal;
+    StageTimer tm(h, BP_STAGE_PREP);
+    CU_TRY(launch_lw_shrink(q, h->stream));
+    h->launches++;
+    return BP_OK;
+}
+
+// S0 Gram of the chunk (intraday rows), finished by run_post when post; S0: its output or nullptr
+int run_s0(bp_handle* h, const Batch& B, const Layout& L, const Chunk& c, int w0, int wc, bool post, double* S0) {
+    int rc = run_gram(h, gram_params(h, B, L, c, w0, wc, GRAM_S0), B.plan.resampled);
+    if (!rc && post) rc = run_post(h, L, c, wc);
+    if (!rc) rc = emit_dense(h, c.S, L, wc, true, S0);
+    return rc;
+}
+
+// S1 (conjugate) or J (Jeffreys) Gram of the chunk, of the base windows only on the chain path; finished by run_post
+// when post, rewritten into the Ledoit-Wolf system for the shrinkage estimator; S1: its output or nullptr
+int run_s1(bp_handle* h, const Batch& B, const Route& r, const Chunk& c, int w0, int wc, const CallDesc& call, bool post,
+           double* S1) {
+    GramParams gp = gram_params(h, B, r.L, c, w0, wc, call.mode == BP_MODE_CONJUGATE ? GRAM_S1 : GRAM_J);
+    if (r.G >= 2) {                      // base windows only
+        gp.w_stride = r.G;
+        gp.n_windows = (wc + r.G - 1) / r.G;
+    }
+    int rc = run_gram(h, gp, B.plan.resampled);
+    if (!rc && post) rc = run_post(h, r.L, c, wc);
+    if (!rc && call.estimator == BP_EST_SHRINKAGE) rc = run_shrink(h, B, r.L, c, w0, wc);
+    if (!rc) rc = emit_dense(h, c.S, r.L, wc, true, S1);
+    return rc;
+}
+
+// Chain path: factorise the base windows of the chunk, then solve the other windows of each group relative to their base
+int run_chain(bp_handle* h, const bp_window_batch* b, const Batch& B, const Route& r, const Chunk& c, int w0, int wc,
+              const CallDesc& call) {
+    const int G = r.G;
+    int rc = solve_batch_windows(h, b, r.L, c, call, 0, (wc + G - 1) / G, G);
     if (rc) return rc;
-    const Chunk c = carve(h->ws.p, L, Wc);
+    ChainParams cp{};
+    cp.n_windows = wc;
+    cp.group = G;
+    cp.n_assets = h->N;
+    cp.n_window = B.plan.n;
+    cp.estimator = call.estimator;
+    cp.ld = h->ld;
+    cp.ldv = r.L.ldv;
+    cp.ldS = r.L.ldS;
+    cp.win_stride = r.L.win_stride;
+    cp.inv_gamma = 1.0 / b->risk_aversion;
+    cp.lr_daily = h->lr_d;
+    cp.day_row = B.day_row + w0;
+    cp.S = c.S;
+    cp.t = c.t;
+    cp.pvec = c.pvec;
+    cp.w1 = c.w1;
+    cp.nu = c.nu;
+    cp.weights = c.weights;
+    cp.scal = c.scal;
+    cp.status = c.status;
+    {
+        StageTimer tm(h, BP_STAGE_CHAIN);
+        CU_TRY(launch_jeffreys_chain(cp, h->stream));
+    }
+    h->launches++;
+    h->work_chained += wc - (wc + G - 1) / G;
+    return BP_OK;
+}
+
+// Pipelined conjugate batch (one workspace chunk) against a segmented asynchronous intraday upload: waits for the
+// segments one by one, runs the prep + S1 Gram of the windows whose bars have arrived, and solves full waves of them
+// between the segments.  *w_solved: the windows it solved.
+int run_pipelined(bp_handle* h, const bp_window_batch* b, const Batch& B, const Route& r, const Chunk& c,
+                  const CallDesc& call, double* S1, int* w_solved) {
+    const BatchPlan& P = B.plan;
+    const PhasePlan& A = P.phase[0];
+    const Layout& L = r.L;
     const int N = h->N;
+    int rc = run_block_precompute(h, B, 1);          // daily blocks do not wait for the bars
+    if (rc) return rc;
+    int w_done = 0, k_done[2] = {0, 0};
+    *w_solved = 0;
+    // S1 has to leave every segment's windows before the full waves below factorise them in place.  A device S1 is
+    // unpacked straight into the output; a host S1 into the staging buffer (grown once, here), which is copied out
+    // after the last segment, so that no segment waits for the host.
+    double* s1_dev = nullptr;
+    const size_t s1_bytes = sizeof(double) * (size_t)P.W * N * N;
+    if (S1) {
+        if (is_device_ptr(S1)) s1_dev = S1;
+        else if ((rc = host_stage(h, s1_bytes, &s1_dev))) return rc;
+    }
+    for (int s = h->seg_waited; s < h->n_seg; ++s) {
+        CU_TRY(cudaStreamWaitEvent(h->stream, h->ev_seg[s], 0));
+        const bool last = s == h->n_seg - 1;
+        const long long r_end = h->seg_end[s];
+        if ((rc = hf_returns(h, h->lr_hf_done, r_end))) return rc;
+        h->lr_hf_done = r_end;
+        int k_ready[2];
+        for (int l = 0; l < 2; ++l) {
+            k_ready[l] = A.nb[l];
+            if (!last && l == 0 && A.inner) {
+                // day block k is complete once the bars below starts[k+1] have arrived
+                const long long k = std::upper_bound(A.starts.begin() + 1, A.starts.end(), (int)std::min<long long>(r_end, 0x7fffffff)) -
+                                    (A.starts.begin() + 1);
+                k_ready[l] = (int)std::min<long long>(A.nb[l], std::max<long long>(k, k_done[l]));
+            } else if (!last && A.blk[l] > 0) {
+                const long long k = floor_div(r_end, A.blk[l]) - A.bmin[l];
+                k_ready[l] = (int)std::min<long long>(A.nb[l], std::max<long long>(k, k_done[l]));
+            }
+        }
+        if (A.inner) {
+            launch_gather_rows_indexed(h->lr_hf, h->ld, B.hf_starts, h->R, k_done[0], k_ready[0], h->stream);
+            h->launches++;
+            CU_TRY(cudaGetLastError());
+        }
+        if ((rc = run_block_precompute(h, B, 0, k_done, k_ready))) return rc;
+        k_done[0] = k_ready[0];
+        k_done[1] = k_ready[1];
+        int w_end = w_done;
+        if (last) w_end = P.W;
+        else while (w_end < P.W && (long long)b->hf_hi[w_end] <= r_end) ++w_end;
+        if (w_end > w_done) {
+            const Chunk cw = chunk_at(c, L, w_done);
+            if ((rc = run_prep(h, b, B, L, cw, w_done, w_end - w_done, call))) return rc;
+            if ((rc = run_gram(h, gram_params(h, B, L, cw, w_done, w_end - w_done, GRAM_S1), P.resampled))) return rc;
+            if (s1_dev) {
+                unpack(h, cw.S, L, w_end - w_done, true, s1_dev + (size_t)w_done * N * N);
+                CU_TRY(cudaGetLastError());
+            }
+            w_done = w_end;
+        }
+        // Solve the full waves of windows that are ready: the compute stream would otherwise idle until the next
+        // segment arrives (the copy takes longer than the statistics / Gram stages), and after the last segment
+        // only the remainder (less than one wave) is left instead of every window.  Full waves cost nothing in
+        // occupancy whichever of the copy and the GPU is the bottleneck.
+        if (!last) {
+            const int wave = chol_wave_windows(h->sm_count);
+            // Full waves only -- a launch costs the latency of one factorisation however few windows it has -- except
+            // before the LAST segment: whatever is ready then is solved while the last segment is on the bus, so that
+            // only the last segment's own windows follow the copy (with the default plan that is a full wave anyway;
+            // plans with several short tail segments were measured slower, windows.plan_wave_fractions)
+            const bool before_last = s == h->n_seg - 2;
+            const int wn = before_last ? w_done - *w_solved : (w_done - *w_solved) / wave * wave;
+            if (wn > 0) {
+                if ((rc = solve_batch_windows(h, b, L, c, call, *w_solved, wn))) return rc;
+                *w_solved += wn;
+            }
+        }
+    }
+    if (s1_dev && s1_dev != S1) {
+        CU_TRY(cudaMemcpyAsync(S1, s1_dev, s1_bytes, cudaMemcpyDeviceToHost, h->stream));
+        h->need_sync = true;
+    }
+    h->seg_waited = h->n_seg;
+    h->hf_pending = false;
+    return BP_OK;
+}
+
+// Shared driver of bp_conjugate_batched / bp_jeffreys_batched / bp_estimator_batched / bp_stats_batched /
+// bp_hf_cov_batched / bp_moments_batched: validate, plan, upload the descriptors, then run the stages
+int run_batches(bp_handle* h, const bp_window_batch* b, const bp_outputs* out, int mode, bool solve, int estimator = BP_EST_NONE) {
+    if (!h || !b) return fail(BP_ERR_INVALID, "null handle or batch");
+    int rc;
+    if (solve && h->has_market && (rc = check_solver_size(h->N, estimator))) return rc;
+    const CallDesc call{mode, solve, estimator, out->T != nullptr, out->S0 != nullptr, out->S1 != nullptr};
+    const bool conj = mode == BP_MODE_CONJUGATE;
+    PlanCtx ctx = plan_ctx(h);
+    if ((rc = check_batch(ctx, b, conj, &g_err)) || (rc = check_call(ctx, b, call, &g_err))) return rc;
+    const int G = plan_chain_group(ctx, b, call);
+    ctx.stride = G >= 2 ? G : 1;       // the chain path runs only the base windows through the Gram kernel
+    Batch B;
+    Route r;
+    if ((rc = plan_batch(ctx, b, conj, &B.plan, &g_err)) || (rc = plan_route(ctx, B.plan, b, call, G, &r, &g_err))) return rc;
+    const BatchPlan& P = B.plan;
+    // every allocation / launch below must land on the handle's device, whatever the calling thread's current device
+    // is (two handles on two GPUs in one thread, or torch having switched)
+    CU_TRY(cudaSetDevice(h->device));
+    if ((rc = upload_batch(h, b, &B))) return rc;
+    if (r.hf_wait_rows > 0 && (rc = wait_hf_rows(h, r.hf_wait_rows))) return rc;
+    if ((rc = grow(h, h->ws, (size_t)r.Wc * r.L.per_window + 256))) return rc;
+    const Chunk c = carve(h->ws.p, r.L, r.Wc);
     if (P.band_ok && ((rc = grow(h, h->band_aw, (size_t)P.W * round_up(P.n - 1, 2))) ||
                       (rc = grow(h, h->band_stats, 2 * (size_t)P.W))))
         return rc;
-    if (solve && (mode == BP_MODE_CONJUGATE || estimator != BP_EST_NONE) && !(b->risk_aversion != 0.0))
-        return fail(BP_ERR_INVALID, "risk_aversion must be non-zero");
-    if (estimator == BP_EST_JORION && P.n - 1 - N - 2 <= 0)
-        return fail(BP_ERR_INVALID, "Jorion needs T - N - 2 > 0 (T = rolling_window - 1 returns, :879)");
 
-    const bool any_gram = out->T || out->S0 || out->S1 || solve;
-    if (any_gram && !pipelined) {
-        if (mode == BP_MODE_CONJUGATE && A.inner && !P.presum) {
-            launch_gather_rows_indexed(h->lr_hf, h->ld, B.hf_starts, h->R, 0, A.nb[0], h->stream);
-            h->launches++;
-            CU_TRY(cudaGetLastError());
-        }
-        if (mode == BP_MODE_CONJUGATE && (out->S0 || out->S1 || solve || P.presum) && (rc = run_block_precompute(h, B, 0))) return rc;
-        if (mode == BP_MODE_CONJUGATE && P.presum) {
-            // scans of the day blocks: column sums (vectors) and Gram tiles, suffix' and prefix per chunk
-            StageTimer tm(h, BP_STAGE_GRAM);
-            const int nt = (N + GRAM_TILE - 1) / GRAM_TILE;
-            launch_block_col_sums(h->lr_hf, h->ld, B.hf_starts, 0, A.nb[0], h->vstore.p, h->stream);
-            launch_vec_scan(h->vstore.p, h->ld, h->lr_hf, B.hf_starts, A.nb[0], A.chunk, h->stream);
-            launch_tile_scan(h->store[0][0].p, nt * (nt + 1) / 2, nt, h->lr_hf, h->ld, B.hf_starts, A.nb[0], A.chunk, h->stream);
-            h->launches += 3;
-            CU_TRY(cudaGetLastError());
-        }
-        if ((out->T || out->S1 || solve) && (rc = run_block_precompute(h, B, 1))) return rc;
-    }
-    // Cholesky + solves of the windows [ws, ws+wn) of the workspace; the reference evaluates (1/gamma) * nu (:836,:849)
-    auto solve_range = [&](int ws, int wn, int stride = 1) -> int {
-        return solve_windows(h, chunk_at(c, L, ws % Wc), L, wn, stride, mode, estimator, P.n - 1, 1.0 / b->risk_aversion);
-    };
+    if ((call.T || call.S0 || call.S1 || solve) && !r.pipelined && (rc = run_blocks(h, B, call))) return rc;
     int w_solved = 0;          // windows already solved by the pipelined path (full waves, between the upload segments)
-    if (pipelined) {
-        if ((rc = run_block_precompute(h, B, 1))) return rc;          // daily blocks do not wait for the bars
-        int w_done = 0, k_done[2] = {0, 0};
-        // S1 has to leave every segment's windows before the full waves below factorise them in place.  A device S1 is
-        // unpacked straight into the output; a host S1 into the staging buffer (grown once, here), which is copied out
-        // after the last segment, so that no segment waits for the host.
-        double* s1_dev = nullptr;
-        const size_t s1_bytes = sizeof(double) * (size_t)P.W * N * N;
-        if (out->S1) {
-            if (is_device_ptr(out->S1)) {
-                s1_dev = out->S1;
-            } else {
-                if (h->need_sync) {
-                    CU_TRY(cudaStreamSynchronize(h->stream));
-                    h->need_sync = false;
-                }
-                if ((rc = grow(h, h->stage, s1_bytes))) return rc;
-                s1_dev = reinterpret_cast<double*>(h->stage.p);
-            }
-        }
-        for (int s = h->seg_waited; s < h->n_seg; ++s) {
-            CU_TRY(cudaStreamWaitEvent(h->stream, h->ev_seg[s], 0));
-            const bool last = s == h->n_seg - 1;
-            const long long r_end = h->seg_end[s];
-            if ((rc = hf_returns(h, h->lr_hf_done, r_end))) return rc;
-            h->lr_hf_done = r_end;
-            int k_ready[2];
-            for (int l = 0; l < 2; ++l) {
-                k_ready[l] = A.nb[l];
-                if (!last && l == 0 && A.inner) {
-                    // day block k is complete once the bars below starts[k+1] have arrived
-                    const long long k = std::upper_bound(A.starts.begin() + 1, A.starts.end(), (int)std::min<long long>(r_end, 0x7fffffff)) -
-                                        (A.starts.begin() + 1);
-                    k_ready[l] = (int)std::min<long long>(A.nb[l], std::max<long long>(k, k_done[l]));
-                } else if (!last && A.blk[l] > 0) {
-                    const long long k = floor_div(r_end, A.blk[l]) - A.bmin[l];
-                    k_ready[l] = (int)std::min<long long>(A.nb[l], std::max<long long>(k, k_done[l]));
-                }
-            }
-            if (A.inner) {
-                launch_gather_rows_indexed(h->lr_hf, h->ld, B.hf_starts, h->R, k_done[0], k_ready[0], h->stream);
-                h->launches++;
-                CU_TRY(cudaGetLastError());
-            }
-            if ((rc = run_block_precompute(h, B, 0, k_done, k_ready))) return rc;
-            k_done[0] = k_ready[0];
-            k_done[1] = k_ready[1];
-            int w_end = w_done;
-            if (last) w_end = P.W;
-            else while (w_end < P.W && (long long)b->hf_hi[w_end] <= r_end) ++w_end;
-            if (w_end > w_done) {
-                const Chunk cw = chunk_at(c, L, w_done);
-                PrepParams pp = prep_params(h, b, B, L, cw, w_done, mode);
-                {
-                    StageTimer tm(h, BP_STAGE_PREP);
-                    CU_TRY(launch_window_prep(pp, w_end - w_done, h->stream, h->D));
-                    h->launches += pp.use_band ? 2 : 0;
-                }
-                h->launches++;
-                if ((rc = run_gram(h, gram_params(h, B, L, cw, w_done, w_end - w_done, GRAM_S1), P.resampled))) return rc;
-                if (s1_dev) {
-                    launch_unpack_sym(cw.S, L.win_stride, L.ldS, N, w_end - w_done, s1_dev + (size_t)w_done * N * N, h->stream);
-                    h->launches++;
-                    CU_TRY(cudaGetLastError());
-                }
-                w_done = w_end;
-            }
-            // Solve the full waves of windows that are ready: the compute stream would otherwise idle until the next
-            // segment arrives (the copy takes longer than the statistics / Gram stages), and after the last segment
-            // only the remainder (less than one wave) is left instead of every window.  Full waves cost nothing in
-            // occupancy whichever of the copy and the GPU is the bottleneck.
-            if (!last) {
-                const int wave = chol_wave_windows(h->sm_count);
-                // Full waves only -- a launch costs the latency of one factorisation however few windows it has -- except
-                // before the LAST segment: whatever is ready then is solved while the last segment is on the bus, so that
-                // only the last segment's own windows follow the copy (with the default plan that is a full wave anyway;
-                // plans with several short tail segments were measured slower, windows.plan_wave_fractions)
-                const bool before_last = s == h->n_seg - 2;
-                const int wn = before_last ? w_done - w_solved : (w_done - w_solved) / wave * wave;
-                if (wn > 0) {
-                    if ((rc = solve_range(w_solved, wn))) return rc;
-                    w_solved += wn;
-                }
-            }
-        }
-        if (s1_dev && s1_dev != out->S1) {
-            CU_TRY(cudaMemcpyAsync(out->S1, s1_dev, s1_bytes, cudaMemcpyDeviceToHost, h->stream));
-            h->need_sync = true;
-        }
-        h->seg_waited = h->n_seg;
-        h->hf_pending = false;
-    }
-    for (int w0 = 0; w0 < P.W; w0 += Wc) {
-        const int wc = std::min(Wc, P.W - w0);
-        const size_t ov = (size_t)w0 * N, om = (size_t)w0 * N * N;
-        if (!pipelined) {
-            PrepParams pp = prep_params(h, b, B, L, c, w0, mode);
-            if (estimator != BP_EST_NONE) pp.beta_den = P.n - 1;       // sample covariance: centre with 1/m, m = n-1 returns
-            {
-                StageTimer tm(h, BP_STAGE_PREP);
-                CU_TRY(launch_window_prep(pp, wc, h->stream, h->D));
-                h->launches += pp.use_band ? (mode == BP_MODE_JEFFREYS ? 1 : 2) : 0;
-            }
-            h->launches++;
-        }
-        if (out->T) {
-            rc = run_gram(h, gram_params(h, B, L, c, w0, wc, GRAM_T), P.resampled);
-            if (rc) return rc;
-            rc = emit_sym(h, c.S, L, wc, out->T + om);
-            if (rc) return rc;
-        }
-        // pre-summed day blocks: S0 w0, v0, c and rhs are finished from the G w0 partials of the first Gram launch
-        // that contracts the intraday phase (it must precede the solve and every emit of rhs / scalars)
-        bool post_pending = mode == BP_MODE_CONJUGATE && P.presum;
-        auto run_post = [&]() -> int {
-            if (!post_pending) return BP_OK;
-            post_pending = false;
-            PostParams q{};
-            q.n_windows = wc;
-            q.n_assets = N;
-            q.ldv = L.ldv;
-            q.mv_part = c.mv;
-            q.w0 = c.w0;
-            q.gvec = c.gvec;
-            q.t = c.t;
-            q.s0w0 = c.s0w0;
-            q.rhs = c.rhs;
-            q.scal = c.scal;
-            StageTimer tm(h, BP_STAGE_PREP);
-            CU_TRY(launch_conj_post(q, h->stream));
-            h->launches++;
-            return BP_OK;
-        };
-        if ((out->S0 || (post_pending && !solve && !out->S1)) && mode == BP_MODE_CONJUGATE) {
-            rc = run_gram(h, gram_params(h, B, L, c, w0, wc, GRAM_S0), P.resampled);
-            if (rc) return rc;
-            if ((rc = run_post())) return rc;
-            rc = emit_sym(h, c.S, L, wc, out->S0 ? out->S0 + om : nullptr);
-            if (rc) return rc;
-        }
-        if (solve || out->S1) {
-            if (!pipelined) {
-                GramParams gp = gram_params(h, B, L, c, w0, wc, mode == BP_MODE_CONJUGATE ? GRAM_S1 : GRAM_J);
-                if (G >= 2) {                      // base windows only
-                    gp.w_stride = G;
-                    gp.n_windows = (wc + G - 1) / G;
-                }
-                rc = run_gram(h, gp, P.resampled);
-                if (rc) return rc;
-                if ((rc = run_post())) return rc;
-            }
-            if (estimator == BP_EST_SHRINKAGE) {
-                // C = X_c'X_c  ->  m Sigma_LW / (1 - shrinkage) = C + rho I, rhs = t / (1 - shrinkage), in place (:727-729)
-                ShrinkParams q{};
-                q.n_windows = wc;
-                q.n_assets = N;
-                q.n_window = P.n;
-                q.ld = h->ld;
-                q.ldv = L.ldv;
-                q.ldS = L.ldS;
-                q.win_stride = L.win_stride;
-                q.lr_daily = P.resampled ? h->lr_w : h->lr_d;
-                q.rf_row = P.resampled ? h->rf_w : h->rf_row;
-                q.day_row = B.day_row + w0;
-                q.extra_row = B.extra_row ? B.extra_row + w0 : nullptr;
-                q.span_days = B.span + w0;
-                q.t = c.t;
-                q.S = c.S;
-                q.rhs = c.rhs;
-                q.scal = c.scal;
-                StageTimer tm(h, BP_STAGE_PREP);
-                CU_TRY(launch_lw_shrink(q, h->stream));
-                h->launches++;
-            }
-            rc = emit_sym(h, c.S, L, wc, out->S1 && !pipelined ? out->S1 + om : nullptr);
-            if (rc) return rc;
-        }
-        if (solve && G >= 2) {
-            // factorise the base windows, then solve the other windows of each group relative to their base
-            if ((rc = solve_range(w0, (wc + G - 1) / G, G))) return rc;
-            ChainParams cp{};
-            cp.n_windows = wc;
-            cp.group = G;
-            cp.n_assets = N;
-            cp.n_window = P.n;
-            cp.estimator = estimator;
-            cp.ld = h->ld;
-            cp.ldv = L.ldv;
-            cp.ldS = L.ldS;
-            cp.win_stride = L.win_stride;
-            cp.inv_gamma = 1.0 / b->risk_aversion;
-            cp.lr_daily = h->lr_d;
-            cp.day_row = B.day_row + w0;
-            cp.S = c.S;
-            cp.t = c.t;
-            cp.pvec = c.pvec;
-            cp.w1 = c.w1;
-            cp.nu = c.nu;
-            cp.weights = c.weights;
-            cp.scal = c.scal;
-            cp.status = c.status;
-            {
-                StageTimer tm(h, BP_STAGE_CHAIN);
-                CU_TRY(launch_jeffreys_chain(cp, h->stream));
-            }
-            h->launches++;
-            h->work_chained += wc - (wc + G - 1) / G;
-        }
-        if (solve) {
-            if (G < 2 && (rc = solve_range(w0 + w_solved, wc - w_solved))) return rc;
-            if ((rc = emit_vec(h, c.weights, L, wc, out->weights ? out->weights + ov : nullptr))) return rc;
-            if ((rc = emit_vec(h, c.nu, L, wc, out->nu ? out->nu + ov : nullptr))) return rc;
-            if ((rc = emit_vec(h, c.w1, L, wc, out->w1 ? out->w1 + ov : nullptr))) return rc;
-            if ((rc = emit_raw(h, c.status, sizeof(int) * (size_t)wc, out->status ? out->status + w0 : nullptr))) return rc;
-        }
-        if ((rc = emit_vec(h, c.t, L, wc, out->t ? out->t + ov : nullptr))) return rc;
-        if (mode == BP_MODE_CONJUGATE) {
-            if ((rc = emit_vec(h, c.w0, L, wc, out->w0 ? out->w0 + ov : nullptr))) return rc;
-        }
-        if ((rc = emit_vec(h, c.rhs, L, wc, out->rhs ? out->rhs + ov : nullptr))) return rc;
-        if ((rc = emit_raw(h, c.scal, sizeof(double) * (size_t)wc * BP_NSCAL,
-                           out->scalars ? out->scalars + (size_t)w0 * BP_NSCAL : nullptr))) return rc;
-        // the workspace is reused by the next chunk: host-bound copies must have drained
-        if (w0 + wc < P.W && h->need_sync) {
-            CU_TRY(cudaStreamSynchronize(h->stream));
-            h->need_sync = false;
-        }
+    if (r.pipelined && (rc = run_pipelined(h, b, B, r, c, call, out->S1, &w_solved))) return rc;
+    const size_t NN = (size_t)h->N * h->N;
+    const bool post = conj && P.presum;        // each chunk's first Gram launch of the intraday phase runs run_post
+    for (int w0 = 0; w0 < P.W; w0 += r.Wc) {
+        const int wc = std::min(r.Wc, P.W - w0);
+        if (!r.pipelined && (rc = run_prep(h, b, B, r.L, c, w0, wc, call))) return rc;
+        if (out->T && ((rc = run_gram(h, gram_params(h, B, r.L, c, w0, wc, GRAM_T), P.resampled)) ||
+                       (rc = emit_dense(h, c.S, r.L, wc, true, out->T + w0 * NN))))
+            return rc;
+        const bool s0 = conj && (out->S0 || (post && !solve && !out->S1));
+        if (s0 && (rc = run_s0(h, B, r.L, c, w0, wc, post, out->S0 ? out->S0 + w0 * NN : nullptr))) return rc;
+        // (the pipelined path has run the S1 Gram and unpacked S1)
+        if ((solve || out->S1) && !r.pipelined &&
+            (rc = run_s1(h, B, r, c, w0, wc, call, post && !s0, out->S1 ? out->S1 + w0 * NN : nullptr)))
+            return rc;
+        if (solve && r.G >= 2 && (rc = run_chain(h, b, B, r, c, w0, wc, call))) return rc;
+        if (solve && r.G < 2 && (rc = solve_batch_windows(h, b, r.L, c, call, w_solved, wc - w_solved))) return rc;
+        if ((rc = emit_chunk(h, c, r.L, out, w0, wc, P.W, solve, conj))) return rc;
     }
     return finish(h);
 }
@@ -1713,7 +1699,7 @@ int bp_backtest_batched(bp_handle* h, const bp_backtest_desc* d) {
 int bp_excess_returns(bp_handle* h, const bp_window_batch* b, double* X) {
     if (!h || !b || !X) return fail(BP_ERR_INVALID, "null argument");
     if (b->n_windows != 1) return fail(BP_ERR_INVALID, "bp_excess_returns handles one window per call");
-    int rc = check_batch(plan_ctx(h, 1), b, false, &g_err);
+    int rc = check_batch(plan_ctx(h), b, false, &g_err);
     if (rc) return rc;
     CU_TRY(cudaSetDevice(h->device));
     const int K = b->rolling_window - 1;
@@ -1812,9 +1798,9 @@ int bp_dense_posterior(bp_handle* h, const bp_dense_problem* in, const bp_dense_
         CU_TRY(cudaStreamSynchronize(st));
         return BP_OK;
     }
+    const Layout L = make_layout(N, ldv, 0, false);
     if (out->S1) {
-        const Layout L{N, ldv, ldS, rowsS, (long long)rowsS * ldS, 2, 0};
-        if ((rc = emit_sym(h, dS, L, 1, out->S1))) return rc;
+        if ((rc = emit_dense(h, dS, L, 1, true, out->S1))) return rc;
         if (h->need_sync) { CU_TRY(cudaStreamSynchronize(st)); h->need_sync = false; }
     }
     const double inv_gamma = 1.0 / in->risk_aversion;
@@ -1824,7 +1810,6 @@ int bp_dense_posterior(bp_handle* h, const bp_dense_problem* in, const bp_dense_
         h->launches++;
         CU_TRY(cudaMemcpyAsync(dw1, dw1in, sizeof(double) * N, cudaMemcpyDeviceToDevice, st));
     } else {
-        const Layout L{N, ldv, ldS, rowsS, (long long)rowsS * ldS, 2, 0};
         Chunk c{};
         c.S = dS; c.rhs = drhs; c.scal = dscal; c.w1 = dw1; c.nu = dnu; c.weights = dwts; c.status = dstatus;
         if ((rc = solve_windows(h, c, L, 1, 1, in->jeffreys ? BP_MODE_JEFFREYS : BP_MODE_CONJUGATE, BP_EST_NONE, 0, inv_gamma)))
@@ -1858,15 +1843,7 @@ int bp_solve_batched(bp_handle* h, const bp_solve_desc* d, const bp_outputs* out
     if (rc) return rc;
     CU_TRY(cudaSetDevice(h->device));
     // the layout of bp_dense_posterior for W windows
-    Layout L{};
-    L.N = N;
-    L.ldv = round_up(N, 16);
-    L.ldS = round_up(N, 32);
-    L.rowsS = L.ldS + 8;
-    L.win_stride = (long long)L.rowsS * L.ldS;
-    L.y_stride = 2;
-    L.mv_stride = 0;
-    L.per_window = sizeof(double) * ((size_t)L.win_stride + 9 * (size_t)L.ldv + BP_NSCAL + (size_t)L.y_stride) + 16;
+    const Layout L = make_layout(N, round_up(N, 16), 0, false);
     const int Wc = (int)std::min<size_t>((size_t)W, std::max<size_t>(1, h->ws_limit / L.per_window));
     if ((rc = grow(h, h->ws, (size_t)Wc * L.per_window + 256))) return rc;
     const Chunk c = carve(h->ws.p, L, Wc);
@@ -1885,18 +1862,8 @@ int bp_solve_batched(bp_handle* h, const bp_solve_desc* d, const bp_outputs* out
             CU_TRY(cudaMemcpy2DAsync(c.scal + BP_SCAL_N1, sizeof(double) * BP_NSCAL, d->n1 + w0, sizeof(double), sizeof(double),
                                      wc, cudaMemcpyHostToDevice, st));
         if ((rc = solve_windows(h, c, L, wc, 1, mode, d->estimator, d->n_returns, 1.0 / d->risk_aversion))) return rc;
-        const size_t ov = (size_t)w0 * N;
-        if ((rc = emit_vec(h, c.weights, L, wc, out->weights ? out->weights + ov : nullptr))) return rc;
-        if ((rc = emit_vec(h, c.nu, L, wc, out->nu ? out->nu + ov : nullptr))) return rc;
-        if ((rc = emit_vec(h, c.w1, L, wc, out->w1 ? out->w1 + ov : nullptr))) return rc;
-        if ((rc = emit_raw(h, c.status, sizeof(int) * (size_t)wc, out->status ? out->status + w0 : nullptr))) return rc;
-        if ((rc = emit_raw(h, c.scal, sizeof(double) * (size_t)wc * BP_NSCAL,
-                           out->scalars ? out->scalars + (size_t)w0 * BP_NSCAL : nullptr))) return rc;
-        // the workspace is reused by the next chunk: host-bound copies must have drained
-        if (w0 + wc < W && h->need_sync) {
-            CU_TRY(cudaStreamSynchronize(st));
-            h->need_sync = false;
-        }
+        // (t, w0 and rhs are not outputs of this call: the checks above rejected them)
+        if ((rc = emit_chunk(h, c, L, out, w0, wc, W, true, false))) return rc;
     }
     return finish(h);
 }

@@ -211,7 +211,7 @@ class knobs:
 
 
 def _per_window(N, max_m):
-    """bp_api.cu make_layout without the pre-summed mat-vec partials (the chunked test asserts the chunk count it
+    """batch_plan.cu make_layout without the pre-summed mat-vec partials (the chunked test asserts the chunk count it
     implies, so a change of the layout fails there rather than silently testing something else)."""
     ld, ldS = -(-N // 16) * 16, -(-N // 32) * 32
     return 8 * ((ldS + 8) * ldS + 9 * ld + 12 + max(max_m, 2) + (max_m & 1)) + 16
