@@ -134,7 +134,11 @@ typedef struct {
     double* w0;                 /* prior weights                 :361-380                            */
     double* rhs;                /* c S0 w0 + t                   :489                                */
     double* scalars;            /* [W][BP_NSCAL]                                                     */
-    int* status;                /* [W] 0 ok; k+1: pivot k not positive (reference would return garbage, F6) */
+    int* status;                /* [W] 0 ok; k+1: pivot k not positive (reference would return garbage, F6).
+                                   A window solved relative to a base window (bp_set_jeffreys_chain) reports its
+                                   base's status when that is non-zero, else N+1 when its own matrix is singular
+                                   relative to the base (a Gauss-Jordan pivot at or below 2^-40 of the largest entry
+                                   of its small system) or v1 <= 0 (Jorion: t'C^-1 t <= 0), else 0. */
     double* T;                  /* canonical statistic T         :180-182                            */
     double* S0;                 /* conjugate prior S             :333                                */
     double* S1;                 /* posterior S (or Jeffreys J)   :358 / :600-601                     */
@@ -188,9 +192,10 @@ int bp_set_hf_presum_min_days(bp_handle* h, int min_days);
 /* Jeffreys batches of CONSECUTIVE trade dates (calculate_mean_jeffreys_posterior_nu, :580-608): consecutive windows
  * differ by a rank 2k+4 term (k rows in, k rows out, the change of the risk-free adjustment and of t t'/n), so only
  * every `group`-th window is factorised and the others are solved relative to it by the Woodbury identity (30
- * triangular solves per group + a small elimination per window instead of a factorisation per window; 3e-14 of the
- * reference-pinned oracle at N = 500).  group in [2, 8]; 0 or 1 factorises every window.  Default 8.  Batches that
- * are not consecutive dates, weekly windows, and calls that ask for T / S1 always take the per-window path. */
+ * triangular solves per group + a small elimination per window instead of a factorisation per window).  Each solved
+ * window is held to an a-priori bound of the extended-precision solution (tests/_chain_ref.py).  group in [2, 8]; 0
+ * or 1 factorises every window.  Default 8.  Batches that are not consecutive dates, weekly windows, and calls that
+ * ask for T / S1 always take the per-window path. */
 int bp_set_jeffreys_chain(bp_handle* h, int group);
 /* Solve-stage work since the previous call (then reset): out2[0] windows factorised, out2[1] windows solved
  * relative to a base window. */

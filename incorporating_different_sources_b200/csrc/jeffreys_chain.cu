@@ -11,9 +11,10 @@
 // Only the base window is factorised (chol_solve_kernel, J_b = L L'); this kernel solves the 30 right-hand sides of a
 // group against L in one pass (Z = L^-1 R, then U'J_b^-1U = Z'Z for every pair of columns at once, then Y = L^-T Z)
 // and finishes each window with a (2k+4)-dimensional elimination: 2 N^2 * 30 / (G-1) flops per window instead of
-// N^3/3.  Measured against the reference-pinned oracle at N = 500, n = 1008: 3e-14 relative at distance k = 15
-// (cond(J) = 4e3; the low-rank identity itself holds to 1e-15) -- far inside the 1e-9 bar, and independent of k
-// because every window is expressed relative to an exactly factorised base, never as a chain of updates.
+// N^3/3.  Every window is expressed relative to an exactly factorised base, never as a chain of updates, so the error
+// does not grow with k.  tests/test_gpu_chain.py holds each window to the a-priori bound of tests/_chain_ref.py,
+// 2 k(J_w) eta_in + 2 (k(J_b) + k(J_w)) (4 sqrt(N) + 2m + 8) u; the worst ratios to it measured on a B200 are 0.05
+// (N = 1), 2e-4 (N = 31 .. 33 at the rank guard's margin) and 1.5e-6 .. 5e-7 (N = 500 .. 640).
 //
 // One CTA per group.  Shared memory: the right-hand-side block Y [Nr][33] (in place: R -> Z -> Y), a ring of six
 // 32 x 32 factor blocks (cp.async, five blocks ahead), the 32 x 32 Gram Z'Z.  Substitutions are right-looking by 32-row panels: one warp
@@ -277,6 +278,17 @@ __global__ void __launch_bounds__(CH_T, 1) jeffreys_chain_kernel(const ChainPara
         }
         row[MMAX] = active ? Wm[mycol * LDY + tcol] : 0.0;       // right-hand side U'y_t
         row[MMAX + 1] = active ? Wm[mycol * LDY + COL_ONE] : 0.0;    // second right-hand side U'y_1 (Jorion: C^-1 1)
+        // Singularity relative to the base.  A window whose own matrix is exactly singular (an asset flat over the
+        // window at a zero risk-free rate) gives a small system that is singular only in exact arithmetic: its
+        // smallest pivot is 1e-21 .. 1e-19 of max |M| in floating point, never exactly 0.  Regular windows keep
+        // pivots above 1e-9 of max |M| even at the rank guard's margin or with an asset flat at a positive rate
+        // (cond(J) ~ 1e7; tests/test_chain_reference.py).  TAU = 2^-40 ~ 9e-13 sits orders of magnitude from both.
+        double scale = 0.0;
+#pragma unroll
+        for (int c = 0; c < MMAX; ++c) scale = fmax(scale, fabs(row[c]));
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) scale = fmax(scale, __shfl_xor_sync(0xffffffffu, scale, o));
+        const double piv_min = 0x1p-40 * scale;
         bool done = !active;
         int mypiv = -1;
         bool singular = false;
@@ -292,7 +304,7 @@ __global__ void __launch_bounds__(CH_T, 1) jeffreys_chain_kernel(const ChainPara
                     const int ol = __shfl_xor_sync(0xffffffffu, bl, o);
                     if (ob > best || (ob == best && ol < bl)) { best = ob; bl = ol; }
                 }
-                if (!(best > 0.0)) singular = true;
+                if (!(best > piv_min)) singular = true;
                 const double pv = __shfl_sync(0xffffffffu, row[s], bl);
                 const double f = (lane == bl || !active) ? 0.0 : row[s] / pv;
 #pragma unroll

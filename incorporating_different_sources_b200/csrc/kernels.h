@@ -290,7 +290,9 @@ struct ChainParams {
     double* nu;
     double* weights;
     double* scal;            // [W][BP_S_COUNT] (writes v1)
-    int* status;             // [W] reads the base's flag, writes the chained windows'
+    int* status;             // [W] reads the base's flag, writes the chained windows': the base's flag when it is
+                             // non-zero, else N+1 for a window singular relative to the base (pivot <= 2^-40 max |M|)
+                             // or with v1 <= 0 (Jorion: t'C^-1 t <= 0), else 0
 };
 size_t chain_smem_bytes(int n_assets);
 int chain_max_group();

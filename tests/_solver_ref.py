@@ -39,10 +39,11 @@ def symmetric_from_lower(S: np.ndarray) -> np.ndarray:
 
 
 def refined_solve(S: np.ndarray, b: np.ndarray, steps: int = 3) -> np.ndarray:
-    """x = S^-1 b (S symmetric positive definite, float64; b [N] or [N][k]) to about kappa * 5e-20, as np.longdouble."""
+    """x = S^-1 b (S symmetric positive definite, float64 or np.longdouble; b [N] or [N][k]) to about kappa * 5e-20, as
+    np.longdouble.  The residuals are taken with S as given (a longdouble S is factorised rounded to float64)."""
     require_extended_precision()
-    cf = sla.cho_factor(S, lower=True, check_finite=True)
-    S_ld = S.astype(LD)
+    cf = sla.cho_factor(np.asarray(S, dtype=np.float64), lower=True, check_finite=True)
+    S_ld = np.asarray(S, dtype=LD)
     b_ld = np.asarray(b, dtype=LD)
     x = sla.cho_solve(cf, np.asarray(b, dtype=np.float64)).astype(LD)
     for _ in range(steps):
@@ -194,14 +195,15 @@ class _Err:
         return _Err(v, np.sum(np.abs(w) * self.e) + n * U * np.sum(np.abs(w * self.v)))
 
 
-def jorion_reference(C: np.ndarray, t: np.ndarray, m: int, risk_aversion: float, kappa: float):
+def jorion_reference(C: np.ndarray, t: np.ndarray, m: int, risk_aversion: float, kappa: float, eps: float = None):
     """Jorion's Bayes-Stein portfolio (oracle.bayes_oracle.jorion_window, portfolio_calculations.py:851-895) restated
     on the centred Gram C = (m-1) V_hat, t = m mu_hat and m, evaluated on the refined y = C^-1 t and z = C^-1 1.
     Returns values and first-order error bounds: y and z carry the forward-error bound, every later operation its
-    own float64 rounding, as the solver's epilogue evaluates it."""
+    own float64 rounding, as the solver's epilogue evaluates it.  ``eps`` replaces the solver's forward-error bound of
+    y and z (relative, infinity norm) where another stage produced them (the chain of tests/_chain_ref.py)."""
     N = C.shape[0]
-    yz = refined_solve(C, np.stack([t, np.ones(N)], axis=1))
-    eps = forward_bound(N, kappa)
+    yz = refined_solve(C, np.stack([np.asarray(t, dtype=LD), np.ones(N, dtype=LD)], axis=1))
+    eps = forward_bound(N, kappa) if eps is None else eps
     y = _Err(yz[:, 0], eps * np.max(np.abs(yz[:, 0])))
     z = _Err(yz[:, 1], eps * np.max(np.abs(yz[:, 1])))
     md, Nd = float(m), float(N)
