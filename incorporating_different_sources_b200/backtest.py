@@ -254,6 +254,8 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
     needs_hf = conj or strat in ("vw", "ew")
     if portfolio_spec["rolling_window_frequency"] not in ("daily", "weekly") and strat not in ("vw", "ew"):
         raise NotImplementedError("monthly windows: resample('M') was removed from pandas (SURVEY F10)")
+    if strat not in ("vw", "ew", "jeffreys", "jorion", "shrinkage") and not conj:
+        raise ValueError("Unknown weights spec.")
     rf_dates = rf_df.index.values.astype("datetime64[ns]")
     rf_vals = rf_df.iloc[:, 0].to_numpy(dtype=np.float64)
     # n0 per rebalance date from the MCM series' OWN calendar (7 observations a week for FRED's EPU index; the
@@ -287,8 +289,8 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
             small.append((idx, rows))
             continue
         try:
-            outcome[idx] = _per_set(engine, portfolio_spec, spec, strat, idx, rows, dates_ns, reb_pos, hf_ts, rf_dates,
-                                    rf_vals, prior_n_all, hf_lookback_days, estimate)
+            outcome[idx] = _per_set(engine, spec, strat, idx, rows, dates_ns, reb_pos, hf_ts, rf_dates, rf_vals,
+                                    prior_n_all, hf_lookback_days, estimate)
         except Exception as e:          # raised below, in its set's turn
             outcome[idx] = e
     n_calls = 0
@@ -306,49 +308,45 @@ def _batched_weights(engine, portfolio_spec, market_data, dates_all, reb_pos, un
     return W, member
 
 
-def _per_set(engine, portfolio_spec, spec, strat, idx, rows, dates_ns, reb_pos, hf_ts, rf_dates, rf_vals, prior_n_all,
+def _plan_windows(spec, strat, dates_ns, d_idx, hf_ts, rf_dates, rf_vals, hf_lookback_days):
+    """The windows of the trade-date rows ``d_idx`` on the full calendar, as both asset-set routes evaluate them:
+    (ResampledRows, WindowBatch) for weekly windows, (None, WindowBatch) for daily ones.  ``spec`` is the spec the
+    windows are planned with (for vw / ew the 3-price daily conjugate spec whose prior weights they read)."""
+    need_hf = strat in ("vw", "ew") or strat.startswith("conjugate")
+    look = hf_lookback_days if strat.startswith("conjugate") else None
+    hf = hf_ts if need_hf else None
+    if spec["rolling_window_frequency"] == "weekly":
+        return plan_weekly_windows(spec, dates_ns, d_idx, rf_dates, rf_vals, None, hf, hf_lookback_days=look,
+                                   need_hf=need_hf)
+    return None, plan_daily_windows(spec, dates_ns, d_idx, hf, hf_lookback_days=look, need_hf=need_hf)
+
+
+def _set_slice(batch, n_days, n_hf_rows):
+    """Pool rows of one asset set's own working market (``select_market``) for a batch planned on the full calendar:
+    daily windows get the rows they read and their intraday look-backs with one row in front (``hf_lo - 1``, as
+    ``stack_windows`` keeps it: an empty selection is not a market), and the batch is shifted onto that slice in place;
+    weekly windows keep the whole history addressable.  Returns (day_lo, day_hi, hf_lo, hf_hi)."""
+    if batch.resampled:
+        return 0, n_days, 0, (0 if batch.hf_lo is None else n_hf_rows)
+    day_lo, day_hi = int(batch.day_row.min()) - (batch.rolling_window - 1), int(batch.day_row.max()) + 1
+    batch.day_row = (batch.day_row - day_lo).astype(np.int32)
+    if batch.hf_lo is None:
+        return day_lo, day_hi, 0, 0
+    hf_lo, hf_hi = max(int(batch.hf_lo.min()) - 1, 0), int(batch.hf_hi.max())
+    batch.hf_lo = (batch.hf_lo - hf_lo).astype(np.int32)
+    batch.hf_hi = (batch.hf_hi - hf_lo).astype(np.int32)
+    return day_lo, day_hi, hf_lo, hf_hi
+
+
+def _per_set(engine, spec, strat, idx, rows, dates_ns, reb_pos, hf_ts, rf_dates, rf_vals, prior_n_all,
              hf_lookback_days, estimate):
     """One asset set on a working market of its own: its columns, the daily rows its windows read and their intraday
     look-backs, gathered from the pool; one batched call."""
-    conj = strat.startswith("conjugate")
-    needs_hf = conj or strat in ("vw", "ew")
-    weekly = portfolio_spec["rolling_window_frequency"] == "weekly" and strat not in ("vw", "ew")
-    day = np.timedelta64(1, "D")
-    cols = list(idx)
     d_idx = np.asarray([reb_pos[r] for r in rows], dtype=np.int64)
-    if weekly:
-        day_lo, hf_lo, hf_hi = 0, 0, (len(hf_ts) if needs_hf else 0)       # weekly closes: the whole history stays addressable
-        day_hi = len(dates_ns)
-    else:
-        n = int(spec["rolling_window"])
-        day_lo, day_hi = int(d_idx.min()) - (n - 1), int(d_idx.max()) + 1
-        if day_lo < 0:
-            raise ValueError(f"a window of {n} prices needs {n - 1} rows before the trade date")
-        hf_lo = hf_hi = 0
-        if needs_hf:
-            Dd = hf_lookback_days if (hf_lookback_days is not None and conj) else HF_LOOKBACK_DAYS[spec["rolling_window_frequency"]]
-            hf_lo = int(np.searchsorted(hf_ts, dates_ns[int(d_idx.min())] - Dd * day + day, side="right"))
-            hf_hi = int(np.searchsorted(hf_ts, dates_ns[int(d_idx.max())] + day, side="right"))
-            hf_lo = max(hf_lo - 1, 0)          # keep one row in front: an empty selection is not a market
-    engine.select_market(cols, day_lo, day_hi, hf_lo, hf_hi)
-    if strat in ("vw", "ew"):
-        batch = plan_daily_windows(spec, dates_ns, d_idx, hf_ts, row_offset=day_lo, hf_row_offset=hf_lo)
-    elif conj:
-        if weekly:
-            rows_w, batch = plan_weekly_windows(portfolio_spec, dates_ns, d_idx, rf_dates, rf_vals, None, hf_ts,
-                                                hf_lookback_days=hf_lookback_days)
-            engine.set_resampled(rows_w)
-        else:
-            batch = plan_daily_windows(portfolio_spec, dates_ns, d_idx, hf_ts, hf_lookback_days=hf_lookback_days,
-                                       row_offset=day_lo, hf_row_offset=hf_lo)
-    elif strat in ("jeffreys", "jorion", "shrinkage"):
-        if weekly:
-            rows_w, batch = plan_weekly_windows(portfolio_spec, dates_ns, d_idx, rf_dates, rf_vals, None, need_hf=False)
-            engine.set_resampled(rows_w)
-        else:
-            batch = plan_daily_windows(portfolio_spec, dates_ns, d_idx, need_hf=False, row_offset=day_lo)
-    else:
-        raise ValueError("Unknown weights spec.")
+    rows_w, batch = _plan_windows(spec, strat, dates_ns, d_idx, hf_ts, rf_dates, rf_vals, hf_lookback_days)
+    engine.select_market(list(idx), *_set_slice(batch, len(dates_ns), len(hf_ts)))
+    if rows_w is not None:
+        engine.set_resampled(rows_w)
     return _evaluate(engine, strat, batch, prior_n_all, rows, estimate)
 
 
@@ -392,19 +390,8 @@ def _stacked_weights(engine, spec, strat, sets, dates_ns, reb_pos, hf_ts, rf_dat
     the per-set route plans them, relocated into stacked working markets (``stack_windows``) of one N each and
     evaluated per batch.  ``outcome[columns]`` receives each set's results, row for row as its own call would return
     them, or the exception its planning or its batch raised.  Returns the number of batched calls."""
-    weekly = spec["rolling_window_frequency"] == "weekly" and strat not in ("vw", "ew")
-    need_hf = strat in ("vw", "ew") or strat.startswith("conjugate")
-    look = hf_lookback_days if strat.startswith("conjugate") else None
-    if strat not in ("vw", "ew", "jeffreys", "jorion", "shrinkage") and not strat.startswith("conjugate"):
-        for idx, _ in sets:
-            outcome[idx] = ValueError("Unknown weights spec.")
-        return 0
-
     def plan(d):
-        if weekly:
-            return plan_weekly_windows(spec, dates_ns, d, rf_dates, rf_vals, None, hf_ts if need_hf else None,
-                                       hf_lookback_days=look, need_hf=need_hf)
-        return None, plan_daily_windows(spec, dates_ns, d, hf_ts if need_hf else None, hf_lookback_days=look, need_hf=need_hf)
+        return _plan_windows(spec, strat, dates_ns, d, hf_ts, rf_dates, rf_vals, hf_lookback_days)
 
     d_of = lambda rows: np.asarray(reb_pos, dtype=np.int64)[np.asarray(rows, dtype=np.int64)]
     sets = sorted(sets, key=lambda s: len(s[0]))                          # windows of one N next to each other

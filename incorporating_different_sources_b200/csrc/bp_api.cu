@@ -1310,12 +1310,18 @@ static int finish_market(bp_handle* h) {
     return BP_OK;
 }
 
-static int upload_market_impl(bp_handle* h, const bp_market_desc* m, bool blocking) {
-    if (!h || !m) return fail(BP_ERR_INVALID, "null handle or market");
+// the checks the working market (noun "market") and the pool (noun "pool") share; the pool ignores mcm
+static int check_market_desc(const bp_market_desc* m, const char* noun) {
     if (m->n_assets <= 0 || m->n_days < 2 || !m->prices || !m->rf_row)
-        return fail(BP_ERR_INVALID, "market needs n_assets > 0, n_days >= 2, prices and rf_row");
+        return fail(BP_ERR_INVALID, "%s needs n_assets > 0, n_days >= 2, prices and rf_row", noun);
     if (m->n_hf_rows < 0 || (m->n_hf_rows > 0 && !m->hf_prices)) return fail(BP_ERR_INVALID, "hf_prices missing");
     if (m->n_hf_rows > 0x7fffffffLL) return fail(BP_ERR_INVALID, "too many intraday rows for int32 row indices");
+    return BP_OK;
+}
+
+static int upload_market_impl(bp_handle* h, const bp_market_desc* m, bool blocking) {
+    if (!h || !m) return fail(BP_ERR_INVALID, "null handle or market");
+    if (int rc = check_market_desc(m, "market")) return rc;
     if (m->n_mcm < 0 || (m->n_mcm > 0 && !m->mcm)) return fail(BP_ERR_INVALID, "mcm missing");
     CU_TRY(cudaSetDevice(h->device));
     const int N = m->n_assets, D = m->n_days;
@@ -1398,10 +1404,7 @@ int bp_upload_pool(bp_handle* h, const bp_market_desc* m) {
     CU_TRY(cudaStreamSynchronize(h->stream));            // earlier gathers may still read the old pool
     free_pool(h);
     if (!m) return BP_OK;                                  // a null market releases the pool
-    if (m->n_assets <= 0 || m->n_days < 2 || !m->prices || !m->rf_row)
-        return fail(BP_ERR_INVALID, "pool needs n_assets > 0, n_days >= 2, prices and rf_row");
-    if (m->n_hf_rows < 0 || (m->n_hf_rows > 0 && !m->hf_prices)) return fail(BP_ERR_INVALID, "hf_prices missing");
-    if (m->n_hf_rows > 0x7fffffffLL) return fail(BP_ERR_INVALID, "too many intraday rows for int32 row indices");
+    if (int rc = check_market_desc(m, "pool")) return rc;
     const size_t N = (size_t)m->n_assets, D = (size_t)m->n_days, R = (size_t)m->n_hf_rows;
     cudaStream_t st = h->stream;
     CU_TRY(cudaMalloc(&h->pool_prices, sizeof(double) * D * N));
@@ -1423,99 +1426,27 @@ int bp_upload_pool(bp_handle* h, const bp_market_desc* m) {
     return BP_OK;
 }
 
-int bp_select_market(bp_handle* h, const bp_pool_select* s) {
-    if (!h || !s) return fail(BP_ERR_INVALID, "null handle or selection");
-    if (!h->pool_prices) return fail(BP_ERR_STATE, "no pool resident: call bp_upload_pool first");
-    if (s->n_cols <= 0 || !s->cols) return fail(BP_ERR_INVALID, "selection needs at least one column");
-    if (s->day_lo < 0 || s->day_hi > h->pool_D || s->day_hi - s->day_lo < 2)
-        return fail(BP_ERR_INVALID, "daily row range [%d, %d) outside the pool's %d rows (or shorter than 2)", s->day_lo, s->day_hi, h->pool_D);
-    if (s->hf_lo < 0 || s->hf_hi < s->hf_lo || s->hf_hi > h->pool_R)
-        return fail(BP_ERR_INVALID, "intraday row range outside the pool");
-    for (int j = 0; j < s->n_cols; ++j)
-        if (s->cols[j] < 0 || s->cols[j] >= h->pool_N) return fail(BP_ERR_INVALID, "column %d outside the pool's %d columns", s->cols[j], h->pool_N);
-    CU_TRY(cudaSetDevice(h->device));
-    const int N = s->n_cols, D = s->day_hi - s->day_lo;
-    const long long R = s->hf_hi - s->hf_lo;
-    int rc;
-    if ((rc = begin_market(h, N, D, R, 0))) return rc;
-    h->has_caps = h->pool_caps != nullptr;
-    cudaStream_t st = h->stream;
-    if ((rc = grow(h, h->pool_cols, (size_t)N))) return rc;
-    // (pageable host memory: the copy is staged before the call returns, so the caller's array may go away; stream
-    // order keeps earlier gathers, which read the previous column list, ahead of it)
-    CU_TRY(cudaMemcpyAsync(h->pool_cols.p, s->cols, sizeof(int) * (size_t)N, cudaMemcpyHostToDevice, st));
-    const long long pN = h->pool_N;
-    launch_gather_cols(h->pool_prices + (size_t)s->day_lo * pN, pN, h->prices, N, D, h->pool_cols.p, h->sm_count, st);
-    h->launches++;
-    if (h->pool_caps) {
-        launch_gather_cols(h->pool_caps + (size_t)s->day_lo * pN, pN, h->caps, N, D, h->pool_cols.p, h->sm_count, st);
-        h->launches++;
-    }
-    CU_TRY(cudaMemcpyAsync(h->rf_row, h->pool_rf + s->day_lo, sizeof(double) * (size_t)D, cudaMemcpyDeviceToDevice, st));
-    if (R > 0) {
-        launch_gather_cols(h->pool_hf + (size_t)s->hf_lo * pN, pN, h->hf_prices, N, R, h->pool_cols.p, h->sm_count, st);
-        h->launches++;
-        CU_TRY(cudaEventRecord(h->ev_hf, st));
-        h->hf_pending = true;            // the first consumer computes the intraday log returns (wait_hf)
-    }
-    CU_TRY(cudaGetLastError());
-    return finish_market(h);
-}
-
-int bp_select_windows(bp_handle* h, const bp_window_select* s) {
-    if (!h || !s) return fail(BP_ERR_INVALID, "null handle or selection");
-    if (!h->pool_prices) return fail(BP_ERR_STATE, "no pool resident: call bp_upload_pool first");
-    const int W = s->n_windows, N = s->n_cols;
-    if (W <= 0 || N <= 0 || !s->cols || !s->day_lo || !s->day_hi || !s->day_off)
-        return fail(BP_ERR_INVALID, "selection needs windows, columns and daily row ranges with their offsets");
-    const bool with_hf = s->hf_lo || s->hf_hi || s->hf_off;
-    if (with_hf && (!s->hf_lo || !s->hf_hi || !s->hf_off))
-        return fail(BP_ERR_INVALID, "intraday row ranges need hf_lo, hf_hi and hf_off");
-    if (N > h->pool_N || N > 12288)      // (the gather keeps a window's column list in 48 KB of shared memory)
-        return fail(BP_ERR_INVALID, "%d columns per window: the pool has %d, a stack takes at most 12288", N, h->pool_N);
-    // [W][3] daily blocks, then [W][3] intraday blocks: (first pool row, first stack row, rows)
-    std::vector<long long> tab(6 * (size_t)W, 0);
+// The device half of every pool selection: window w's daily pool rows [tab[3w], tab[3w] + tab[3w+2]) in its columns
+// cols[w][0..N) go to working rows tab[3w+1] on, its intraday rows likewise by the [W][3] table behind (tab[3W..6W)).
+// The caller has checked columns and rows, and that the blocks tile the working market in window order.
+static int gather_pool(bp_handle* h, int W, int N, const int* cols, const std::vector<long long>& tab) {
     long long D = 0, R = 0, max_d = 0, max_r = 0;
     for (int w = 0; w < W; ++w) {
-        const int* c = s->cols + (size_t)w * N;
-        for (int j = 0; j < N; ++j)
-            if (c[j] < 0 || c[j] >= h->pool_N)
-                return fail(BP_ERR_INVALID, "window %d: column %d outside the pool's %d columns", w, c[j], h->pool_N);
-        const int lo = s->day_lo[w], hi = s->day_hi[w];
-        if (lo < 0 || hi > h->pool_D || hi <= lo)
-            return fail(BP_ERR_INVALID, "window %d: daily row range [%d, %d) outside the pool's %d rows (or empty)", w, lo, hi, h->pool_D);
-        if (s->day_off[w] != D)
-            return fail(BP_ERR_INVALID, "window %d: daily block starts at stack row %d, the blocks before it end at %lld: the blocks must tile the stack",
-                        w, s->day_off[w], D);
-        tab[3 * (size_t)w] = lo;
-        tab[3 * (size_t)w + 1] = D;
-        tab[3 * (size_t)w + 2] = hi - lo;
-        D += hi - lo;
-        max_d = std::max<long long>(max_d, hi - lo);
-        if (D > 0x7fffffffLL) return fail(BP_ERR_INVALID, "too many daily rows in the stack for int32 row indices");
-        if (!with_hf) continue;
-        const long long hlo = s->hf_lo[w], hhi = s->hf_hi[w];
-        if (hlo < 0 || hhi < hlo || hhi > h->pool_R)
-            return fail(BP_ERR_INVALID, "window %d: intraday row range [%lld, %lld) outside the pool's %lld rows", w, hlo, hhi, h->pool_R);
-        if (s->hf_off[w] != R)
-            return fail(BP_ERR_INVALID, "window %d: intraday block starts at stack row %lld, the blocks before it end at %lld: the blocks must tile the stack",
-                        w, s->hf_off[w], R);
-        tab[3 * ((size_t)W + w)] = hlo;
-        tab[3 * ((size_t)W + w) + 1] = R;
-        tab[3 * ((size_t)W + w) + 2] = hhi - hlo;
-        R += hhi - hlo;
-        max_r = std::max(max_r, hhi - hlo);
-        if (R > 0x7fffffffLL) return fail(BP_ERR_INVALID, "too many intraday rows in the stack for int32 row indices");
+        const long long nd = tab[3 * (size_t)w + 2], nh = tab[3 * ((size_t)W + w) + 2];
+        D += nd;
+        R += nh;
+        max_d = std::max(max_d, nd);
+        max_r = std::max(max_r, nh);
     }
-    if (D < 2) return fail(BP_ERR_INVALID, "the stack needs at least 2 daily rows");
     CU_TRY(cudaSetDevice(h->device));
     int rc;
     if ((rc = begin_market(h, N, (int)D, R, 0))) return rc;
     h->has_caps = h->pool_caps != nullptr;
     cudaStream_t st = h->stream;
     if ((rc = grow(h, h->pool_cols, (size_t)W * N)) || (rc = grow(h, h->stack_rows, tab.size()))) return rc;
-    // (pageable host memory: staged before the call returns, as in bp_select_market)
-    CU_TRY(cudaMemcpyAsync(h->pool_cols.p, s->cols, sizeof(int) * (size_t)W * N, cudaMemcpyHostToDevice, st));
+    // (pageable host memory: the copies are staged before the call returns, so the caller's arrays may go away; stream
+    // order keeps earlier gathers, which read the previous lists, ahead of them)
+    CU_TRY(cudaMemcpyAsync(h->pool_cols.p, cols, sizeof(int) * (size_t)W * N, cudaMemcpyHostToDevice, st));
     CU_TRY(cudaMemcpyAsync(h->stack_rows.p, tab.data(), sizeof(long long) * tab.size(), cudaMemcpyHostToDevice, st));
     const long long pN = h->pool_N;
     const long long* day_tab = h->stack_rows.p;
@@ -1534,7 +1465,68 @@ int bp_select_windows(bp_handle* h, const bp_window_select* s) {
         h->hf_pending = true;            // the first consumer computes the intraday log returns (wait_hf)
     }
     CU_TRY(cudaGetLastError());
-    if ((rc = finish_market(h))) return rc;
+    return finish_market(h);
+}
+
+int bp_select_market(bp_handle* h, const bp_pool_select* s) {
+    if (!h || !s) return fail(BP_ERR_INVALID, "null handle or selection");
+    if (!h->pool_prices) return fail(BP_ERR_STATE, "no pool resident: call bp_upload_pool first");
+    if (s->n_cols <= 0 || !s->cols) return fail(BP_ERR_INVALID, "selection needs at least one column");
+    if (s->day_lo < 0 || s->day_hi > h->pool_D || s->day_hi - s->day_lo < 2)
+        return fail(BP_ERR_INVALID, "daily row range [%d, %d) outside the pool's %d rows (or shorter than 2)", s->day_lo, s->day_hi, h->pool_D);
+    if (s->hf_lo < 0 || s->hf_hi < s->hf_lo || s->hf_hi > h->pool_R)
+        return fail(BP_ERR_INVALID, "intraday row range outside the pool");
+    for (int j = 0; j < s->n_cols; ++j)
+        if (s->cols[j] < 0 || s->cols[j] >= h->pool_N) return fail(BP_ERR_INVALID, "column %d outside the pool's %d columns", s->cols[j], h->pool_N);
+    // one window: a stack of one block
+    return gather_pool(h, 1, s->n_cols, s->cols, {s->day_lo, 0, s->day_hi - s->day_lo, s->hf_lo, 0, s->hf_hi - s->hf_lo});
+}
+
+int bp_select_windows(bp_handle* h, const bp_window_select* s) {
+    if (!h || !s) return fail(BP_ERR_INVALID, "null handle or selection");
+    if (!h->pool_prices) return fail(BP_ERR_STATE, "no pool resident: call bp_upload_pool first");
+    const int W = s->n_windows, N = s->n_cols;
+    if (W <= 0 || N <= 0 || !s->cols || !s->day_lo || !s->day_hi || !s->day_off)
+        return fail(BP_ERR_INVALID, "selection needs windows, columns and daily row ranges with their offsets");
+    const bool with_hf = s->hf_lo || s->hf_hi || s->hf_off;
+    if (with_hf && (!s->hf_lo || !s->hf_hi || !s->hf_off))
+        return fail(BP_ERR_INVALID, "intraday row ranges need hf_lo, hf_hi and hf_off");
+    if (N > h->pool_N) return fail(BP_ERR_INVALID, "%d columns per window: the pool has %d", N, h->pool_N);
+    // [W][3] daily blocks, then [W][3] intraday blocks: (first pool row, first stack row, rows)
+    std::vector<long long> tab(6 * (size_t)W, 0);
+    long long D = 0, R = 0;
+    for (int w = 0; w < W; ++w) {
+        const int* c = s->cols + (size_t)w * N;
+        for (int j = 0; j < N; ++j)
+            if (c[j] < 0 || c[j] >= h->pool_N)
+                return fail(BP_ERR_INVALID, "window %d: column %d outside the pool's %d columns", w, c[j], h->pool_N);
+        const int lo = s->day_lo[w], hi = s->day_hi[w];
+        if (lo < 0 || hi > h->pool_D || hi <= lo)
+            return fail(BP_ERR_INVALID, "window %d: daily row range [%d, %d) outside the pool's %d rows (or empty)", w, lo, hi, h->pool_D);
+        if (s->day_off[w] != D)
+            return fail(BP_ERR_INVALID, "window %d: daily block starts at stack row %d, the blocks before it end at %lld: the blocks must tile the stack",
+                        w, s->day_off[w], D);
+        tab[3 * (size_t)w] = lo;
+        tab[3 * (size_t)w + 1] = D;
+        tab[3 * (size_t)w + 2] = hi - lo;
+        D += hi - lo;
+        if (D > 0x7fffffffLL) return fail(BP_ERR_INVALID, "too many daily rows in the stack for int32 row indices");
+        if (!with_hf) continue;
+        const long long hlo = s->hf_lo[w], hhi = s->hf_hi[w];
+        if (hlo < 0 || hhi < hlo || hhi > h->pool_R)
+            return fail(BP_ERR_INVALID, "window %d: intraday row range [%lld, %lld) outside the pool's %lld rows", w, hlo, hhi, h->pool_R);
+        if (s->hf_off[w] != R)
+            return fail(BP_ERR_INVALID, "window %d: intraday block starts at stack row %lld, the blocks before it end at %lld: the blocks must tile the stack",
+                        w, s->hf_off[w], R);
+        tab[3 * ((size_t)W + w)] = hlo;
+        tab[3 * ((size_t)W + w) + 1] = R;
+        tab[3 * ((size_t)W + w) + 2] = hhi - hlo;
+        R += hhi - hlo;
+        if (R > 0x7fffffffLL) return fail(BP_ERR_INVALID, "too many intraday rows in the stack for int32 row indices");
+    }
+    if (D < 2) return fail(BP_ERR_INVALID, "the stack needs at least 2 daily rows");
+    int rc;
+    if ((rc = gather_pool(h, W, N, s->cols, tab))) return rc;
     h->stacked = true;
     h->stack_day_start.resize(W);
     h->stack_hf_start.resize(with_hf ? W : 0);

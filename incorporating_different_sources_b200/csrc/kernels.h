@@ -147,10 +147,8 @@ void launch_block_col_sums(const double* M, int ld, const int* starts, int b0, i
 void launch_vec_scan(double* vsum, int ld, const double* M, const int* starts, int nb, int chunk, cudaStream_t st);
 void launch_tile_scan(double* store, int npairs, int n_tiles_side, const double* M, int ld, const int* starts, int nb,
                       int chunk, cudaStream_t st);
-void launch_gather_cols(const double* src, long long ld_src, double* dst, int n, long long rows, const int* cols,
-                        int sm_count, cudaStream_t st);
 // per-window blocks of rows and columns stacked into one dense [sum rows][n] matrix; rows = [W][3] (first pool row,
-// first stack row, row count), cols = [W][n] or nullptr (columns 0..n-1); max_rows = the largest row count
+// first stack row, row count), cols = [W][n] or nullptr (columns 0..n-1); max_rows = the largest row count.  Any n.
 void launch_gather_window_blocks(const double* src, long long ld_src, double* dst, int n, int n_windows, const int* cols,
                                  const long long* rows, long long max_rows, cudaStream_t st);
 void launch_gather_rows_indexed(double* M, int ld, const int* src_rows, long long dst_row0, int k0, int k1, cudaStream_t st);

@@ -615,50 +615,39 @@ void launch_range_sum(const double* store, const int* ranges, int n_ranges, int 
     range_sum_kernel<<<grid, 256, 0, st>>>(store, ranges, npairs, out);
 }
 
-// dst[r][j] = src[r][cols[j]]: a column subset (any order) of a row-major matrix, dense output.  HBM bound; the reads
-// of a row are scattered over its 128-byte lines, the writes are coalesced.
-__global__ void gather_cols_kernel(const double* __restrict__ src, long long ld_src, double* __restrict__ dst, int n,
-                                   long long rows, const int* __restrict__ cols) {
-    for (long long r = blockIdx.x; r < rows; r += gridDim.x) {
-        const double* s = src + r * ld_src;
-        double* d = dst + r * n;
-        for (int j = threadIdx.x; j < n; j += blockDim.x) d[j] = s[cols[j]];
-    }
-}
+// Columns of a window staged in shared memory at a time: 48 KB, the dynamic shared memory a launch gets without opting in
+constexpr int GATHER_COL_CHUNK = 12288;
 
-void launch_gather_cols(const double* src, long long ld_src, double* dst, int n, long long rows, const int* cols,
-                        int sm_count, cudaStream_t st) {
-    if (rows <= 0 || n <= 0) return;
-    const long long want = (long long)sm_count * 16;
-    const int grid = (int)(rows < want ? rows : want);
-    gather_cols_kernel<<<grid, n >= 256 ? 256 : 128, 0, st>>>(src, ld_src, dst, n, rows, cols);
-}
-
-// Stacked working market (bp_select_windows): block w = pool rows [rows[3w], rows[3w] + rows[3w+2]) of its own columns
-// cols[w][0..n) (cols == nullptr: columns 0..n-1), written densely from stack row rows[3w+1] on.  One CTA per (window,
-// slice of rows); the window's column list sits in shared memory.  A thread keeps one column (and, for n below the
-// CTA size, one of the blockDim / n rows handled per step), so the loop has no index division, and each step stores
-// a contiguous run of the output.
+// Working market gathered from the resident pool (bp_select_market, bp_select_windows): block w = pool rows [rows[3w],
+// rows[3w] + rows[3w+2]) of its own columns cols[w][0..n) (cols == nullptr: columns 0..n-1), written densely from
+// working row rows[3w+1] on.  One CTA per (window, slice of rows); the window's column list sits in shared memory, in
+// chunks of GATHER_COL_CHUNK columns (one chunk up to that width).  A thread keeps one column (and, for a chunk narrower
+// than the CTA, one of the blockDim / nc rows handled per step), so the loop has no index division, and each step
+// stores a contiguous run of the output.  HBM bound; the reads of a row are scattered over its 128-byte lines.
 __global__ void gather_window_blocks_kernel(const double* __restrict__ src, long long ld_src, double* __restrict__ dst,
                                             int n, const int* __restrict__ cols, const long long* __restrict__ rows,
                                             int slice_rows) {
     extern __shared__ int wcols[];
     const int w = blockIdx.x;
-    for (int j = threadIdx.x; j < n; j += blockDim.x) wcols[j] = cols ? cols[(long long)w * n + j] : j;
-    __syncthreads();
     const long long s0 = rows[3 * (long long)w], d0 = rows[3 * (long long)w + 1], nr = rows[3 * (long long)w + 2];
-    const bool wide = n >= (int)blockDim.x;
-    const int per_step = wide ? 1 : blockDim.x / n;          // rows per step
-    const int tr = wide ? 0 : threadIdx.x / n;               // this thread's row within a step
-    const int tc = wide ? threadIdx.x : threadIdx.x % n;     // and its first column
-    const int cstep = wide ? blockDim.x : n;
-    if (tr >= per_step) return;
-    for (long long r0 = (long long)blockIdx.y * slice_rows; r0 < nr; r0 += (long long)gridDim.y * slice_rows) {
-        const long long r1 = nr - r0 < slice_rows ? nr : r0 + slice_rows;
-        for (long long r = r0 + tr; r < r1; r += per_step) {
-            const double* s = src + (s0 + r) * ld_src;
-            double* d = dst + (d0 + r) * n;
-            for (int j = tc; j < n; j += cstep) d[j] = s[wcols[j]];
+    for (int c0 = 0; c0 < n; c0 += GATHER_COL_CHUNK) {
+        const int nc = n - c0 < GATHER_COL_CHUNK ? n - c0 : GATHER_COL_CHUNK;
+        if (c0 > 0) __syncthreads();                         // every thread is done with the previous chunk
+        for (int j = threadIdx.x; j < nc; j += blockDim.x) wcols[j] = cols ? cols[(long long)w * n + c0 + j] : c0 + j;
+        __syncthreads();
+        const bool wide = nc >= (int)blockDim.x;
+        const int per_step = wide ? 1 : blockDim.x / nc;     // rows per step
+        const int tr = wide ? 0 : threadIdx.x / nc;          // this thread's row within a step
+        const int tc = wide ? threadIdx.x : threadIdx.x % nc; // and its first column
+        const int cstep = wide ? blockDim.x : nc;
+        if (tr >= per_step) continue;
+        for (long long r0 = (long long)blockIdx.y * slice_rows; r0 < nr; r0 += (long long)gridDim.y * slice_rows) {
+            const long long r1 = nr - r0 < slice_rows ? nr : r0 + slice_rows;
+            for (long long r = r0 + tr; r < r1; r += per_step) {
+                const double* s = src + (s0 + r) * ld_src;
+                double* d = dst + (d0 + r) * n + c0;
+                for (int j = tc; j < nc; j += cstep) d[j] = s[wcols[j]];
+            }
         }
     }
 }
@@ -669,7 +658,8 @@ void launch_gather_window_blocks(const double* src, long long ld_src, double* ds
     const int slice_rows = n >= 2048 ? 1 : 2048 / n;
     const long long slices = (max_rows + slice_rows - 1) / slice_rows;
     const dim3 grid(n_windows, (unsigned)(slices < 65535 ? slices : 65535));
-    gather_window_blocks_kernel<<<grid, 256, sizeof(int) * (size_t)n, st>>>(src, ld_src, dst, n, cols, rows, slice_rows);
+    const size_t smem = sizeof(int) * (size_t)(n < GATHER_COL_CHUNK ? n : GATHER_COL_CHUNK);
+    gather_window_blocks_kernel<<<grid, 256, smem, st>>>(src, ld_src, dst, n, cols, rows, slice_rows);
 }
 
 // dst row (dst_row0 + k) = src row src_rows[k], k in [k0, k1): the overnight returns of arbitrary day blocks, gathered

@@ -36,6 +36,36 @@ def _c64(a) -> np.ndarray:
     return np.ascontiguousarray(a, dtype=np.float64)
 
 
+def _market_desc(prices, rf_row, caps, hf_prices):
+    """The descriptor of a market or pool upload (no MCM series) and the coerced arrays it points into, which must stay
+    alive as long as the library reads them."""
+    prices = _c64(prices)
+    rf_row = _c64(rf_row)
+    D, N = prices.shape
+    if rf_row.shape != (D,):
+        raise ValueError("rf_row must have one entry per daily row")
+    if np.isnan(rf_row).any():
+        raise ValueError("risk-free rate undefined on some window dates (the reference would drop rows, :60)")
+    desc = MarketDesc()                   # unset pointers are NULL, unset counts 0
+    desc.n_assets, desc.n_days = N, D
+    desc.prices, desc.rf_row = prices.ctypes.data, rf_row.ctypes.data
+    keep = [prices, rf_row]
+    if caps is not None:
+        caps = _c64(caps)
+        if caps.shape != (D, N):
+            raise ValueError("caps must match prices")
+        keep.append(caps)
+        desc.caps = caps.ctypes.data
+    if hf_prices is not None and len(hf_prices):
+        hf_prices = _c64(hf_prices)
+        if hf_prices.shape[1] != N:
+            raise ValueError("hf_prices must have N columns")
+        keep.append(hf_prices)
+        desc.hf_prices = hf_prices.ctypes.data
+        desc.n_hf_rows = hf_prices.shape[0]
+    return desc, keep
+
+
 class BayesEngine:
     """One CUDA device, one resident market.
 
@@ -244,41 +274,12 @@ class BayesEngine:
         ``hf_prices`` may hold NaN (missing bars).  As the reference's ``dropna`` (:314), an intraday return row with a
         NaN in any column is dropped: a NaN bar removes the returns on both sides of it.  A conjugate window uses the
         m returns it keeps (scalar ``m``); with m < 2 its S0 and weights are NaN and its status is non-zero."""
-        prices = _c64(prices)
-        rf_row = _c64(rf_row)
-        D, N = prices.shape
-        if rf_row.shape != (D,):
-            raise ValueError("rf_row must have one entry per daily row")
-        if np.isnan(rf_row).any():
-            raise ValueError("risk-free rate undefined on some window dates (the reference would drop rows, :60)")
-        keep = [prices, rf_row]
-        desc = MarketDesc()
-        desc.n_assets, desc.n_days = N, D
-        desc.prices = prices.ctypes.data
-        desc.rf_row = rf_row.ctypes.data
-        desc.caps = None
-        desc.hf_prices = None
-        desc.n_hf_rows = 0
-        desc.mcm = None
-        desc.n_mcm = 0
-        if caps is not None:
-            caps = _c64(caps)
-            if caps.shape != (D, N):
-                raise ValueError("caps must match prices")
-            keep.append(caps)
-            desc.caps = caps.ctypes.data
-        if hf_prices is not None and len(hf_prices):
-            hf_prices = _c64(hf_prices)
-            if hf_prices.shape[1] != N:
-                raise ValueError("hf_prices must have N columns")
-            keep.append(hf_prices)
-            desc.hf_prices = hf_prices.ctypes.data
-            desc.n_hf_rows = hf_prices.shape[0]
+        desc, keep = _market_desc(prices, rf_row, caps, hf_prices)
         if mcm is not None:
             mcm = _c64(mcm)
             if mcm.ndim == 1:
                 mcm = mcm[None, :]
-            if mcm.shape[1] != D:
+            if mcm.shape[1] != desc.n_days:
                 raise ValueError("mcm series must be aligned with the daily rows")
             keep.append(mcm)
             desc.mcm = mcm.ctypes.data
@@ -287,7 +288,7 @@ class BayesEngine:
         rc = fn(self._h, C.byref(desc))
         if rc:
             _raise(rc)
-        self.n_assets, self.n_days, self.n_hf_rows = N, D, int(desc.n_hf_rows)
+        self.n_assets, self.n_days, self.n_hf_rows = desc.n_assets, desc.n_days, int(desc.n_hf_rows)
         self._inflight = keep if async_copy else None
 
     def upload_pool(self, prices, rf_row, caps=None, hf_prices=None):
@@ -301,37 +302,12 @@ class BayesEngine:
                 _raise(rc)
             self.pool_shape = None
             return
-        prices = _c64(prices)
-        rf_row = _c64(rf_row)
-        D, N = prices.shape
-        if rf_row.shape != (D,):
-            raise ValueError("rf_row must have one entry per daily row")
-        if np.isnan(rf_row).any():
-            raise ValueError("risk-free rate undefined on some window dates (the reference would drop rows, :60)")
-        desc = MarketDesc()
-        desc.n_assets, desc.n_days = N, D
-        desc.prices, desc.rf_row = prices.ctypes.data, rf_row.ctypes.data
-        desc.caps = desc.hf_prices = desc.mcm = None
-        desc.n_hf_rows = desc.n_mcm = 0
-        keep = [prices, rf_row]
-        if caps is not None:
-            caps = _c64(caps)
-            if caps.shape != (D, N):
-                raise ValueError("caps must match prices")
-            keep.append(caps)
-            desc.caps = caps.ctypes.data
-        if hf_prices is not None and len(hf_prices):
-            hf_prices = _c64(hf_prices)
-            if hf_prices.shape[1] != N:
-                raise ValueError("hf_prices must have N columns")
-            keep.append(hf_prices)
-            desc.hf_prices = hf_prices.ctypes.data
-            desc.n_hf_rows = hf_prices.shape[0]
+        desc, keep = _market_desc(prices, rf_row, caps, hf_prices)
         rc = self._lib.bp_upload_pool(self._h, C.byref(desc))
         del keep
         if rc:
             _raise(rc)
-        self.pool_shape = (D, N, int(desc.n_hf_rows))
+        self.pool_shape = (desc.n_days, desc.n_assets, int(desc.n_hf_rows))
 
     def select_market(self, cols, day_lo: int = 0, day_hi: Optional[int] = None, hf_lo: int = 0, hf_hi: Optional[int] = None):
         """Working market = pool columns ``cols`` (in that order), daily rows [day_lo, day_hi), intraday rows

@@ -267,6 +267,41 @@ def test_error_paths(engine, mkt):
         engine.upload_pool(None, None)
 
 
+@pytest.mark.parametrize("N", [12289, 25000])
+def test_wide_selections_equal_direct_upload(engine, N):
+    """Working markets wider than the 12,288 columns the gather stages in shared memory at a time: a select_market slice
+    and each window of a select_windows stack give the excess returns (prices and risk-free rate) that a direct upload
+    of the same columns gives, bit for bit."""
+    from incorporating_different_sources_b200.windows import plan_daily_windows, slice_batch, stack_windows
+    rng = np.random.default_rng(N)
+    P, D, H, n = N + 1000, 40, 30, 20
+    dates = np.busday_offset("2020-01-01", np.arange(D), roll="forward").astype("datetime64[ns]")
+    prices = 100.0 * np.exp(np.cumsum(rng.normal(0.0, 0.01, (D, P)), axis=0))
+    caps = prices * rng.uniform(1e6, 1e9, P)
+    hf = rng.uniform(50.0, 150.0, (H, P))
+    rf = rng.uniform(0.0, 1e-4, D)
+    spec = dict(weighting_strategy="jeffreys", rolling_window=n, rolling_window_frequency="daily", risk_aversion=1)
+    d_idx = [25, 39]
+    cols = np.stack([rng.permutation(P)[:N] for _ in d_idx]).astype(np.int32)
+    plan = plan_daily_windows(spec, dates, d_idx, need_hf=False)
+    want = []
+    for w in range(len(d_idx)):
+        engine.upload_market(prices=prices[:, cols[w]], rf_row=rf, caps=caps[:, cols[w]], hf_prices=hf[:, cols[w]])
+        want.append(engine.excess_returns(slice_batch(plan, w, w + 1)))
+    engine.upload_pool(prices=prices, rf_row=rf, caps=caps, hf_prices=hf)
+    try:
+        for w, d in enumerate(d_idx):
+            engine.select_market(cols[w], d - (n - 1), d + 1, 0, H)
+            b = plan_daily_windows(spec, dates, [d], need_hf=False, row_offset=d - (n - 1))
+            assert np.array_equal(engine.excess_returns(b), want[w]), w
+        stk = stack_windows(plan)
+        engine.select_windows(cols, np.stack([stk.day_lo, stk.day_hi], axis=1), [[0, H], [5, H]])
+        for w in range(len(d_idx)):
+            assert np.array_equal(engine.excess_returns(slice_batch(stk.batch, w, w + 1)), want[w]), w
+    finally:
+        engine.upload_pool(None, None)
+
+
 # ------------------------------------------------------------------ backtest level: stacking on == stacking off
 def _backtest_both(engine, spec, md, start, end, **kw):
     from incorporating_different_sources_b200 import portfolio_calculations as pc

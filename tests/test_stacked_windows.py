@@ -25,15 +25,25 @@ def _sets(rng, n_pool, size, dates_pos):
 
 
 def _per_set_daily(spec, mkt, d_idx, look, need_hf):
-    """The plan of one set as backtest._batched_weights makes it for its own select_market slice."""
+    """The plan of one set as backtest._batched_weights makes it for its own select_market slice; the slice and the
+    shifted batch are also checked against the set's trade dates and look-back, searched directly."""
+    from incorporating_different_sources_b200 import backtest as bt
     n = spec["rolling_window"]
-    day_lo = min(d_idx) - (n - 1)
-    hf_lo = 0
+    _, b = bt._plan_windows(spec, spec["weighting_strategy"], mkt.dates, np.asarray(d_idx), mkt.hf_ts, mkt.dates, mkt.rf,
+                            look)
+    day_lo, day_hi, hf_lo, hf_hi = bt._set_slice(b, mkt.n_days, len(mkt.hf_ts))
+    assert (day_lo, day_hi) == (min(d_idx) - (n - 1), max(d_idx) + 1)
+    want_lo = want_hi = 0
     if need_hf:
         D = look if look is not None else HF_LOOKBACK_DAYS[spec["rolling_window_frequency"]]
-        hf_lo = max(int(np.searchsorted(mkt.hf_ts, mkt.dates[min(d_idx)] - D * _DAY + _DAY, side="right")) - 1, 0)
-    b = plan_daily_windows(spec, mkt.dates, d_idx, mkt.hf_ts if need_hf else None, hf_lookback_days=look,
-                           need_hf=need_hf, row_offset=day_lo, hf_row_offset=hf_lo)
+        want_lo = max(int(np.searchsorted(mkt.hf_ts, mkt.dates[min(d_idx)] - D * _DAY + _DAY, side="right")) - 1, 0)
+        want_hi = int(np.searchsorted(mkt.hf_ts, mkt.dates[max(d_idx)] + _DAY, side="right"))
+    assert (hf_lo, hf_hi) == (want_lo, want_hi)
+    ref = plan_daily_windows(spec, mkt.dates, d_idx, mkt.hf_ts if need_hf else None, hf_lookback_days=look,
+                             need_hf=need_hf, row_offset=day_lo, hf_row_offset=hf_lo)
+    for name in ("day_row", "span_days", "hf_lo", "hf_hi"):
+        a, r = getattr(b, name), getattr(ref, name)
+        assert (a is None and r is None) or (a.dtype == r.dtype and np.array_equal(a, r)), name
     return b, day_lo, hf_lo
 
 

@@ -6,12 +6,15 @@ and one batched call per asset set (``set_stack_max_windows(0)``).  One process:
 alternate; every pass records the wall-clock phases of ``backtest_portfolio`` (``timings``), the stacked windows and
 calls and the kernel launches, and splits the weights phase into the pool upload, the working-market selections
 (``select_market`` / ``select_windows`` / ``set_resampled``), the batched calls (which return with the weights in host
-memory) and the host work between them.  The outputs of both routes are compared bit for bit.  The card's name and power
-limit are read in the same run.
+memory) and the host work between them.  The outputs of both routes are compared bit for bit, and their sha256 is
+recorded so that two builds can be compared too.  The card's name and power limit are read in the same run.
 
-    python tools/asset_sets_bench.py [--reps 5] [--out profiles/asset_sets_bench.json]
+    python tools/asset_sets_bench.py [--reps 5] [--lib PATH] [--out profiles/asset_sets_bench.json]
+
+--lib loads another build of libbayes_portfolio.so (e.g. one of an earlier commit) in place of the package's.
 """
 import argparse
+import hashlib
 import json
 import os
 import subprocess
@@ -42,10 +45,14 @@ def main():
     ap.add_argument("--n-assets", type=int, default=500)
     ap.add_argument("--windows", type=int, default=4150)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "asset_sets_bench.json"))
+    ap.add_argument("--lib", help="libbayes_portfolio.so to load instead of the package's")
     args = ap.parse_args()
     import pandas as pd
     import bench
+    from incorporating_different_sources_b200 import _lib
     from incorporating_different_sources_b200 import portfolio_calculations as pc
+    if args.lib:
+        _lib.LIB_PATH = os.path.abspath(args.lib)
     from incorporating_different_sources_b200.engine import BayesEngine
 
     mkt, _, _, d_idx = bench.make_workload(args, 0)
@@ -104,10 +111,12 @@ def main():
         med = sorted(recs, key=lambda r: r["weights_s"])[len(recs) // 2]
         summary[name] = dict(median=med, weights_s_all=[r["weights_s"] for r in recs],
                              total_s_all=[r["total_s"] for r in recs], passes=recs)
-    out = dict(tool="tools/asset_sets_bench.py", card=card(), spec="top 50 of 500 by cap, monthly rebalancing, 250-week "
-               "window, conjugate HF-VIX VW, 7-day intraday look-back", market=dict(n_assets=args.n_assets,
-               n_days=int(mkt.n_days), hf_rows=int(mkt.hf_prices.shape[0])), reps=args.reps,
-               outputs_bit_identical=bool(identical), routes=summary)
+    out = dict(tool="tools/asset_sets_bench.py", lib=os.path.relpath(_lib.LIB_PATH, ROOT), card=card(),
+               spec="top 50 of 500 by cap, monthly rebalancing, 250-week window, conjugate HF-VIX VW, 7-day intraday look-back",
+               market=dict(n_assets=args.n_assets, n_days=int(mkt.n_days), hf_rows=int(mkt.hf_prices.shape[0])), reps=args.reps,
+               outputs_bit_identical=bool(identical), routes=summary,
+               output_sha256={k: hashlib.sha256(np.ascontiguousarray(v.to_numpy()).tobytes()).hexdigest()
+                              for k, v in outputs["per_set"].items()})
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
         json.dump(out, f, indent=1, default=float)

@@ -8,6 +8,8 @@ two runs is flagged ("deterministic": false), and a case whose second run differ
     python tools/driver_fingerprint.py [--lib PATH] --out FILE.json
 
 --lib loads another build of libbayes_portfolio.so (e.g. one of an earlier commit) in place of the package's.
+The working-market selections from the pool (select_market, select_windows) are cases of their own too: their launch
+counts are the gathers and the daily log returns.
 """
 import argparse
 import hashlib
@@ -95,6 +97,7 @@ def main():
     if args.lib:
         _lib.LIB_PATH = os.path.abspath(args.lib)
     import torch
+    from incorporating_different_sources_b200.backtest import _set_slice
     from incorporating_different_sources_b200.engine import BayesEngine, upload_synthetic
     from incorporating_different_sources_b200.synthetic import generate_market
     from incorporating_different_sources_b200.windows import (ffill_rows, plan_daily_windows, plan_weekly_windows,
@@ -198,13 +201,27 @@ def main():
     eng.set_resampled(rows)
     R.run("conj_weekly", None, lambda: eng.conjugate(wk, outputs=ALL))
 
-    # ---- stacked working market (select_windows)
+    # ---- one asset set's working market gathered from the pool (select_market), sliced as backtest's per-set route
+    # cuts it: the selection on its own, then a conjugate call with block reuse and a Jeffreys call with the chain
     pm = generate_market(40, 200, seed=31)
     eng.upload_pool(prices=pm.prices, rf_row=ffill_rows(pm.dates, pm.dates, pm.rf), caps=pm.caps, hf_prices=pm.hf_prices)
+    pcols = np.random.default_rng(3).permutation(40)[:N]
+    pb = plan_daily_windows(_spec(N, 60), pm.dates, list(range(100, 140)), pm.hf_ts, hf_lookback_days=7)
+    psl = _set_slice(pb, pm.n_days, len(pm.hf_ts))
+    pb.prior_n = np.full(pb.n_windows, 30.0)
+    jpb = plan_daily_windows(_spec(N, 60, "jeffreys"), pm.dates, list(range(100, 140)), need_hf=False)
+    jsl = _set_slice(jpb, pm.n_days, len(pm.hf_ts))
+    R.run("select_market", None, lambda: eng.select_market(pcols, *psl))
+    R.run("conj_pool_block_reuse", lambda: eng.select_market(pcols, *psl), conj(pb))
+    R.run("jeffreys_pool_chain", lambda: eng.select_market(pcols, *jsl),
+          lambda: eng.jeffreys(jpb, outputs=("weights", "nu", "w1", "status", "scalars")))
+
+    # ---- stacked working market (select_windows)
     sb = plan_daily_windows(_spec(N, 60), pm.dates, list(range(100, 140, 2)), pm.hf_ts, hf_lookback_days=7)
     stk = stack_windows(sb, None)
     cols = np.stack([np.sort(np.random.default_rng(i).choice(40, N, replace=False)) for i in range(sb.n_windows)])
-    eng.select_windows(cols, np.stack([stk.day_lo, stk.day_hi], axis=1), np.stack([stk.hf_lo, stk.hf_hi], axis=1))
+    R.run("select_windows", None, lambda: eng.select_windows(cols, np.stack([stk.day_lo, stk.day_hi], axis=1),
+                                                             np.stack([stk.hf_lo, stk.hf_hi], axis=1)))
     stk.batch.prior_n = np.full(sb.n_windows, 30.0)
     R.run("conj_stacked", None, lambda: eng.conjugate(stk.batch, outputs=ALL))
     jstk = stack_windows(plan_daily_windows(_spec(N, 60, "jeffreys"), pm.dates, list(range(100, 140)), need_hf=False), None)
