@@ -288,7 +288,9 @@ int bp_jeffreys_batched(bp_handle* h, const bp_window_batch* b, const bp_outputs
  *                          reference returns these weights after a cvxpy solve and clean_weights() rounding; the
  *                          rounding is the Python shim's job.  scalars: BP_SCAL_LW_*.
  * Outputs honoured: weights, nu (weights before 1/gamma), w1 (C^-1 t), t, rhs, scalars, status, S1 (Jorion: the
- * centred Gram C = (m-1) V_hat; shrinkage: m Sigma_LW / (1 - shrinkage intensity)), m = rolling_window - 1. */
+ * centred Gram C = (m-1) V_hat; shrinkage: m Sigma_LW / (1 - s) with s the shrinkage intensity, and rhs = t / (1 - s)),
+ * m = rolling_window - 1.  As in sklearn, s = 0 for one asset, and s = 1 exactly when beta >= delta (the intensity
+ * clips): Sigma_LW = mu I, and then S1 = m Sigma_LW = mu m I and rhs = t. */
 #define BP_ESTIMATOR_JORION 1
 #define BP_ESTIMATOR_SHRINKAGE 2
 #define BP_SCAL_JORION_MU_G 0          /* grand mean                                  :882               */

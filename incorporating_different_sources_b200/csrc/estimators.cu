@@ -13,6 +13,9 @@
 //   stage) m Sigma = (1 - shrinkage) C + shrinkage mu m I, and (m Sigma) w = t = m mu_hat is solved by the unchanged
 //   Cholesky kernel as (C + rho I) w = t / (1 - shrinkage), rho = shrinkage mu m / (1 - shrinkage): only the diagonal of
 //   the workspace and the right-hand side are rewritten (a full rescaling pass would re-read and re-write 2 MB per window).
+//   Two cases follow sklearn where that form does not apply: one asset (N = 1) has shrinkage 0, and a clipped window
+//   (beta >= delta, shrinkage exactly 1) has Sigma = mu I, solved as mu m I w = t: its lower triangle is rewritten to
+//   zero off the diagonal and mu m on it, and rhs = t.
 //   The only O(m N) work is beta_: one pass over the window's rows (L2 resident: consecutive windows share them).
 #include "common.cuh"
 #include "kernels.h"
@@ -27,6 +30,7 @@ __global__ void __launch_bounds__(LW_THREADS) lw_shrink_kernel(ShrinkParams p) {
     double* xbar = lw_sm;                  // [ldv]
     double* scratch = xbar + p.ldv;        // [40]
     __shared__ double sh_scale, sh_diag;
+    __shared__ bool sh_clip;
 
     const int w = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int N = p.n_assets, K = p.n_window - 1;
@@ -104,18 +108,29 @@ __global__ void __launch_bounds__(LW_THREADS) lw_shrink_kernel(ShrinkParams p) {
         delta /= Nd;
         const double beta_raw = beta;
         beta = fmin(beta, delta);
-        const double shrink = beta == 0.0 ? 0.0 : beta / delta;
+        // sklearn: shrinkage 0 for one feature (delta is 0 in exact arithmetic there, rounding leaves it either sign)
+        const double shrink = (N == 1 || beta == 0.0) ? 0.0 : beta / delta;
         double* scal = p.scal + (long long)w * BP_S_COUNT;
         scal[BP_S_LW_SHRINKAGE] = shrink;
         scal[BP_S_LW_MU] = mu;
         scal[BP_S_LW_BETA] = beta_raw;
         scal[BP_S_LW_DELTA] = delta;
-        sh_scale = 1.0 / (1.0 - shrink);                 // shrink < 1: beta <= delta and the data are not constant
-        sh_diag = shrink * mu * m / (1.0 - shrink);
+        // beta >= delta (also any delta <= 0 left by rounding) clips the intensity to exactly 1: Sigma_LW = mu I, and
+        // the window's system is m Sigma_LW w = mu m I w = t (1/(1 - shrink) would be inf)
+        sh_clip = shrink == 1.0;
+        sh_scale = sh_clip ? 1.0 : 1.0 / (1.0 - shrink);
+        sh_diag = sh_clip ? mu * m : shrink * mu * m / (1.0 - shrink);
     }
     __syncthreads();
     const double scale = sh_scale, diag = sh_diag;
-    for (int i = tid; i < N; i += LW_THREADS) S[(long long)i * p.ldS + i] += diag;
+    if (sh_clip) {                                       // uniform per block; only clipped windows pay the O(N^2) write
+        for (int i = warp; i < N; i += LW_WARPS) {
+            double* row = S + (long long)i * p.ldS;
+            for (int j = lane; j <= i; j += 32) row[j] = j == i ? diag : 0.0;
+        }
+    } else {
+        for (int i = tid; i < N; i += LW_THREADS) S[(long long)i * p.ldS + i] += diag;
+    }
     for (int j = tid; j < p.ldv; j += LW_THREADS) p.rhs[(long long)w * p.ldv + j] = j < N ? scale * p.t[(long long)w * p.ldv + j] : 0.0;
 }
 

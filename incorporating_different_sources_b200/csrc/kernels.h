@@ -253,9 +253,10 @@ constexpr int GRAM_KT = 32;        // rows per TMA k-tile
 constexpr int GRAM_TILE = 128;     // output tile edge
 cudaError_t launch_gram(const GramParams& p, const CUtensorMap& map0, const CUtensorMap& map1, int sm_count,
                         cudaStream_t st);
-// Ledoit-Wolf shrinkage of the centred Gram C = X_c'X_c in the solver workspace (in place):
-// S <- C + rho I, rhs <- t / (1 - delta), rho = delta mu m / (1 - delta): Sigma_LW w = mu_hat scaled by m / (1 - delta) (sklearn.covariance.ledoit_wolf
-// as called by pypfopt's CovarianceShrinkage.ledoit_wolf(), portfolio_calculations.py:727-729)
+// Ledoit-Wolf shrinkage of the centred Gram C = X_c'X_c in the solver workspace (in place), s the shrinkage intensity:
+// S <- C + rho I, rhs <- t / (1 - s), rho = s mu m / (1 - s): Sigma_LW w = mu_hat scaled by m / (1 - s) (sklearn.covariance.ledoit_wolf
+// as called by pypfopt's CovarianceShrinkage.ledoit_wolf(), portfolio_calculations.py:727-729).  s = 0 for N = 1; a clipped
+// window (s = 1, Sigma_LW = mu I) gets S <- mu m I (lower triangle) and rhs <- t
 struct ShrinkParams {
     int n_windows, n_assets, n_window, ld, ldv, ldS;
     long long win_stride;

@@ -492,7 +492,10 @@ class BayesEngine:
     def shrinkage(self, batch: WindowBatch, outputs: Sequence[str] = ("weights", "status"),
                   device_out: bool = False, into: Optional[dict] = None) -> Dict[str, object]:
         """``calculate_shrinkage_portfolio`` (:703-758) in closed form, ``(1/gamma) Sigma_LW^-1 mu_hat`` with the
-        Ledoit-Wolf covariance (unrounded: the reference's ``clean_weights()`` rounding is the facade's job)."""
+        Ledoit-Wolf covariance (unrounded: the reference's ``clean_weights()`` rounding is the facade's job).  With s
+        the shrinkage intensity (``scalars[:, SCAL_LW["shrinkage"]]``), ``S1`` is ``m Sigma_LW / (1 - s)`` and ``rhs``
+        ``t / (1 - s)``, m = rolling_window - 1.  As in sklearn, s = 0 for one asset, and a window whose intensity
+        clips (s = 1 exactly) has Sigma_LW = mu I: its ``S1`` is ``m Sigma_LW = mu m I`` and its ``rhs`` is ``t``."""
         from ._lib import EST_SHRINKAGE
         return self._estimator(EST_SHRINKAGE, batch, outputs, device_out, into)
 

@@ -275,6 +275,8 @@ def ledoit_wolf(X):
     pinned against the installed sklearn in ``tests/test_oracle_golden.py``.  Returns (shrunk_cov, shrinkage)."""
     n_samples, n_features = X.shape
     Xc = X - X.mean(0)
+    if n_features == 1:           # sklearn's one-feature rule: "the result is the same whatever the shrinkage"
+        return np.atleast_2d((Xc ** 2).mean()), 0.0
     X2 = Xc ** 2
     emp_cov_trace = np.sum(X2, axis=0) / n_samples
     mu = np.sum(emp_cov_trace) / n_features

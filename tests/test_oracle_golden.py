@@ -83,6 +83,20 @@ def test_ledoit_wolf_restatement_matches_installed_sklearn():
         assert relerr(cov2, cov) <= 1e-13
 
 
+def test_ledoit_wolf_one_feature_has_zero_shrinkage_as_in_sklearn():
+    """sklearn returns shrinkage 0 and the plain variance for one feature, whatever its beta and delta round to (the
+    general formula's delta is 0 in exact arithmetic there, and rounding leaves it of either sign)."""
+    sk = pytest.importorskip("sklearn.covariance")
+    rng = np.random.default_rng(12)
+    for m in (2, 3, 17, 120, 251):
+        for _ in range(20):
+            X = rng.standard_normal((m, 1)) * rng.uniform(0.005, 0.03) + 4e-4
+            cov, sh = sk.ledoit_wolf(X)
+            cov2, sh2 = bo.ledoit_wolf(X)
+            assert sh == 0.0 and sh2 == 0.0
+            assert cov2.shape == (1, 1) and relerr(cov2, cov) <= 1e-15
+
+
 def test_weekly_resample_matches_pandas():
     import pandas as pd
     from incorporating_different_sources_b200.synthetic import generate_market
