@@ -333,7 +333,11 @@ int bp_backtest_batched(bp_handle* h, const bp_backtest_desc* d);
  * strategies): one row of BP_PM_COUNT statistics per series.  returns / excess: [n_paths][n_obs] HOST arrays (simple
  * returns after adjust_returns, :46-72, and excess returns, :703-719); years = (index[-1] - index[0]).days / 365 (:524);
  * out: [n_paths][BP_PM_COUNT] host.  The probabilistic Sharpe ratio (:78-120) follows on the host from BP_PM_SKEW,
- * BP_PM_KURT and BP_PM_SHARPE_1 of the series and of the benchmark. */
+ * BP_PM_KURT and BP_PM_SHARPE_1 of the series and of the benchmark.
+ * BP_PM_SKEW and BP_PM_KURT are NaN for a flat excess series, by scipy.stats' rule m2 <= (DBL_EPSILON * mean)^2 on the
+ * kernel's mean and the two-pass corrected m2 = (sum b^2 - (sum b)^2 / n) / n, b = excess - mean: the correction
+ * cancels the rounding error of the mean, so a constant series is NaN even when its computed mean is a few ulp off.
+ * The other statistics use the uncorrected m2 = sum b^2 / n. */
 enum {
     BP_PM_CUM_RETURN = 0, BP_PM_CAGR, BP_PM_SHARPE, BP_PM_SORTINO, BP_PM_MAX_DD, BP_PM_CALMAR, BP_PM_AVG_LOSS,
     BP_PM_AVG_RETURN, BP_PM_AVG_WIN, BP_PM_BEST, BP_PM_WORST, BP_PM_ANN_VOL, BP_PM_DAILY_VAR, BP_PM_SKEW, BP_PM_KURT,

@@ -9,6 +9,8 @@
 // thread in index order).  HBM bound and tiny: T = 4,149 returns per series; the point is that a path ensemble never
 // goes back to pandas.  Formulas: QuantStats 0.0.62 (requirements.txt:10, not vendored) as restated in
 // oracle/eval_oracle.py, which pins them on the reference's own CHECK expressions (:520-650).
+#include <cfloat>
+
 #include "common.cuh"
 #include "../../include/bayes_portfolio.h"
 #include "kernels.h"
@@ -59,16 +61,18 @@ __global__ void __launch_bounds__(PM_THREADS) path_metrics_kernel(PathMetricsPar
     mn = -block_max(-mn, s8);
     const double n = (double)T, mr = sr / n, mxs = sx / n;
 
-    // ---- pass 2: central moments
-    double r2 = 0, x2 = 0, x3 = 0, x4 = 0;
+    // ---- pass 2: central moments (x1 = sum of the excess deviations, for the flat-sample rule of the skewness)
+    double r2 = 0, x1 = 0, x2 = 0, x3 = 0, x4 = 0;
     for (int i = tid; i < T; i += PM_THREADS) {
         const double a = r[i] - mr, b = x[i] - mxs, b2 = b * b;
         r2 = fma(a, a, r2);
+        x1 += b;
         x2 += b2;
         x3 = fma(b2, b, x3);
         x4 = fma(b2, b2, x4);
     }
     r2 = block_sum(r2, scratch); x2 = block_sum(x2, scratch); x3 = block_sum(x3, scratch); x4 = block_sum(x4, scratch);
+    x1 = block_sum(x1, scratch);
 
     // ---- cumulative product and drawdown: contiguous chunk per thread
     const int chunk = (T + PM_THREADS - 1) / PM_THREADS;
@@ -119,8 +123,13 @@ __global__ void __launch_bounds__(PM_THREADS) path_metrics_kernel(PathMetricsPar
         out[BP_PM_ANN_VOL] = sd_r * sqrt(252.0);
         out[BP_PM_DAILY_VAR] = fma(sd_r, -1.6448536269514729, mr);     // norm.ppf(0.05, mu, sigma)
         const double m2 = x2 / n;
-        out[BP_PM_SKEW] = (x3 / n) / (m2 * sqrt(m2));                   // scipy.stats.skew (biased)
-        out[BP_PM_KURT] = (x4 / n) / (m2 * m2);                         // scipy.stats.kurtosis(fisher=False)
+        // scipy's rule: NaN when m2 <= (eps mean)^2.  It is tested on the two-pass corrected m2, from which the
+        // error of the mean cancels: a constant series whose computed mean is a few ulp off has b = delta != 0 in
+        // every term, so x2 / n = delta^2 would pass for a spread (and give skew = +-1, kurtosis = 1).
+        const double m2c = (x2 - x1 * x1 / n) / n, eps_mean = DBL_EPSILON * mxs;
+        const bool flat = m2c <= eps_mean * eps_mean;
+        out[BP_PM_SKEW] = flat ? nan : (x3 / n) / (m2 * sqrt(m2));      // scipy.stats.skew (biased)
+        out[BP_PM_KURT] = flat ? nan : (x4 / n) / (m2 * m2);            // scipy.stats.kurtosis(fisher=False)
         out[BP_PM_SHARPE_1] = mxs / sd_x;                               // periods = 1 (:81-82)
     }
 }
